@@ -5,7 +5,7 @@ path timed beside it, an end-to-end number through the public API with host
 buffers, and short sub-benchmarks of the other hot-path rows (memory, pixel
 loss, frame scoring).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic tokens:
   C1+L1  EuclidDistance_Assign_Module.forward with the fused cluster loss
@@ -187,9 +187,10 @@ def reference_step_fn(device):
     return step, "port", "oracle/ref_port.py (the reference's ATen op chain restated; baseline/_ref not staged)"
 
 
-def cpu_reference_run(steps, warmup, budget_s=25.0):
+def cpu_reference_run(steps, warmup, budget_s=None):
     """time the reference step on a bounded sample of the workload (CPU_SAMPLE_CLIPS of the 64 clips) with every
-    host core; returns tokens/s etc."""
+    host core; returns tokens/s etc.  With ``budget_s`` the warm-up stops after half of it and the timed loop after
+    all of it (at least 3 steps); without, exactly ``warmup`` and ``steps`` steps run."""
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     step, kind, what = reference_step_fn(torch.device("cpu"))
@@ -201,14 +202,14 @@ def cpu_reference_run(steps, warmup, budget_s=25.0):
     t_start = time.perf_counter()
     for _ in range(warmup):
         step(x, gR)
-        if time.perf_counter() - t_start > budget_s / 2:
+        if budget_s is not None and time.perf_counter() - t_start > budget_s / 2:
             break
     times = []
     for _ in range(steps):
         t0 = time.perf_counter()
         step(x, gR)
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_start > budget_s and len(times) >= 3:
+        if budget_s is not None and time.perf_counter() - t_start > budget_s and len(times) >= 3:
             break
     ms = statistics.median(times) * 1e3
     return dict(value=ntok / (ms * 1e-3), ms_per_step=ms, cores=cores, steps=len(times), tokens=ntok, kind=kind,
@@ -240,7 +241,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_reference_run(args.steps, args.warmup, budget_s=150.0)
+    r = cpu_reference_run(args.steps, args.warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -265,6 +266,7 @@ class Step:
         self.graph, self.launches = None, None
         self.marks = []
         self.out = {}
+        self.keep_outputs = False       # also hold on to the forward outputs of the last step (--dump-outputs)
 
     def __call__(self, x_src=None, record=False):
         V, mod = self.V, self.mod
@@ -286,6 +288,8 @@ class Step:
         if self.collectives:
             V.allreduce_sum_packed([p.grad for p in self.params])
         self.out = {"loss": loss, "gx": x.grad}
+        if self.keep_outputs:
+            self.out.update(D=D, A=A, S=S, R=R, F=F, label=lab)
         return loss, x.grad
 
     def capture(self):
@@ -306,6 +310,36 @@ class Step:
 
     def release(self):
         self.graph = None
+
+
+DUMP_TOKENS = 16384               # token rows sampled from the per-token outputs by --dump-outputs (~42 MB in all)
+
+
+def gather_outputs(st, params):
+    """-> {name: numpy array} of what the step ``st`` computed in its last call: the loss, the centroid self-distances
+    and the parameter gradients in full; of the per-token outputs (distances, soft assignments, x_rec, LayerNorm
+    features, labels, token gradients) the rows of DUMP_TOKENS tokens drawn once from a fixed seed, in token order"""
+    o = st.out
+    ntok = o["F"].shape[0]
+    idx = torch.randperm(ntok, generator=torch.Generator().manual_seed(0))[:DUMP_TOKENS].sort().values
+    idx = idx.to(o["F"].device)
+    tensors = {"loss": o["loss"], "cluster_dist": o["S"],
+               "grad_cluster_center": params[0].grad, "grad_norm_weight": params[1].grad, "grad_norm_bias": params[2].grad}
+    for name, key in (("distance", "D"), ("assignment", "A"), ("x_rec", "R"), ("feature", "F"), ("label", "label"),
+                      ("x_grad", "gx")):
+        tensors[name] = o[key].reshape(ntok, -1).index_select(0, idx).squeeze(1)
+    out = {}
+    for name, t in tensors.items():
+        t = t.detach()
+        out[name] = t.cpu().numpy() if t.dtype == torch.float32 else t.double().cpu().numpy()   # labels: exact in float64
+    return out
+
+
+def write_outputs(arrays, out_dir):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_ours(args):
@@ -383,6 +417,7 @@ def run_ours(args):
         return float(tm) / steps
 
     head = make_step(head_clips, True)
+    head.keep_outputs = args.dump_outputs is not None
     ntok = head.x_buf.numel() // C
     need_flush = ntok * C * 8 <= (200 << 20)
     sampler = ClockSampler(local) if rank == 0 else None
@@ -463,6 +498,7 @@ def run_ours(args):
     wall0 = time.time()
     ms_step = timed(head, args.steps, need_flush)
     wall1 = time.time()
+    dumped = gather_outputs(head, params) if args.dump_outputs is not None and rank == 0 else None
     launches = V.launch_count() - launches0 if head.graph is None else head.launches * args.steps
     # clocks: the timed region is a fraction of a second, so every rank keeps the same load running (untimed,
     # same step count on all ranks: the step has collectives) until the 20 ms sampler has ~0.6 s under load
@@ -634,6 +670,8 @@ def run_ours(args):
             line["gpu_reference"] = {"unavailable": repr(e)[:200]}
         if not args.no_extra:
             line["extra"] = extra_benchmarks(V, dev, peak)
+    if dumped is not None:
+        write_outputs(dumped, args.dump_outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         V.disable_peer_allreduce()
@@ -851,7 +889,16 @@ def main():
     ap.add_argument("--no-reference-legs", action="store_true",
                     help="skip the cpu_baseline / gpu_reference legs (ncu launch lists of this repo's kernels only)")
     ap.add_argument("--no-graph", action="store_true", help="launch every step eagerly instead of replaying a CUDA graph of it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, labels "
+                         "float64; rank 0): loss, cluster_dist, grad_cluster_center, grad_norm_weight, grad_norm_bias in "
+                         "full, and distance, assignment, x_rec, feature, label, x_grad for a fixed seeded sample of "
+                         f"{DUMP_TOKENS} tokens. The inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repository's step (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

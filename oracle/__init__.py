@@ -8,8 +8,8 @@ the timed CPU baseline), never as something the CUDA path routes through.
 * ``np_oracle``  – numpy restatement of the reference algorithms (fp32 in the
   reference's operation order by default, fp64 on request for adjudicating
   near-ties).  Every function cites the reference ``file:line`` it follows.
-* ``ref_loader`` – imports the UNMODIFIED reference (``/root/reference`` here, the staged copy ``baseline/_ref``
-  on the GPU box) with stubs for its absent, unused dependencies: the reference arm of bench.py (``kind:
+* ``ref_loader`` – imports the UNMODIFIED reference (the checkout named by ``VADC_REFERENCE_ROOT``, or the staged
+  copy ``baseline/_ref``) with stubs for its absent, unused dependencies: the reference arm of bench.py (``kind:
   "reference"``), its ``gpu_reference`` leg and the model-level drop-in test use the reference's own classes.
 * ``ref_port``   – the same op chain written with torch CPU ops, used as the
   timed CPU baseline (the reference itself is a torch program, so this is the

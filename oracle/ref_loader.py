@@ -1,5 +1,7 @@
-"""TEST / BENCH INFRASTRUCTURE — imports the UNMODIFIED reference (``/root/reference`` in the build container, the
-staged copy ``baseline/_ref`` on the GPU box: scripts/stage_reference.py) with the stub recipe of SURVEY.md 8(c).
+"""TEST / BENCH INFRASTRUCTURE — imports the UNMODIFIED reference (a checkout of the original project named by the
+environment variable ``VADC_REFERENCE_ROOT``, or the copy staged under ``baseline/_ref`` by scripts/stage_reference.py)
+with the stub recipe of SURVEY.md 8(c).  Neither is part of this repository: without them the tests that build the
+reference's own model skip.
 Only tests/, ``__graft_entry__.smoke()`` and bench.py's reference legs may import this module; the product never does.
 
 Stubs (packages the reference imports at module level but that are absent here and unused on the path):
@@ -14,7 +16,7 @@ import types
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = (os.environ.get("VADC_REFERENCE_ROOT") or "/root/reference", os.path.join(ROOT, "baseline", "_ref"))
+CANDIDATES = tuple(c for c in (os.environ.get("VADC_REFERENCE_ROOT"), os.path.join(ROOT, "baseline", "_ref")) if c)
 
 
 def ref_root():
@@ -106,7 +108,7 @@ _ref = None
 
 
 def load():
-    """-> Reference, or None when neither /root/reference nor baseline/_ref exists"""
+    """-> Reference, or None when neither $VADC_REFERENCE_ROOT nor baseline/_ref holds the reference"""
     global _ref
     if _ref is None:
         root = ref_root()

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Stage the reference's own Python sources for the hot path under the git-ignored ``baseline/_ref/`` so that they
-travel to the GPU box with the repo snapshot (``/root/reference`` does not exist there).
+"""Stage the reference's own Python sources for the hot path under the git-ignored ``baseline/_ref/`` so that a copy
+of this working tree carries them to a machine without the original project's checkout.
 
-    python scripts/stage_reference.py            # no-op when /root/reference is absent (the GPU box)
+    VADC_REFERENCE_ROOT=<checkout of the original project> python scripts/stage_reference.py   # no-op without it
 
 The reference is not pip-installable (no setup.py / pyproject, SURVEY.md 2), so "installing" it is a copy of the
 package directories the path imports: model/ (cluster, Memory, backbone + the encoder / decoder files backbone
@@ -17,15 +17,15 @@ import shutil
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("VADC_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("VADC_REFERENCE_ROOT", "")
 DST = os.path.join(ROOT, "baseline", "_ref")
 PACKAGES = ["model", "loss_tool", "misc", "utils", "tool"]
 
 
 def stage(verbose=True):
-    if not os.path.isdir(os.path.join(REF, "model")):
+    if not REF or not os.path.isdir(os.path.join(REF, "model")):
         if verbose:
-            print(f"stage_reference: {REF} not present; keeping {DST} as it is")
+            print(f"stage_reference: no reference checkout at VADC_REFERENCE_ROOT={REF!r}; keeping {DST} as it is")
         return False
     manifest = {}
     for pkg in PACKAGES:

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/*.npz by running the
-REFERENCE'S OWN modules (imported from /root/reference, unmodified) on seeded
-synthetic inputs.  Runs only in the build container (the reference does not
-travel to the GPU box); the fixtures it writes are committed.
+REFERENCE'S OWN modules (imported unmodified from a checkout of the original
+project) on seeded synthetic inputs, on the CPU; the fixtures it writes are
+committed.
 
-    python tests/golden/make_golden.py
+    VADC_REFERENCE_ROOT=<checkout of the original project> python tests/golden/make_golden.py
 
 Stubs: misc/utils.py imports matplotlib / skimage / cv2 at module import;
 they are not installed here and are not used by psnr()/anomly_score(), so
@@ -19,7 +19,10 @@ import types
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("VADC_REFERENCE_ROOT", "")
+if not os.path.isfile(os.path.join(REF, "model", "cluster.py")):
+    sys.exit("make_golden.py: set VADC_REFERENCE_ROOT to a checkout of the original project, e.g.\n"
+             "    VADC_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 

@@ -67,17 +67,26 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo():
+def test_two_rank_gloo(monkeypatch):
+    # the workers see no GPU, so they take the gloo path on any host (with CUDA, init_distributed_mode picks nccl and
+    # binds rank r to cuda:r, which a one-GPU machine does not have)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]
-    for p in procs:
-        p.start()
-    res = dict(q.get(timeout=120) for _ in range(world))
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    try:
+        for p in procs:
+            p.start()
+        res = dict(q.get(timeout=120) for _ in range(world))
+        for p in procs:
+            p.join(timeout=60)
+            assert p.exitcode == 0
+    finally:
+        for p in procs:                                  # a worker left waiting for a dead peer must not outlive the test
+            if p.is_alive():
+                p.kill()
+                p.join()
     assert res[0]["shard"] == (0, 4) and res[1]["shard"] == (4, 7)
     for i in range(3):
         want = res[0]["local"][i] + res[1]["local"][i]

@@ -2,7 +2,7 @@
 videoad_b200 classes into ``model.backbone`` (``patch_reference``) and build the reference's own ``Mymodel`` with
 them — parameter names and shapes must equal those of the unpatched model, and the reference's substring-based
 grad toggles (backbone.py:44-76) must act on the same parameters.  CPU only (construction and state_dict; the
-forward needs a B200) and skipped where ``/root/reference`` does not exist (the GPU box)."""
+forward needs a B200) and skipped where ``oracle.ref_loader`` finds no copy of the original project."""
 import os
 import sys
 import types
@@ -10,8 +10,10 @@ import types
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "model")), reason="reference tree not present")
+from oracle import ref_loader
+
+REF = ref_loader.ref_root()
+pytestmark = pytest.mark.skipif(REF is None, reason="reference sources not staged (baseline/_ref or VADC_REFERENCE_ROOT)")
 
 
 def _stub(name, **attrs):

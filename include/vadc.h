@@ -311,6 +311,24 @@ size_t vadc_memory_separateness_workspace_bytes(int m, int d);
 int vadc_memory_separateness(const float* keys, int m, int d, float* out,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/* Backward of read with respect to the memory items (autograd of Memory.py:255, keys learnable):
+ *   g_keys [m,d] = score_memory^T G_r,  G_r[b*HW + hw, c] = g_updated_query[b, d + c, hw]
+ * score_memory [B*HW, m] as returned by vadc_memory_score; g_updated_query [B,2d,HW] (only channels d..2d-1 are
+ * read).  g_keys is overwritten.  Split-K over the tokens on the tcgen05 GEMM, the partials summed in a fixed order
+ * (bit-identical across launches); operand terms as in vadc_memory_read (VADC_MEMORY_TERMS=3: bf16 x3).
+ * Under a token-sharded global batch the result is this rank's share; the sum over ranks is the full gradient.
+ * d >= 8 (VADC_ERR_UNSUPPORTED otherwise). */
+size_t vadc_memory_keys_bwd_workspace_bytes(int B, int d, int64_t HW, int m);
+int vadc_memory_keys_bwd(const float* score_memory, const float* g_updated_query, int B, int d, int64_t HW,
+                         int m, float* g_keys, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Backward of MemoryLoss  Memory.py:52-59 with respect to keys [m,d]; g_out is a device scalar:
+ *   S = K K^T/2 + 1/2 - I (recomputed as vadc_memory_separateness does), G = sgn(S) with sgn(0) = 0,
+ *   g_keys = g_out / (m (m-1)) * (G + G^T)/2 K   (G is symmetric bit for bit).  g_keys is overwritten. */
+size_t vadc_memory_separateness_bwd_workspace_bytes(int m, int d);
+int vadc_memory_separateness_bwd(const float* keys, const float* g_out, int m, int d, float* g_keys,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------ *
  * Debug / self-test: one CTA runs out[128,N] = A * B on tcgen05 (TMEM
  * accumulator, SWIZZLE_128B shared-memory operands).  mode bit0: B is [Kd,N]

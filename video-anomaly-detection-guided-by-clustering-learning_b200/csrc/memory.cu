@@ -671,6 +671,110 @@ sum_all_kernel(const float* __restrict__ a, long long n, double scale, float* __
   if (threadIdx.x == 0) out[0] = (float)(s * scale);
 }
 
+// ---- gradient with respect to the memory items ------------------------------------------------------------------
+// read (Memory.py:255): updated_query[:, d:2d] = score_memory.detach() @ keys, so g_keys = score_memory^T G_r with
+// G_r[n, c] = g_updated_query[b, d + c, hw], n = b HW + hw.  One GEMM, M = slots, N = channels, contraction over the
+// tokens: score_memory is the A operand read MN-major ([tokens, slots] = [Kd, M]), G_r the K-major B operand
+// ([channels, tokens]).  Both are split into their operand terms with row pitches padded to eight elements (TMA: 16-byte
+// pitches) and zeros in the padding, so any m and any token count take the tensor-core path.
+template <int TERMS>
+__device__ __forceinline__ void split_terms(float a, __half (&h)[2], __nv_bfloat16 (&b)[3]) {
+  if constexpr (TERMS == 2) {
+    h[0] = __float2half_rn(a);
+    h[1] = __float2half_rn(a - __half2float(h[0]));
+  } else {
+    b[0] = __float2bfloat16_rn(a);
+    const float r1 = a - __bfloat162float(b[0]);
+    b[1] = __float2bfloat16_rn(r1);
+    b[2] = __float2bfloat16_rn(r1 - __bfloat162float(b[1]));
+  }
+}
+
+template <int TERMS>
+__device__ __forceinline__ void store_terms(void* dst, long long plane, long long i, float a) {
+  __half h[2];
+  __nv_bfloat16 b[3];
+  split_terms<TERMS>(a, h, b);
+  if constexpr (TERMS == 2) {
+    __half* o = static_cast<__half*>(dst) + i;
+    o[0] = h[0]; o[plane] = h[1];
+  } else {
+    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(dst) + i;
+    o[0] = b[0]; o[plane] = b[1]; o[2 * plane] = b[2];
+  }
+}
+
+// score_memory [N, m] -> terms [TERMS][Np][m8] of score_memory * scale (fp16 x2: scale = 2^13, bf16 x3: 1)
+template <int TERMS>
+__global__ void __launch_bounds__(256)
+keys_bwd_split_scores_kernel(const float* __restrict__ sm, long long N, int m, long long Np, int m8, float scale,
+                             void* __restrict__ dst) {
+  const long long plane = Np * m8;
+  for (long long r = blockIdx.x; r < Np; r += gridDim.x) {
+    const float* row = sm + r * m;
+    for (int c = threadIdx.x; c < m8; c += blockDim.x) {
+      const float v = (r < N && c < m) ? __ldg(row + c) * scale : 0.f;
+      store_terms<TERMS>(dst, plane, r * m8 + c, v);
+    }
+  }
+}
+
+// g_updated_query [B, 2d, HW], channels d..2d-1 -> terms [TERMS][d][Np] of G_r^T * scale[0] (scale == NULL: 1), read
+// and written along hw; the last batch's blocks also zero the padding columns N..Np-1
+template <int TERMS>
+__global__ void __launch_bounds__(256)
+keys_bwd_split_grad_kernel(const float* __restrict__ g_uq, int B, int d, long long HW, long long Np,
+                           const float* __restrict__ scale, void* __restrict__ dst) {
+  const long long hw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int c = blockIdx.y, b = blockIdx.z;
+  const long long n = (long long)b * HW + hw;
+  float v = 0.f;
+  if (hw < HW) v = __ldg(g_uq + ((long long)b * 2 * d + d + c) * HW + hw) * (scale ? __ldg(scale) : 1.0f);
+  else if (b != B - 1 || n >= Np) return;
+  store_terms<TERMS>(dst, (long long)d * Np, (long long)c * Np + n, v);
+}
+
+// g_keys[i, c] = sum over split slots s (in slot order) of part[s][i][c]: repeated launches give identical bits
+__global__ void __launch_bounds__(256)
+keys_bwd_sum_partials_kernel(const float* __restrict__ part, int splits, long long split_stride, long long n,
+                    float* __restrict__ out) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    float s = 0.f;
+    for (int k = 0; k < splits; ++k) s += __ldg(part + k * split_stride + i);
+    out[i] = s;
+  }
+}
+
+// MemoryLoss (Memory.py:52-59) backward: G = sgn(S), S = K K^T / 2 + 1/2 - I from the same product and the same
+// expression as SeparatenessEpilogue (sgn(0) = 0, the subgradient torch's abs backward takes)
+struct SeparatenessSignEpilogue {
+  float* out; int m;
+  __device__ __forceinline__ void operator()(int, int, int r, int c, float v) const {
+    const float s = v * 0.5f + 0.5f - (r == c ? 1.0f : 0.0f);
+    out[(long long)r * m + c] = (s > 0.f) ? 1.0f : ((s < 0.f) ? -1.0f : 0.0f);
+  }
+};
+
+// g_keys = g_out / (m (m - 1)) * (G K); G is symmetric by construction (the entries (r, c) and (c, r) come from the same
+// operands in the same accumulation order), so G K = (G + G^T) / 2 K
+struct ScaledStoreEpilogue {
+  float* out; int ld; const float* g_out; float scale;
+  __device__ __forceinline__ void operator()(int, int, int r, int c, float v) const {
+    out[(long long)r * ld + c] = v * (__ldg(g_out) * scale);
+  }
+};
+
+// split-K factor of the g_keys contraction ([m, d] output, contraction over the tokens): ~2 tiles per SM of a B200
+// (148 SMs).  A function of the shape alone, so that the workspace query makes no CUDA call.
+static int keys_bwd_splits(long long Np, int m8, int d) {
+  const long long tiles = (long long)((m8 + 127) / 128) * ((d + 127) / 128);
+  const long long nkb = (Np + 63) / 64;
+  long long s = (2ll * 148 + tiles - 1) / tiles;
+  if (s > nkb) s = nkb;
+  if (s < 1) s = 1;
+  return (int)s;
+}
+
 static int col_chunks(long long N) {
   long long c = (N + 255) / 256;
   if (c > 2048) c = 2048;
@@ -1013,5 +1117,89 @@ extern "C" int vadc_memory_separateness(const float* keys, int m, int d, float* 
   if (e != cudaSuccess) return record_cuda_error(e, "separateness sgemm");
   sum_all_kernel<<<1, 256, 0, st>>>(sim, (long long)m * m, 1.0 / ((double)m * (m - 1)), out);
   VADC_CHECK_LAUNCH("sum_all_kernel");
+  return VADC_OK;
+}
+
+static long long pad8(long long v) { return (v + 7) / 8 * 8; }
+
+extern "C" size_t vadc_memory_keys_bwd_workspace_bytes(int B, int d, int64_t HW, int m) {
+  const long long Np = pad8((long long)(B > 0 ? B : 1) * (HW > 0 ? HW : 1)), m8 = pad8(m > 0 ? m : 1);
+  const int dd = d > 0 ? d : 1;
+  return tc_gemm_split_bytes(Np, m8) + tc_gemm_split_bytes(dd, Np) +       // operand terms (room for three)
+         align_up((size_t)keys_bwd_splits(Np, (int)m8, dd) * m8 * dd * sizeof(float), 256) + 1024;   // partials, scales
+}
+
+extern "C" int vadc_memory_keys_bwd(const float* score_memory, const float* g_updated_query, int B, int d, int64_t HW,
+                                    int m, float* g_keys, void* workspace, size_t workspace_bytes, void* stream) {
+  VADC_REQUIRE(B >= 0 && d > 0 && HW > 0 && m > 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(g_keys && workspace, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(B == 0 || (score_memory && g_updated_query), VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(d >= 8 && d <= 65535 && B <= 65535 && (long long)B * HW < (1ll << 31) - 8, VADC_ERR_UNSUPPORTED);
+  VADC_REQUIRE(workspace_bytes >= vadc_memory_keys_bwd_workspace_bytes(B, d, HW, m), VADC_ERR_WORKSPACE);
+  if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (B == 0) {                                          // no tokens: the read contributes nothing
+    VADC_CUDA(cudaMemsetAsync(g_keys, 0, (size_t)m * d * sizeof(float), st));
+    return VADC_OK;
+  }
+  const long long N = (long long)B * HW, Np = pad8(N);
+  const int m8 = (int)pad8(m);
+  const int sk = keys_bwd_splits(Np, m8, d);
+  Carver ws(workspace, workspace_bytes);
+  void* sms = ws.take<uint8_t>(tc_gemm_split_bytes(Np, m8));
+  void* gs = ws.take<uint8_t>(tc_gemm_split_bytes(d, Np));
+  float* part = ws.take<float>((size_t)sk * m8 * d);
+  const TcPartialEpi epi{part, d, (long long)m8 * d};
+  const unsigned srows = (unsigned)std::min<long long>(Np, 16ll * sm_count());
+  const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
+  int rc;
+  if (env_int("VADC_MEMORY_TERMS", 2) == 3) {            // fp32-faithful three-term bf16 split, six products
+    keys_bwd_split_scores_kernel<3><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 1.0f, sms);
+    VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
+    keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(g_updated_query, B, d, HW, Np, nullptr, gs);
+    VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+    rc = launch_tc_gemm_ex<true, false>(sms, gs, m8, d, Np, sk, epi, st);
+  } else {
+    // two fp16 terms: the softmax weights scaled by 2^13 as in vadc_memory_read, G_r by the power of two of its measured
+    // bound (over the channels d..2d-1 of every batch)
+    unsigned* bits = ws.take<unsigned>(64);
+    float* sc = ws.take<float>(64);
+    if ((rc = tc_absmax_bits_seg(g_updated_query + (long long)d * HW, (long long)d * HW, B, 2ll * d * HW, bits, st))) return rc;
+    if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
+    keys_bwd_split_scores_kernel<2><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 8192.0f, sms);
+    VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
+    keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(g_updated_query, B, d, HW, Np, sc + 1, gs);
+    VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+    rc = launch_tc_gemm_ex_h2<true, false>(sms, gs, m8, d, Np, sk, sc + 2, epi, st);
+  }
+  if (rc) return rc;
+  const long long md = (long long)m * d;
+  keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
+      part, sk, (long long)m8 * d, md, g_keys);
+  VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
+  return VADC_OK;
+}
+
+extern "C" size_t vadc_memory_separateness_bwd_workspace_bytes(int m, int d) {
+  (void)d;
+  return align_up((size_t)(m > 0 ? m : 1) * (m > 0 ? m : 1) * sizeof(float), 256) + 256;
+}
+
+extern "C" int vadc_memory_separateness_bwd(const float* keys, const float* g_out, int m, int d, float* g_keys,
+                                            void* workspace, size_t workspace_bytes, void* stream) {
+  VADC_REQUIRE(m > 1 && d > 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(keys && g_out && g_keys && workspace, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(workspace_bytes >= vadc_memory_separateness_bwd_workspace_bytes(m, d), VADC_ERR_WORKSPACE);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* sgn = static_cast<float*>(workspace);
+  {
+    Operand Aop{keys, d, 1}, Bop{keys, 1, d};                // K K^T exactly as vadc_memory_separateness forms it
+    cudaError_t e = sgemm_auto(m, m, d, Aop, Bop, 0, 0, 1, 1, SeparatenessSignEpilogue{sgn, m}, st);
+    if (e != cudaSuccess) return record_cuda_error(e, "separateness bwd sgemm K.K^T");
+  }
+  Operand Aop{sgn, m, 1}, Bop{keys, d, 1};
+  cudaError_t e = sgemm_auto(m, d, m, Aop, Bop, 0, 0, 1, 1,
+                             ScaledStoreEpilogue{g_keys, d, g_out, (float)(1.0 / ((double)m * (m - 1)))}, st);
+  if (e != cudaSuccess) return record_cuda_error(e, "separateness bwd sgemm G.K");
   return VADC_OK;
 }

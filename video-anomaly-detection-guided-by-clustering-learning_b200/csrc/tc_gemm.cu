@@ -606,9 +606,11 @@ int tc_split2h(const float* src, long long rows, long long cols, const float* sc
 }
 
 namespace tg {
-// max |src| as the bit pattern of a non-negative float (ordered like unsigned integers): deterministic atomicMax
+// max |src| as the bit pattern of a non-negative float (ordered like unsigned integers): deterministic atomicMax;
+// blockIdx.y walks segments of n elements `stride` apart
 __global__ void __launch_bounds__(256)
-absmax_bits_kernel(const float* __restrict__ src, long long n, unsigned* __restrict__ out) {
+absmax_bits_kernel(const float* __restrict__ src, long long n, long long stride, unsigned* __restrict__ out) {
+  src += (long long)blockIdx.y * stride;
   float m = 0.f;
   const long long n4 = ((reinterpret_cast<uintptr_t>(src) & 15u) == 0) ? n / 4 : 0;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
@@ -690,12 +692,18 @@ int tc_cluster_bwd_scales(const unsigned* bits, int stage, float* out, cudaStrea
   return VADC_OK;
 }
 
-int tc_absmax_bits(const float* src, long long n, unsigned* out, cudaStream_t st) {
+int tc_absmax_bits_seg(const float* src, long long n, int nseg, long long stride, unsigned* out, cudaStream_t st) {
+  if (nseg < 1 || nseg > 65535) return VADC_ERR_UNSUPPORTED;
   VADC_CUDA(cudaMemsetAsync(out, 0, sizeof(unsigned), st));
-  const int grid = (int)std::max<long long>(1, std::min<long long>((n / 4 + 255) / 256, (long long)sm_count() * 8));
-  tg::absmax_bits_kernel<<<grid, 256, 0, st>>>(src, n, out);
+  const long long per = std::max<long long>(1, (long long)sm_count() * 8 / nseg);
+  const int grid = (int)std::max<long long>(1, std::min<long long>((n / 4 + 255) / 256, per));
+  tg::absmax_bits_kernel<<<dim3(grid, nseg), 256, 0, st>>>(src, n, stride, out);
   VADC_CHECK_LAUNCH("absmax_bits_kernel");
   return VADC_OK;
+}
+
+int tc_absmax_bits(const float* src, long long n, unsigned* out, cudaStream_t st) {
+  return tc_absmax_bits_seg(src, n, 1, 0, out, st);
 }
 
 int tc_pair_scales(const unsigned* a_bits, float a_given, const unsigned* b_bits, float b_given, float* out3, cudaStream_t st) {
@@ -720,6 +728,7 @@ template int launch_tc_gemm_h2<true, TcGzEpi>(const void*, const void*, long lon
 template int launch_tc_gemm_ex_h2<true, false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcStoreTEpi, cudaStream_t);
 template int launch_tc_gemm_ex_h2<true, false, TcReadTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcReadTEpi, cudaStream_t);
 template int launch_tc_gemm_ex_h2<true, false, TcGzTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcGzTEpi, cudaStream_t);
+template int launch_tc_gemm_ex_h2<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex_h2<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
 
 template <bool B_MN, class Epi>
@@ -735,6 +744,7 @@ template int launch_tc_gemm<false, TcDistEpi>(const void*, const void*, long lon
 template int launch_tc_gemm<true, TcReadEpi>(const void*, const void*, long long, long long, long long, TcReadEpi, cudaStream_t);
 template int launch_tc_gemm<true, TcGzEpi>(const void*, const void*, long long, long long, long long, TcGzEpi, cudaStream_t);
 template int launch_tc_gemm<false, TcTimeDebedEpi>(const void*, const void*, long long, long long, long long, TcTimeDebedEpi, cudaStream_t);
+template int launch_tc_gemm_ex<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex<true, false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, int, TcStoreTEpi, cudaStream_t);
 template int launch_tc_gemm<false, TcBiasEpi>(const void*, const void*, long long, long long, long long, TcBiasEpi, cudaStream_t);

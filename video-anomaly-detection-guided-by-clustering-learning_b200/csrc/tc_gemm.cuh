@@ -33,6 +33,8 @@ int launch_tc_gemm_h2(const void* a_split, const void* b_split, long long M, lon
 // scales for operands whose bound has to be measured: max |src| as float bits (memset + atomicMax), then
 // out3 = {s_a, s_b, 1 / (s_a s_b)} with s = the power of two that puts the bound in [4, 8), or the given constant
 int tc_absmax_bits(const float* src, long long n, unsigned* out, cudaStream_t st);
+// the same over nseg segments of n elements, `stride` elements apart (e.g. a channel slice of a [B, C, HW] tensor)
+int tc_absmax_bits_seg(const float* src, long long n, int nseg, long long stride, unsigned* out, cudaStream_t st);
 int tc_pair_scales(const unsigned* a_bits, float a_given, const unsigned* b_bits, float b_given, float* out3, cudaStream_t st);
 int tc_fwd_scales_from_bits(const unsigned* cen_bits, const float* ln_w, const float* ln_b, int C, float* out6, cudaStream_t st);
 int tc_cluster_bwd_scales(const unsigned* bits4, int stage, float* out9, cudaStream_t st);   // see tc_gemm.cu

@@ -14,17 +14,41 @@ from . import _lib
 from ._lib import check, f32c, ptr, stream, workspace
 
 
+class _MemoryLoss(torch.autograd.Function):
+    """separateness of the memory items and its gradient: with S = K K^T/2 + 1/2 - I and G = sgn(S) (sgn(0) = 0, as
+    torch's abs backward), d/dK = g / (m (m-1)) (G + G^T)/2 K"""
+
+    @staticmethod
+    def forward(ctx, memory):
+        k = f32c(memory)
+        m, d = k.shape
+        out = torch.empty((), device=k.device, dtype=torch.float32)
+        l = _lib.lib()
+        ws = workspace(l.vadc_memory_separateness_workspace_bytes(m, d), k.device)
+        check(l.vadc_memory_separateness(ptr(k), m, d, ptr(out), ptr(ws), ws.numel(), stream()),
+              "vadc_memory_separateness")
+        if ctx.needs_input_grad[0]:
+            ctx.save_for_backward(k)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_out):
+        (k,) = ctx.saved_tensors
+        m, d = k.shape
+        g = f32c(g_out).reshape(1)
+        gk = torch.empty_like(k)
+        l = _lib.lib()
+        ws = workspace(l.vadc_memory_separateness_bwd_workspace_bytes(m, d), k.device)
+        check(l.vadc_memory_separateness_bwd(ptr(k), ptr(g), m, d, ptr(gk), ptr(ws), ws.numel(), stream()),
+              "vadc_memory_separateness_bwd")
+        return gk
+
+
 def MemoryLoss(memory):
-    """model/Memory.py:52-59: separateness sum |K K^T/2 + 1/2 - I| / (m (m-1))"""
+    """model/Memory.py:52-59: separateness sum |K K^T/2 + 1/2 - I| / (m (m-1)); differentiable with respect to
+    ``memory`` (the regulariser of learnable memory items)"""
     _lib.require_cuda(memory)
-    k = f32c(memory)
-    m, d = k.shape
-    out = torch.empty((1,), device=k.device, dtype=torch.float32)
-    l = _lib.lib()
-    ws = workspace(l.vadc_memory_separateness_workspace_bytes(m, d), k.device)
-    check(l.vadc_memory_separateness(ptr(k), m, d, ptr(out), ptr(ws), ws.numel(), stream()),
-          "vadc_memory_separateness")
-    return out[0]
+    return _MemoryLoss.apply(memory)
 
 
 def _dist_reduce(t, op):
@@ -66,9 +90,13 @@ class _MemoryForward(torch.autograd.Function):
     """Memory.forward (Memory.py:145-175) as one autograd node.  Gradients flow to ``query`` exactly where
     the reference graph lets them: through the first half of ``updated_query`` (the read softmax is
     ``.detach()``ed, :255), ``gathering_loss`` (:245) and ``spreading_loss`` (:229), back through
-    ``F.normalize`` (:148).  ``keys`` are constants (every use is detached or, for the read product, the
-    caller passes a plain tensor: main.py:131); ``updated_memory`` is detached (:204); the two score
-    matrices are returned for inspection and are not differentiable here."""
+    ``F.normalize`` (:148).  ``keys`` get a gradient only through the read product (:255, ``score_memory`` detached):
+    g_keys = score_memory^T G_r, computed when ``keys`` requires grad (e.g. an ``nn.Parameter``; main.py:131 passes
+    a plain tensor, and then nothing extra is saved or launched).  Every other use of ``keys`` is detached (:229,
+    :245), ``updated_memory`` is detached (:204); the two score matrices are returned for inspection and are not
+    differentiable here.  Under ``Memory.global_batch`` the read softmax is per token, so each rank's g_keys is the
+    contribution of its own tokens: their sum over ranks is the full-batch gradient, and summing it is left to the
+    caller (DDP's gradient all-reduce, or ``allreduce_sum_packed``)."""
 
     @staticmethod
     def forward(ctx, mod, query, keys, train):
@@ -92,7 +120,10 @@ class _MemoryForward(torch.autograd.Function):
             gathering_loss = mod._reduce(gathering_loss.reshape(1) * ctx.loss_scale, "sum")[0]
             if spreading_loss is not None:
                 spreading_loss = mod._reduce(spreading_loss.reshape(1) * ctx.loss_scale, "sum")[0]
-        ctx.save_for_backward(qc, keys_c, s.top1, s.top2)
+        if ctx.needs_input_grad[2]:                       # learnable memory items: the read needs score_memory back
+            ctx.save_for_backward(qc, keys_c, s.top1, s.top2, s.score_memory)
+        else:
+            ctx.save_for_backward(qc, keys_c, s.top1, s.top2)
         ctx.train = bool(train)
         ctx.set_materialize_grads(False)
         if train:
@@ -105,7 +136,7 @@ class _MemoryForward(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, *grads):
-        qc, keys_c, top1, top2 = ctx.saved_tensors
+        qc, keys_c, top1, top2 = ctx.saved_tensors[:4]
         if ctx.train:
             g_uq, _, _, _, g_gather, g_spread = grads
         else:
@@ -117,17 +148,27 @@ class _MemoryForward(torch.autograd.Function):
         # (global batch: the kernel divides by the local token count; loss_scale turns that into the global mean)
         g_gather = None if g_gather is None else f32c(g_gather).reshape(1) * ctx.loss_scale
         g_spread = None if g_spread is None else f32c(g_spread).reshape(1) * ctx.loss_scale
-        gq = torch.empty_like(qc)
-        check(_lib.lib().vadc_memory_query_bwd(ptr(qc), ptr(keys_c), ptr(top1), ptr(top2) if ctx.train else None,
-                                               ptr(g_uq), ptr(g_gather), ptr(g_spread), B, d, h * w,
-                                               keys_c.shape[0], ptr(gq), stream()), "vadc_memory_query_bwd")
-        return None, gq, None, None
+        l = _lib.lib()
+        gq = gk = None
+        if ctx.needs_input_grad[1]:
+            gq = torch.empty_like(qc)
+            check(l.vadc_memory_query_bwd(ptr(qc), ptr(keys_c), ptr(top1), ptr(top2) if ctx.train else None,
+                                          ptr(g_uq), ptr(g_gather), ptr(g_spread), B, d, h * w,
+                                          keys_c.shape[0], ptr(gq), stream()), "vadc_memory_query_bwd")
+        if ctx.needs_input_grad[2] and g_uq is not None:   # the losses reach keys only through detached copies
+            score_memory = ctx.saved_tensors[4]
+            m = keys_c.shape[0]
+            gk = torch.empty_like(keys_c)
+            ws = workspace(l.vadc_memory_keys_bwd_workspace_bytes(B, d, h * w, m), gk.device)
+            check(l.vadc_memory_keys_bwd(ptr(score_memory), ptr(g_uq), B, d, h * w, m, ptr(gk), ptr(ws), ws.numel(),
+                                         stream()), "vadc_memory_keys_bwd")
+        return None, gq, gk, None
 
 
 class Memory(nn.Module):
-    """Drop-in for model/Memory.py:62-261.  ``forward`` is differentiable with respect to ``query``
-    (``_MemoryForward``); the stand-alone public methods (``read``, ``gather_loss``, ...) are
-    forward-only.  The reference module is not wired into ``Mymodel`` (SURVEY.md D5)."""
+    """Drop-in for model/Memory.py:62-261.  ``forward`` is differentiable with respect to ``query`` and, when they
+    require grad, the memory items ``keys`` (``_MemoryForward``); the stand-alone public methods (``read``,
+    ``gather_loss``, ...) are forward-only.  The reference module is not wired into ``Mymodel`` (SURVEY.md D5)."""
 
     def __init__(self, memory_size, feature_dim, key_dim, temp_update, temp_gather):
         super().__init__()

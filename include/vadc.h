@@ -251,6 +251,14 @@ int vadc_memory_query_bwd(const float* query, const float* keys, const int64_t* 
                           const float* g_gather, const float* g_spread, int B, int d,
                           int64_t HW, int m, float* g_query, void* stream);
 
+/* The same with g_qhat [B,d,HW] (may be NULL): a gradient with respect to the normalised query q-hat (in the query's
+ * layout) added to what is pulled back through F.normalize, in the same single pass — the share of the returned score
+ * matrices (vadc_memory_scores_bwd). */
+int vadc_memory_query_bwd_ex(const float* query, const float* keys, const int64_t* top1,
+                             const int64_t* top2, const float* g_updated_query,
+                             const float* g_gather, const float* g_spread, const float* g_qhat, int B, int d,
+                             int64_t HW, int m, float* g_query, void* stream);
+
 /* get_score  Memory.py:133-143 (+ the top-1 / top-2 of score_memory that
  * gather_loss :241, spread_loss :223 and update :185 take with torch.topk):
  *   logits = q keys^T [N,m]; score_query = softmax over N; score_memory =
@@ -321,6 +329,30 @@ int vadc_memory_separateness(const float* keys, int m, int d, float* out,
 size_t vadc_memory_keys_bwd_workspace_bytes(int B, int d, int64_t HW, int m);
 int vadc_memory_keys_bwd(const float* score_memory, const float* g_updated_query, int B, int d, int64_t HW,
                          int m, float* g_keys, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Backward through the two score matrices Memory.forward returns (get_score, Memory.py:133-143: s = q-hat K^T,
+ * score_query sq = softmax(s, dim=0), score_memory sm = softmax(s, dim=1)), given their gradients Gq, Gm [N,m]:
+ *   coldot c_i = sum_n Gq[n,i] sq[n,i]                     (vadc_memory_score_coldot; over ALL tokens of the batch:
+ *                                                           under a token-sharded global batch, all-reduce SUM it)
+ *   r_n = sum_i Gm[n,i] sm[n,i],  g_s = sq (Gq - 1 c^T) + sm (Gm - r 1^T)
+ *   g_qhat [B,d,HW] = g_s K   (overwritten; in the query's layout: hand it to vadc_memory_query_bwd_ex)
+ *   g_keys [m,d]   += g_s^T q-hat   (accumulated: added, in a fixed order, to what g_keys holds, e.g. the result of
+ *                                    vadc_memory_keys_bwd; bit-identical across launches)
+ * The column dots are a two-level reduction in a fixed order (no atomics).  g_s is formed in one pass and written
+ * directly as the operand terms of both contractions on the tcgen05 GEMM (g_qhat: one GEMM with rows = tokens;
+ * g_keys: split-K over the tokens with the q-hat terms written from query and its norms).  Precision as the module's
+ * forward: fp16 x2 with power-of-two scales from the measured bounds of Gq, Gm, c and K (no host sync), or
+ * VADC_MEMORY_TERMS=3: bf16 x3.  Either gradient may be NULL (Gq also needs score_query and coldot, Gm needs
+ * score_memory), but not both; one of g_qhat / g_keys may be NULL.  query [B,d,HW], keys [m,d] as in the forward.
+ * d >= 8 (VADC_ERR_UNSUPPORTED otherwise). */
+size_t vadc_memory_score_coldot_workspace_bytes(int64_t N, int m);
+int vadc_memory_score_coldot(const float* score_query, const float* g_score_query, int64_t N, int m,
+                             float* coldot, void* workspace, size_t workspace_bytes, void* stream);
+size_t vadc_memory_scores_bwd_workspace_bytes(int B, int d, int64_t HW, int m);
+int vadc_memory_scores_bwd(const float* query, const float* keys, const float* score_query,
+                           const float* score_memory, const float* g_score_query, const float* g_score_memory,
+                           const float* coldot, int B, int d, int64_t HW, int m, float* g_qhat, float* g_keys,
+                           void* workspace, size_t workspace_bytes, void* stream);
 
 /* Backward of MemoryLoss  Memory.py:52-59 with respect to keys [m,d]; g_out is a device scalar:
  *   S = K K^T/2 + 1/2 - I (recomputed as vadc_memory_separateness does), G = sgn(S) with sgn(0) = 0,

@@ -78,14 +78,15 @@ query_transpose_kernel(const float* __restrict__ query, const float* __restrict_
 // F.normalize(query, dim=1) (:148).  Everything is per token, so one kernel does it in the query's own
 // [B, d, HW] layout: lanes run along hw (coalesced), the 8 warps of a block split the channels and meet
 // in shared memory for the three per-token reductions (|x|^2; the two triplet distances; q . g).
-//   g[c]  = gU[b,c,hw] + ag (q - k1) + cp (q - k1 + eps) - cn (q - k2 + eps)
+//   g[c]  = gU[b,c,hw] + gQ[b,c,hw] + ag (q - k1) + cp (q - k1 + eps) - cn (q - k2 + eps)
 //   gx[c] = (g[c] - q[c] (q . g)) / |x|            (g / 1e-12 where |x| < 1e-12: the clamp is constant)
+// gQ (optional) is the gradient with respect to q-hat that the score matrices contribute (vadc_memory_scores_bwd).
 __global__ void __launch_bounds__(256)
 memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict__ keys,
                         const long long* __restrict__ top1, const long long* __restrict__ top2,
                         const float* __restrict__ g_uq, const float* __restrict__ g_gather,
-                        const float* __restrict__ g_spread, int d, long long HW, long long N,
-                        float* __restrict__ gquery) {
+                        const float* __restrict__ g_spread, const float* __restrict__ g_qhat, int d, long long HW,
+                        long long N, float* __restrict__ gquery) {
   __shared__ float red[2][8][32];
   __shared__ float tot[2][32];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -95,6 +96,7 @@ memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict
   const long long n = (long long)b * HW + hw;
   const float* xp = query + (long long)b * d * HW + hw;
   const float* gp = g_uq ? g_uq + (long long)b * 2 * d * HW + hw : nullptr;
+  const float* hp = g_qhat ? g_qhat + (long long)b * d * HW + hw : nullptr;
   const float* k1 = live ? keys + top1[n] * d : keys;
   const float* k2 = (live && top2) ? keys + top2[n] * d : nullptr;
   const float ag = g_gather ? 2.0f * __ldg(g_gather) / ((float)N * (float)d) : 0.f;
@@ -137,6 +139,7 @@ memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict
   auto grad_at = [&](int c, float q) {
     const float a = q - __ldg(k1 + c);
     float g = gp ? __ldg(gp + (long long)c * HW) : 0.f;
+    if (hp) g += __ldg(hp + (long long)c * HW);
     g += ag * a + cp * (a + kEps);
     if (k2) g -= cn * (q - __ldg(k2 + c) + kEps);
     return g;
@@ -719,31 +722,201 @@ keys_bwd_split_scores_kernel(const float* __restrict__ sm, long long N, int m, l
   }
 }
 
-// g_updated_query [B, 2d, HW], channels d..2d-1 -> terms [TERMS][d][Np] of G_r^T * scale[0] (scale == NULL: 1), read
-// and written along hw; the last batch's blocks also zero the padding columns N..Np-1
+// channels c0..c0+d-1 of a [B, C, HW] tensor -> terms [TERMS][d][Np] of its transpose times scale[0] (NULL: 1) and,
+// per token, tok[n] (NULL: 1); read and written along hw; the last batch's blocks also zero the padding columns N..Np-1.
+// (G_r: g_updated_query with C = 2d, c0 = d; q-hat: query with C = d, c0 = 0, tok = 1 / |x|)
 template <int TERMS>
 __global__ void __launch_bounds__(256)
-keys_bwd_split_grad_kernel(const float* __restrict__ g_uq, int B, int d, long long HW, long long Np,
-                           const float* __restrict__ scale, void* __restrict__ dst) {
+keys_bwd_split_grad_kernel(const float* __restrict__ src, int B, int C, int c0, int d, long long HW, long long Np,
+                           const float* __restrict__ scale, const float* __restrict__ tok, void* __restrict__ dst) {
   const long long hw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int c = blockIdx.y, b = blockIdx.z;
   const long long n = (long long)b * HW + hw;
   float v = 0.f;
-  if (hw < HW) v = __ldg(g_uq + ((long long)b * 2 * d + d + c) * HW + hw) * (scale ? __ldg(scale) : 1.0f);
-  else if (b != B - 1 || n >= Np) return;
+  if (hw < HW) {
+    v = __ldg(src + ((long long)b * C + c0 + c) * HW + hw) * (scale ? __ldg(scale) : 1.0f);
+    if (tok) v *= __ldg(tok + n);
+  } else if (b != B - 1 || n >= Np) {
+    return;
+  }
   store_terms<TERMS>(dst, (long long)d * Np, (long long)c * Np + n, v);
 }
 
-// g_keys[i, c] = sum over split slots s (in slot order) of part[s][i][c]: repeated launches give identical bits
+// g_keys[i, c] (+)= sum over split slots s (in slot order) of part[s][i][c]: repeated launches give identical bits
 __global__ void __launch_bounds__(256)
 keys_bwd_sum_partials_kernel(const float* __restrict__ part, int splits, long long split_stride, long long n,
-                    float* __restrict__ out) {
+                             bool accumulate, float* __restrict__ out) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     float s = 0.f;
     for (int k = 0; k < splits; ++k) s += __ldg(part + k * split_stride + i);
-    out[i] = s;
+    out[i] = accumulate ? out[i] + s : s;
   }
 }
+
+// ---- gradient through the returned score matrices -------------------------------------------------------------
+// get_score (Memory.py:133-143): s = q-hat K^T, sq = softmax(s, dim=0), sm = softmax(s, dim=1).  With Gq, Gm the
+// gradients of score_query, score_memory:
+//   c_i = sum_n Gq[n,i] sq[n,i]  (over every token of the batch),  r_n = sum_i Gm[n,i] sm[n,i]
+//   g_s = sq (Gq - 1 c^T) + sm (Gm - r 1^T);   g_qhat = g_s K,  g_keys += g_s^T q-hat
+
+// column dots, first level: block y sums rows [y rpb, (y+1) rpb) of its column in four interleaved chains
+__global__ void __launch_bounds__(256)
+score_coldot_stage1_kernel(const float* __restrict__ sq, const float* __restrict__ gq, long long N, int m,
+                           long long rpb, float* __restrict__ part) {
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= m) return;
+  const long long r0 = (long long)blockIdx.y * rpb, r1 = min(N, r0 + rpb);
+  float a[4] = {0.f, 0.f, 0.f, 0.f};
+  long long r = r0;
+  for (; r + 3 < r1; r += 4) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) a[j] += __ldg(sq + (r + j) * m + col) * __ldg(gq + (r + j) * m + col);
+  }
+  for (; r < r1; ++r) a[0] += __ldg(sq + r * m + col) * __ldg(gq + r * m + col);
+  part[(long long)blockIdx.y * m + col] = (a[0] + a[1]) + (a[2] + a[3]);
+}
+
+// second level: 32 columns per block, eight warps stride the chunks, merged through shared memory in warp order
+__global__ void __launch_bounds__(256)
+score_coldot_stage2_kernel(const float* __restrict__ part, int chunks, int m, float* __restrict__ coldot) {
+  __shared__ float red[8][32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int col = blockIdx.x * 32 + lane;
+  float s = 0.f;
+  if (col < m)
+    for (int c = wid; c < chunks; c += 8) s += part[(long long)c * m + col];
+  red[wid][lane] = s;
+  __syncthreads();
+  if (wid == 0 && col < m) {
+#pragma unroll
+    for (int w = 1; w < 8; ++w) s += red[w][lane];
+    coldot[col] = s;
+  }
+}
+
+template <int TERMS>
+__device__ __forceinline__ void store4_terms(void* dst, long long plane, long long i, const float (&a)[4]) {
+  if constexpr (TERMS == 2) {
+    __half h[2][4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { h[0][j] = __float2half_rn(a[j]); h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j])); }
+    __half* o = static_cast<__half*>(dst) + i;
+    *reinterpret_cast<uint2*>(o) = *reinterpret_cast<uint2*>(h[0]);
+    *reinterpret_cast<uint2*>(o + plane) = *reinterpret_cast<uint2*>(h[1]);
+  } else {
+    __nv_bfloat16 b[3][4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      b[0][j] = __float2bfloat16_rn(a[j]);
+      const float r1 = a[j] - __bfloat162float(b[0][j]);
+      b[1][j] = __float2bfloat16_rn(r1);
+      b[2][j] = __float2bfloat16_rn(r1 - __bfloat162float(b[1][j]));
+    }
+    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(dst) + i;
+#pragma unroll
+    for (int t = 0; t < 3; ++t) *reinterpret_cast<uint2*>(o + t * plane) = *reinterpret_cast<uint2*>(b[t]);
+  }
+}
+
+// g_s in one pass, one warp per token row, written straight as operand terms [TERMS][Np][m8] of g_s * scale[0]
+// (scale == NULL: 1; rows N..Np-1 and columns m..m8-1 zero).  Gq / Gm == NULL: that term is absent.
+// V4 > 0 (m % 4 == 0, m <= 128 V4, 16-byte aligned rows): the row of sm and Gm stays in registers between the row dot
+// and g_s, as in row_softmax_top2_reg_kernel; V4 == 0: two passes over the row, the second one served by L1.
+template <int TERMS, int V4>
+__global__ void __launch_bounds__(256)
+scores_bwd_gs_kernel(const float* __restrict__ sq, const float* __restrict__ sm, const float* __restrict__ gq,
+                     const float* __restrict__ gm, const float* __restrict__ coldot, long long N, int m, long long Np,
+                     int m8, const float* __restrict__ scale, void* __restrict__ dst) {
+  const int lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (row >= Np) return;
+  const long long plane = Np * m8;
+  if (row >= N) {                                        // padding token: zeros for the contraction over the tokens
+    for (int c = lane; c < m8; c += 32) store_terms<TERMS>(dst, plane, row * m8 + c, 0.f);
+    return;
+  }
+  const float s = scale ? __ldg(scale) : 1.0f;
+  const float* sqr = sq ? sq + row * m : nullptr;
+  const float* gqr = gq ? gq + row * m : nullptr;
+  const float* smr = gm ? sm + row * m : nullptr;
+  const float* gmr = gm ? gm + row * m : nullptr;
+  if constexpr (V4 > 0) {
+    const int n4 = m >> 2;
+    float4 vs[V4], vg[V4];
+    float r = 0.f;
+    if (gmr) {
+#pragma unroll
+      for (int k = 0; k < V4; ++k) {
+        const int i = lane + 32 * k;
+        vs[k] = i < n4 ? ld_stream(reinterpret_cast<const float4*>(smr) + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+        vg[k] = i < n4 ? ld_stream(reinterpret_cast<const float4*>(gmr) + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+        r += (vs[k].x * vg[k].x + vs[k].y * vg[k].y) + (vs[k].z * vg[k].z + vs[k].w * vg[k].w);
+      }
+      r = warp_sum(r);
+    }
+#pragma unroll
+    for (int k = 0; k < V4; ++k) {
+      const int i = lane + 32 * k;
+      if (i >= n4) continue;
+      float a[4] = {0.f, 0.f, 0.f, 0.f};
+      if (gqr) {
+        const float4 p = ld_stream(reinterpret_cast<const float4*>(sqr) + i);
+        const float4 g = ld_stream(reinterpret_cast<const float4*>(gqr) + i);
+        const float4 c = __ldg(reinterpret_cast<const float4*>(coldot) + i);
+        a[0] = p.x * (g.x - c.x); a[1] = p.y * (g.y - c.y); a[2] = p.z * (g.z - c.z); a[3] = p.w * (g.w - c.w);
+      }
+      if (gmr) {
+        a[0] += vs[k].x * (vg[k].x - r); a[1] += vs[k].y * (vg[k].y - r);
+        a[2] += vs[k].z * (vg[k].z - r); a[3] += vs[k].w * (vg[k].w - r);
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) a[j] *= s;
+      store4_terms<TERMS>(dst, plane, row * m8 + 4 * i, a);
+    }
+  } else {
+    float r = 0.f;
+    if (gmr) {
+      for (int i = lane; i < m; i += 32) r += __ldg(smr + i) * __ldg(gmr + i);
+      r = warp_sum(r);
+    }
+    for (int i = lane; i < m; i += 32) {
+      float a = 0.f;
+      if (gqr) a = __ldg(sqr + i) * (__ldg(gqr + i) - __ldg(coldot + i));
+      if (gmr) a += __ldg(smr + i) * (__ldg(gmr + i) - r);
+      store_terms<TERMS>(dst, plane, row * m8 + i, a * s);
+    }
+  }
+  for (int c = m + lane; c < m8; c += 32) store_terms<TERMS>(dst, plane, row * m8 + c, 0.f);
+}
+
+// keys [m, d] -> terms [TERMS][m8][d8] of keys * scale[0] (NULL: 1), zero padded: the MN-major B operand of g_s K
+template <int TERMS>
+__global__ void __launch_bounds__(256)
+scores_bwd_split_keys_kernel(const float* __restrict__ keys, int m, int d, int m8, int d8,
+                             const float* __restrict__ scale, void* __restrict__ dst) {
+  const float s = scale ? __ldg(scale) : 1.0f;
+  for (int r = blockIdx.x; r < m8; r += gridDim.x)
+    for (int c = threadIdx.x; c < d8; c += blockDim.x)
+      store_terms<TERMS>(dst, (long long)m8 * d8, (long long)r * d8 + c,
+                         (r < m && c < d) ? __ldg(keys + (long long)r * d + c) * s : 0.f);
+}
+
+// power-of-two scales of the two contractions, from the measured bounds (float bits) of Gq, Gm, the column dots and K:
+//   |g_s| <= max|Gq| + max|c| + 2 max|Gm|   (sq, sm in [0, 1]; |r_n| <= max|Gm|), put in [2^12, 2^13) like the softmax
+//   weights of the read (small entries stay normal fp16 numbers); K in [4, 8) as in the forward; q-hat has unit rows: 2^13
+//   out = {s_g, s_k, 1 / (s_g s_k), s_q, 1 / (s_g s_q)}
+__global__ void scores_bwd_scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ out) {
+  auto pow2 = [](float bound, int top) {                // 2^e with 2^e bound in [2^(top-1), 2^top); 1 for 0 / non-finite
+    if (!(bound > 0.f) || !isfinite(bound)) return 1.0f;
+    int e;
+    (void)frexpf(bound, &e);
+    return ldexpf(1.0f, max(-100, min(100, top - e)));
+  };
+  const float sg = pow2(__uint_as_float(bits[0]) + __uint_as_float(bits[2]) + 2.0f * __uint_as_float(bits[1]), 13);
+  const float sk = pow2(__uint_as_float(bits[3]), 3), sq = 8192.0f;
+  out[0] = sg; out[1] = sk; out[2] = 1.0f / (sg * sk); out[3] = sq; out[4] = 1.0f / (sg * sq);
+}
+
 
 // MemoryLoss (Memory.py:52-59) backward: G = sgn(S), S = K K^T / 2 + 1/2 - I from the same product and the same
 // expression as SeparatenessEpilogue (sgn(0) = 0, the subgradient torch's abs backward takes)
@@ -812,6 +985,14 @@ extern "C" int vadc_memory_query_bwd(const float* query, const float* keys, cons
                                      const int64_t* top2, const float* g_updated_query,
                                      const float* g_gather, const float* g_spread, int B, int d,
                                      int64_t HW, int m, float* g_query, void* stream) {
+  return vadc_memory_query_bwd_ex(query, keys, top1, top2, g_updated_query, g_gather, g_spread, nullptr, B, d, HW, m,
+                                  g_query, stream);
+}
+
+extern "C" int vadc_memory_query_bwd_ex(const float* query, const float* keys, const int64_t* top1,
+                                        const int64_t* top2, const float* g_updated_query,
+                                        const float* g_gather, const float* g_spread, const float* g_qhat, int B,
+                                        int d, int64_t HW, int m, float* g_query, void* stream) {
   VADC_REQUIRE(B >= 0 && d > 0 && HW > 0 && m > 0, VADC_ERR_BAD_SHAPE);
   if (B == 0) return VADC_OK;
   VADC_REQUIRE(query && keys && top1 && g_query, VADC_ERR_NULL_POINTER);
@@ -821,7 +1002,7 @@ extern "C" int vadc_memory_query_bwd(const float* query, const float* keys, cons
   dim3 grid((unsigned)((HW + 31) / 32), B);
   memory_query_bwd_kernel<<<grid, 256, 0, st>>>(query, keys, reinterpret_cast<const long long*>(top1),
                                                 reinterpret_cast<const long long*>(top2), g_updated_query,
-                                                g_gather, g_spread, d, HW, (long long)B * HW, g_query);
+                                                g_gather, g_spread, g_qhat, d, HW, (long long)B * HW, g_query);
   VADC_CHECK_LAUNCH("memory_query_bwd_kernel");
   return VADC_OK;
 }
@@ -1156,7 +1337,7 @@ extern "C" int vadc_memory_keys_bwd(const float* score_memory, const float* g_up
   if (env_int("VADC_MEMORY_TERMS", 2) == 3) {            // fp32-faithful three-term bf16 split, six products
     keys_bwd_split_scores_kernel<3><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 1.0f, sms);
     VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
-    keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(g_updated_query, B, d, HW, Np, nullptr, gs);
+    keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(g_updated_query, B, 2 * d, d, d, HW, Np, nullptr, nullptr, gs);
     VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
     rc = launch_tc_gemm_ex<true, false>(sms, gs, m8, d, Np, sk, epi, st);
   } else {
@@ -1168,14 +1349,14 @@ extern "C" int vadc_memory_keys_bwd(const float* score_memory, const float* g_up
     if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
     keys_bwd_split_scores_kernel<2><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 8192.0f, sms);
     VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
-    keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(g_updated_query, B, d, HW, Np, sc + 1, gs);
+    keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(g_updated_query, B, 2 * d, d, d, HW, Np, sc + 1, nullptr, gs);
     VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
     rc = launch_tc_gemm_ex_h2<true, false>(sms, gs, m8, d, Np, sk, sc + 2, epi, st);
   }
   if (rc) return rc;
   const long long md = (long long)m * d;
   keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
-      part, sk, (long long)m8 * d, md, g_keys);
+      part, sk, (long long)m8 * d, md, false, g_keys);
   VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
   return VADC_OK;
 }
@@ -1201,5 +1382,139 @@ extern "C" int vadc_memory_separateness_bwd(const float* keys, const float* g_ou
   cudaError_t e = sgemm_auto(m, d, m, Aop, Bop, 0, 0, 1, 1,
                              ScaledStoreEpilogue{g_keys, d, g_out, (float)(1.0 / ((double)m * (m - 1)))}, st);
   if (e != cudaSuccess) return record_cuda_error(e, "separateness bwd sgemm G.K");
+  return VADC_OK;
+}
+
+extern "C" size_t vadc_memory_score_coldot_workspace_bytes(int64_t N, int m) {
+  return align_up((size_t)col_chunks(N) * (m > 0 ? m : 1) * sizeof(float), 256) + 256;
+}
+
+extern "C" int vadc_memory_score_coldot(const float* score_query, const float* g_score_query, int64_t N, int m,
+                                        float* coldot, void* workspace, size_t workspace_bytes, void* stream) {
+  VADC_REQUIRE(N >= 0 && m > 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(coldot && workspace, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(N == 0 || (score_query && g_score_query), VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(workspace_bytes >= vadc_memory_score_coldot_workspace_bytes(N, m), VADC_ERR_WORKSPACE);
+  if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (N == 0) {
+    VADC_CUDA(cudaMemsetAsync(coldot, 0, (size_t)m * sizeof(float), st));
+    return VADC_OK;
+  }
+  const int chunks = col_chunks(N);
+  const long long rpb = (N + chunks - 1) / chunks;
+  float* part = static_cast<float*>(workspace);
+  score_coldot_stage1_kernel<<<dim3((m + 255) / 256, chunks), 256, 0, st>>>(score_query, g_score_query, N, m, rpb, part);
+  VADC_CHECK_LAUNCH("score_coldot_stage1_kernel");
+  score_coldot_stage2_kernel<<<(m + 31) / 32, 256, 0, st>>>(part, chunks, m, coldot);
+  VADC_CHECK_LAUNCH("score_coldot_stage2_kernel");
+  return VADC_OK;
+}
+
+extern "C" size_t vadc_memory_scores_bwd_workspace_bytes(int B, int d, int64_t HW, int m) {
+  const long long Np = pad8((long long)(B > 0 ? B : 1) * (HW > 0 ? HW : 1)), m8 = pad8(m > 0 ? m : 1);
+  const int dd = d > 0 ? d : 1;
+  return tc_gemm_split_bytes(Np, m8) + tc_gemm_split_bytes(m8, pad8(dd)) + tc_gemm_split_bytes(dd, Np) +  // terms
+         align_up((size_t)Np * sizeof(float), 256) +                                                     // 1 / |x|
+         align_up((size_t)keys_bwd_splits(Np, (int)m8, dd) * m8 * dd * sizeof(float), 256) + 1024;        // partials, scales
+}
+
+extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, const float* score_query,
+                                      const float* score_memory, const float* g_score_query,
+                                      const float* g_score_memory, const float* coldot, int B, int d, int64_t HW,
+                                      int m, float* g_qhat, float* g_keys, void* workspace, size_t workspace_bytes,
+                                      void* stream) {
+  VADC_REQUIRE(B >= 0 && d > 0 && HW > 0 && m > 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(query && keys && workspace, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(g_score_query || g_score_memory, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(g_qhat || g_keys, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(!g_score_query || (score_query && coldot), VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(!g_score_memory || score_memory, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(d >= 8 && d <= 65535 && B <= 65535 && (long long)B * HW < (1ll << 31) - 8, VADC_ERR_UNSUPPORTED);
+  VADC_REQUIRE(workspace_bytes >= vadc_memory_scores_bwd_workspace_bytes(B, d, HW, m), VADC_ERR_WORKSPACE);
+  if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
+  if (B == 0) return VADC_OK;                            // no tokens: nothing to add to g_keys, g_qhat is empty
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long N = (long long)B * HW, Np = pad8(N);
+  const int m8 = (int)pad8(m), d8 = (int)pad8(d);
+  const int sk = keys_bwd_splits(Np, m8, d);
+  const bool three = env_int("VADC_MEMORY_TERMS", 2) == 3;   // fp32-faithful three-term bf16 split, six products
+  Carver ws(workspace, workspace_bytes);
+  void* gst = ws.take<uint8_t>(tc_gemm_split_bytes(Np, m8));
+  void* kst = ws.take<uint8_t>(tc_gemm_split_bytes(m8, d8));
+  void* qst = ws.take<uint8_t>(tc_gemm_split_bytes(d, Np));
+  float* inv = ws.take<float>(Np);
+  float* part = ws.take<float>((size_t)sk * m8 * d);
+  unsigned* bits = ws.take<unsigned>(64);
+  float* sc = ws.take<float>(64);
+  int rc;
+  if (!three) {
+    // fp16 x2: g_s scaled from the bounds of the incoming gradients (no host sync), K from its measured max
+    VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
+    if (g_score_query) {
+      if ((rc = tc_absmax_bits(g_score_query, N * m, bits, st))) return rc;
+      if ((rc = tc_absmax_bits(coldot, m, bits + 2, st))) return rc;
+    }
+    if (g_score_memory && (rc = tc_absmax_bits(g_score_memory, N * m, bits + 1, st))) return rc;
+    if (g_qhat && (rc = tc_absmax_bits(keys, (long long)m * d, bits + 3, st))) return rc;
+    scores_bwd_scales_kernel<<<1, 1, 0, st>>>(bits, sc);
+    VADC_CHECK_LAUNCH("scores_bwd_scales_kernel");
+  }
+  const float* s_g = three ? nullptr : sc;
+  {
+    const unsigned rg = (unsigned)((Np + 7) / 8);
+    const bool regs = (m % 4) == 0 && m <= 2048 && (!score_query || aligned16(score_query)) &&
+                      (!score_memory || aligned16(score_memory)) && (!g_score_query || aligned16(g_score_query)) &&
+                      (!g_score_memory || aligned16(g_score_memory)) && (!coldot || aligned16(coldot));
+    const float* sq = g_score_query ? score_query : nullptr;
+    const int V4 = !regs ? 0 : (m <= 512 ? 4 : (m <= 1024 ? 8 : 16));
+#define VADC_GS_LAUNCH(T, V)                                                                                       \
+  scores_bwd_gs_kernel<T, V><<<rg, 256, 0, st>>>(sq, score_memory, g_score_query, g_score_memory, coldot, N, m, Np, \
+                                                 m8, s_g, gst)
+    if (three) {
+      if (V4 == 4) VADC_GS_LAUNCH(3, 4); else if (V4 == 8) VADC_GS_LAUNCH(3, 8);
+      else if (V4 == 16) VADC_GS_LAUNCH(3, 16); else VADC_GS_LAUNCH(3, 0);
+    } else {
+      if (V4 == 4) VADC_GS_LAUNCH(2, 4); else if (V4 == 8) VADC_GS_LAUNCH(2, 8);
+      else if (V4 == 16) VADC_GS_LAUNCH(2, 16); else VADC_GS_LAUNCH(2, 0);
+    }
+#undef VADC_GS_LAUNCH
+    VADC_CHECK_LAUNCH("scores_bwd_gs_kernel");
+  }
+  if (g_qhat) {
+    // g_qhat [tokens, d8] = g_s [Np, m8] (K-major A) . K [m8, d8] (MN-major B), stored into [B, d, HW]
+    const unsigned kr = (unsigned)std::min<long long>(m8, 16ll * sm_count());
+    const ScoresQhatEpi epi{g_qhat, N, HW, d};
+    if (three) {
+      scores_bwd_split_keys_kernel<3><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, nullptr, kst);
+      VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
+      if ((rc = launch_tc_gemm_ex<false, true>(gst, kst, Np, d8, m8, 1, epi, st))) return rc;
+    } else {
+      scores_bwd_split_keys_kernel<2><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, sc + 1, kst);
+      VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
+      if ((rc = launch_tc_gemm_ex_h2<false, true>(gst, kst, Np, d8, m8, 1, sc + 2, epi, st))) return rc;
+    }
+  }
+  if (g_keys) {
+    // g_keys [m8, d] += g_s^T q-hat: g_s [Np, m8] the MN-major A operand, q-hat^T [d, Np] (K-major B) written straight
+    // from query and 1 / |x|; split-K over the tokens, the partials then added to g_keys in slot order
+    query_norm_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, st>>>(query, d, HW, inv);
+    VADC_CHECK_LAUNCH("query_norm_kernel");
+    const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
+    const TcPartialEpi epi{part, d, (long long)m8 * d};
+    if (three) {
+      keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, nullptr, inv, qst);
+      VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+      if ((rc = launch_tc_gemm_ex<true, false>(gst, qst, m8, d, Np, sk, epi, st))) return rc;
+    } else {
+      keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, sc + 3, inv, qst);
+      VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+      if ((rc = launch_tc_gemm_ex_h2<true, false>(gst, qst, m8, d, Np, sk, sc + 4, epi, st))) return rc;
+    }
+    const long long md = (long long)m * d;
+    keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
+        part, sk, (long long)m8 * d, md, true, g_keys);
+    VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
+  }
   return VADC_OK;
 }

@@ -346,6 +346,19 @@ struct TcTimeDebedEpi {
   }
 };
 
+// Memory: gradient with respect to q-hat through the score matrices, g_qhat = g_s K (vadc_memory_scores_bwd).  The
+// GEMM's rows (TMEM lanes = epilogue threads) are the tokens, its columns the channels: for each channel a warp stores
+// 32 consecutive tokens, one 128-byte line of the query's [B, d, HW] layout (two where the 32 tokens straddle a batch
+// boundary, n = b HW + hw).  Rows N..Np-1 and channels d..d8-1 are padding.
+struct ScoresQhatEpi {
+  float* out; long long N, HW; int d;
+  __device__ __forceinline__ void operator()(long long n, int c, float (&v)[32], int nvalid, int = 0) const {
+    if (n >= N) return;
+    const long long b = n / HW, hw = n - b * HW;
+    tc_store_col32(out + (b * d + c) * HW + hw, HW, v, min(nvalid, d - c));
+  }
+};
+
 // split-K partial: out[split][m][n]
 struct TcPartialEpi {
   float* out; long long ld, split_stride;

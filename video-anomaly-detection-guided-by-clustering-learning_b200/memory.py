@@ -93,8 +93,11 @@ class _MemoryForward(torch.autograd.Function):
     ``F.normalize`` (:148).  ``keys`` get a gradient only through the read product (:255, ``score_memory`` detached):
     g_keys = score_memory^T G_r, computed when ``keys`` requires grad (e.g. an ``nn.Parameter``; main.py:131 passes
     a plain tensor, and then nothing extra is saved or launched).  Every other use of ``keys`` is detached (:229,
-    :245), ``updated_memory`` is detached (:204); the two score matrices are returned for inspection and are not
-    differentiable here.  Under ``Memory.global_batch`` the read softmax is per token, so each rank's g_keys is the
+    :245), ``updated_memory`` is detached (:204).  The two score matrices are not differentiable unless
+    ``Memory.differentiable_scores`` is set: then, as in the reference graph (get_score, :133-143), their gradients
+    reach the query through F.normalize and, when ``keys`` require grad, the keys (vadc_memory_score_coldot,
+    vadc_memory_scores_bwd), and both matrices are kept for the backward.  Under ``Memory.global_batch`` the read
+    softmax is per token and the column dots of score_query are all-reduced, so each rank's g_keys is the
     contribution of its own tokens: their sum over ranks is the full-batch gradient, and summing it is left to the
     caller (DDP's gradient all-reduce, or ``allreduce_sum_packed``)."""
 
@@ -120,7 +123,12 @@ class _MemoryForward(torch.autograd.Function):
             gathering_loss = mod._reduce(gathering_loss.reshape(1) * ctx.loss_scale, "sum")[0]
             if spreading_loss is not None:
                 spreading_loss = mod._reduce(spreading_loss.reshape(1) * ctx.loss_scale, "sum")[0]
-        if ctx.needs_input_grad[2]:                       # learnable memory items: the read needs score_memory back
+        # differentiable score matrices: both are kept for the backward (2 N m floats, as the reference's softmax nodes)
+        ctx.scores = bool(mod.differentiable_scores) and any(ctx.needs_input_grad[1:3])
+        ctx.reduce = mod._reduce if (ctx.scores and glob) else None
+        if ctx.scores:
+            ctx.save_for_backward(qc, keys_c, s.top1, s.top2, s.score_query, s.score_memory)
+        elif ctx.needs_input_grad[2]:                     # learnable memory items: the read needs score_memory back
             ctx.save_for_backward(qc, keys_c, s.top1, s.top2, s.score_memory)
         else:
             ctx.save_for_backward(qc, keys_c, s.top1, s.top2)
@@ -128,20 +136,26 @@ class _MemoryForward(torch.autograd.Function):
         ctx.set_materialize_grads(False)
         if train:
             updated_memory = mod._dp_update(s, keys_c, cm_g) if glob else mod._update(s, keys_c)
-            ctx.mark_non_differentiable(updated_memory, s.score_query, s.score_memory)
+            if ctx.scores:
+                ctx.mark_non_differentiable(updated_memory)
+            else:
+                ctx.mark_non_differentiable(updated_memory, s.score_query, s.score_memory)
             return (updated_query, updated_memory, s.score_query, s.score_memory,
                     gathering_loss, spreading_loss)
-        ctx.mark_non_differentiable(s.score_query, s.score_memory)
+        if not ctx.scores:
+            ctx.mark_non_differentiable(s.score_query, s.score_memory)
         return updated_query, s.score_query, s.score_memory, gathering_loss
 
     @staticmethod
     def backward(ctx, *grads):
         qc, keys_c, top1, top2 = ctx.saved_tensors[:4]
         if ctx.train:
-            g_uq, _, _, _, g_gather, g_spread = grads
+            g_uq, _, g_sq, g_sm, g_gather, g_spread = grads
         else:
-            (g_uq, _, _, g_gather), g_spread = grads, None
-        if g_uq is None and g_gather is None and g_spread is None:
+            (g_uq, g_sq, g_sm, g_gather), g_spread = grads, None
+        if not ctx.scores:
+            g_sq = g_sm = None
+        if g_uq is None and g_gather is None and g_spread is None and g_sq is None and g_sm is None:
             return None, None, None, None
         B, d, h, w = qc.shape
         g_uq = None if g_uq is None else f32c(g_uq)                  # [B,2d,h,w]; the first d channels reach q
@@ -149,26 +163,63 @@ class _MemoryForward(torch.autograd.Function):
         g_gather = None if g_gather is None else f32c(g_gather).reshape(1) * ctx.loss_scale
         g_spread = None if g_spread is None else f32c(g_spread).reshape(1) * ctx.loss_scale
         l = _lib.lib()
+        m = keys_c.shape[0]
         gq = gk = None
-        if ctx.needs_input_grad[1]:
-            gq = torch.empty_like(qc)
-            check(l.vadc_memory_query_bwd(ptr(qc), ptr(keys_c), ptr(top1), ptr(top2) if ctx.train else None,
-                                          ptr(g_uq), ptr(g_gather), ptr(g_spread), B, d, h * w,
-                                          keys_c.shape[0], ptr(gq), stream()), "vadc_memory_query_bwd")
         if ctx.needs_input_grad[2] and g_uq is not None:   # the losses reach keys only through detached copies
-            score_memory = ctx.saved_tensors[4]
-            m = keys_c.shape[0]
+            score_memory = ctx.saved_tensors[-1]
             gk = torch.empty_like(keys_c)
             ws = workspace(l.vadc_memory_keys_bwd_workspace_bytes(B, d, h * w, m), gk.device)
             check(l.vadc_memory_keys_bwd(ptr(score_memory), ptr(g_uq), B, d, h * w, m, ptr(gk), ptr(ws), ws.numel(),
                                          stream()), "vadc_memory_keys_bwd")
+        g_qhat = None
+        if g_sq is not None or g_sm is not None:
+            g_qhat, gk = _scores_backward(ctx, qc, keys_c, f32c(g_sq), f32c(g_sm), gk)
+        if ctx.needs_input_grad[1]:
+            gq = torch.empty_like(qc)
+            if g_qhat is None:
+                check(l.vadc_memory_query_bwd(ptr(qc), ptr(keys_c), ptr(top1), ptr(top2) if ctx.train else None,
+                                              ptr(g_uq), ptr(g_gather), ptr(g_spread), B, d, h * w,
+                                              m, ptr(gq), stream()), "vadc_memory_query_bwd")
+            else:
+                check(l.vadc_memory_query_bwd_ex(ptr(qc), ptr(keys_c), ptr(top1), ptr(top2) if ctx.train else None,
+                                                 ptr(g_uq), ptr(g_gather), ptr(g_spread), ptr(g_qhat), B, d, h * w,
+                                                 m, ptr(gq), stream()), "vadc_memory_query_bwd_ex")
         return None, gq, gk, None
+
+
+def _scores_backward(ctx, qc, keys_c, g_sq, g_sm, gk):
+    """the share of the returned score matrices: (g_qhat [B,d,h,w] or None, g_keys) with g_keys = gk + g_s^T q-hat
+    when the keys require grad (gk None: the read contributed nothing)"""
+    sq, sm = ctx.saved_tensors[-2:]
+    B, d, h, w = qc.shape
+    N, m = sm.shape
+    l = _lib.lib()
+    coldot = None
+    if g_sq is not None:
+        coldot = torch.empty((m,), device=qc.device, dtype=torch.float32)
+        ws = workspace(l.vadc_memory_score_coldot_workspace_bytes(N, m), qc.device)
+        check(l.vadc_memory_score_coldot(ptr(sq), ptr(g_sq), N, m, ptr(coldot), ptr(ws), ws.numel(), stream()),
+              "vadc_memory_score_coldot")
+        if ctx.reduce is not None:                        # global batch: the column softmax spans every rank's tokens
+            coldot = ctx.reduce(coldot, "sum")
+    g_qhat = torch.empty_like(qc) if ctx.needs_input_grad[1] else None
+    if ctx.needs_input_grad[2] and gk is None:
+        gk = torch.zeros_like(keys_c)
+    elif not ctx.needs_input_grad[2]:
+        gk = None
+    ws = workspace(l.vadc_memory_scores_bwd_workspace_bytes(B, d, h * w, m), qc.device)
+    check(l.vadc_memory_scores_bwd(ptr(qc), ptr(keys_c), ptr(sq), ptr(sm), ptr(g_sq), ptr(g_sm), ptr(coldot),
+                                   B, d, h * w, m, ptr(g_qhat), ptr(gk), ptr(ws), ws.numel(), stream()),
+          "vadc_memory_scores_bwd")
+    return g_qhat, gk
 
 
 class Memory(nn.Module):
     """Drop-in for model/Memory.py:62-261.  ``forward`` is differentiable with respect to ``query`` and, when they
-    require grad, the memory items ``keys`` (``_MemoryForward``); the stand-alone public methods (``read``,
-    ``gather_loss``, ...) are forward-only.  The reference module is not wired into ``Mymodel`` (SURVEY.md D5)."""
+    require grad, the memory items ``keys`` (``_MemoryForward``); with ``differentiable_scores`` set, also through
+    the returned ``score_query`` / ``score_memory``.  The stand-alone public methods (``get_score``, ``read``,
+    ``gather_loss``, ...) are forward-only, and ``updated_memory`` carries no gradient to ``keys`` (detached in the
+    reference too).  The reference module is not wired into ``Mymodel`` (SURVEY.md D5)."""
 
     def __init__(self, memory_size, feature_dim, key_dim, temp_update, temp_gather):
         super().__init__()
@@ -182,6 +233,11 @@ class Memory(nn.Module):
         # single-process full-batch result: all-reduce MAX of the column maxima [m], SUM of the column sums [m],
         # SUM of the update sums [m,d] and of three scalars
         self.global_batch = False
+        # True: score_query and score_memory returned by forward are differentiable, as in the reference (a loss on
+        # the addressing weights, e.g. an entropy penalty, reaches the query and learnable keys).  False (default):
+        # they are returned for inspection only, and nothing extra is kept for the backward.  When True, the two
+        # [N, m] matrices stay alive until the backward (2 N m floats: 1 GB at N = 65536, m = 2000).
+        self.differentiable_scores = False
         self._reduce = _dist_reduce
 
     # -- helpers ------------------------------------------------------------

@@ -354,6 +354,41 @@ int vadc_memory_scores_bwd(const float* query, const float* keys, const float* s
                            const float* coldot, int B, int d, int64_t HW, int m, float* g_qhat, float* g_keys,
                            void* workspace, size_t workspace_bytes, void* stream);
 
+/* Backward of the stand-alone methods (get_score :133-143, read :249-261, gather_loss :233-247, spread_loss :214-231),
+ * which take the query channel-last, [B,h,w,d] flattened to q [N,d], and do not normalise it.
+ *
+ * vadc_memory_scores_bwd_rows: the channel-last twin of vadc_memory_scores_bwd, with s = q K^T for q as passed:
+ *   g_q_rows [N,d] = g_s K      (overwritten; one GEMM with rows = channels, stored one 128-byte line of a row per warp)
+ *   g_keys [m,d]  += g_s^T q    (accumulated in a fixed order, bit-identical across launches; split-K over the tokens,
+ *                                the operand terms of q written in one transposing pass)
+ * coldot from vadc_memory_score_coldot.  Precision as vadc_memory_scores_bwd, except that in fp16 x2 q is scaled by the
+ * power of two of its measured bound (no host sync).  Either gradient may be NULL (Gq also needs score_query and
+ * coldot, Gm needs score_memory), but not both; one of g_q_rows / g_keys may be NULL.  d >= 8 (VADC_ERR_UNSUPPORTED
+ * otherwise). */
+size_t vadc_memory_scores_bwd_rows_workspace_bytes(int64_t N, int d, int m);
+int vadc_memory_scores_bwd_rows(const float* q, const float* keys, const float* score_query,
+                                const float* score_memory, const float* g_score_query, const float* g_score_memory,
+                                const float* coldot, int64_t N, int d, int m, float* g_q_rows, float* g_keys,
+                                void* workspace, size_t workspace_bytes, void* stream);
+
+/* vadc_memory_rows_bwd: the query gradient of read / gather_loss / spread_loss, channel-last and without the
+ * normalisation (the counterpart of vadc_memory_query_bwd_ex), one per-token pass:
+ *   g_query[n,c] = g_updated_query[b,c,hw] + g_q_rows[n,c] + g_gather 2 (q - keys[top1]) / (N d)
+ *                + g_spread / N (TripletMarginLoss(margin=1,p=2,eps=1e-6) gradient of (q, keys[top1], keys[top2]))
+ * with n = b HW + hw.  q, g_q_rows, g_query [N,d]; g_updated_query [B,2d,HW] (only channels 0..d-1 are read).  Each
+ * term may be NULL, but not all of them; g_gather and g_spread are device scalars; the gather term needs top1, the
+ * spread term top1 and top2.  g_q_rows may be g_query (updated in place).  No workspace. */
+int vadc_memory_rows_bwd(const float* q, const float* keys, const int64_t* top1, const int64_t* top2,
+                         const float* g_updated_query, const float* g_gather, const float* g_spread,
+                         const float* g_q_rows, int B, int d, int64_t HW, int m, float* g_query, void* stream);
+
+/* vadc_memory_prepare_query_bwd: backward of vadc_memory_prepare_query (F.normalize(query, dim=1) + permute, :148-149):
+ *   g_x[b,:,hw] = (g - q-hat (q-hat . g)) / max(|x|, 1e-12),  q-hat = x / max(|x|, 1e-12),  x = query[b,:,hw]
+ * (q-hat . g taken as 0 where |x| < 1e-12: the clamp is a constant).  g [B,HW,d] channel-last, query and g_x [B,d,HW];
+ * one pass.  No workspace. */
+int vadc_memory_prepare_query_bwd(const float* g, const float* query, int B, int d, int64_t HW, float* g_x,
+                                  void* stream);
+
 /* Backward of MemoryLoss  Memory.py:52-59 with respect to keys [m,d]; g_out is a device scalar:
  *   S = K K^T/2 + 1/2 - I (recomputed as vadc_memory_separateness does), G = sgn(S) with sgn(0) = 0,
  *   g_keys = g_out / (m (m-1)) * (G + G^T)/2 K   (G is symmetric bit for bit).  g_keys is overwritten. */

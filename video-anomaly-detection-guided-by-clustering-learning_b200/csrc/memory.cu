@@ -81,6 +81,33 @@ query_transpose_kernel(const float* __restrict__ query, const float* __restrict_
 //   g[c]  = gU[b,c,hw] + gQ[b,c,hw] + ag (q - k1) + cp (q - k1 + eps) - cn (q - k2 + eps)
 //   gx[c] = (g[c] - q[c] (q . g)) / |x|            (g / 1e-12 where |x| < 1e-12: the clamp is constant)
 // gQ (optional) is the gradient with respect to q-hat that the score matrices contribute (vadc_memory_scores_bwd).
+// The per-token loss maths below is shared with the channel-last twin (memory_rows_bwd_kernel).
+constexpr float kTripletEps = 1e-6f;            // pairwise_distance eps (TripletMarginLoss)
+
+// the loss weights: ag = 2 g_gather / (N d) (MSELoss mean), gs = g_spread / N (TripletMarginLoss mean)
+__device__ __forceinline__ void memory_loss_weights(const float* g_gather, const float* g_spread, bool spread,
+                                                    long long N, int d, float& ag, float& gs) {
+  ag = g_gather ? 2.0f * __ldg(g_gather) / ((float)N * (float)d) : 0.f;
+  gs = (g_spread && spread) ? __ldg(g_spread) / (float)N : 0.f;
+}
+
+// triplet coefficients from the two squared distances |q - k1 + eps|^2, |q - k2 + eps|^2 (clamp_min(., 0) backward)
+__device__ __forceinline__ void triplet_coefs(float dp2, float dn2, float gs, float& cp, float& cn) {
+  const float dap = sqrtf(dp2), dan = sqrtf(dn2);
+  const bool active = dap - dan + 1.0f >= 0.f;
+  cp = (active && dap > 0.f) ? gs / dap : 0.f;
+  cn = (active && dan > 0.f) ? gs / dan : 0.f;
+}
+
+// g + the gathering and spreading terms at one channel: ag (q - k1) + cp (q - k1 + eps) - cn (q - k2 + eps)
+__device__ __forceinline__ float add_loss_grads(float g, float q, float k1, const float* k2, int c, float ag, float cp,
+                                                float cn) {
+  const float a = q - k1;
+  g += ag * a + cp * (a + kTripletEps);
+  if (k2) g -= cn * (q - __ldg(k2 + c) + kTripletEps);
+  return g;
+}
+
 __global__ void __launch_bounds__(256)
 memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict__ keys,
                         const long long* __restrict__ top1, const long long* __restrict__ top2,
@@ -99,9 +126,9 @@ memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict
   const float* hp = g_qhat ? g_qhat + (long long)b * d * HW + hw : nullptr;
   const float* k1 = live ? keys + top1[n] * d : keys;
   const float* k2 = (live && top2) ? keys + top2[n] * d : nullptr;
-  const float ag = g_gather ? 2.0f * __ldg(g_gather) / ((float)N * (float)d) : 0.f;
-  const float gs = (g_spread && top2) ? __ldg(g_spread) / (float)N : 0.f;
-  constexpr float kEps = 1e-6f;
+  float ag, gs;
+  memory_loss_weights(g_gather, g_spread, top2 != nullptr, N, d, ag, gs);
+  constexpr float kEps = kTripletEps;
   auto reduce2 = [&](float a, float c) {      // block-wide sums per lane (token) of two values
     red[0][wid][lane] = a; red[1][wid][lane] = c;
     __syncthreads();
@@ -130,19 +157,13 @@ memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict
       dp += a * a; dn += e * e;
     }
     reduce2(dp, dn);
-    const float dap = sqrtf(tot[0][lane]), dan = sqrtf(tot[1][lane]);
-    const bool active = dap - dan + 1.0f >= 0.f;          // clamp_min(., 0) backward
-    cp = (active && dap > 0.f) ? gs / dap : 0.f;
-    cn = (active && dan > 0.f) ? gs / dan : 0.f;
+    triplet_coefs(tot[0][lane], tot[1][lane], gs, cp, cn);
     __syncthreads();
   }
   auto grad_at = [&](int c, float q) {
-    const float a = q - __ldg(k1 + c);
     float g = gp ? __ldg(gp + (long long)c * HW) : 0.f;
     if (hp) g += __ldg(hp + (long long)c * HW);
-    g += ag * a + cp * (a + kEps);
-    if (k2) g -= cn * (q - __ldg(k2 + c) + kEps);
-    return g;
+    return add_loss_grads(g, q, __ldg(k1 + c), k2, c, ag, cp, cn);
   };
   // 3: q . g
   float dot = 0.f;
@@ -156,6 +177,118 @@ memory_query_bwd_kernel(const float* __restrict__ query, const float* __restrict
   if (live) for (int c = wid; c < d; c += 8) {
     const float q = __ldg(xp + (long long)c * HW) * inv;
     gquery[((long long)b * d + c) * HW + hw] = (grad_at(c, q) - q * dot) * inv;
+  }
+}
+
+// ---- backward of the stand-alone methods, channel-last and without the normalisation -------------------------------
+// read / gather_loss / spread_loss (Memory.py:214-261) take q [N, d] as passed, so the query gradient is per token:
+//   g[n, c] = gU[b, c, hw] + gR[n, c] + ag (q - k1) + cp (q - k1 + eps) - cn (q - k2 + eps),   n = b HW + hw
+// A block owns 32 tokens of one batch and each warp four of them.  The triplet distances are warp sums along the
+// token's row (lanes along channels); gU ([B, 2d, HW], lanes along hw) is staged through shared memory 32 channels at
+// a time, so that its reads and the [N, d] writes are both 128-byte lines.  g_rows may be the output (read, then
+// written by the same thread).
+__global__ void __launch_bounds__(256)
+memory_rows_bwd_kernel(const float* __restrict__ q, const float* __restrict__ keys, const long long* __restrict__ top1,
+                       const long long* __restrict__ top2, const float* __restrict__ g_uq,
+                       const float* __restrict__ g_gather, const float* __restrict__ g_spread, const float* g_rows,
+                       int d, long long HW, long long N, float* gquery) {
+  __shared__ float tile[32][33];               // [channel][token]
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int b = blockIdx.y;
+  const long long hw0 = (long long)blockIdx.x * 32;
+  float ag, gs;
+  memory_loss_weights(g_gather, g_spread, top2 != nullptr, N, d, ag, gs);
+  const bool losses = g_gather || (g_spread && top2);
+  const float* k1[4];
+  const float* k2[4];
+  float cp[4], cn[4];
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    const long long hw = hw0 + wid * 4 + t, n = (long long)b * HW + hw;
+    const bool live = hw < HW && losses;
+    k1[t] = live ? keys + top1[n] * d : keys;
+    k2[t] = (live && top2) ? keys + top2[n] * d : nullptr;
+    cp[t] = cn[t] = 0.f;
+    if (k2[t]) {                               // warp-uniform
+      const float* qr = q + n * d;
+      float dp = 0.f, dn = 0.f;
+      for (int c = lane; c < d; c += 32) {
+        const float v = __ldg(qr + c);
+        const float a = v - __ldg(k1[t] + c) + kTripletEps, e = v - __ldg(k2[t] + c) + kTripletEps;
+        dp += a * a; dn += e * e;
+      }
+      triplet_coefs(warp_sum(dp), warp_sum(dn), gs, cp[t], cn[t]);
+    }
+  }
+  for (int c0 = 0; c0 < d; c0 += 32) {
+    if (g_uq) {                                // block-uniform
+      const long long hw = hw0 + lane;
+      for (int i = wid; i < 32; i += 8)
+        tile[i][lane] = (hw < HW && c0 + i < d) ? __ldg(g_uq + ((long long)b * 2 * d + c0 + i) * HW + hw) : 0.f;
+      __syncthreads();
+    }
+    const int c = c0 + lane;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const int j = wid * 4 + t;
+      const long long n = (long long)b * HW + hw0 + j;
+      if (hw0 + j >= HW || c >= d) continue;
+      float g = g_uq ? tile[lane][j] : 0.f;
+      if (g_rows) g += g_rows[n * d + c];
+      if (losses) g = add_loss_grads(g, __ldg(q + n * d + c), __ldg(k1[t] + c), k2[t], c, ag, cp[t], cn[t]);
+      gquery[n * d + c] = g;
+    }
+    if (g_uq) __syncthreads();
+  }
+}
+
+// prepare_query backward (F.normalize(query, dim=1) + permute, Memory.py:148-149): g arrives channel-last [B, HW, d],
+// g_x [B, d, HW] = (g - q-hat (q-hat . g)) / max(|x|, 1e-12) per token (dot = 0 where the clamp holds: the clamp is a
+// constant).  A block owns 32 positions (lanes along hw: query reads and g_x writes are 128-byte lines); g is staged
+// through shared memory 32 channels at a time (read along its rows), once for |x|^2 and x . g, once for g_x.
+__global__ void __launch_bounds__(256)
+prepare_query_bwd_kernel(const float* __restrict__ g, const float* __restrict__ query, int d, long long HW,
+                         float* __restrict__ gx) {
+  __shared__ float tile[32][33];               // [channel][position]
+  __shared__ float red[2][8][32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int b = blockIdx.y;
+  const long long hw0 = (long long)blockIdx.x * 32, hw = hw0 + lane;
+  const bool live = hw < HW;
+  const float* xp = query + (long long)b * d * HW + hw;
+  const float* gb = g + ((long long)b * HW + hw0) * d;
+  auto stage = [&](int c0) {
+    for (int j = wid; j < 32; j += 8)
+      tile[lane][j] = (hw0 + j < HW && c0 + lane < d) ? __ldg(gb + (long long)j * d + c0 + lane) : 0.f;
+    __syncthreads();
+  };
+  float s = 0.f, t = 0.f;
+  for (int c0 = 0; c0 < d; c0 += 32) {
+    stage(c0);
+    for (int i = wid; i < 32; i += 8) {
+      const int c = c0 + i;
+      if (live && c < d) { const float x = __ldg(xp + (long long)c * HW); s += x * x; t += x * tile[i][lane]; }
+    }
+    __syncthreads();
+  }
+  red[0][wid][lane] = s; red[1][wid][lane] = t;
+  __syncthreads();
+  s = 0.f; t = 0.f;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) { s += red[0][w][lane]; t += red[1][w][lane]; }
+  const float nrm = sqrtf(s);
+  const float inv = 1.0f / fmaxf(nrm, 1e-12f);
+  const float dot = nrm < 1e-12f ? 0.f : t * inv;      // q-hat . g
+  for (int c0 = 0; c0 < d; c0 += 32) {
+    stage(c0);
+    for (int i = wid; i < 32; i += 8) {
+      const int c = c0 + i;
+      if (live && c < d) {
+        const float qh = __ldg(xp + (long long)c * HW) * inv;
+        gx[((long long)b * d + c) * HW + hw] = (tile[i][lane] - qh * dot) * inv;
+      }
+    }
+    __syncthreads();
   }
 }
 
@@ -889,6 +1022,51 @@ scores_bwd_gs_kernel(const float* __restrict__ sq, const float* __restrict__ sm,
   for (int c = m + lane; c < m8; c += 32) store_terms<TERMS>(dst, plane, row * m8 + c, 0.f);
 }
 
+// q [N, d] row-major -> terms [TERMS][d][Np] of its transpose times scale[0] (NULL: 1), tokens N..Np-1 zero: the
+// K-major B operand of g_s^T q for the channel-last query.  A block moves 64 tokens x 32 channels through shared memory:
+// a warp reads 128 bytes of a token row, and writes two tokens per lane along a channel row (128 bytes per term).
+template <int TERMS>
+__global__ void __launch_bounds__(256)
+rows_transpose_terms_kernel(const float* __restrict__ q, long long N, int d, long long Np,
+                            const float* __restrict__ scale, void* __restrict__ dst) {
+  __shared__ float tile[32][65];               // [channel][token]
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const long long n0 = (long long)blockIdx.x * 64;
+  const int c0 = blockIdx.y * 32;
+  for (int j = wid; j < 64; j += 8) {
+    const long long n = n0 + j;
+    tile[lane][j] = (n < N && c0 + lane < d) ? __ldg(q + n * d + c0 + lane) : 0.f;
+  }
+  __syncthreads();
+  const float s = scale ? __ldg(scale) : 1.0f;
+  const long long plane = (long long)d * Np, n = n0 + 2 * lane;
+  if (n >= Np) return;                         // Np is a multiple of eight: both tokens of a pair are in or out
+  for (int i = wid; i < 32 && c0 + i < d; i += 8) {
+    const float a0 = tile[i][2 * lane] * s, a1 = tile[i][2 * lane + 1] * s;
+    const long long o = (long long)(c0 + i) * Np + n;
+    if constexpr (TERMS == 2) {
+      const __half h0 = __float2half_rn(a0), h1 = __float2half_rn(a1);
+      __half2* t = reinterpret_cast<__half2*>(static_cast<__half*>(dst) + o);
+      t[0] = __halves2half2(h0, h1);
+      *reinterpret_cast<__half2*>(static_cast<__half*>(dst) + plane + o) =
+          __halves2half2(__float2half_rn(a0 - __half2float(h0)), __float2half_rn(a1 - __half2float(h1)));
+    } else {
+      __nv_bfloat16 b[2][3];
+      const float a[2] = {a0, a1};
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        b[k][0] = __float2bfloat16_rn(a[k]);
+        const float r1 = a[k] - __bfloat162float(b[k][0]);
+        b[k][1] = __float2bfloat16_rn(r1);
+        b[k][2] = __float2bfloat16_rn(r1 - __bfloat162float(b[k][1]));
+      }
+      __nv_bfloat16* t = static_cast<__nv_bfloat16*>(dst) + o;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) *reinterpret_cast<__nv_bfloat162*>(t + k * plane) = __halves2bfloat162(b[0][k], b[1][k]);
+    }
+  }
+}
+
 // keys [m, d] -> terms [TERMS][m8][d8] of keys * scale[0] (NULL: 1), zero padded: the MN-major B operand of g_s K
 template <int TERMS>
 __global__ void __launch_bounds__(256)
@@ -903,9 +1081,10 @@ scores_bwd_split_keys_kernel(const float* __restrict__ keys, int m, int d, int m
 
 // power-of-two scales of the two contractions, from the measured bounds (float bits) of Gq, Gm, the column dots and K:
 //   |g_s| <= max|Gq| + max|c| + 2 max|Gm|   (sq, sm in [0, 1]; |r_n| <= max|Gm|), put in [2^12, 2^13) like the softmax
-//   weights of the read (small entries stay normal fp16 numbers); K in [4, 8) as in the forward; q-hat has unit rows: 2^13
+//   weights of the read (small entries stay normal fp16 numbers); K in [4, 8) as in the forward; q-hat has unit rows: 2^13,
+//   an unnormalised q (q_measured: its bound in bits[4]) is put in [2^12, 2^13) like g_s
 //   out = {s_g, s_k, 1 / (s_g s_k), s_q, 1 / (s_g s_q)}
-__global__ void scores_bwd_scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ out) {
+__global__ void scores_bwd_scales_kernel(const unsigned* __restrict__ bits, bool q_measured, float* __restrict__ out) {
   auto pow2 = [](float bound, int top) {                // 2^e with 2^e bound in [2^(top-1), 2^top); 1 for 0 / non-finite
     if (!(bound > 0.f) || !isfinite(bound)) return 1.0f;
     int e;
@@ -913,7 +1092,7 @@ __global__ void scores_bwd_scales_kernel(const unsigned* __restrict__ bits, floa
     return ldexpf(1.0f, max(-100, min(100, top - e)));
   };
   const float sg = pow2(__uint_as_float(bits[0]) + __uint_as_float(bits[2]) + 2.0f * __uint_as_float(bits[1]), 13);
-  const float sk = pow2(__uint_as_float(bits[3]), 3), sq = 8192.0f;
+  const float sk = pow2(__uint_as_float(bits[3]), 3), sq = q_measured ? pow2(__uint_as_float(bits[4]), 13) : 8192.0f;
   out[0] = sg; out[1] = sk; out[2] = 1.0f / (sg * sk); out[3] = sq; out[4] = 1.0f / (sg * sq);
 }
 
@@ -1419,21 +1598,23 @@ extern "C" size_t vadc_memory_scores_bwd_workspace_bytes(int B, int d, int64_t H
          align_up((size_t)keys_bwd_splits(Np, (int)m8, dd) * m8 * dd * sizeof(float), 256) + 1024;        // partials, scales
 }
 
-extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, const float* score_query,
-                                      const float* score_memory, const float* g_score_query,
-                                      const float* g_score_memory, const float* coldot, int B, int d, int64_t HW,
-                                      int m, float* g_qhat, float* g_keys, void* workspace, size_t workspace_bytes,
-                                      void* stream) {
+// shared by vadc_memory_scores_bwd (query [B, d, HW], normalised where its operand terms are written) and
+// vadc_memory_scores_bwd_rows (q [N, d] as passed: B = 1, HW = N): checks, scales, the g_s pass and the two contractions,
+// whose query-side operand and epilogue follow the query's layout
+static int scores_bwd_impl(const float* query, bool rows, const float* keys, const float* score_query,
+                           const float* score_memory, const float* g_score_query, const float* g_score_memory,
+                           const float* coldot, int B, int d, int64_t HW, int m, float* g_q, float* g_keys,
+                           void* workspace, size_t workspace_bytes, void* stream) {
   VADC_REQUIRE(B >= 0 && d > 0 && HW > 0 && m > 0, VADC_ERR_BAD_SHAPE);
   VADC_REQUIRE(query && keys && workspace, VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(g_score_query || g_score_memory, VADC_ERR_NULL_POINTER);
-  VADC_REQUIRE(g_qhat || g_keys, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(g_q || g_keys, VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(!g_score_query || (score_query && coldot), VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(!g_score_memory || score_memory, VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(d >= 8 && d <= 65535 && B <= 65535 && (long long)B * HW < (1ll << 31) - 8, VADC_ERR_UNSUPPORTED);
   VADC_REQUIRE(workspace_bytes >= vadc_memory_scores_bwd_workspace_bytes(B, d, HW, m), VADC_ERR_WORKSPACE);
   if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
-  if (B == 0) return VADC_OK;                            // no tokens: nothing to add to g_keys, g_qhat is empty
+  if (B == 0) return VADC_OK;                            // no tokens: nothing to add to g_keys, g_q is empty
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const long long N = (long long)B * HW, Np = pad8(N);
   const int m8 = (int)pad8(m), d8 = (int)pad8(d);
@@ -1449,15 +1630,18 @@ extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, con
   float* sc = ws.take<float>(64);
   int rc;
   if (!three) {
-    // fp16 x2: g_s scaled from the bounds of the incoming gradients (no host sync), K from its measured max
+    // fp16 x2: g_s scaled from the bounds of the incoming gradients (no host sync), K from its measured max, and an
+    // unnormalised q (rows) from its measured max
     VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
     if (g_score_query) {
       if ((rc = tc_absmax_bits(g_score_query, N * m, bits, st))) return rc;
       if ((rc = tc_absmax_bits(coldot, m, bits + 2, st))) return rc;
     }
     if (g_score_memory && (rc = tc_absmax_bits(g_score_memory, N * m, bits + 1, st))) return rc;
-    if (g_qhat && (rc = tc_absmax_bits(keys, (long long)m * d, bits + 3, st))) return rc;
-    scores_bwd_scales_kernel<<<1, 1, 0, st>>>(bits, sc);
+    if (g_q && (rc = tc_absmax_bits(keys, (long long)m * d, bits + 3, st))) return rc;
+    const bool q_measured = rows && g_keys;
+    if (q_measured && (rc = tc_absmax_bits(query, N * d, bits + 4, st))) return rc;
+    scores_bwd_scales_kernel<<<1, 1, 0, st>>>(bits, q_measured, sc);
     VADC_CHECK_LAUNCH("scores_bwd_scales_kernel");
   }
   const float* s_g = three ? nullptr : sc;
@@ -1481,40 +1665,108 @@ extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, con
 #undef VADC_GS_LAUNCH
     VADC_CHECK_LAUNCH("scores_bwd_gs_kernel");
   }
-  if (g_qhat) {
-    // g_qhat [tokens, d8] = g_s [Np, m8] (K-major A) . K [m8, d8] (MN-major B), stored into [B, d, HW]
+  if (g_q) {
+    // g_q = g_s [Np, m8] . K [m8, d8].  Channel-first query: rows = tokens (g_s the K-major A operand, K the MN-major B),
+    // stored into [B, d, HW].  Channel-last (rows): rows = channels (K the MN-major A operand, g_s the K-major B), stored
+    // into [N, d] one 128-byte line of a token row per warp.
     const unsigned kr = (unsigned)std::min<long long>(m8, 16ll * sm_count());
-    const ScoresQhatEpi epi{g_qhat, N, HW, d};
     if (three) {
       scores_bwd_split_keys_kernel<3><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, nullptr, kst);
       VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
-      if ((rc = launch_tc_gemm_ex<false, true>(gst, kst, Np, d8, m8, 1, epi, st))) return rc;
+      rc = rows ? launch_tc_gemm_ex<true, false>(kst, gst, d8, Np, m8, 1, ScoresQRowsTEpi{g_q, N, d}, st)
+                : launch_tc_gemm_ex<false, true>(gst, kst, Np, d8, m8, 1, ScoresQhatEpi{g_q, N, HW, d}, st);
     } else {
       scores_bwd_split_keys_kernel<2><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, sc + 1, kst);
       VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
-      if ((rc = launch_tc_gemm_ex_h2<false, true>(gst, kst, Np, d8, m8, 1, sc + 2, epi, st))) return rc;
+      rc = rows ? launch_tc_gemm_ex_h2<true, false>(kst, gst, d8, Np, m8, 1, sc + 2, ScoresQRowsTEpi{g_q, N, d}, st)
+                : launch_tc_gemm_ex_h2<false, true>(gst, kst, Np, d8, m8, 1, sc + 2, ScoresQhatEpi{g_q, N, HW, d}, st);
     }
+    if (rc) return rc;
   }
   if (g_keys) {
-    // g_keys [m8, d] += g_s^T q-hat: g_s [Np, m8] the MN-major A operand, q-hat^T [d, Np] (K-major B) written straight
-    // from query and 1 / |x|; split-K over the tokens, the partials then added to g_keys in slot order
-    query_norm_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, st>>>(query, d, HW, inv);
-    VADC_CHECK_LAUNCH("query_norm_kernel");
-    const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
-    const TcPartialEpi epi{part, d, (long long)m8 * d};
-    if (three) {
-      keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, nullptr, inv, qst);
-      VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
-      if ((rc = launch_tc_gemm_ex<true, false>(gst, qst, m8, d, Np, sk, epi, st))) return rc;
+    // g_keys [m8, d] += g_s^T q: g_s [Np, m8] the MN-major A operand, q^T [d, Np] (K-major B) written straight from the
+    // query (channel-first: times 1 / |x|, i.e. q-hat; rows: one transposing pass); split-K over the tokens, the
+    // partials then added to g_keys in slot order
+    const float* s_q = three ? nullptr : sc + 3;
+    if (rows) {
+      const dim3 tgrid((unsigned)((Np + 63) / 64), (unsigned)((d + 31) / 32));
+      if (three) rows_transpose_terms_kernel<3><<<tgrid, 256, 0, st>>>(query, N, d, Np, s_q, qst);
+      else rows_transpose_terms_kernel<2><<<tgrid, 256, 0, st>>>(query, N, d, Np, s_q, qst);
+      VADC_CHECK_LAUNCH("rows_transpose_terms_kernel");
     } else {
-      keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, sc + 3, inv, qst);
+      query_norm_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, st>>>(query, d, HW, inv);
+      VADC_CHECK_LAUNCH("query_norm_kernel");
+      const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
+      if (three) keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, s_q, inv, qst);
+      else keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, s_q, inv, qst);
       VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
-      if ((rc = launch_tc_gemm_ex_h2<true, false>(gst, qst, m8, d, Np, sk, sc + 4, epi, st))) return rc;
     }
+    const TcPartialEpi epi{part, d, (long long)m8 * d};
+    if (three) rc = launch_tc_gemm_ex<true, false>(gst, qst, m8, d, Np, sk, epi, st);
+    else rc = launch_tc_gemm_ex_h2<true, false>(gst, qst, m8, d, Np, sk, sc + 4, epi, st);
+    if (rc) return rc;
     const long long md = (long long)m * d;
     keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
         part, sk, (long long)m8 * d, md, true, g_keys);
     VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
   }
+  return VADC_OK;
+}
+
+extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, const float* score_query,
+                                      const float* score_memory, const float* g_score_query,
+                                      const float* g_score_memory, const float* coldot, int B, int d, int64_t HW,
+                                      int m, float* g_qhat, float* g_keys, void* workspace, size_t workspace_bytes,
+                                      void* stream) {
+  return scores_bwd_impl(query, false, keys, score_query, score_memory, g_score_query, g_score_memory, coldot, B, d, HW,
+                         m, g_qhat, g_keys, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t vadc_memory_scores_bwd_rows_workspace_bytes(int64_t N, int d, int m) {
+  return vadc_memory_scores_bwd_workspace_bytes(1, d, N > 0 ? N : 1, m);
+}
+
+extern "C" int vadc_memory_scores_bwd_rows(const float* q, const float* keys, const float* score_query,
+                                           const float* score_memory, const float* g_score_query,
+                                           const float* g_score_memory, const float* coldot, int64_t N, int d, int m,
+                                           float* g_q_rows, float* g_keys, void* workspace, size_t workspace_bytes,
+                                           void* stream) {
+  VADC_REQUIRE(N >= 0, VADC_ERR_BAD_SHAPE);
+  return scores_bwd_impl(q, true, keys, score_query, score_memory, g_score_query, g_score_memory, coldot,
+                         N > 0 ? 1 : 0, d, N > 0 ? N : 1, m, g_q_rows, g_keys, workspace, workspace_bytes, stream);
+}
+
+extern "C" int vadc_memory_rows_bwd(const float* q, const float* keys, const int64_t* top1, const int64_t* top2,
+                                    const float* g_updated_query, const float* g_gather, const float* g_spread,
+                                    const float* g_q_rows, int B, int d, int64_t HW, int m, float* g_query,
+                                    void* stream) {
+  VADC_REQUIRE(B >= 0 && d > 0 && HW > 0 && m > 0, VADC_ERR_BAD_SHAPE);
+  if (B == 0) return VADC_OK;
+  VADC_REQUIRE(q && keys && g_query, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(g_updated_query || g_gather || g_spread || g_q_rows, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(!(g_gather || g_spread) || top1, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(!g_spread || top2, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(B <= 65535 && (long long)B * HW < (1ll << 31), VADC_ERR_UNSUPPORTED);
+  if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  dim3 grid((unsigned)((HW + 31) / 32), B);
+  memory_rows_bwd_kernel<<<grid, 256, 0, st>>>(q, keys, reinterpret_cast<const long long*>(top1),
+                                               g_spread ? reinterpret_cast<const long long*>(top2) : nullptr,
+                                               g_updated_query, g_gather, g_spread, g_q_rows, d, HW,
+                                               (long long)B * HW, g_query);
+  VADC_CHECK_LAUNCH("memory_rows_bwd_kernel");
+  return VADC_OK;
+}
+
+extern "C" int vadc_memory_prepare_query_bwd(const float* g, const float* query, int B, int d, int64_t HW,
+                                             float* g_x, void* stream) {
+  VADC_REQUIRE(B >= 0 && d > 0 && HW > 0, VADC_ERR_BAD_SHAPE);
+  if (B == 0) return VADC_OK;
+  VADC_REQUIRE(g && query && g_x, VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(B <= 65535, VADC_ERR_UNSUPPORTED);
+  if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
+  prepare_query_bwd_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      g, query, d, HW, g_x);
+  VADC_CHECK_LAUNCH("prepare_query_bwd_kernel");
   return VADC_OK;
 }

@@ -731,6 +731,7 @@ template int launch_tc_gemm_ex_h2<true, false, TcGzTEpi>(const void*, const void
 template int launch_tc_gemm_ex_h2<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex_h2<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex_h2<false, true, ScoresQhatEpi>(const void*, const void*, long long, long long, long long, int, const float*, ScoresQhatEpi, cudaStream_t);
+template int launch_tc_gemm_ex_h2<true, false, ScoresQRowsTEpi>(const void*, const void*, long long, long long, long long, int, const float*, ScoresQRowsTEpi, cudaStream_t);
 
 template <bool B_MN, class Epi>
 int launch_tc_gemm(const void* a_split, const void* b_split, long long M, long long N, long long Kd, Epi epi,
@@ -748,6 +749,7 @@ template int launch_tc_gemm<false, TcTimeDebedEpi>(const void*, const void*, lon
 template int launch_tc_gemm_ex<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
 template int launch_tc_gemm_ex<false, true, ScoresQhatEpi>(const void*, const void*, long long, long long, long long, int, ScoresQhatEpi, cudaStream_t);
+template int launch_tc_gemm_ex<true, false, ScoresQRowsTEpi>(const void*, const void*, long long, long long, long long, int, ScoresQRowsTEpi, cudaStream_t);
 template int launch_tc_gemm_ex<true, false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, int, TcStoreTEpi, cudaStream_t);
 template int launch_tc_gemm<false, TcBiasEpi>(const void*, const void*, long long, long long, long long, TcBiasEpi, cudaStream_t);
 template int launch_tc_gemm<false, TcBiasTEpi>(const void*, const void*, long long, long long, long long, TcBiasTEpi, cudaStream_t);

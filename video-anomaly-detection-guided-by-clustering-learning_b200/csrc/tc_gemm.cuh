@@ -359,6 +359,17 @@ struct ScoresQhatEpi {
   }
 };
 
+// Memory: g_q = g_s K for the stand-alone methods' channel-last query [N, d] (vadc_memory_scores_bwd_rows), transposed:
+// the GEMM's rows are the channels (K's terms [m8, d8] the MN-major A operand), its columns the tokens, so for each token
+// a warp stores 32 consecutive channels, one 128-byte line of its row.  Channels d..d8-1 and tokens N..Np-1 are padding.
+struct ScoresQRowsTEpi {
+  float* out; long long N; int d;
+  __device__ __forceinline__ void operator()(long long c, int r0, float (&v)[32], int nvalid, int = 0) const {
+    if (c >= d) return;
+    tc_store_col32(out + (long long)r0 * d + c, d, v, (int)min((long long)nvalid, N - r0));
+  }
+};
+
 // split-K partial: out[split][m][n]
 struct TcPartialEpi {
   float* out; long long ld, split_stride;

@@ -214,12 +214,169 @@ def _scores_backward(ctx, qc, keys_c, g_sq, g_sm, gk):
     return g_qhat, gk
 
 
+def _grad_possible(*tensors):
+    """True when autograd would record a graph for a call on these tensors"""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
+
+
+def _prepare_query(qc):
+    B, d, h, w = qc.shape
+    out = torch.empty((B, h, w, d), device=qc.device, dtype=torch.float32)
+    l = _lib.lib()
+    ws = workspace(l.vadc_memory_prepare_query_workspace_bytes(B, h * w), qc.device)
+    check(l.vadc_memory_prepare_query(ptr(qc), B, d, h * w, ptr(out), ptr(ws), ws.numel(), stream()),
+          "vadc_memory_prepare_query")
+    return out
+
+
+class _PrepareQuery(torch.autograd.Function):
+    """F.normalize(query, dim=1).permute(0, 2, 3, 1) (Memory.py:148-149) as an autograd node: per token,
+    g_x = (g - q-hat (q-hat . g)) / max(|x|, 1e-12), with g channel-last and g_x channel-first"""
+
+    @staticmethod
+    def forward(ctx, query):
+        qc = f32c(query)
+        ctx.save_for_backward(qc)
+        return _prepare_query(qc)
+
+    @staticmethod
+    def backward(ctx, g):
+        (qc,) = ctx.saved_tensors
+        B, d, h, w = qc.shape
+        g = f32c(g)
+        gx = torch.empty_like(qc)
+        check(_lib.lib().vadc_memory_prepare_query_bwd(ptr(g), ptr(qc), B, d, h * w, ptr(gx), stream()),
+              "vadc_memory_prepare_query_bwd")
+        return gx
+
+
+def _scores_rows_backward(q, keys_c, sq, sm, g_sq, g_sm, need_q, need_k, gk):
+    """the share of get_score's two matrices for a channel-last, unnormalised q [N,d]: (g_q [N,d] or None, g_keys),
+    g_keys = gk + g_s^T q when ``need_k`` (gk None: nothing else reached the keys).  Launches nothing when no score
+    gradient arrived."""
+    if (g_sq is None and g_sm is None) or not (need_q or need_k):
+        return None, gk
+    g_sq, g_sm = f32c(g_sq), f32c(g_sm)
+    N, m = sm.shape
+    d = q.shape[1]
+    l = _lib.lib()
+    coldot = None
+    if g_sq is not None:
+        coldot = torch.empty((m,), device=q.device, dtype=torch.float32)
+        ws = workspace(l.vadc_memory_score_coldot_workspace_bytes(N, m), q.device)
+        check(l.vadc_memory_score_coldot(ptr(sq), ptr(g_sq), N, m, ptr(coldot), ptr(ws), ws.numel(), stream()),
+              "vadc_memory_score_coldot")
+    g_rows = torch.empty_like(q) if need_q else None
+    if need_k and gk is None:
+        gk = torch.zeros_like(keys_c)
+    ws = workspace(l.vadc_memory_scores_bwd_rows_workspace_bytes(N, d, m), q.device)
+    check(l.vadc_memory_scores_bwd_rows(ptr(q), ptr(keys_c), ptr(sq), ptr(sm), ptr(g_sq), ptr(g_sm), ptr(coldot),
+                                        N, d, m, ptr(g_rows), ptr(gk if need_k else None), ptr(ws), ws.numel(),
+                                        stream()), "vadc_memory_scores_bwd_rows")
+    return g_rows, gk
+
+
+class _GetScore(torch.autograd.Function):
+    """get_score (Memory.py:133-143) on a channel-last query as an autograd node, differentiable with respect to the
+    query and the memory: g_s = sq (Gq - 1 c^T) + sm (Gm - r 1^T), g_q = g_s K, g_K = g_s^T q"""
+
+    @staticmethod
+    def forward(ctx, query, mem):
+        q, _ = Memory._flat(query)
+        keys_c = f32c(mem)
+        s = _compute_scores(q, keys_c)
+        ctx.save_for_backward(q, keys_c, s.score_query, s.score_memory)
+        ctx.qshape = query.shape
+        ctx.set_materialize_grads(False)
+        return s.score_query, s.score_memory
+
+    @staticmethod
+    def backward(ctx, g_sq, g_sm):
+        q, keys_c, sq, sm = ctx.saved_tensors
+        gq, gk = _scores_rows_backward(q, keys_c, sq, sm, g_sq, g_sm, ctx.needs_input_grad[0],
+                                       ctx.needs_input_grad[1], None)
+        return (None if gq is None else gq.view(ctx.qshape)), gk
+
+
+class _Read(torch.autograd.Function):
+    """read (Memory.py:249-261) as an autograd node: updated_query = cat(q, score_memory.detach() K) permuted to
+    [B,2d,h,w], plus the two score matrices.  The query gets the first d channels of G_uq (transposed to channel-last)
+    and the score share g_s K; the memory gets score_memory^T G_r (vadc_memory_keys_bwd) and the score share g_s^T q."""
+
+    @staticmethod
+    def forward(ctx, mod, query, mem):
+        q, shp = mod._flat(query)
+        keys_c = f32c(mem)
+        s = _compute_scores(q, keys_c, want_read_terms=True)
+        uq = mod._read(s, keys_c, shp)
+        ctx.save_for_backward(q, keys_c, s.score_query, s.score_memory)
+        ctx.shp = shp
+        ctx.set_materialize_grads(False)
+        return uq, s.score_query, s.score_memory
+
+    @staticmethod
+    def backward(ctx, g_uq, g_sq, g_sm):
+        q, keys_c, sq, sm = ctx.saved_tensors
+        need_q, need_k = ctx.needs_input_grad[1], ctx.needs_input_grad[2]
+        B, h, w, d = ctx.shp
+        m = keys_c.shape[0]
+        g_uq = None if g_uq is None else f32c(g_uq)                  # [B,2d,h,w]
+        l = _lib.lib()
+        gk = None
+        if need_k and g_uq is not None:
+            gk = torch.empty_like(keys_c)
+            ws = workspace(l.vadc_memory_keys_bwd_workspace_bytes(B, d, h * w, m), gk.device)
+            check(l.vadc_memory_keys_bwd(ptr(sm), ptr(g_uq), B, d, h * w, m, ptr(gk), ptr(ws), ws.numel(), stream()),
+                  "vadc_memory_keys_bwd")
+        gq, gk = _scores_rows_backward(q, keys_c, sq, sm, g_sq, g_sm, need_q, need_k, gk)
+        if need_q and g_uq is not None:
+            out = gq if gq is not None else torch.empty_like(q)
+            check(l.vadc_memory_rows_bwd(ptr(q), ptr(keys_c), None, None, ptr(g_uq), None, None, ptr(gq), B, d,
+                                         h * w, m, ptr(out), stream()), "vadc_memory_rows_bwd")
+            gq = out
+        return None, (None if gq is None else gq.view(B, h, w, d)), gk
+
+
+class _MemoryLossTerm(torch.autograd.Function):
+    """gather_loss (Memory.py:233-247) or spread_loss (:214-231) as an autograd node, differentiable with respect to
+    the query only (the reference detaches the keys, :229, :245); keeps top1 (and top2), no [N, m] matrix"""
+
+    @staticmethod
+    def forward(ctx, mod, query, keys, spread):
+        q, _ = mod._flat(query)
+        keys_c = f32c(keys)
+        s = _compute_scores(q, keys_c, False)
+        gathering, spreading = mod._losses(s, keys_c, spread)
+        ctx.save_for_backward(q, keys_c, s.top1, s.top2 if spread else None)
+        ctx.qshape = query.shape
+        return spreading if spread else gathering
+
+    @staticmethod
+    def backward(ctx, g):
+        q, keys_c, top1, top2 = ctx.saved_tensors
+        g = f32c(g).reshape(1)
+        B, h, w, d = ctx.qshape
+        gq = torch.empty_like(q)
+        check(_lib.lib().vadc_memory_rows_bwd(ptr(q), ptr(keys_c), ptr(top1), ptr(top2), None,
+                                              None if top2 is not None else ptr(g), ptr(g) if top2 is not None else None,
+                                              None, B, d, h * w, keys_c.shape[0], ptr(gq), stream()),
+              "vadc_memory_rows_bwd")
+        return None, gq.view(ctx.qshape), None, None
+
+
 class Memory(nn.Module):
     """Drop-in for model/Memory.py:62-261.  ``forward`` is differentiable with respect to ``query`` and, when they
     require grad, the memory items ``keys`` (``_MemoryForward``); with ``differentiable_scores`` set, also through
-    the returned ``score_query`` / ``score_memory``.  The stand-alone public methods (``get_score``, ``read``,
-    ``gather_loss``, ...) are forward-only, and ``updated_memory`` carries no gradient to ``keys`` (detached in the
-    reference too).  The reference module is not wired into ``Mymodel`` (SURVEY.md D5)."""
+    the returned ``score_query`` / ``score_memory``.  The stand-alone public methods are differentiable where the
+    reference's are: ``prepare_query`` (our helper for F.normalize + permute) to its query, ``get_score`` and ``read``
+    to the query and the memory argument, ``gather_loss`` and ``spread_loss`` to the query (the keys are detached there,
+    as in the reference).  They take the query channel-last, [B,h,w,d], as the reference's do, and do not normalise it.
+    Under ``torch.no_grad()``, or when no tensor argument requires grad, they launch and return exactly what a
+    forward-only call does, with no ``grad_fn``.  They stay per rank: ``global_batch`` applies to ``forward`` only.
+    Not differentiable, by design: ``update`` (its result is detached in the reference, :204) and
+    ``get_update_query`` (only ever called inside ``update``); ``updated_memory`` carries no gradient to ``keys``.
+    ``pointwise_gather_loss`` is plain torch indexing and differentiable as such.  The reference module is not wired
+    into ``Mymodel`` (SURVEY.md D5)."""
 
     def __init__(self, memory_size, feature_dim, key_dim, temp_update, temp_gather):
         super().__init__()
@@ -251,20 +408,19 @@ class Memory(nn.Module):
     @staticmethod
     def prepare_query(query):
         """F.normalize(query, dim=1) + permute(0,2,3,1)  (Memory.py:148-149):
-        [B,d,h,w] -> [B,h,w,d] contiguous"""
+        [B,d,h,w] -> [B,h,w,d] contiguous; differentiable with respect to ``query``"""
         _lib.require_cuda(query)
-        qc = f32c(query)
-        B, d, h, w = qc.shape
-        out = torch.empty((B, h, w, d), device=qc.device, dtype=torch.float32)
-        l = _lib.lib()
-        ws = workspace(l.vadc_memory_prepare_query_workspace_bytes(B, h * w), qc.device)
-        check(l.vadc_memory_prepare_query(ptr(qc), B, d, h * w, ptr(out), ptr(ws), ws.numel(), stream()),
-              "vadc_memory_prepare_query")
-        return out
+        if _grad_possible(query):
+            return _PrepareQuery.apply(query)
+        return _prepare_query(f32c(query))
 
     # -- reference API --------------------------------------------------------
     def get_score(self, mem, query):
-        """Memory.py:133-143 -> (softmax over tokens, softmax over slots), [N,m] each"""
+        """Memory.py:133-143 -> (softmax over tokens, softmax over slots), [N,m] each; differentiable with respect to
+        ``query`` (channel-last, as passed) and ``mem``.  Per rank: ignores ``global_batch``."""
+        if _grad_possible(query, mem):
+            _lib.require_cuda(query, mem)
+            return _GetScore.apply(query, mem)
         q, _ = self._flat(query)
         s = _compute_scores(q, f32c(mem))
         return s.score_query, s.score_memory
@@ -278,14 +434,15 @@ class Memory(nn.Module):
         return uq, keys, sq, sm, gl
 
     def update(self, query, keys, train):
-        """Memory.py:177-204"""
+        """Memory.py:177-204 (forward-only: the reference detaches the result, :204)"""
         with torch.no_grad():
             q, _ = self._flat(query)
             keys_c = f32c(keys)
             return self._update(_compute_scores(q, keys_c), keys_c)
 
     def get_update_query(self, mem, max_indices, update_indices, score, query, train):
-        """Memory.py:94-131: weighted sum of the queries assigned to each slot"""
+        """Memory.py:94-131: weighted sum of the queries assigned to each slot (forward-only: only ever called
+        inside ``update``, whose result the reference detaches)"""
         with torch.no_grad():
             q = f32c(query)
             return self._segmented_update(q, f32c(mem), f32c(score),
@@ -296,21 +453,34 @@ class Memory(nn.Module):
         return (query_reshape - keys[gathering_indices].squeeze(1).detach()) ** 2
 
     def spread_loss(self, query, keys, train):
-        """Memory.py:214-231"""
+        """Memory.py:214-231; differentiable with respect to ``query`` (the keys are detached, :229).  Per rank:
+        ignores ``global_batch``."""
+        if _grad_possible(query):
+            _lib.require_cuda(query, keys)
+            return _MemoryLossTerm.apply(self, query, keys.detach(), True)
         with torch.no_grad():
             q, _ = self._flat(query)
             keys_c = f32c(keys)
             return self._losses(_compute_scores(q, keys_c, False), keys_c, True)[1]
 
     def gather_loss(self, query, keys, train):
-        """Memory.py:233-247"""
+        """Memory.py:233-247; differentiable with respect to ``query`` (the keys are detached, :245).  Per rank:
+        ignores ``global_batch``."""
+        if _grad_possible(query):
+            _lib.require_cuda(query, keys)
+            return _MemoryLossTerm.apply(self, query, keys.detach(), False)
         with torch.no_grad():
             q, _ = self._flat(query)
             keys_c = f32c(keys)
             return self._losses(_compute_scores(q, keys_c, False), keys_c, False)[0]
 
     def read(self, query, updated_memory):
-        """Memory.py:249-261"""
+        """Memory.py:249-261 -> (updated_query [B,2d,h,w], score_query, score_memory); differentiable with respect to
+        ``query`` and ``updated_memory`` (through the read product and the two score matrices).  Per rank: ignores
+        ``global_batch``."""
+        if _grad_possible(query, updated_memory):
+            _lib.require_cuda(query, updated_memory)
+            return _Read.apply(self, query, updated_memory)
         with torch.no_grad():
             q, shp = self._flat(query)
             keys_c = f32c(updated_memory)

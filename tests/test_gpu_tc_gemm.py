@@ -28,9 +28,10 @@ def run(A, B, b_mn):
 
 
 @pytest.mark.parametrize("M,Nn,Kd", [(128, 128, 64), (300, 32, 192), (1000, 256, 768), (515, 1024, 192),
-                                     (2048, 2000, 768), (77, 16, 768), (129, 136, 200), (4096, 64, 768),
-                                     (3001, 1096, 200),        # more tiles than SMs: the persistent kernel, ragged M / N / Kd
-                                     (20000, 136, 64)])        # persistent, one k-block per tile, 157 x 2 tiles
+                                     (77, 16, 768), (129, 136, 200), (4096, 64, 768),   # fewer tiles than SMs: grid < SMs
+                                     (2048, 2000, 768),        # 256 tiles: CTAs walk several tiles each
+                                     (3001, 1096, 200),        # more tiles than SMs, ragged M / N / Kd
+                                     (20000, 136, 64)])        # more tiles than SMs, one k-block per tile, 157 x 2 tiles
 @pytest.mark.parametrize("b_mn", [0, 1])
 def test_tc_gemm_vs_float64(M, Nn, Kd, b_mn):
     rng = np.random.default_rng(M + Nn + Kd + b_mn)

@@ -293,14 +293,12 @@ static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b
   VADC_REQUIRE(workspace_bytes >= vadc_cluster_fwd_workspace_bytes(N, C, K, impl), VADC_ERR_WORKSPACE);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 
-  if (impl != VADC_IMPL_SIMT && !env_on("VADC_FWD_NO_WS")) {
+  if (impl != VADC_IMPL_SIMT) {
     int rc = vadc_cluster_fwd_ws(x, ln_w, ln_b, centers, N, C, K, alpha, eps, D, A, x_rec, feature,
                                  label, mu, rstd, rowstats, loss_sq, workspace, workspace_bytes, st);
     if (rc != VADC_ERR_UNSUPPORTED) return rc;
-  }
-  if (impl != VADC_IMPL_SIMT) {
-    int rc = vadc_cluster_fwd_tc(x, ln_w, ln_b, centers, N, C, K, alpha, eps, D, A, x_rec, feature,
-                                 label, mu, rstd, loss_sq, workspace, workspace_bytes, st);
+    rc = vadc_cluster_fwd_tc(x, ln_w, ln_b, centers, N, C, K, alpha, eps, D, A, x_rec, feature,
+                             label, mu, rstd, loss_sq, workspace, workspace_bytes, st);
     if (rc == VADC_OK) return launch_rowstats(x, feature, mu, rstd, ln_w, N, C, rowstats, st);
     if (rc != VADC_ERR_UNSUPPORTED || impl == VADC_IMPL_TCGEN05) return rc;
   }
@@ -327,12 +325,12 @@ static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b
     if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
     if ((rc = tc_split2h(centers, K, C, sc + 1, cs, st))) return rc;
     // from K = 128 up the distance GEMM runs with the operands swapped (rows = centroids): coalesced stores of D
-    if (K >= 128 && !env_on("VADC_TC_ROW_EPILOGUE")) {
+    if (K >= 128) {
       if ((rc = launch_tc_gemm_h2<false>(cs, fs, K, N, C, sc + 2, TcDistTEpi{D, cc, zz, K}, st))) return rc;
     } else if ((rc = launch_tc_gemm_h2<false>(fs, cs, N, K, C, sc + 2, TcDistEpi{D, zz, cc, K}, st))) return rc;
     // softmin writes A and, in the same pass, its two fp16 terms scaled by s_a = 2^13 (the value fwd_scales_kernel puts in sc[3])
     if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid, as, 8192.0f))) return rc;
-    if (C >= 128 && !env_on("VADC_TC_ROW_EPILOGUE"))       // rows = channels (centers [K,C] as the MN-major A operand): coalesced x_rec
+    if (C >= 128)   // rows = channels (centers [K,C] as the MN-major A operand): coalesced x_rec
       return launch_tc_gemm_ex_h2<true, false>(cs, as, C, N, K, 1, sc + 4, TcStoreTEpi{x_rec, C}, st);
     return launch_tc_gemm_h2<true>(as, cs, N, C, K, sc + 4, TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
   }
@@ -527,7 +525,7 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
   if (want_tc && rowstats && ln_b && gR && !gD && !gA && !gF && bwd_tc2_shape_ok(N, C, K))
     return launch_cluster_bwd_tc2(x, mu, rstd, rowstats, ln_w, ln_b, centers, D, A, gR, g_loss_sq, N, C, K, alpha, gx,
                                   gcenters, g_ln_w, g_ln_b, workspace, workspace_bytes, st);
-  if (bwd_fused_shape_ok(N, C, K) && !env_on("VADC_BWD_GENERIC") && !(bimpl && !strcmp(bimpl, "generic")))
+  if (bwd_fused_shape_ok(N, C, K) && !(bimpl && !strcmp(bimpl, "generic")))
     return launch_cluster_bwd_fused(x, mu, rstd, feature, ln_w, centers, D, A, gD, gA, gR, gF, g_loss_sq,
                                     N, C, K, alpha, gx, gcenters, g_ln_w, g_ln_b, workspace,
                                     workspace_bytes, st);
@@ -568,7 +566,7 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
       if ((rc = tc_split2h(centers, K, C, sc + 1, cs, st))) return rc;
       if (gR) {
         if ((rc = tc_split2h(gR, N, C, sc + 0, gRs, st))) return rc;
-        if (K >= 128 && !env_on("VADC_TC_ROW_EPILOGUE")) {      // operands swapped: rows = centroids, coalesced stores
+        if (K >= 128) {   // operands swapped: rows = centroids, coalesced stores
           if ((rc = launch_tc_gemm_h2<false>(cs, gRs, K, N, C, sc + 5, TcStoreTEpi{gemm, K}, st))) return rc;
         } else if ((rc = launch_tc_gemm_h2<false>(gRs, cs, N, K, C, sc + 5, TcStoreEpi{gemm, K}, st))) return rc;
       }
@@ -576,7 +574,7 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
       if ((rc = launch_bwd_rows(D, A, gR ? gemm : nullptr, gD, gA, g_loss_sq, N, K, alpha, r, rsum, st, bits + 3))) return rc;
       if ((rc = tc_cluster_bwd_scales(bits, 1, sc, st))) return rc;
       if ((rc = tc_split2h(r, N, K, sc + 4, rs, st))) return rc;
-      if (C >= 128 && !env_on("VADC_TC_ROW_EPILOGUE")) {     // rows = channels: coalesced loads of feature / gF and stores of gz
+      if (C >= 128) {   // rows = channels: coalesced loads of feature / gF and stores of gz
         if ((rc = launch_tc_gemm_ex_h2<true, false>(cs, rs, C, N, K, 1, sc + 7, TcGzTEpi{gz, feature, rsum, gF, C}, st))) return rc;
       } else if ((rc = launch_tc_gemm_h2<true>(rs, cs, N, C, K, sc + 7, TcGzEpi{gz, feature, rsum, gF, C}, st))) return rc;
       if (gR) {

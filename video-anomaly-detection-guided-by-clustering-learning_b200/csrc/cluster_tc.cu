@@ -25,8 +25,8 @@
 //   P4  1 thread: 6 x K/16 tcgen05.mma (M=128, N=C) against the SAME centroid
 //       tiles read MN-major -> TMEM cols [K, K+C)
 //   P5  8 warps: tcgen05.ld -> swizzled staging -> TMA tensor store of x_rec
-// Shared memory (C=192, K=32): 144 KB token operand (re-used as staging after
-// GEMM1), 36 KB centroid operand, loaded once per CTA by a bulk TMA copy.
+// Shared memory (C=192, K=64): 144 KB token operand (re-used as staging after
+// GEMM1), 72 KB centroid operand, loaded once per CTA by a bulk TMA copy.
 #include <cuda.h>
 #include <algorithm>
 #include <stdio.h>
@@ -323,46 +323,30 @@ cluster_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapD, const __grid_con
       const float nalpha = -p.alpha * 1.4426950408889634f;     // exp(-a t) = 2^(-a log2(e) t)
       float best = INFINITY; int bidx = 0;
       float dv[32];
-      if (KCH == 1) {
-        tmem_ld32(tmemD + lane_addr, dv);
+      for (int c0 = 0; c0 < K; c0 += 32) {
+        tmem_ld32(tmemD + lane_addr + c0, dv);
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
-          dv[j] = fast_sqrt(fmaxf(zz + sCC[j] - 2.0f * dv[j], 0.f));
-          if (dv[j] < best) { best = dv[j]; bidx = j; }
-        }
-      } else {
-        for (int c0 = 0; c0 < K; c0 += 32) {
-          tmem_ld32(tmemD + lane_addr + c0, dv);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            float d = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
-            if (d < best) { best = d; bidx = c0 + j; }
-          }
+          float d = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
+          if (d < best) { best = d; bidx = c0 + j; }
         }
       }
       float sum = 0.f;
-      if (KCH > 1) {
-        for (int c0 = 0; c0 < K; c0 += 32) {
-          tmem_ld32(tmemD + lane_addr + c0, dv);
+      for (int c0 = 0; c0 < K; c0 += 32) {
+        tmem_ld32(tmemD + lane_addr + c0, dv);
 #pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            float d = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
-            sum += exp2f(nalpha * (d - best));
-          }
+        for (int j = 0; j < 32; ++j) {
+          float d = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
+          sum += exp2f(nalpha * (d - best));
         }
       }
       for (int c0 = 0; c0 < K; c0 += 32) {
         float ev[32];
-        if (KCH > 1) {
-          tmem_ld32(tmemD + lane_addr + c0, dv);
+        tmem_ld32(tmemD + lane_addr + c0, dv);
 #pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            dv[j] = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
-            ev[j] = exp2f(nalpha * (dv[j] - best));
-          }
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) { ev[j] = exp2f(nalpha * (dv[j] - best)); sum += ev[j]; }
+        for (int j = 0; j < 32; ++j) {
+          dv[j] = fast_sqrt(fmaxf(zz + sCC[c0 + j] - 2.0f * dv[j], 0.f));
+          ev[j] = exp2f(nalpha * (dv[j] - best));
         }
         const float inv = fast_rcp(sum);
         uint8_t* dblk = smem + pl.dst_off + (c0 >> 5) * (kTileM * 128u);
@@ -499,8 +483,8 @@ static int make_map(CUtensorMap* m, float* base, long long rows, int cols) {
 
 static bool tc_shape_ok(long long N, int C, int K) {
   if (N < 1 || N >= (1ll << 31)) return false;
-  if (C != 64 && C != 128 && C != 192) return false;   // instantiated (C/32, K/32) combinations
-  if (K != 32 && K != 64) return false;
+  // the one instantiated shape: K = 32 runs cluster_fwd_ws, and at C = 64 / 128 the K = 64 staging does not fit
+  if (C != 192 || K != 64) return false;
   TcSmemPlan pl = tc_plan(C, K);
   if (pl.alias_end > pl.z_bytes) return false;          // staging must fit in the dead operand tiles
   if (pl.total + 1024 > 227 * 1024) return false;
@@ -543,17 +527,8 @@ int vadc_cluster_fwd_tc(const float* x, const float* ln_w, const float* ln_b, co
   const size_t smem = pl.total + 1024;
   TcParams p{x, ln_w, ln_b, image, cc, feature, reinterpret_cast<long long*>(label), mu, rstd, partial,
              (long long)N, C, K, alpha, eps};
-#define TC_CASE(F4_, KCH_)                                                                              \
-  if (C == 32 * F4_ && K == 32 * KCH_) {                                                                \
-    VADC_CUDA(cudaFuncSetAttribute(cluster_fwd_tc_kernel<F4_, KCH_>,                                     \
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-    cluster_fwd_tc_kernel<F4_, KCH_><<<grid, kTcThreads, smem, st>>>(mD, mA, mR, p);                     \
-    launched = true;                                                                                    \
-  }
-  bool launched = false;
-  TC_CASE(2, 1) TC_CASE(4, 1) TC_CASE(6, 1) TC_CASE(4, 2) TC_CASE(6, 2)
-#undef TC_CASE
-  if (!launched) return VADC_ERR_UNSUPPORTED;
+  VADC_CUDA(cudaFuncSetAttribute(cluster_fwd_tc_kernel<6, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cluster_fwd_tc_kernel<6, 2><<<grid, kTcThreads, smem, st>>>(mD, mA, mR, p);
   VADC_CHECK_LAUNCH("cluster_fwd_tc_kernel");
   finalize_sum_kernel<<<1, 1024, 0, st>>>(partial, grid, loss_sq);
   VADC_CHECK_LAUNCH("finalize_sum_kernel");

@@ -1235,8 +1235,8 @@ extern "C" int vadc_memory_score(const float* q, const float* keys, int64_t N, i
       if ((rc = tc_split2h(q, N, d, sc, qs, st))) return rc;
       if ((rc = tc_split2h(keys, m, d, sc + 1, ks, st))) return rc;
       // operands swapped from m = 128 up (rows = memory slots): coalesced stores of the logits
-      if (m >= 128 && !env_on("VADC_TC_ROW_EPILOGUE")) {
-        if (score_query && !env_on("VADC_MEMORY_NO_FUSED_STATS")) {
+      if (m >= 128) {
+        if (score_query) {
           if ((rc = launch_tc_gemm_h2<false>(ks, qs, m, N, d, sc + 2, TcLogitsColStatsTEpi{logits, m, pmax, psum}, st))) return rc;
           have_groups = true;
         } else if ((rc = launch_tc_gemm_h2<false>(ks, qs, m, N, d, sc + 2, TcStoreTEpi{logits, m}, st))) return rc;
@@ -1332,7 +1332,7 @@ extern "C" int vadc_memory_read(const float* q, const float* score_memory, const
       sst = ss;
     }
     if ((rc = tc_split2h(keys, m, d, sc + 1, ks, st))) return rc;
-    if (d >= 128 && !env_on("VADC_TC_ROW_EPILOGUE"))       // rows = channels (keys [m,d] as the MN-major A operand): coalesced output
+    if (d >= 128)   // rows = channels (keys [m,d] as the MN-major A operand): coalesced output
       return launch_tc_gemm_ex_h2<true, false>(ks, sst, d, N, m, 1, sc + 2, TcReadTEpi{updated_query, q, d}, st);
     return launch_tc_gemm_h2<true>(sst, ks, N, d, m, sc + 2, TcReadEpi{updated_query, q, d}, st);
   }

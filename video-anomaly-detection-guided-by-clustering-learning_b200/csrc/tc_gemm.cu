@@ -10,10 +10,10 @@
 // the GEMM keeps the six products t0t0, t0t1, t1t0, t0t2, t1t1, t2t0 in the fp32 TMEM accumulator
 // (dropped terms <= 2^-24 relative), which is what keeps argmin bit-exact against the fp32 reference.
 //
-// One CTA = one 128 x BN output tile: warp 0 = TMA producer (3-D tensor maps {cols, rows, term},
-// SWIZZLE_128B boxes land directly as UMMA operand tiles), warp 1 = MMA issuer, warps 2-5 = epilogue
-// (thread = output row = TMEM lane, functor per 32 columns).  One 96 KB stage per CTA and two CTAs per SM
-// (a CTA's load / MMA / epilogue phases overlap with its neighbour's: 1.63 -> 1.30 ms on the C=768, K=256 distance GEMM).
+// One kernel for every launch, plain, batched and split-K: tc_gemm_persist_kernel on min(work items, SMs) CTAs, one per
+// SM, each walking 128 x BN output tiles.  Warp 0 = TMA producer (3-D tensor maps {cols, rows, term}, SWIZZLE_128B boxes
+// land directly as UMMA operand tiles), warp 1 = MMA issuer, warps 2-9 = epilogue (thread = output row = TMEM lane,
+// functor per 32 columns).
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -28,24 +28,8 @@ using namespace tc;
 
 namespace tg {
 
-constexpr int BM = 128, BK = 64, kThreads = 192;
-// bf16 x3: one 96 KB stage per CTA, two CTAs per SM.  fp16 x2: one 64 KB stage, three CTAs per SM — measured against a
-// 3-stage ring in ONE CTA per SM (-DVADC_TC_STAGES_H=3): 169 vs 124 us on the C=768, K=256 distance GEMM and 499 vs 251 us at
-// K=1024: without a second accumulator the lone CTA's epilogue idles the tensor pipe; co-resident CTAs overlap it for free
-#ifndef VADC_TC_STAGES_H
-#define VADC_TC_STAGES_H 1
-#endif
-constexpr int kStagesH = VADC_TC_STAGES_H;
-// co-resident CTAs per SM for a ring of STAGES stages: one-stage CTAs share an SM (two at 96 KB, three at 64 KB), a deeper
-// ring owns it.
-template <int TERMS, int STAGES> struct StageCfg { static constexpr int ctas = STAGES > 1 ? 1 : (TERMS == 2 ? 3 : 2); };
-
-// per-blockIdx.z coordinate offsets of a batched launch: output-row / contraction offsets of A, output-column /
-// contraction offsets of B (in elements of the respective tensor-map dimension)
-// m_fast: blockIdx.x walks the m-tiles (the launcher
-// lets the dimension with FEWER tiles vary fastest, so that the CTAs in flight share the small operand and stream the
-// big one from DRAM once: with 16 m-tiles x 512 n-tiles the other order re-read the n-side operand 16 times)
-struct ZOffsets { int batched, a_m, a_k, b_n, b_k, m_fast; };
+constexpr int BM = 128, BK = 64;
+constexpr int kThreads = 320;            // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue
 
 __global__ void __launch_bounds__(256)
 split3_kernel(const float* __restrict__ src, long long n4, __nv_bfloat16* __restrict__ t0,
@@ -72,140 +56,27 @@ __device__ __forceinline__ void tma_load_3d(const void* tmap, uint32_t smem_dst,
                ::"r"(smem_dst), "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 
+// One CTA per SM walks the work items (output tiles, the nz slices along z slowest).  Within a slice the dimension with
+// FEWER tiles varies fastest (m_fast = the m-tiles): the CTAs in flight then share the small operand and stream the big
+// one from DRAM once (with 16 m-tiles x 512 n-tiles the other order re-read the n-side operand 16 times).  The operand
+// ring (STAGES stages) runs across tile boundaries, the accumulator is double-buffered in TMEM (2 x BN columns), and EIGHT
+// epilogue warps (two per TMEM lane quarter, splitting the columns) drain tile i while the MMA warp is already in tile
+// i+1: load, MMA and epilogue are three concurrent streams.  A CTA with a single tile still overlaps its loads with the
+// MMAs of the k-loop.
+//
 // TERMS = 3: three bf16 terms per operand, six products (fp32-faithful for any fp32 data).
 // TERMS = 2: two fp16 terms of operands pre-scaled by a power of two into fp16's range (bounded data: LayerNorm
 // output, centroids, softmax weights), three products hh + hl + lh (22 significant bits) — two thirds of the operand
-// bytes, half the MMAs, and a 64 KB stage so that three CTAs share an SM; the accumulators are multiplied by
-// *acc_scale (= 1 / (s_a s_b)) before the epilogue sees them.
-template <int BN, int TERMS, int STAGES, bool A_MN, bool B_MN, class Epi>
-__global__ void __launch_bounds__(kThreads, StageCfg<TERMS, STAGES>::ctas)
-tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-               int M, int N, int Kd, int kb_per_split, const ZOffsets zo, const float* __restrict__ acc_scale, Epi epi) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  constexpr uint32_t kATerm = BM * 128u, kBTerm = BN * 128u;           // bytes per bf16 term of a stage's operand
-  constexpr uint32_t kStage = (uint32_t)TERMS * (kATerm + kBTerm);
-  constexpr int kStages = STAGES;
-  __shared__ uint64_t full[kStages], empty[kStages], accfull;
-  __shared__ uint32_t tmem_slot;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m0 = (zo.m_fast ? blockIdx.x : blockIdx.y) * BM, n0 = (zo.m_fast ? blockIdx.y : blockIdx.x) * BN;
-  // blockIdx.z is either a split-K slot (k-blocks [kb0, kb1), partial outputs) or, with zo.batched, the index
-  // of an independent problem whose operands sit zo.* coordinates further along the same tensors; either way
-  // the epilogue receives it
-  const int nkb_all = (Kd + BK - 1) / BK;
-  const int z = blockIdx.z;
-  const int kb0 = zo.batched ? 0 : z * kb_per_split, kb1 = zo.batched ? nkb_all : min(nkb_all, kb0 + kb_per_split);
-  const int nkb = max(kb1 - kb0, 0);
-  const int am = m0 + z * zo.a_m, ak = z * zo.a_k, bn = n0 + z * zo.b_n, bk = z * zo.b_k;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    mbar_init(&accfull, 1);
-    fence_mbar_init();
-    prefetch_tmap(&mapA); prefetch_tmap(&mapB);
-  }
-  if (warp == 1) tmem_alloc(&tmem_slot, BN);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = tmem_slot;
-  const uint32_t s0 = smem_u32(smem);
-
-  if (warp == 0 && lane == 0) {
-    // ---------------------------------------------------------------- TMA producer
-    for (int kb = 0; kb < nkb; ++kb) {
-      const int s = kb % kStages;
-      mbar_wait(&empty[s], (uint32_t)(((kb / kStages) & 1) ^ 1));
-      mbar_expect_tx(&full[s], kStage);
-      const uint32_t a = s0 + s * kStage, b = a + (uint32_t)TERMS * kATerm;
-      const int k0 = (kb0 + kb) * BK;
-#pragma unroll
-      for (int t = 0; t < TERMS; ++t) {
-        if constexpr (!A_MN) {
-          tma_load_3d(&mapA, a + t * kATerm, &full[s], k0 + ak, am, t);
-        } else {
-#pragma unroll
-          for (int mb = 0; mb < BM / 64; ++mb)                // A given as [Kd, M]: [64 k-rows x 64 m-cols] boxes, 8 KB apart
-            tma_load_3d(&mapA, a + t * kATerm + mb * 8192u, &full[s], am + mb * 64, k0 + ak, t);
-        }
-        if constexpr (!B_MN) {
-          tma_load_3d(&mapB, b + t * kBTerm, &full[s], k0 + bk, bn, t);
-        } else {
-#pragma unroll
-          for (int nb = 0; nb < BN / 64; ++nb)                // [64 k-rows x 64 n-cols] boxes, 8 KB apart
-            tma_load_3d(&mapB, b + t * kBTerm + nb * 8192u, &full[s], bn + nb * 64, k0 + bk, t);
-        }
-      }
-    }
-  } else if (warp == 1 && lane == 0) {
-    // ---------------------------------------------------------------- MMA issuer
-    const uint32_t idesc = instr_desc(TERMS == 2 ? 0u /* fp16 */ : kFmtBF16, BM, BN, A_MN ? 1 : 0, B_MN ? 1 : 0);
-    constexpr int kProducts = TERMS == 2 ? 3 : 6;
-    constexpr int ta[6] = {TERMS == 2 ? 1 : 2, TERMS == 2 ? 0 : 1, 0, 1, 0, 0};   // small products first
-    constexpr int tb[6] = {0, 1, TERMS == 2 ? 0 : 2, 0, 1, 0};
-    for (int kb = 0; kb < nkb; ++kb) {
-      const int s = kb % kStages;
-      mbar_wait(&full[s], (uint32_t)((kb / kStages) & 1));
-      tc_fence_after();
-      const uint32_t a = s0 + s * kStage, b = a + (uint32_t)TERMS * kATerm;
-#pragma unroll
-      for (int pr = 0; pr < kProducts; ++pr) {
-#pragma unroll
-        for (int kk = 0; kk < BK / 16; ++kk) {
-          const uint64_t ad = A_MN ? smem_desc_sw128(a + ta[pr] * kATerm + kk * 2048u, 8192, 1024)
-                                   : smem_desc_sw128(a + ta[pr] * kATerm + kk * 32u, 0, 1024);
-          const uint64_t bd = B_MN ? smem_desc_sw128(b + tb[pr] * kBTerm + kk * 2048u, 8192, 1024)
-                                   : smem_desc_sw128(b + tb[pr] * kBTerm + kk * 32u, 0, 1024);
-          mma_f16(tmem, ad, bd, idesc, (kb > 0 || pr > 0 || kk > 0) ? 1u : 0u);
-        }
-      }
-      mma_commit(&empty[s]);
-    }
-    if (nkb > 0) mma_commit(&accfull);
-  } else if (warp >= 2) {
-    // ---------------------------------------------------------------- epilogue: thread = row = TMEM lane
-    const int q = warp & 3;
-    const long long m = (long long)m0 + q * 32 + lane;
-    if (nkb > 0) { mbar_wait(&accfull, 0); tc_fence_after(); }
-    const float sc = acc_scale ? __ldg(acc_scale) : 1.0f;
-#pragma unroll 1
-    for (int c = 0; c < BN / 32; ++c) {
-      float v[32];
-      if (nkb > 0) {
-        tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), v);
-        if (TERMS == 2) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) v[j] *= sc;
-        }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = 0.f;             // an empty split still writes its (zero) partial
-      }
-      const int n = n0 + c * 32;
-      if (m < M && n < N) epi(m, n, v, min(32, N - n), (int)blockIdx.z);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem, BN); }
-}
-
-// ---- persistent form ------------------------------------------------------------------------------------------------
-// One CTA per SM walks the output tiles (the dimension with fewer tiles fastest).  The operand ring (STAGES stages) runs
-// across tile boundaries, the accumulator is double-buffered in TMEM (2 x BN columns), and EIGHT epilogue warps (two per
-// TMEM lane quarter, splitting the columns) drain tile i while the MMA warp is already in tile i+1: the load -> MMA ->
-// epilogue chain of the one-tile-per-CTA kernel above — per-tile barrier set-up, TMEM allocation, a serial k-loop per CTA and
-// an epilogue that only overlaps a neighbour CTA's work — becomes three concurrent streams.  Short contraction loops with a
-// large output (distance / logits / x_rec GEMMs) gain the most: there the tile time is the epilogue's store time.
-constexpr int kThreadsP = 320;           // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue
+// bytes, half the MMAs, and a 64 KB stage; the accumulators are multiplied by *acc_scale (= 1 / (s_a s_b)) before the
+// epilogue sees them.
 __device__ __forceinline__ void mbar_arrive1(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
 template <int BN, int TERMS, int STAGES, bool A_MN, bool B_MN, class Epi>
-__global__ void __launch_bounds__(kThreadsP, 1)
+__global__ void __launch_bounds__(kThreads, 1)
 tc_gemm_persist_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                       int M, int N, int Kd, int mt, int nt, int nz, int m_fast, int kb_per_split, const ZOffsets zo,
+                       int M, int N, int Kd, int mt, int nt, int nz, int m_fast, int kb_per_split, const TcBatchOffsets zo,
                        const float* __restrict__ acc_scale, Epi epi) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -409,48 +280,41 @@ int tc_split3(const float* src, long long rows, long long cols, void* dst, cudaS
   return VADC_OK;
 }
 
+// The launch of every front-end: nz slices along z of an [M, N] output on min(work items, SMs) persistent CTAs with three
+// 64 KB (fp16 x2) or two 96 KB (bf16 x3) operand stages.  The split matrices are a_rows x a_cols and b_rows x b_cols
+// (MN-major: [Kd rows, M / N cols], boxes of 64 k-rows x 64 cols; K-major: [M / N rows, Kd cols], boxes of 128 rows x
+// 64 k-cols).  kb_per_split > 0: split-K slots of kb_per_split k-blocks; 0: nz problems, operands zo further along.
 template <int TERMS, bool A_MN, bool B_MN, class Epi>
-static int launch_tc_gemm_ex_t(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                               const float* acc_scale, Epi epi, cudaStream_t st) {
-  constexpr int BN = 128;
+static int launch_tc_gemm_t(const void* a_split, long long a_rows, long long a_cols, const void* b_split, long long b_rows,
+                            long long b_cols, long long M, long long N, long long Kd, int nz, int kb_per_split,
+                            TcBatchOffsets zo, const float* acc_scale, Epi epi, cudaStream_t st) {
+  constexpr int BN = 128, kStages = TERMS == 2 ? 3 : 2;
   if (TERMS == 2 && !acc_scale) return VADC_ERR_NULL_POINTER;
   CUtensorMap mA, mB;
   int rc;
-  if (A_MN) rc = tg::make_map3(&mA, a_split, Kd, M, 64, TERMS);   // [Kd rows, M cols]: boxes of 64 k-rows x 64 m-cols
-  else rc = tg::make_map3(&mA, a_split, M, Kd, tg::BM, TERMS);
-  if (rc) return rc;
-  if (B_MN) rc = tg::make_map3(&mB, b_split, Kd, N, 64, TERMS);   // [Kd rows, N cols]: boxes of 64 k-rows x 64 n-cols
-  else rc = tg::make_map3(&mB, b_split, N, Kd, BN, TERMS);        // [N rows, Kd cols]: boxes of BN rows x 64 k-cols
-  if (rc) return rc;
-  const unsigned ntl = (unsigned)((N + BN - 1) / BN), mtl = (unsigned)((M + tg::BM - 1) / tg::BM);
-  if (splits < 1) splits = 1;
-  if ((long long)ntl * mtl * splits > sm_count() && !env_on("VADC_TC_NO_PERSIST")) {
-    // persistent CTAs: three 64 KB (fp16 x2) or two 96 KB (bf16 x3) stages, double-buffered accumulator
-    constexpr int kStP = TERMS == 2 ? 3 : 2;
-    const size_t smemp = (size_t)kStP * TERMS * (tg::BM * 128 + BN * 128) + 1024;
-    auto kp = tg::tc_gemm_persist_kernel<BN, TERMS, kStP, A_MN, B_MN, Epi>;
-    VADC_CUDA(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemp));
-    const int m_fast = mtl < ntl ? 1 : 0;
-    const int nkbp = (int)((Kd + tg::BK - 1) / tg::BK);
-    const int perp = splits > 1 ? (nkbp + splits - 1) / splits : 0;          // split-K: k-blocks per slot
-    kp<<<sm_count(), tg::kThreadsP, smemp, st>>>(mA, mB, (int)M, (int)N, (int)Kd, (int)mtl, (int)ntl, splits, m_fast, perp,
-                                                  tg::ZOffsets{0, 0, 0, 0, 0, 0}, acc_scale, epi);
-    VADC_CHECK_LAUNCH("tc_gemm_persist_kernel");
-    return VADC_OK;
-  }
-  constexpr int kSt = TERMS == 2 ? tg::kStagesH : 1;
-  const size_t smem = (size_t)kSt * TERMS * (tg::BM * 128 + BN * 128) + 1024;
-  auto kern = tg::tc_gemm_kernel<BN, TERMS, kSt, A_MN, B_MN, Epi>;
+  if ((rc = tg::make_map3(&mA, a_split, a_rows, a_cols, A_MN ? 64 : tg::BM, TERMS))) return rc;
+  if ((rc = tg::make_map3(&mB, b_split, b_rows, b_cols, B_MN ? 64 : BN, TERMS))) return rc;
+  const int mt = (int)((M + tg::BM - 1) / tg::BM), nt = (int)((N + BN - 1) / BN);
+  const int grid = (int)std::min<long long>((long long)mt * nt * nz, sm_count());
+  const size_t smem = (size_t)kStages * TERMS * (tg::BM * 128 + BN * 128) + 1024;
+  auto kern = tg::tc_gemm_persist_kernel<BN, TERMS, kStages, A_MN, B_MN, Epi>;
   VADC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int nkb = (int)((Kd + tg::BK - 1) / tg::BK);
-  if (splits < 1) splits = 1;
-  const int per = (nkb + splits - 1) / splits;
-  const unsigned nt = (unsigned)((N + BN - 1) / BN), mt = (unsigned)((M + tg::BM - 1) / tg::BM);
-  const int m_fast = (mt < nt && nt <= 65535u) ? 1 : 0;
-  dim3 grid(m_fast ? mt : nt, m_fast ? nt : mt, (unsigned)splits);
-  kern<<<grid, tg::kThreads, smem, st>>>(mA, mB, (int)M, (int)N, (int)Kd, per, tg::ZOffsets{0, 0, 0, 0, 0, m_fast}, acc_scale, epi);
-  VADC_CHECK_LAUNCH("tc_gemm_kernel");
+  kern<<<grid, tg::kThreads, smem, st>>>(mA, mB, (int)M, (int)N, (int)Kd, mt, nt, nz, mt < nt ? 1 : 0, kb_per_split, zo,
+                                         acc_scale, epi);
+  VADC_CHECK_LAUNCH("tc_gemm_persist_kernel");
   return VADC_OK;
+}
+
+// one problem; splits > 1 slots along the contraction, each handing its index to the epilogue (split-K partials)
+template <int TERMS, bool A_MN, bool B_MN, class Epi>
+static int launch_tc_gemm_ex_t(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
+                               const float* acc_scale, Epi epi, cudaStream_t st) {
+  if (splits < 1) splits = 1;
+  const int nkb = (int)((Kd + tg::BK - 1) / tg::BK);
+  const int per = splits > 1 ? (nkb + splits - 1) / splits : 0;          // k-blocks per slot
+  return launch_tc_gemm_t<TERMS, A_MN, B_MN, Epi>(a_split, A_MN ? Kd : M, A_MN ? M : Kd, b_split, B_MN ? Kd : N,
+                                                  B_MN ? N : Kd, M, N, Kd, splits, per, TcBatchOffsets{0, 0, 0, 0},
+                                                  acc_scale, epi, st);
 }
 
 template <bool A_MN, bool B_MN, class Epi>
@@ -466,43 +330,16 @@ int launch_tc_gemm_ex_h2(const void* a_split, const void* b_split, long long M, 
   return launch_tc_gemm_ex_t<2, A_MN, B_MN, Epi>(a_split, b_split, M, N, Kd, splits, acc_scale, epi, st);
 }
 
-// nbatch independent [M,N,Kd] problems in ONE launch (blockIdx.z = batch): the operands of batch z start
+// nbatch independent [M,N,Kd] problems in ONE launch (z = batch): the operands of batch z start
 // z * off.{m,k} coordinates further along tensors of the given full extents (rows x cols of the split matrices)
 // TERMS = 3: bf16 x3 operands from tc_split3; TERMS = 2: fp16 x2 operands from tc_split2h, accumulators scaled by *acc_scale
 template <int TERMS, bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_batched_t(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                             long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                             TcBatchOffsets off, const float* acc_scale, Epi epi, cudaStream_t st) {
-  constexpr int BN = 128;
+static int launch_tc_gemm_batched_t(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
+                                    long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
+                                    TcBatchOffsets off, const float* acc_scale, Epi epi, cudaStream_t st) {
   if (nbatch < 1 || nbatch > 65535) return VADC_ERR_UNSUPPORTED;
-  if (TERMS == 2 && !acc_scale) return VADC_ERR_NULL_POINTER;
-  CUtensorMap mA, mB;
-  int rc;
-  if ((rc = tg::make_map3(&mA, a_split, a_rows, a_cols, A_MN ? 64 : tg::BM, TERMS))) return rc;
-  if ((rc = tg::make_map3(&mB, b_split, b_rows, b_cols, B_MN ? 64 : BN, TERMS))) return rc;
-  const int nkb = (int)((Kd + tg::BK - 1) / tg::BK);
-  const size_t stage = (size_t)TERMS * (tg::BM * 128 + BN * 128);
-  dim3 grid((unsigned)((N + BN - 1) / BN), (unsigned)((M + tg::BM - 1) / tg::BM), (unsigned)nbatch);
-  const tg::ZOffsets zo{1, off.a_m, off.a_k, off.b_n, off.b_k, 0};
-  if ((long long)grid.x * grid.y * grid.z > sm_count() && !env_on("VADC_TC_NO_PERSIST") && !env_on("VADC_TC_NO_PERSIST_BATCHED")) {
-    constexpr int kStP = TERMS == 2 ? 3 : 2;
-    const size_t smemp = kStP * stage + 1024;
-    auto kp = tg::tc_gemm_persist_kernel<BN, TERMS, kStP, A_MN, B_MN, Epi>;
-    VADC_CUDA(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemp));
-    const int m_fast = grid.y < grid.x ? 1 : 0;
-    kp<<<sm_count(), tg::kThreadsP, smemp, st>>>(mA, mB, (int)M, (int)N, (int)Kd, (int)grid.y, (int)grid.x, nbatch, m_fast, 0, zo,
-                                                  acc_scale, epi);
-    VADC_CHECK_LAUNCH("tc_gemm_persist_kernel(batched)");
-    return VADC_OK;
-  }
-  // (a two-stage ring with one CTA per SM and an L2 prefetch of the following k-blocks were both measured on the space
-  // head's long contraction loops and were no better than two co-resident one-stage CTAs: 251 vs 210 us, no change)
-  auto kern = tg::tc_gemm_kernel<BN, TERMS, 1, A_MN, B_MN, Epi>;
-  const size_t smem = stage + 1024;
-  VADC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<grid, tg::kThreads, smem, st>>>(mA, mB, (int)M, (int)N, (int)Kd, nkb, zo, acc_scale, epi);
-  VADC_CHECK_LAUNCH("tc_gemm_kernel(batched)");
-  return VADC_OK;
+  return launch_tc_gemm_t<TERMS, A_MN, B_MN, Epi>(a_split, a_rows, a_cols, b_split, b_rows, b_cols, M, N, Kd, nbatch, 0, off,
+                                                  acc_scale, epi, st);
 }
 
 template <bool A_MN, bool B_MN, class Epi>

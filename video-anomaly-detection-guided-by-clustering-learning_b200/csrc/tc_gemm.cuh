@@ -14,7 +14,7 @@ int tc_split3(const float* src, long long rows, long long cols, void* dst, cudaS
 template <bool B_MN, class Epi>
 int launch_tc_gemm(const void* a_split, const void* b_split, long long M, long long N, long long Kd, Epi epi,
                    cudaStream_t st);
-// general form: A_MN = A given as [Kd, M] (e.g. a transposed token matrix), `splits` CTAs along the contraction,
+// general form: A_MN = A given as [Kd, M] (e.g. a transposed token matrix), `splits` slots along the contraction,
 // each handing its index to the epilogue (split-K partials for the centroid-gradient GEMMs, Kd = tokens)
 template <bool A_MN, bool B_MN, class Epi>
 int launch_tc_gemm_ex(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
@@ -44,7 +44,7 @@ template <bool A_MN, bool B_MN, class Epi>
 int launch_tc_gemm_ex_h2(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
                          const float* acc_scale, Epi epi, cudaStream_t st);
 
-// batched form (blockIdx.z = batch): per-batch coordinate offsets along the operands' tensors — a_m / b_n along the
+// batched form (z = batch, handed to the epilogue): per-batch coordinate offsets along the operands' tensors — a_m / b_n along the
 // output-row / output-column dimension, a_k / b_k along the contraction dimension
 struct TcBatchOffsets { int a_m, a_k, b_n, b_k; };
 template <bool A_MN, bool B_MN, class Epi>

@@ -105,6 +105,15 @@ int vadc_soft_assign_bwd(const float* y, const float* g, int64_t rows, int K, fl
 size_t vadc_cdist_workspace_bytes(int nb, int64_t R, int64_t P, int C);
 int vadc_cdist(const float* a, const float* b, int nb, int64_t R, int64_t P, int C,
                float* out, void* workspace, size_t workspace_bytes, void* stream);
+/* Its backward (torch.cdist's gradient, ATen's _euclidean_dist_backward), per batch:
+ *   r = g / dist (0 where dist == 0), ga = a rowsum(r) - r b, gb = b colsum(r) - r^T a.
+ * a [nb,R,C], b [nb,P,C], dist [nb,R,P] (vadc_cdist's output), g [nb,R,P] -> ga [nb,R,C], gb [nb,P,C];
+ * either output may be NULL (not computed).  self != 0: a == b (b may be NULL), R == P, ga receives the whole
+ * gradient of cdist(a, a) and gb must be NULL; the diagonal is skipped (its exact contribution is 0).  Empty problems
+ * (nb, R or P == 0) write zero gradients.  nb <= 65535.  Deterministic; no allocation, no synchronisation. */
+size_t vadc_cdist_bwd_workspace_bytes(int nb, int64_t R, int64_t P, int C);
+int vadc_cdist_bwd(const float* a, const float* b, const float* dist, const float* g, int nb, int64_t R, int64_t P,
+                   int C, int self, float* ga, float* gb, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------ *
  * C2: autograd of C1 — the reference's "centroid update" (SURVEY.md D4):

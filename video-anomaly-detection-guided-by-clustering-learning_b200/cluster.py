@@ -3,6 +3,7 @@ of libvadc.so.  Class names, constructor / forward signatures, parameter names
 and state_dict keys are the reference's (SURVEY.md §8b) so the classes drop into
 ``Mymodel`` (model/backbone.py:40-41) unchanged."""
 import ctypes
+import math
 
 import numpy as np
 import torch
@@ -111,49 +112,104 @@ class _ClusterAssign(torch.autograd.Function):
         return gx.view(*ctx.lead, C), (gc if Kv == K else gc[:Kv]), gw, gb, None, None, None
 
 
-def cdist(a, b):
-    """batched ``torch.cdist(a, b)`` (p=2, mm form) on the vadc kernels.
-    a [..., R, C], b [..., P, C] with equal leading dims.  Forward only."""
-    _lib.require_cuda(a, b)
-    a3, b3 = f32c(a), f32c(b)
-    if a3.shape[-1] != b3.shape[-1]:
-        raise RuntimeError("X1 and X2 must have the same number of columns. X1: %d X2: %d"
-                           % (a3.shape[-1], b3.shape[-1]))
-    lead = a3.shape[:-2]
-    R, P, C = a3.shape[-2], b3.shape[-2], a3.shape[-1]
-    nbatch = int(np.prod(lead)) if len(lead) else 1
-    out = torch.empty((*lead, R, P), device=a3.device, dtype=torch.float32)
+def _cdist_fwd(a3, b3):
+    """vadc_cdist of a3 [nb,R,C] and b3 [nb,P,C] (fp32, contiguous) -> [nb,R,P]"""
+    nbatch, R, C = a3.shape
+    P = b3.shape[1]
+    out = torch.empty((nbatch, R, P), device=a3.device, dtype=torch.float32)
     l = _lib.lib()
     nb = l.vadc_cdist_workspace_bytes(nbatch, R, P, C)
     ws = workspace(nb, a3.device)
-    check(l.vadc_cdist(ptr(a3), ptr(b3), nbatch, R, P, C, ptr(out), ptr(ws), ws.numel(), stream()),
-          "vadc_cdist")
+    check(l.vadc_cdist(ptr(a3), ptr(b3), nbatch, R, P, C, ptr(out), ptr(ws), ws.numel(), stream()), "vadc_cdist")
     return out
 
 
-class _SelfDist(torch.autograd.Function):
-    """self_similarity(): cdist(centers, centers) (model/cluster.py:77-79,124-125).
-    The reference never back-propagates through it (backbone.py:95-97 are
-    commented out); the backward is provided for completeness via autograd's
-    own formula on the saved output."""
+def _cdist_bwd(a3, b3, D, g, need_a, need_b, self_mode=False):
+    """(ga, gb) of cdist(a3, b3) for the upstream gradient g [nb,R,P] (vadc_cdist_bwd); an unrequested one is None.
+    self_mode: b3 is a3, and ga is the whole gradient of cdist(a3, a3)."""
+    nbatch, R, C = a3.shape
+    P = b3.shape[1]
+    g = f32c(g)
+    ga = torch.empty_like(a3) if need_a else None
+    gb = torch.empty_like(b3) if need_b and not self_mode else None
+    l = _lib.lib()
+    nb = l.vadc_cdist_bwd_workspace_bytes(nbatch, R, P, C)
+    ws = workspace(nb, a3.device)
+    check(l.vadc_cdist_bwd(ptr(a3), None if self_mode else ptr(b3), ptr(D), ptr(g), nbatch, R, P, C, int(self_mode),
+                           ptr(ga), ptr(gb), ptr(ws), ws.numel(), stream()), "vadc_cdist_bwd")
+    return ga, gb
+
+
+class _CDist(torch.autograd.Function):
+    """cdist(a [nb,R,C], b [nb,P,C]) -> [nb,R,P] and its backward on the vadc kernels"""
 
     @staticmethod
-    def forward(ctx, centers):
-        S = cdist(centers, centers)
-        ctx.save_for_backward(centers, S)
+    def forward(ctx, a3, b3):
+        D = _cdist_fwd(a3, b3)
+        ctx.save_for_backward(a3, b3, D)
+        ctx.set_materialize_grads(False)
+        return D
+
+    @staticmethod
+    def backward(ctx, g):
+        if g is None:
+            return None, None
+        a3, b3, D = ctx.saved_tensors
+        return _cdist_bwd(a3, b3, D, g, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+
+
+class _SelfDist(torch.autograd.Function):
+    """cdist(c, c) of c [nb,K,C] -> [nb,K,K] (self_similarity(), model/cluster.py:77-79,124-125).  The reference never
+    back-propagates through it (backbone.py:95-97 are commented out); the backward is vadc_cdist_bwd's self mode."""
+
+    @staticmethod
+    def forward(ctx, c3):
+        S = _cdist_fwd(c3, c3)
+        ctx.save_for_backward(c3, S)
+        ctx.set_materialize_grads(False)
         return S
 
     @staticmethod
     def backward(ctx, gS):
-        c, S = ctx.saved_tensors
-        return _selfdist_grad(c, S, gS)
+        if gS is None:
+            return None
+        c3, S = ctx.saved_tensors
+        return _cdist_bwd(c3, c3, S, gS, True, False, self_mode=True)[0]
 
 
-def _selfdist_grad(c, S, gS):
-    """d cdist(c, c) / dc applied to gS (autograd's own formula on the saved output)"""
-    r = torch.where(S == 0, torch.zeros_like(S), gS / S)
-    r = r + r.transpose(-1, -2)
-    return c * r.sum(-1, keepdim=True) - r @ c
+def cdist(a, b):
+    """``torch.cdist(a, b)`` (p=2, mm form) on the vadc kernels, differentiable in both arguments.
+    a [..., R, C], b [..., P, C]; the leading dimensions broadcast as torch.cdist's do.  ``cdist(c, c)`` (the same
+    tensor twice, as in self_similarity()) takes the self-distance path."""
+    _lib.require_cuda(a, b)
+    for name, t in (("X1", a), ("X2", b)):
+        if t.dim() < 2:
+            raise RuntimeError("cdist only supports at least 2D tensors, %s got: %dD" % (name, t.dim()))
+    if a.shape[-1] != b.shape[-1]:
+        raise RuntimeError("X1 and X2 must have the same number of columns. X1: %d X2: %d"
+                           % (a.shape[-1], b.shape[-1]))
+    R, P, C = a.shape[-2], b.shape[-2], a.shape[-1]
+    # every reshape names its sizes: a -1 next to a zero-sized dimension is ambiguous to torch, and empty inputs (R, P
+    # or a leading dimension 0) give torch.cdist's empty result and zero / empty gradients
+    if a is b:
+        lead = a.shape[:-2]
+        return _SelfDist.apply(f32c(a).reshape(math.prod(lead), R, C)).view(*lead, R, P)
+    if a.dim() == 2 and b.dim() == 2:
+        return _CDist.apply(f32c(a)[None], f32c(b)[None]).view(R, P)      # a view: its backward copies nothing
+    if b.dim() == 2:              # b's rows are shared by every batch of a: a's leading dimensions fold into its rows
+        lead = a.shape[:-2]
+        return _CDist.apply(f32c(a).reshape(1, math.prod(lead) * R, C), f32c(b)[None]).view(*lead, R, P)
+    if a.dim() == 2:              # a's rows are shared: b's leading dimensions fold into its rows, D^T per batch
+        lead = b.shape[:-2]
+        Dt = _CDist.apply(f32c(b).reshape(1, math.prod(lead) * P, C), f32c(a)[None])          # [1, n P, R]
+        return Dt.view(*lead, P, R).transpose(-1, -2).contiguous()
+    lead = a.shape[:-2]
+    if b.shape[:-2] != lead:      # the smaller side is expanded (autograd sums its gradient back); torch's error otherwise
+        lead = torch.broadcast_tensors(torch.empty(lead, device="meta"), torch.empty(b.shape[:-2], device="meta"))[0].shape
+    nbatch = math.prod(lead)
+    a3 = f32c(a.expand(*lead, R, C)).reshape(nbatch, R, C)
+    b3 = f32c(b.expand(*lead, P, C)).reshape(nbatch, P, C)
+    return _CDist.apply(a3, b3).view(*lead, R, P)
 
 
 class PosSoftAssign(nn.Module):
@@ -246,7 +302,7 @@ class EuclidDistance_Assign_Module(nn.Module):
         return
 
     def self_similarity(self):
-        return _SelfDist.apply(self.cluster_center)
+        return cdist(self.cluster_center, self.cluster_center)
 
     def forward(self, x, alpha=None):
         if not alpha == None:  # noqa: E711  (cluster.py:49-50: persists on assign_func)
@@ -347,7 +403,8 @@ class _SpaceClusterAssign(torch.autograd.Function):
               "vadc_space_cluster_bwd")
         gc = gc if Kv == K else gc[:, :Kv].contiguous()
         if gS is not None:     # the reference never back-propagates through the self-distance (backbone.py:95-97 are comments)
-            gc = gc + _selfdist_grad(cen[:, :Kv], Sd, gS)
+            c3 = cen if Kv == K else cen[:, :Kv].contiguous()
+            gc = gc + _cdist_bwd(c3, c3, Sd, gS, True, False, self_mode=True)[0]
         return gx.view(B, Dd, H, W, C), gc, gw, gb, None, None
 
 
@@ -378,7 +435,7 @@ class Space_EuclidDistance_Assign_Module(nn.Module):
         return
 
     def self_similarity(self):
-        return _SelfDist.apply(self.cluster_center)
+        return cdist(self.cluster_center, self.cluster_center)
 
     def forward(self, x, alpha=None):
         if not alpha == None:  # noqa: E711

@@ -30,12 +30,13 @@ struct StoreEpilogue {
   }
 };
 
-// gz = feature * rsum - acc + gF
+// gz = feature * rsum - acc + gF   (batch z: out / feature / gF batch_out, rsum batch_rsum further)
 struct GzEpilogue {
   float* out; const float* feature; const float* rsum; const float* gF; long long ld;
-  __device__ __forceinline__ void operator()(int, int, int m, int n, float v) const {
-    long long i = (long long)m * ld + n;
-    float o = feature[i] * rsum[m] - v;
+  long long batch_out = 0, batch_rsum = 0;
+  __device__ __forceinline__ void operator()(int batch, int, int m, int n, float v) const {
+    long long i = batch * batch_out + (long long)m * ld + n;
+    float o = feature[i] * rsum[batch * batch_rsum + m] - v;
     if (gF) o += gF[i];
     out[i] = o;
   }
@@ -645,6 +646,317 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
   }
   // (5) LayerNorm backward
   return launch_ln_bwd(gz, x, mu, rstd, ln_w, N, C, gx, lnpart, g_ln_w, g_ln_b, st);
+}
+
+// ---------------------------------------------------------------------------
+// backward of the stand-alone batched cdist (ATen's _euclidean_dist_backward), per batch z:
+//   r = g / D (0 where D == 0),  rho_a = rowsum(r),  rho_b = colsum(r)
+//   ga = a rho_a - r b,  gb = b rho_b - r^T a
+// self (cdist(c, c)): r + r^T with the diagonal zeroed, gc = c rowsum(r + r^T) - (r + r^T) c — one contraction.
+// Both sums of r come out of the pass that writes r, as per-block partials reduced in a fixed order, rather than from
+// launch_colsum / launch_space_colsum over r afterwards: that would read r (4 nb R P bytes, 256 MB for 65536 tokens
+// against 1024 centroids) a second time, and launch_space_colsum sums the space head's [M, C K] layout (a batch = a
+// K-column window), not [nb, R, P] (a batch = R rows).
+// ---------------------------------------------------------------------------
+namespace vadc {
+// Ratio pass: one block = 32 S rows of one batch (blockIdx.z) by a range of `tpc` 32-wide column tiles (blockIdx.y;
+// warp = rows, lanes = columns: coalesced).  Writes r (batch stride Rp P; rows R..Rp-1 zero, so that a contraction over
+// a batch's rows never reaches the next batch), the row sums (to rho with one column range, else the range's partials
+// rowpart[blockIdx.y, z R + i]), the block's column partials colpart[blockIdx.x, z P + j] (optional) and max |r| as
+// float bits.  SYM (R == P): r + r^T, the transposed tile through shared memory; the diagonal is skipped — its exact
+// contribution is r_ii (c_i - c_i) = 0, and the mm-form D_ii is fp32 cancellation noise, not 0.
+template <bool SYM, int S>
+__global__ void __launch_bounds__(256, 2)      // (256) alone left SYM at 64 registers and a spill
+cdist_ratio_kernel(const float* __restrict__ g, const float* __restrict__ D, long long R, long long P, long long Rp,
+                   int tpc, float* __restrict__ r, float* __restrict__ rho, float* __restrict__ rowpart,
+                   float* __restrict__ colpart, unsigned* __restrict__ absmax_bits) {
+  __shared__ float tile[32][33];
+  __shared__ float csum[8][33];
+  __shared__ float bmax[8];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const long long z = blockIdx.z, i0 = (long long)blockIdx.x * 32 * S, nbt = gridDim.z;
+  const float* gz = g + z * R * P;
+  const float* dz = D + z * R * P;
+  float* rz = r + z * Rp * P;
+  float rs[4 * S];
+#pragma unroll
+  for (int q = 0; q < 4 * S; ++q) rs[q] = 0.f;
+  float amax = 0.f;
+  const long long jend = min(P, (long long)(blockIdx.y + 1) * tpc * 32);
+  for (long long j0 = (long long)blockIdx.y * tpc * 32; j0 < jend; j0 += 32) {
+    const long long j = j0 + tx;
+    float cs = 0.f;
+#pragma unroll
+    for (int s = 0; s < S; ++s) {
+      const long long ib = i0 + 32 * s;
+      if (SYM) {                  // tile[jj][ii] = ratio at (row j0 + jj, column ib + ii)
+        float dv[4], gv[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const long long jr = j0 + ty + 8 * q, ic = ib + tx;
+          const bool in = jr < P && ic < R;
+          dv[q] = in ? dz[jr * P + ic] : 0.f;
+          gv[q] = in ? gz[jr * P + ic] : 0.f;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < 4; ++q) tile[ty + 8 * q][tx] = dv[q] != 0.f ? gv[q] / dv[q] : 0.f;
+        __syncthreads();
+      }
+      float dv[4], gv[4];         // every load of the tile issued before the first use
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const long long i = ib + ty + 8 * q;
+        const bool in = i < R && j < P;
+        dv[q] = in ? dz[i * P + j] : 0.f;
+        gv[q] = in ? gz[i * P + j] : 0.f;
+      }
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const int ii = ty + 8 * q;
+        const long long i = ib + ii;
+        float v = dv[q] != 0.f ? gv[q] / dv[q] : 0.f;
+        if (SYM) v = i == j ? 0.f : v + tile[tx][ii];
+        if (i < Rp && j < P) rz[i * P + j] = v;
+        rs[4 * s + q] += v;
+        cs += v;
+        amax = fmaxf(amax, fabsf(v));
+      }
+    }
+    if (colpart) {               // the block's column sums, fixed order (deterministic)
+      csum[ty][tx] = cs;
+      __syncthreads();
+      if (ty == 0 && j < P) {
+        float t = 0.f;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) t += csum[w][tx];
+        colpart[(long long)blockIdx.x * nbt * P + z * P + j] = t;
+      }
+      __syncthreads();
+    }
+  }
+  float* rout = gridDim.y == 1 ? rho : rowpart + (long long)blockIdx.y * nbt * R;
+#pragma unroll
+  for (int s = 0; s < S; ++s)
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float t = warp_sum(rs[4 * s + q]);
+      const long long i = i0 + 32 * s + ty + 8 * q;
+      if (tx == 0 && i < R) rout[z * R + i] = t;
+    }
+  amax = warp_max(amax);
+  if (tx == 0) bmax[ty] = amax;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float m = bmax[0];
+#pragma unroll
+    for (int w = 1; w < 8; ++w) m = fmaxf(m, bmax[w]);
+    if (m > 0.f && isfinite(m)) atomicMax(absmax_bits, __float_as_uint(m));
+  }
+}
+
+// out[w] = sum_c partial[c, w] over nchunks rows, fixed order: a block owns 32 columns, its eight warps take every
+// eighth chunk.  (colsum_stage2_kernel runs one thread per column through all chunks: with the ratio pass's ~1000
+// chunks of 1024 columns that is four blocks of 1000 dependent loads each; ln_bwd_finalize_kernel has this shape but
+// writes two fixed outputs.)
+__global__ void __launch_bounds__(256)
+colsum_chunks_kernel(const float* __restrict__ partial, int nchunks, long long W, float* __restrict__ out) {
+  __shared__ float red[8][33];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const long long w = (long long)blockIdx.x * 32 + lane;
+  float s = 0.f;
+  if (w < W)
+    for (int c = wid; c < nchunks; c += 8) s += partial[(long long)c * W + w];
+  red[wid][lane] = s;
+  __syncthreads();
+  if (wid == 0 && w < W) {
+    float t = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) t += red[k][lane];
+    out[w] = t;
+  }
+}
+
+// rows of one batch of r: batches of a batched launch start on a k-block boundary of the contraction over the rows
+static long long cdist_bwd_rows(int nb, long long R) { return nb > 1 ? (R + 63) / 64 * 64 : R; }
+// rows per ratio-pass block / 32: tall blocks for many rows keep the column partials few
+static int cdist_ratio_s(bool self, long long R) { return !self && R >= 1024 ? 2 : 1; }
+static long long cdist_ratio_chunks(long long Rp, int S) { return (Rp + 32ll * S - 1) / (32ll * S); }
+// column ranges of the ratio pass: ~1024 blocks in all (a [K, K] self-distance alone is K / 32 row strips)
+static int cdist_ratio_colchunks(int nb, long long Rp, long long P, int S) {
+  const long long tiles = (P + 31) / 32, blocks = cdist_ratio_chunks(Rp, S) * nb;
+  return (int)std::max<long long>(1, std::min<long long>(tiles, (1024 + blocks - 1) / blocks));
+}
+static int cdist_ratio_colchunks_max(int nb, long long Rp, long long P) {
+  return std::max(cdist_ratio_colchunks(nb, Rp, P, 1), cdist_ratio_colchunks(nb, Rp, P, 2));
+}
+// split-K slots of the one-problem gb contraction (over the R rows): the larger of the tensor-core and SIMT counts
+static int cdist_bwd_sk_tc(long long R, long long P, int C) { return bwd_tc_splits(R, C, (int)P); }
+static int cdist_bwd_sk_simt(long long R, long long P, int C) {
+  return split_count(R, (int)(((P + 63) / 64) * ((C + 63) / 64)));
+}
+
+// the two contractions on the tcgen05 GEMM: tensor-bound sizes (the operand splits cost a pass each), TMA row pitches
+// (C, P multiples of 8) and every launch's shape predicate
+static bool cdist_bwd_tc_ok(int nb, long long R, long long P, int C, const float* a, const float* b) {
+  const long long Rp = cdist_bwd_rows(nb, R);
+  return !env_on("VADC_NO_TC_GEMM") && (C % 8) == 0 && (P % 8) == 0 && (long long)nb * Rp < (1ll << 31) &&
+         (long long)nb * P < (1ll << 31) && (double)nb * R * P * C >= (double)(1ll << 24) && aligned16(a) && aligned16(b) &&
+         tc_gemm_shape_ok(R, C, P, true) && tc_gemm_shape_ok(C, R, P, false) && tc_gemm_shape_ok(P, C, Rp, true);
+}
+}  // namespace vadc
+
+extern "C" size_t vadc_cdist_bwd_workspace_bytes(int nb, int64_t R, int64_t P, int C) {
+  if (nb < 0 || R < 0 || P < 0 || C <= 0) return 0;
+  const size_t n = nb > 0 ? (size_t)nb : 1, r1 = R > 0 ? (size_t)R : 1, p1 = P > 0 ? (size_t)P : 1;
+  const size_t Rp = (size_t)cdist_bwd_rows((int)n, (long long)r1);
+  size_t b = 0;
+  b += align_up(n * Rp * p1 * sizeof(float), 256);                                             // r
+  b += align_up(n * r1 * sizeof(float), 256) + align_up(n * p1 * sizeof(float), 256);          // rho_a, rho_b
+  b += align_up((size_t)cdist_ratio_colchunks_max((int)n, (long long)Rp, (long long)p1) * n * r1 * sizeof(float), 256);  // row partials
+  b += align_up((size_t)cdist_ratio_chunks((long long)Rp, 1) * n * p1 * sizeof(float), 256);  // column partials
+  b += 2 * 256;                                                                                  // max bits, scales
+  if (n == 1)                                                                                    // split-K partials
+    b += align_up((size_t)std::max(cdist_bwd_sk_tc(r1, p1, C), cdist_bwd_sk_simt(r1, p1, C)) * p1 * C * sizeof(float), 256);
+  if ((C % 8) == 0 && (p1 % 8) == 0)                                                             // operand terms
+    b += tc_gemm_split_bytes((long long)(n * Rp), p1) + tc_gemm_split_bytes((long long)(n * r1), C) +
+         tc_gemm_split_bytes((long long)(n * p1), C);
+  return b + 256;
+}
+
+namespace vadc {
+static int cdist_bwd_impl(const float* a, const float* b, const float* dist, const float* g, int nb, long long R,
+                          long long P, int C, bool self, float* ga, float* gb, void* workspace, size_t workspace_bytes,
+                          cudaStream_t st) {
+  const long long Rp = cdist_bwd_rows(nb, R), PC = P * C;
+  const int S = cdist_ratio_s(self, R);
+  const long long chunks = cdist_ratio_chunks(Rp, S);
+  Carver ws(workspace, workspace_bytes);
+  float* r = ws.take<float>((size_t)nb * Rp * P);
+  float* rho_a = ws.take<float>((size_t)nb * R);
+  float* rho_b = ws.take<float>((size_t)nb * P);
+  float* colpart = ws.take<float>((size_t)cdist_ratio_chunks(Rp, 1) * nb * P);
+  float* rowpart = ws.take<float>((size_t)cdist_ratio_colchunks_max(nb, Rp, P) * nb * R);
+  unsigned* bits = ws.take<unsigned>(64);
+  float* sc = ws.take<float>(64);
+  float* q = nb == 1 ? ws.take<float>((size_t)std::max(cdist_bwd_sk_tc(R, P, C), cdist_bwd_sk_simt(R, P, C)) * PC) : nullptr;
+  int rc;
+  // (1) r, rho_a, max |r| in one pass over g and D; rho_b from the column partials
+  VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
+  float* cp = gb ? colpart : nullptr;
+  const int cch = cdist_ratio_colchunks(nb, Rp, P, S), tpc = (int)(((P + 31) / 32 + cch - 1) / cch);
+  const dim3 grid((unsigned)chunks, (unsigned)cch, (unsigned)nb);
+  if (self) cdist_ratio_kernel<true, 1><<<grid, 256, 0, st>>>(g, dist, R, P, Rp, tpc, r, rho_a, rowpart, nullptr, bits);
+  else if (S == 2) cdist_ratio_kernel<false, 2><<<grid, 256, 0, st>>>(g, dist, R, P, Rp, tpc, r, rho_a, rowpart, cp, bits);
+  else cdist_ratio_kernel<false, 1><<<grid, 256, 0, st>>>(g, dist, R, P, Rp, tpc, r, rho_a, rowpart, cp, bits);
+  VADC_CHECK_LAUNCH("cdist_ratio_kernel");
+  if (cch > 1) {
+    colsum_chunks_kernel<<<(unsigned)((nb * R + 31) / 32), 256, 0, st>>>(rowpart, cch, (long long)nb * R, rho_a);
+    VADC_CHECK_LAUNCH("colsum_chunks_kernel");
+  }
+  if (gb) {
+    colsum_chunks_kernel<<<(unsigned)((nb * P + 31) / 32), 256, 0, st>>>(colpart, (int)chunks, (long long)nb * P, rho_b);
+    VADC_CHECK_LAUNCH("colsum_chunks_kernel");
+  }
+  const float* bb = self ? a : b;              // self: the one contraction is the ga form with b = a
+  if (cdist_bwd_tc_ok(nb, R, P, C, a, bb)) {
+    // (2) ga = a rho_a - r b  and  gb = b rho_b - r^T a  on the tcgen05 GEMM.  r as [nb Rp, P], a as [nb R, C], b as
+    //     [nb P, C]; ga: rows = channels from C = 128 up (coalesced stores), gb: contraction over the rows, split-K
+    //     for one problem, one batched launch otherwise
+    const int sk = cdist_bwd_sk_tc(R, P, C);
+    void* rs = ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * Rp, P));
+    void* as = ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * R, C));
+    void* bs = self ? as : ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * P, C));
+    const TcBatchOffsets oga{0, (int)P, (int)Rp, 0}, ogb{0, (int)Rp, 0, (int)R};
+    const TcGzEpi ega{ga, a, rho_a, nullptr, C};
+    const TcCdistGaTEpi egat{ga, a, rho_a, R, C};
+    const TcPartialEpi egbp{q, C, PC};
+    const TcSpaceGcEpi egb{gb, b, rho_b, PC, C, (int)P};
+    if (!env_on("VADC_TC_BF16X3")) {
+      // two fp16 terms of power-of-two-scaled operands; r has no a-priori bound, its scale comes from the measured max:
+      // sc[0..2] = {s_r, s_b, 1 / (s_r s_b)} (ga; self: s_b = s_a), sc[4..6] = {s_r, s_a, 1 / (s_r s_a)} (gb); no host sync
+      if ((gb || self) && (rc = tc_absmax_bits(a, (long long)nb * R * C, bits + 1, st))) return rc;
+      if (ga && !self && (rc = tc_absmax_bits(b, (long long)nb * P * C, bits + 2, st))) return rc;
+      if (ga && (rc = tc_pair_scales(bits, 0.f, self ? bits + 1 : bits + 2, 0.f, sc, st))) return rc;
+      if (gb && (rc = tc_pair_scales(bits, 0.f, bits + 1, 0.f, sc + 4, st))) return rc;
+      if ((rc = tc_split2h(r, (long long)nb * Rp, P, ga ? sc : sc + 4, rs, st))) return rc;
+      if (ga) {
+        if ((rc = tc_split2h(bb, (long long)nb * P, C, sc + 1, bs, st))) return rc;
+        if (nb > 1) rc = launch_tc_gemm_batched_h2<true, false>(bs, (long long)nb * P, C, rs, (long long)nb * Rp, P, C, R, P, nb,
+                                                                oga, sc + 2, egat, st);
+        else if (C >= 128) rc = launch_tc_gemm_ex_h2<true, false>(bs, rs, C, R, P, 1, sc + 2,
+                                                                  TcGzTEpi{ga, a, rho_a, nullptr, C}, st);
+        else rc = launch_tc_gemm_h2<true>(rs, bs, R, C, P, sc + 2, ega, st);
+        if (rc) return rc;
+      }
+      if (gb) {
+        if ((rc = tc_split2h(a, (long long)nb * R, C, sc + 5, as, st))) return rc;
+        if (nb > 1) return launch_tc_gemm_batched_h2<true, true>(rs, (long long)nb * Rp, P, as, (long long)nb * R, C, P, C, Rp, nb,
+                                                                 ogb, sc + 6, egb, st);
+        if ((rc = launch_tc_gemm_ex_h2<true, true>(rs, as, P, C, R, sk, sc + 6, egbp, st))) return rc;
+      }
+    } else {
+      // VADC_TC_BF16X3: three bf16 terms per operand (fp32-faithful for any data, no scales)
+      if ((rc = tc_split3(r, (long long)nb * Rp, P, rs, st))) return rc;
+      if ((gb || self) && (rc = tc_split3(a, (long long)nb * R, C, as, st))) return rc;
+      if (ga) {
+        if (!self && (rc = tc_split3(b, (long long)nb * P, C, bs, st))) return rc;
+        rc = nb > 1 ? launch_tc_gemm_batched<true, false>(bs, (long long)nb * P, C, rs, (long long)nb * Rp, P, C, R, P, nb, oga, egat, st)
+                    : launch_tc_gemm<true>(rs, bs, R, C, P, ega, st);
+        if (rc) return rc;
+      }
+      if (gb) {
+        if (nb > 1) return launch_tc_gemm_batched<true, true>(rs, (long long)nb * Rp, P, as, (long long)nb * R, C, P, C, Rp, nb, ogb,
+                                                              egb, st);
+        if ((rc = launch_tc_gemm_ex<true, true>(rs, as, P, C, R, sk, egbp, st))) return rc;
+      }
+    }
+    if (gb) {                    // one problem: gb = b rho_b - sum of the split-K partials
+      gcenters_finalize_kernel<<<(unsigned)((PC + 255) / 256), 256, 0, st>>>(nullptr, q, sk, b, rho_b, (int)P, C, gb);
+      VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
+    }
+    return VADC_OK;
+  }
+  // (2') fp32 SIMT GEMM: shapes the tensor-core path does not take, and launch-bound sizes
+  cudaError_t e;
+  if (ga) {
+    Operand Aop{r, P, 1}, Bop{bb, C, 1};
+    GzEpilogue epi{ga, a, rho_a, nullptr, C, R * C, R};
+    e = sgemm_auto((int)R, C, (int)P, Aop, Bop, Rp * P, PC, nb, 1, epi, st);
+    if (e != cudaSuccess) return record_cuda_error(e, "cdist bwd sgemm r.b");
+  }
+  if (gb) {
+    Operand Aop{r, 1, P}, Bop{a, C, 1};
+    if (nb > 1) {
+      e = sgemm_auto((int)P, C, (int)R, Aop, Bop, Rp * P, R * C, nb, 1, SpaceGcEpilogue{gb, b, rho_b, PC, C, (int)P}, st);
+      if (e != cudaSuccess) return record_cuda_error(e, "cdist bwd sgemm rT.a");
+      return VADC_OK;
+    }
+    const int sks = cdist_bwd_sk_simt(R, P, C);
+    e = launch_sgemm<64, 64>((int)P, C, (int)R, Aop, Bop, 0, 0, 1, sks, PartialEpilogue{q, C, PC}, st);
+    if (e != cudaSuccess) return record_cuda_error(e, "cdist bwd sgemm rT.a");
+    gcenters_finalize_kernel<<<(unsigned)((PC + 255) / 256), 256, 0, st>>>(nullptr, q, sks, b, rho_b, (int)P, C, gb);
+    VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
+  }
+  return VADC_OK;
+}
+}  // namespace vadc
+
+extern "C" int vadc_cdist_bwd(const float* a, const float* b, const float* dist, const float* g, int nb, int64_t R, int64_t P,
+                              int C, int self, float* ga, float* gb, void* workspace, size_t workspace_bytes, void* stream) {
+  VADC_REQUIRE(nb >= 0 && R >= 0 && P >= 0 && C > 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(!self || (gb == nullptr && R == P && (b == nullptr || b == a)), VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(nb <= 65535 && R < (1ll << 31) && P < (1ll << 31), VADC_ERR_UNSUPPORTED);
+  if (!ga && !gb) return VADC_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (nb == 0 || R == 0 || P == 0) {           // empty distance matrix: zero gradients
+    if (ga && (long long)nb * R > 0) VADC_CUDA(cudaMemsetAsync(ga, 0, (size_t)nb * R * C * sizeof(float), st));
+    if (gb && (long long)nb * P > 0) VADC_CUDA(cudaMemsetAsync(gb, 0, (size_t)nb * P * C * sizeof(float), st));
+    return VADC_OK;
+  }
+  VADC_REQUIRE(a && g && dist && workspace && (self || b), VADC_ERR_NULL_POINTER);
+  VADC_REQUIRE(workspace_bytes >= vadc_cdist_bwd_workspace_bytes(nb, R, P, C), VADC_ERR_WORKSPACE);
+  return cdist_bwd_impl(a, self ? a : b, dist, g, nb, R, P, C, self != 0, ga, gb, workspace, workspace_bytes, st);
 }
 
 // ---------------------------------------------------------------------------

@@ -23,6 +23,14 @@ int launch_ln_bwd(const float* gz, const float* x, const float* mu, const float*
 int launch_dist(const float* a, const float* b, const float* aa, const float* bb, int nb,
                 long long R, long long P, int C, float* out, cudaStream_t st);
 int split_count(long long Ntok, int tiles);
+// gcenters[c,k,p] = centers[c,k,p] * rcol[c,k] - acc   (SIMT epilogue of the space head and the batched cdist backward)
+struct SpaceGcEpilogue {
+  float* out; const float* centers; const float* rcol; long long KP; int P, K;
+  __device__ __forceinline__ void operator()(int batch, int, int m, int n, float v) const {
+    long long i = (long long)batch * KP + (long long)m * P + n;
+    out[i] = centers[i] * rcol[(long long)batch * K + m] - v;
+  }
+};
 // fused small-K backward (cluster_bwd_fused.cu)
 bool bwd_fused_shape_ok(long long N, int C, int K);
 size_t bwd_fused_workspace_bytes(long long N, int C, int K);

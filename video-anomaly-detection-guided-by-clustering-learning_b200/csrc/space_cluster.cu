@@ -390,14 +390,6 @@ struct SpaceGzEpilogue {
   }
 };
 
-// gcenters[c,k,p] = centers[c,k,p] * rcol[c,k] - acc
-struct SpaceGcEpilogue {
-  float* out; const float* centers; const float* rcol; long long KP; int P, K;
-  __device__ __forceinline__ void operator()(int batch, int, int m, int n, float v) const {
-    long long i = (long long)batch * KP + (long long)m * P + n;
-    out[i] = centers[i] * rcol[(long long)batch * K + m] - v;
-  }
-};
 
 // The three contractions of the head as batched tcgen05 GEMMs (three-term bf16 split, fp32-faithful): worth it
 // from a few GFLOP up; P, K multiples of 8 for the TMA row pitches, K a multiple of 64 so that a batch's window

@@ -599,6 +599,7 @@ template int launch_tc_gemm<false, TcBiasGeluTEpi>(const void*, const void*, lon
 VADC_TC_BATCHED(false, false, TcBatchDistEpi)
 VADC_TC_BATCHED(true, false, TcSpaceGzEpi)
 VADC_TC_BATCHED(true, true, TcSpaceGcEpi)
+VADC_TC_BATCHED(true, false, TcCdistGaTEpi)
 #undef VADC_TC_BATCHED
 #define VADC_TC_BATCHED_H2(AMN, BMN, EPI)                                                                              \
   template int launch_tc_gemm_batched_h2<AMN, BMN, EPI>(const void*, long long, long long, const void*, long long,      \
@@ -607,6 +608,7 @@ VADC_TC_BATCHED(true, true, TcSpaceGcEpi)
 VADC_TC_BATCHED_H2(false, false, TcBatchDistEpi)
 VADC_TC_BATCHED_H2(true, false, TcSpaceGzEpi)
 VADC_TC_BATCHED_H2(true, true, TcSpaceGcEpi)
+VADC_TC_BATCHED_H2(true, false, TcCdistGaTEpi)
 #undef VADC_TC_BATCHED_H2
 
 }  // namespace vadc

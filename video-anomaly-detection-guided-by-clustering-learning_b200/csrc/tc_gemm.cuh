@@ -296,6 +296,25 @@ struct TcSpaceGcEpi {
   }
 };
 
+// batched cdist backward (vadc_cdist_bwd): ga[z,i,c] = a[z,i,c] rho[z,i] - (r b)[z,i,c], transposed like TcSpaceGzEpi
+// (the GEMM's rows are the channels c, its columns the rows i of batch z): a warp stores 32 consecutive channels per row
+struct TcCdistGaTEpi {
+  float* out; const float* a; const float* rho; long long R; int C;
+  __device__ __forceinline__ void operator()(long long c, int r0, float (&v)[32], int nvalid, int z) const {
+    const long long base = (long long)z * R * C + (long long)r0 * C + c;
+    const float* rz = rho + (long long)z * R + r0;
+    float t[32], rs[32];
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const int jj = min(j, nvalid - 1);
+      t[j] = __ldg(a + base + (long long)jj * C); rs[j] = __ldg(rz + jj);
+    }
+#pragma unroll
+    for (int j = 0; j < 32; ++j) v[j] = t[j] * rs[j] - v[j];
+    tc_store_col32(out + base, C, v, nvalid);
+  }
+};
+
 // Memory.read (Memory.py:249-261): uq[m, 0:d] = q[m], uq[m, d:2d] = score_memory @ keys
 // (the row loads of these two are unconditional — 128-bit where the row is aligned, clamped indices otherwise: a
 // predicated load + use per column compiles to one branch region per column, every load waited for alone)

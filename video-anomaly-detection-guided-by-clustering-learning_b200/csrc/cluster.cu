@@ -274,8 +274,47 @@ extern "C" size_t vadc_cluster_fwd_workspace_bytes(int64_t N, int C, int K, int 
   b += align_up((size_t)(softmin_blocks(N, K) + 1) * sizeof(double), 256);
   b += std::max(vadc_cluster_tc_extra_workspace_bytes(N, C, K), vadc_cluster_ws_extra_workspace_bytes(N, C, K));
   if (impl != VADC_IMPL_SIMT && N > 0)                                   // term copies for the tcgen05 GEMMs + scales
-    b += tc_gemm_split_bytes(N, C) + tc_gemm_split_bytes(K, C) + tc_gemm_split_bytes(N, K) + 256;
+    b += tc_terms_bytes(3, N, C) + tc_terms_bytes(3, K, C) + tc_terms_bytes(3, N, K) + 256;
   return b + 256;
+}
+
+// the generic forward's two contractions on the tcgen05 GEMM.  TERMS = 3: bf16 x3 (fp32-faithful).  TERMS = 2: every
+// operand is bounded (LayerNorm output, centroids, softmin weights in [0, 1]), so two fp16 terms after a power-of-two
+// scaling carry 22 significant bits (the fused K = 32 kernel's recipe): 2/3 of the operand bytes and half the MMAs; the
+// scales stay in device memory (no host sync)
+template <int TERMS>
+static int cluster_fwd_tc(const float* x, const float* ln_w, const float* ln_b, const float* centers, int64_t N, int C,
+                          int K, int k_valid, float alpha, float eps, float* D, float* A, float* x_rec, float* feature,
+                          int64_t* label, float* mu, float* rstd, float* rowstats, float* loss_sq, float* zz, float* cc,
+                          double* partial, Carver& ws, cudaStream_t st) {
+  void* fs = ws.take<uint8_t>(tc_terms_bytes(TERMS, N, C));
+  void* cs = ws.take<uint8_t>(tc_terms_bytes(TERMS, K, C));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(TERMS, N, K));
+  float* sc = nullptr;
+  int rc;
+  if constexpr (TERMS == 2) {
+    sc = ws.take<float>(8);
+    if ((rc = tc_fwd_scales(centers, ln_w, ln_b, (long long)K * C, C, sc, st))) return rc;
+  }
+  if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, feature, mu, rstd, zz, st, rowstats, fs, sc))) return rc;
+  if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
+  if ((rc = tc_split<TERMS>(centers, K, C, sc ? sc + 1 : nullptr, cs, st))) return rc;
+  const float* sc2 = sc ? sc + 2 : nullptr;
+  if constexpr (TERMS == 2) {
+    // fp16 x2 only: from K = 128 up the distance GEMM runs with the operands swapped (rows = centroids): coalesced stores of D
+    if (K >= 128) {
+      if ((rc = tc_gemm<2, false, false>({cs, fs, K, N, C, sc2}, TcDistTEpi{D, cc, zz, K}, st))) return rc;
+    } else if ((rc = tc_gemm<2, false, false>({fs, cs, N, K, C, sc2}, TcDistEpi{D, zz, cc, K}, st))) return rc;
+    // softmin writes A and, in the same pass, its two fp16 terms scaled by s_a = 2^13 (the value fwd_scales_kernel puts in sc[3])
+    if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid, as, 8192.0f))) return rc;
+    if (C >= 128)   // rows = channels (centers [K,C] as the MN-major A operand): coalesced x_rec
+      return tc_gemm<2, true, false>({cs, as, C, N, K, sc + 4}, TcStoreTEpi{x_rec, C}, st);
+  } else {
+    if ((rc = tc_gemm<3, false, false>({fs, cs, N, K, C}, TcDistEpi{D, zz, cc, K}, st))) return rc;
+    if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid))) return rc;
+    if ((rc = tc_split<3>(A, N, K, nullptr, as, st))) return rc;
+  }
+  return tc_gemm<TERMS, false, true>({as, cs, N, C, K, sc ? sc + 4 : nullptr}, TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
 }
 
 static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b,
@@ -313,40 +352,12 @@ static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b
   // stay row kernels
   const bool use_tc = impl != VADC_IMPL_SIMT && N > 0 && !env_on("VADC_NO_TC_GEMM") &&
                       tc_gemm_shape_ok(N, K, C, false) && tc_gemm_shape_ok(N, C, K, true);
-  if (use_tc && !env_on("VADC_TC_BF16X3")) {
-    // every operand of the forward is bounded (LayerNorm output, centroids, softmin weights in [0, 1]): two fp16
-    // terms after a power-of-two scaling carry 22 significant bits (the fused K = 32 kernel's recipe): 2/3 of the
-    // operand bytes and half the MMAs of the three-term bf16 split; the scales stay in device memory (no host sync)
-    void* fs = ws.take<uint8_t>(tc_gemm_split2_bytes(N, C));
-    void* cs = ws.take<uint8_t>(tc_gemm_split2_bytes(K, C));
-    void* as = ws.take<uint8_t>(tc_gemm_split2_bytes(N, K));
-    float* sc = ws.take<float>(8);
-    if ((rc = tc_fwd_scales(centers, ln_w, ln_b, (long long)K * C, C, sc, st))) return rc;
-    if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, feature, mu, rstd, zz, st, rowstats, fs, sc + 0))) return rc;
-    if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
-    if ((rc = tc_split2h(centers, K, C, sc + 1, cs, st))) return rc;
-    // from K = 128 up the distance GEMM runs with the operands swapped (rows = centroids): coalesced stores of D
-    if (K >= 128) {
-      if ((rc = launch_tc_gemm_h2<false>(cs, fs, K, N, C, sc + 2, TcDistTEpi{D, cc, zz, K}, st))) return rc;
-    } else if ((rc = launch_tc_gemm_h2<false>(fs, cs, N, K, C, sc + 2, TcDistEpi{D, zz, cc, K}, st))) return rc;
-    // softmin writes A and, in the same pass, its two fp16 terms scaled by s_a = 2^13 (the value fwd_scales_kernel puts in sc[3])
-    if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid, as, 8192.0f))) return rc;
-    if (C >= 128)   // rows = channels (centers [K,C] as the MN-major A operand): coalesced x_rec
-      return launch_tc_gemm_ex_h2<true, false>(cs, as, C, N, K, 1, sc + 4, TcStoreTEpi{x_rec, C}, st);
-    return launch_tc_gemm_h2<true>(as, cs, N, C, K, sc + 4, TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
-  }
-  if (use_tc) {
-    void* fs = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-    void* cs = ws.take<uint8_t>(tc_gemm_split_bytes(K, C));
-    void* as = ws.take<uint8_t>(tc_gemm_split_bytes(N, K));
-    if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, feature, mu, rstd, zz, st, rowstats, fs))) return rc;
-    if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
-    if ((rc = tc_split3(centers, K, C, cs, st))) return rc;
-    if ((rc = launch_tc_gemm<false>(fs, cs, N, K, C, TcDistEpi{D, zz, cc, K}, st))) return rc;
-    if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid))) return rc;
-    if ((rc = tc_split3(A, N, K, as, st))) return rc;
-    return launch_tc_gemm<true>(as, cs, N, C, K, TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
-  }
+  if (use_tc)
+    return env_on("VADC_TC_BF16X3")
+               ? cluster_fwd_tc<3>(x, ln_w, ln_b, centers, N, C, K, k_valid, alpha, eps, D, A, x_rec, feature, label, mu,
+                                   rstd, rowstats, loss_sq, zz, cc, partial, ws, st)
+               : cluster_fwd_tc<2>(x, ln_w, ln_b, centers, N, C, K, k_valid, alpha, eps, D, A, x_rec, feature, label, mu,
+                                   rstd, rowstats, loss_sq, zz, cc, partial, ws, st);
   if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, feature, mu, rstd, zz, st, rowstats))) return rc;
   if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
   if ((rc = launch_dist(feature, centers, zz, cc, 1, N, K, C, D, st))) return rc;
@@ -425,7 +436,7 @@ static bool cdist_tc_ok(int nb, long long R, long long P, int C) {
 extern "C" size_t vadc_cdist_workspace_bytes(int nb, int64_t R, int64_t P, int C) {
   size_t b = align_up((size_t)nb * R * sizeof(float), 256) + align_up((size_t)nb * P * sizeof(float), 256) + 256;
   if (nb > 0 && R > 0 && P > 0 && C > 0 && (C % 8) == 0)
-    b += tc_gemm_split_bytes((long long)nb * R, C) + tc_gemm_split_bytes((long long)nb * P, C);
+    b += tc_terms_bytes(3, (long long)nb * R, C) + tc_terms_bytes(3, (long long)nb * P, C);
   return b;
 }
 
@@ -457,13 +468,13 @@ extern "C" int vadc_cdist(const float* a, const float* b, int nb, int64_t R, int
   if (!self && (rc = launch_row_sqnorm(b, (long long)nb * P, C, bb, st))) return rc;
   if (cdist_tc_ok(nb, R, P, C)) {
     // one launch for all batches: A = a as [nb R, C], B = b as [nb P, C], batch z starts z R / z P rows further
-    void* as = ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * R, C));
-    void* bs = self ? as : ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * P, C));
-    if ((rc = tc_split3(a, (long long)nb * R, C, as, st))) return rc;
-    if (!self && (rc = tc_split3(b, (long long)nb * P, C, bs, st))) return rc;
+    void* as = ws.take<uint8_t>(tc_terms_bytes(3, (long long)nb * R, C));
+    void* bs = self ? as : ws.take<uint8_t>(tc_terms_bytes(3, (long long)nb * P, C));
+    if ((rc = tc_split<3>(a, (long long)nb * R, C, nullptr, as, st))) return rc;
+    if (!self && (rc = tc_split<3>(b, (long long)nb * P, C, nullptr, bs, st))) return rc;
     TcBatchDistEpi epi{out, aa, bb, P, R * P, R, P};
-    return launch_tc_gemm_batched<false, false>(as, (long long)nb * R, C, bs, (long long)nb * P, C, R, P, C, nb,
-                                                TcBatchOffsets{(int)R, 0, (int)P, 0}, epi, st);
+    return tc_gemm<3, false, false>({as, bs, R, P, C, nullptr, 1, nb, {(int)R, 0, (int)P, 0}, (long long)nb * R, C, (long long)nb * P, C},
+                                    epi, st);
   }
   return launch_dist(a, b, aa, bb, nb, R, P, C, out, st);
 }
@@ -477,6 +488,81 @@ static int bwd_tc_splits(long long N, int C, int K) {
   if (s > nkb) s = nkb;
   if (s < 1) s = 1;
   return (int)s;
+}
+}  // namespace vadc
+
+namespace vadc {
+// the generic backward's five contractions on the tcgen05 GEMM: G1 = gR c^T; gz = z rsum - r c + gF;
+// gcenters = A^T gR - r^T z + c colsum(r) with the token matrices read MN-major and split-K over the tokens.
+// TERMS = 2: two fp16 terms per operand, each scaled by the power of two of its measured bound (A: 2^13): 22 significant
+// bits, 2/3 of the operand bytes and half the MMAs of the bf16 x3 split (TERMS = 3)
+template <int TERMS>
+static int cluster_bwd_tc(const float* x, const float* mu, const float* rstd, const float* feature, const float* ln_w,
+                          const float* centers, const float* D, const float* A, const float* gD, const float* gA,
+                          const float* gR, const float* gF, const float* g_loss_sq, int64_t N, int C, int K, float alpha,
+                          float* gx, float* gcenters, float* g_ln_w, float* g_ln_b, float* gemm, float* r, float* rsum,
+                          float* gz, float* cpart, float* rcol, float* lnpart, Carver& ws, cudaStream_t st) {
+  const long long KC = (long long)K * C;
+  const int sk = bwd_tc_splits(N, C, K);
+  void* gRs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* fs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(3, N, K));
+  void* rs = ws.take<uint8_t>(tc_terms_bytes(3, N, K));
+  void* cs = ws.take<uint8_t>(tc_terms_bytes(3, K, C));
+  float* q1 = ws.take<float>((size_t)sk * KC);
+  float* q2 = ws.take<float>((size_t)sk * KC);
+  unsigned* bits = nullptr;
+  float* sc = nullptr;
+  // the scales' slots (tc_cluster_bwd_scales): inputs s_g, s_c, s_f, s_a, s_r; accumulators 1/(s_g s_c), 1/(s_a s_g),
+  // 1/(s_r s_c), 1/(s_r s_f) — all NULL in bf16 x3
+  auto at = [&](int i) -> const float* { return sc ? sc + i : nullptr; };
+  int rc;
+  if constexpr (TERMS == 2) {
+    bits = ws.take<unsigned>(64);
+    sc = ws.take<float>(64);
+    VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
+    if (gR && (rc = tc_absmax_bits(gR, (long long)N * C, bits + 0, st))) return rc;
+    if ((rc = tc_absmax_bits(centers, (long long)K * C, bits + 1, st))) return rc;
+    if ((rc = tc_absmax_bits(feature, (long long)N * C, bits + 2, st))) return rc;
+    if ((rc = tc_cluster_bwd_scales(bits, 0, sc, st))) return rc;
+  }
+  if ((rc = tc_split<TERMS>(centers, K, C, at(1), cs, st))) return rc;
+  if (gR) {
+    if ((rc = tc_split<TERMS>(gR, N, C, at(0), gRs, st))) return rc;
+    // fp16 x2 only: from K = 128 up the operands are swapped (rows = centroids): coalesced stores
+    if constexpr (TERMS == 2) {
+      if (K >= 128) rc = tc_gemm<2, false, false>({cs, gRs, K, N, C, at(5)}, TcStoreTEpi{gemm, K}, st);
+      else rc = tc_gemm<2, false, false>({gRs, cs, N, K, C, at(5)}, TcStoreEpi{gemm, K}, st);
+    } else {
+      rc = tc_gemm<3, false, false>({gRs, cs, N, K, C}, TcStoreEpi{gemm, K}, st);
+    }
+    if (rc) return rc;
+  }
+  // (fp16 x2: max |r| for the scale of r comes out of the row pass itself)
+  if ((rc = launch_bwd_rows(D, A, gR ? gemm : nullptr, gD, gA, g_loss_sq, N, K, alpha, r, rsum, st, bits ? bits + 3 : nullptr)))
+    return rc;
+  if constexpr (TERMS == 2)
+    if ((rc = tc_cluster_bwd_scales(bits, 1, sc, st))) return rc;
+  if ((rc = tc_split<TERMS>(r, N, K, at(4), rs, st))) return rc;
+  // fp16 x2 only: from C = 128 up rows = channels, coalesced loads of feature / gF and stores of gz
+  if constexpr (TERMS == 2) {
+    if (C >= 128) rc = tc_gemm<2, true, false>({cs, rs, C, N, K, at(7)}, TcGzTEpi{gz, feature, rsum, gF, C}, st);
+    else rc = tc_gemm<2, false, true>({rs, cs, N, C, K, at(7)}, TcGzEpi{gz, feature, rsum, gF, C}, st);
+  } else {
+    rc = tc_gemm<3, false, true>({rs, cs, N, C, K}, TcGzEpi{gz, feature, rsum, gF, C}, st);
+  }
+  if (rc) return rc;
+  if (gR) {
+    if ((rc = tc_split<TERMS>(A, N, K, at(3), as, st))) return rc;
+    if ((rc = tc_gemm<TERMS, true, true>({as, gRs, K, C, N, at(6), sk}, TcPartialEpi{q1, C, KC}, st))) return rc;
+  }
+  if ((rc = tc_split<TERMS>(feature, N, C, at(2), fs, st))) return rc;
+  if ((rc = tc_gemm<TERMS, true, true>({rs, fs, K, C, N, at(8), sk}, TcPartialEpi{q2, C, KC}, st))) return rc;
+  cudaError_t e2 = launch_colsum(r, N, K, cpart, rcol, st);
+  if (e2 != cudaSuccess) return record_cuda_error(e2, "colsum r");
+  gcenters_finalize_kernel<<<(unsigned)((KC + 255) / 256), 256, 0, st>>>(gR ? q1 : nullptr, q2, sk, centers, rcol, K, C, gcenters);
+  VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
+  return launch_ln_bwd(gz, x, mu, rstd, ln_w, N, C, gx, lnpart, g_ln_w, g_ln_b, st);
 }
 }  // namespace vadc
 
@@ -494,7 +580,7 @@ extern "C" size_t vadc_cluster_bwd_workspace_bytes(int64_t N, int C, int K) {
   b += align_up((size_t)K * sizeof(float), 256);             // rcol
   b += align_up((size_t)ln_bwd_blocks(N) * 2 * C * sizeof(float), 256);
   // generic path on the tcgen05 GEMM: bf16 term copies of gR, feature, A, r and the centroids + split-K partials
-  b += 2 * tc_gemm_split_bytes((long long)n, C) + 2 * tc_gemm_split_bytes((long long)n, K) + tc_gemm_split_bytes(K, C) + 1024;
+  b += 2 * tc_terms_bytes(3, (long long)n, C) + 2 * tc_terms_bytes(3, (long long)n, K) + tc_terms_bytes(3, K, C) + 1024;
   b += 2 * align_up((size_t)bwd_tc_splits(N, C, K) * K * C * sizeof(float), 256);
   return std::max(std::max(b + 256, bwd_fused_workspace_bytes(N, C, K)), bwd_tc2_workspace_bytes(N, C, K));
 }
@@ -543,72 +629,11 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
   float* rcol = ws.take<float>(K);
   float* lnpart = ws.take<float>((size_t)ln_bwd_blocks(N) * 2 * C);
   if (!env_on("VADC_NO_TC_GEMM") && vadc_device_ok() && (K % 8) == 0 && (C % 8) == 0 && K >= 8 && C >= 8) {
-    // ---- the five contractions on the tcgen05 GEMM (three-term bf16 split): G1 = gR c^T; gz = z rsum - r c + gF;
-    //      gcenters = A^T gR - r^T z + c colsum(r) with the token matrices read MN-major and split-K over the tokens
-    const int sk = bwd_tc_splits(N, C, K);
-    void* gRs = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-    void* fs = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-    void* as = ws.take<uint8_t>(tc_gemm_split_bytes(N, K));
-    void* rs = ws.take<uint8_t>(tc_gemm_split_bytes(N, K));
-    void* cs = ws.take<uint8_t>(tc_gemm_split_bytes(K, C));
-    float* q1 = ws.take<float>((size_t)sk * KC);
-    float* q2 = ws.take<float>((size_t)sk * KC);
-    int rc;
-    if (!env_on("VADC_TC_BF16X3")) {
-      // two fp16 terms per operand, each scaled by the power of two of its measured bound (A: 2^13): 22 significant bits,
-      // 2/3 of the operand bytes and half the MMAs of the bf16 x3 split (VADC_TC_BF16X3 keeps that one)
-      unsigned* bits = ws.take<unsigned>(64);
-      float* sc = ws.take<float>(64);
-      VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
-      if (gR && (rc = tc_absmax_bits(gR, (long long)N * C, bits + 0, st))) return rc;
-      if ((rc = tc_absmax_bits(centers, (long long)K * C, bits + 1, st))) return rc;
-      if ((rc = tc_absmax_bits(feature, (long long)N * C, bits + 2, st))) return rc;
-      if ((rc = tc_cluster_bwd_scales(bits, 0, sc, st))) return rc;
-      if ((rc = tc_split2h(centers, K, C, sc + 1, cs, st))) return rc;
-      if (gR) {
-        if ((rc = tc_split2h(gR, N, C, sc + 0, gRs, st))) return rc;
-        if (K >= 128) {   // operands swapped: rows = centroids, coalesced stores
-          if ((rc = launch_tc_gemm_h2<false>(cs, gRs, K, N, C, sc + 5, TcStoreTEpi{gemm, K}, st))) return rc;
-        } else if ((rc = launch_tc_gemm_h2<false>(gRs, cs, N, K, C, sc + 5, TcStoreEpi{gemm, K}, st))) return rc;
-      }
-      // (max |r| for the fp16 scale of r comes out of the row pass itself)
-      if ((rc = launch_bwd_rows(D, A, gR ? gemm : nullptr, gD, gA, g_loss_sq, N, K, alpha, r, rsum, st, bits + 3))) return rc;
-      if ((rc = tc_cluster_bwd_scales(bits, 1, sc, st))) return rc;
-      if ((rc = tc_split2h(r, N, K, sc + 4, rs, st))) return rc;
-      if (C >= 128) {   // rows = channels: coalesced loads of feature / gF and stores of gz
-        if ((rc = launch_tc_gemm_ex_h2<true, false>(cs, rs, C, N, K, 1, sc + 7, TcGzTEpi{gz, feature, rsum, gF, C}, st))) return rc;
-      } else if ((rc = launch_tc_gemm_h2<true>(rs, cs, N, C, K, sc + 7, TcGzEpi{gz, feature, rsum, gF, C}, st))) return rc;
-      if (gR) {
-        if ((rc = tc_split2h(A, N, K, sc + 3, as, st))) return rc;
-        if ((rc = launch_tc_gemm_ex_h2<true, true>(as, gRs, K, C, N, sk, sc + 6, TcPartialEpi{q1, C, KC}, st))) return rc;
-      }
-      if ((rc = tc_split2h(feature, N, C, sc + 2, fs, st))) return rc;
-      if ((rc = launch_tc_gemm_ex_h2<true, true>(rs, fs, K, C, N, sk, sc + 8, TcPartialEpi{q2, C, KC}, st))) return rc;
-      cudaError_t e2 = launch_colsum(r, N, K, cpart, rcol, st);
-      if (e2 != cudaSuccess) return record_cuda_error(e2, "colsum r");
-      gcenters_finalize_kernel<<<(unsigned)((KC + 255) / 256), 256, 0, st>>>(gR ? q1 : nullptr, q2, sk, centers, rcol, K, C, gcenters);
-      VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
-      return launch_ln_bwd(gz, x, mu, rstd, ln_w, N, C, gx, lnpart, g_ln_w, g_ln_b, st);
-    }
-    if ((rc = tc_split3(centers, K, C, cs, st))) return rc;
-    if (gR) {
-      if ((rc = tc_split3(gR, N, C, gRs, st))) return rc;
-      if ((rc = launch_tc_gemm<false>(gRs, cs, N, K, C, TcStoreEpi{gemm, K}, st))) return rc;
-    }
-    if ((rc = launch_bwd_rows(D, A, gR ? gemm : nullptr, gD, gA, g_loss_sq, N, K, alpha, r, rsum, st))) return rc;
-    if ((rc = tc_split3(r, N, K, rs, st))) return rc;
-    if ((rc = launch_tc_gemm<true>(rs, cs, N, C, K, TcGzEpi{gz, feature, rsum, gF, C}, st))) return rc;
-    if (gR) {
-      if ((rc = tc_split3(A, N, K, as, st))) return rc;
-      if ((rc = launch_tc_gemm_ex<true, true>(as, gRs, K, C, N, sk, TcPartialEpi{q1, C, KC}, st))) return rc;
-    }
-    if ((rc = tc_split3(feature, N, C, fs, st))) return rc;
-    if ((rc = launch_tc_gemm_ex<true, true>(rs, fs, K, C, N, sk, TcPartialEpi{q2, C, KC}, st))) return rc;
-    cudaError_t e2 = launch_colsum(r, N, K, cpart, rcol, st);
-    if (e2 != cudaSuccess) return record_cuda_error(e2, "colsum r");
-    gcenters_finalize_kernel<<<(unsigned)((KC + 255) / 256), 256, 0, st>>>(gR ? q1 : nullptr, q2, sk, centers, rcol, K, C, gcenters);
-    VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
-    return launch_ln_bwd(gz, x, mu, rstd, ln_w, N, C, gx, lnpart, g_ln_w, g_ln_b, st);
+    return env_on("VADC_TC_BF16X3")
+               ? cluster_bwd_tc<3>(x, mu, rstd, feature, ln_w, centers, D, A, gD, gA, gR, gF, g_loss_sq, N, C, K, alpha,
+                                   gx, gcenters, g_ln_w, g_ln_b, gemm, r, rsum, gz, cpart, rcol, lnpart, ws, st)
+               : cluster_bwd_tc<2>(x, mu, rstd, feature, ln_w, centers, D, A, gD, gA, gR, gF, g_loss_sq, N, C, K, alpha,
+                                   gx, gcenters, g_ln_w, g_ln_b, gemm, r, rsum, gz, cpart, rcol, lnpart, ws, st);
   }
   cudaError_t e;
   int rc;
@@ -819,12 +844,68 @@ extern "C" size_t vadc_cdist_bwd_workspace_bytes(int nb, int64_t R, int64_t P, i
   if (n == 1)                                                                                    // split-K partials
     b += align_up((size_t)std::max(cdist_bwd_sk_tc(r1, p1, C), cdist_bwd_sk_simt(r1, p1, C)) * p1 * C * sizeof(float), 256);
   if ((C % 8) == 0 && (p1 % 8) == 0)                                                             // operand terms
-    b += tc_gemm_split_bytes((long long)(n * Rp), p1) + tc_gemm_split_bytes((long long)(n * r1), C) +
-         tc_gemm_split_bytes((long long)(n * p1), C);
+    b += tc_terms_bytes(3, (long long)(n * Rp), p1) + tc_terms_bytes(3, (long long)(n * r1), C) +
+         tc_terms_bytes(3, (long long)(n * p1), C);
   return b + 256;
 }
 
 namespace vadc {
+// (2) of cdist_bwd_impl: ga = a rho_a - r b  and  gb = b rho_b - r^T a  on the tcgen05 GEMM.  r as [nb Rp, P], a as
+//     [nb R, C], b as [nb P, C]; gb: contraction over the rows, split-K for one problem, one batched launch otherwise.
+// TERMS = 2: two fp16 terms of power-of-two-scaled operands; r has no a-priori bound, its scale comes from the measured
+// max: sc[0..2] = {s_r, s_b, 1 / (s_r s_b)} (ga; self: s_b = s_a), sc[4..6] = {s_r, s_a, 1 / (s_r s_a)} (gb); no host sync.
+// TERMS = 3: three bf16 terms per operand (fp32-faithful for any data, no scales)
+template <int TERMS>
+static int cdist_bwd_tc(const float* a, const float* b, const float* r, const float* rho_a, const float* rho_b, float* q,
+                        unsigned* bits, float* sc, int nb, long long R, long long P, int C, bool self, float* ga, float* gb,
+                        Carver& ws, cudaStream_t st) {
+  const long long Rp = cdist_bwd_rows(nb, R), PC = P * C;
+  const float* bb = self ? a : b;              // self: the one contraction is the ga form with b = a
+  const int sk = cdist_bwd_sk_tc(R, P, C);
+  void* rs = ws.take<uint8_t>(tc_terms_bytes(3, (long long)nb * Rp, P));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(3, (long long)nb * R, C));
+  void* bs = self ? as : ws.take<uint8_t>(tc_terms_bytes(3, (long long)nb * P, C));
+  const TcBatchOffsets oga{0, (int)P, (int)Rp, 0}, ogb{0, (int)Rp, 0, (int)R};
+  const TcGzEpi ega{ga, a, rho_a, nullptr, C};
+  auto at = [&](int i) -> const float* { return TERMS == 2 ? sc + i : nullptr; };
+  int rc;
+  if constexpr (TERMS == 2) {
+    if ((gb || self) && (rc = tc_absmax_bits(a, (long long)nb * R * C, bits + 1, st))) return rc;
+    if (ga && !self && (rc = tc_absmax_bits(b, (long long)nb * P * C, bits + 2, st))) return rc;
+    if (ga && (rc = tc_pair_scales(bits, 0.f, self ? bits + 1 : bits + 2, 0.f, sc, st))) return rc;
+    if (gb && (rc = tc_pair_scales(bits, 0.f, bits + 1, 0.f, sc + 4, st))) return rc;
+  }
+  if ((rc = tc_split<TERMS>(r, (long long)nb * Rp, P, at(ga ? 0 : 4), rs, st))) return rc;
+  // bf16 x3 splits a once for both contractions; fp16 x2 splits each operand with the scale of its contraction
+  if constexpr (TERMS == 3)
+    if ((gb || self) && (rc = tc_split<3>(a, (long long)nb * R, C, nullptr, as, st))) return rc;
+  if (ga) {
+    if ((TERMS == 2 || !self) && (rc = tc_split<TERMS>(bb, (long long)nb * P, C, at(1), bs, st))) return rc;
+    if (nb > 1) {
+      rc = tc_gemm<TERMS, true, false>({bs, rs, C, R, P, at(2), 1, nb, oga, (long long)nb * P, C, (long long)nb * Rp, P},
+                                       TcCdistGaTEpi{ga, a, rho_a, R, C}, st);
+    } else if constexpr (TERMS == 2) {   // fp16 x2 only: one problem with C >= 128 runs transposed (coalesced stores)
+      rc = C >= 128 ? tc_gemm<2, true, false>({bs, rs, C, R, P, sc + 2}, TcGzTEpi{ga, a, rho_a, nullptr, C}, st)
+                    : tc_gemm<2, false, true>({rs, bs, R, C, P, sc + 2}, ega, st);
+    } else {
+      rc = tc_gemm<3, false, true>({rs, bs, R, C, P}, ega, st);
+    }
+    if (rc) return rc;
+  }
+  if (gb) {
+    if constexpr (TERMS == 2)
+      if ((rc = tc_split<2>(a, (long long)nb * R, C, sc + 5, as, st))) return rc;
+    if (nb > 1)
+      return tc_gemm<TERMS, true, true>({rs, as, P, C, Rp, at(6), 1, nb, ogb, (long long)nb * Rp, P, (long long)nb * R, C},
+                                        TcSpaceGcEpi{gb, b, rho_b, PC, C, (int)P}, st);
+    if ((rc = tc_gemm<TERMS, true, true>({rs, as, P, C, R, at(6), sk}, TcPartialEpi{q, C, PC}, st))) return rc;
+    // one problem: gb = b rho_b - sum of the split-K partials
+    gcenters_finalize_kernel<<<(unsigned)((PC + 255) / 256), 256, 0, st>>>(nullptr, q, sk, b, rho_b, (int)P, C, gb);
+    VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
+  }
+  return VADC_OK;
+}
+
 static int cdist_bwd_impl(const float* a, const float* b, const float* dist, const float* g, int nb, long long R,
                           long long P, int C, bool self, float* ga, float* gb, void* workspace, size_t workspace_bytes,
                           cudaStream_t st) {
@@ -840,7 +921,6 @@ static int cdist_bwd_impl(const float* a, const float* b, const float* dist, con
   unsigned* bits = ws.take<unsigned>(64);
   float* sc = ws.take<float>(64);
   float* q = nb == 1 ? ws.take<float>((size_t)std::max(cdist_bwd_sk_tc(R, P, C), cdist_bwd_sk_simt(R, P, C)) * PC) : nullptr;
-  int rc;
   // (1) r, rho_a, max |r| in one pass over g and D; rho_b from the column partials
   VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
   float* cp = gb ? colpart : nullptr;
@@ -859,64 +939,10 @@ static int cdist_bwd_impl(const float* a, const float* b, const float* dist, con
     VADC_CHECK_LAUNCH("colsum_chunks_kernel");
   }
   const float* bb = self ? a : b;              // self: the one contraction is the ga form with b = a
-  if (cdist_bwd_tc_ok(nb, R, P, C, a, bb)) {
-    // (2) ga = a rho_a - r b  and  gb = b rho_b - r^T a  on the tcgen05 GEMM.  r as [nb Rp, P], a as [nb R, C], b as
-    //     [nb P, C]; ga: rows = channels from C = 128 up (coalesced stores), gb: contraction over the rows, split-K
-    //     for one problem, one batched launch otherwise
-    const int sk = cdist_bwd_sk_tc(R, P, C);
-    void* rs = ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * Rp, P));
-    void* as = ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * R, C));
-    void* bs = self ? as : ws.take<uint8_t>(tc_gemm_split_bytes((long long)nb * P, C));
-    const TcBatchOffsets oga{0, (int)P, (int)Rp, 0}, ogb{0, (int)Rp, 0, (int)R};
-    const TcGzEpi ega{ga, a, rho_a, nullptr, C};
-    const TcCdistGaTEpi egat{ga, a, rho_a, R, C};
-    const TcPartialEpi egbp{q, C, PC};
-    const TcSpaceGcEpi egb{gb, b, rho_b, PC, C, (int)P};
-    if (!env_on("VADC_TC_BF16X3")) {
-      // two fp16 terms of power-of-two-scaled operands; r has no a-priori bound, its scale comes from the measured max:
-      // sc[0..2] = {s_r, s_b, 1 / (s_r s_b)} (ga; self: s_b = s_a), sc[4..6] = {s_r, s_a, 1 / (s_r s_a)} (gb); no host sync
-      if ((gb || self) && (rc = tc_absmax_bits(a, (long long)nb * R * C, bits + 1, st))) return rc;
-      if (ga && !self && (rc = tc_absmax_bits(b, (long long)nb * P * C, bits + 2, st))) return rc;
-      if (ga && (rc = tc_pair_scales(bits, 0.f, self ? bits + 1 : bits + 2, 0.f, sc, st))) return rc;
-      if (gb && (rc = tc_pair_scales(bits, 0.f, bits + 1, 0.f, sc + 4, st))) return rc;
-      if ((rc = tc_split2h(r, (long long)nb * Rp, P, ga ? sc : sc + 4, rs, st))) return rc;
-      if (ga) {
-        if ((rc = tc_split2h(bb, (long long)nb * P, C, sc + 1, bs, st))) return rc;
-        if (nb > 1) rc = launch_tc_gemm_batched_h2<true, false>(bs, (long long)nb * P, C, rs, (long long)nb * Rp, P, C, R, P, nb,
-                                                                oga, sc + 2, egat, st);
-        else if (C >= 128) rc = launch_tc_gemm_ex_h2<true, false>(bs, rs, C, R, P, 1, sc + 2,
-                                                                  TcGzTEpi{ga, a, rho_a, nullptr, C}, st);
-        else rc = launch_tc_gemm_h2<true>(rs, bs, R, C, P, sc + 2, ega, st);
-        if (rc) return rc;
-      }
-      if (gb) {
-        if ((rc = tc_split2h(a, (long long)nb * R, C, sc + 5, as, st))) return rc;
-        if (nb > 1) return launch_tc_gemm_batched_h2<true, true>(rs, (long long)nb * Rp, P, as, (long long)nb * R, C, P, C, Rp, nb,
-                                                                 ogb, sc + 6, egb, st);
-        if ((rc = launch_tc_gemm_ex_h2<true, true>(rs, as, P, C, R, sk, sc + 6, egbp, st))) return rc;
-      }
-    } else {
-      // VADC_TC_BF16X3: three bf16 terms per operand (fp32-faithful for any data, no scales)
-      if ((rc = tc_split3(r, (long long)nb * Rp, P, rs, st))) return rc;
-      if ((gb || self) && (rc = tc_split3(a, (long long)nb * R, C, as, st))) return rc;
-      if (ga) {
-        if (!self && (rc = tc_split3(b, (long long)nb * P, C, bs, st))) return rc;
-        rc = nb > 1 ? launch_tc_gemm_batched<true, false>(bs, (long long)nb * P, C, rs, (long long)nb * Rp, P, C, R, P, nb, oga, egat, st)
-                    : launch_tc_gemm<true>(rs, bs, R, C, P, ega, st);
-        if (rc) return rc;
-      }
-      if (gb) {
-        if (nb > 1) return launch_tc_gemm_batched<true, true>(rs, (long long)nb * Rp, P, as, (long long)nb * R, C, P, C, Rp, nb, ogb,
-                                                              egb, st);
-        if ((rc = launch_tc_gemm_ex<true, true>(rs, as, P, C, R, sk, egbp, st))) return rc;
-      }
-    }
-    if (gb) {                    // one problem: gb = b rho_b - sum of the split-K partials
-      gcenters_finalize_kernel<<<(unsigned)((PC + 255) / 256), 256, 0, st>>>(nullptr, q, sk, b, rho_b, (int)P, C, gb);
-      VADC_CHECK_LAUNCH("gcenters_finalize_kernel");
-    }
-    return VADC_OK;
-  }
+  if (cdist_bwd_tc_ok(nb, R, P, C, a, bb))
+    return env_on("VADC_TC_BF16X3")
+               ? cdist_bwd_tc<3>(a, b, r, rho_a, rho_b, q, bits, sc, nb, R, P, C, self, ga, gb, ws, st)
+               : cdist_bwd_tc<2>(a, b, r, rho_a, rho_b, q, bits, sc, nb, R, P, C, self, ga, gb, ws, st);
   // (2') fp32 SIMT GEMM: shapes the tensor-core path does not take, and launch-bound sizes
   cudaError_t e;
   if (ga) {

@@ -76,27 +76,16 @@ centroid_prep_kernel(const float* __restrict__ centers, int K, int C, uint8_t* _
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     float v = centers[(size_t)k * C + c];
     s += v * v;
-    __nv_bfloat16 t1 = __float2bfloat16_rn(v);
-    float r1 = v - __bfloat162float(t1);
-    __nv_bfloat16 t2 = __float2bfloat16_rn(r1);
-    float r2 = r1 - __bfloat162float(t2);
-    __nv_bfloat16 t3 = __float2bfloat16_rn(r2);
+    __nv_bfloat16 t[3];
+    split_bf16x3(v, t);
     uint32_t off = (uint32_t)(c / 64) * (K * 128u) + sw128(k, (c % 64) * 2);
     const uint32_t term = (uint32_t)K * C * 2u;
-    *reinterpret_cast<__nv_bfloat16*>(image + off) = t1;
-    *reinterpret_cast<__nv_bfloat16*>(image + term + off) = t2;
-    *reinterpret_cast<__nv_bfloat16*>(image + 2 * term + off) = t3;
+    *reinterpret_cast<__nv_bfloat16*>(image + off) = t[0];
+    *reinterpret_cast<__nv_bfloat16*>(image + term + off) = t[1];
+    *reinterpret_cast<__nv_bfloat16*>(image + 2 * term + off) = t[2];
   }
   s = block_sum<float>(s, red);
   if (threadIdx.x == 0) cc[k] = s;
-}
-
-__device__ __forceinline__ void split3(float v, __nv_bfloat16& t1, __nv_bfloat16& t2, __nv_bfloat16& t3) {
-  t1 = __float2bfloat16_rn(v);
-  float r1 = v - __bfloat162float(t1);
-  t2 = __float2bfloat16_rn(r1);
-  float r2 = r1 - __bfloat162float(t2);
-  t3 = __float2bfloat16_rn(r2);
 }
 
 // packed 3-term split of two floats: one F2FP per term converts and packs both values

@@ -23,7 +23,7 @@ namespace vadc {
 // gY [2N, C] channel-last (frames 2f, 2f+1 of token frame f) -> the three bf16 terms of gYm [N, 2C]:
 // gYm[n, j*C + c] = gY[((f*2 + j)*HW + hw), c],  n = f*HW + hw
 __global__ void __launch_bounds__(256)
-split3_frames_kernel(const float* __restrict__ gy, long long N, int C, long long HW, __nv_bfloat16* __restrict__ t0) {
+split3_frames_kernel(const float* __restrict__ gy, long long N, int C, long long HW, void* __restrict__ t0) {
   const long long total4 = N * 2 * (C / 4);
   const long long term = N * 2 * C;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total4; i += (long long)gridDim.x * blockDim.x) {
@@ -34,18 +34,7 @@ split3_frames_kernel(const float* __restrict__ gy, long long N, int C, long long
     const int j = (int)(fj & 1);
     const float4 v = __ldg(reinterpret_cast<const float4*>(gy) + i);
     const float a[4] = {v.x, v.y, v.z, v.w};
-    __nv_bfloat16 h[3][4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      h[0][e] = __float2bfloat16_rn(a[e]);
-      const float r1 = a[e] - __bfloat162float(h[0][e]);
-      h[1][e] = __float2bfloat16_rn(r1);
-      h[2][e] = __float2bfloat16_rn(r1 - __bfloat162float(h[1][e]));
-    }
-    const long long o = (f * HW + hw) * 2 * C + (long long)j * C + c4 * 4;
-    *reinterpret_cast<uint2*>(t0 + o) = *reinterpret_cast<uint2*>(h[0]);
-    *reinterpret_cast<uint2*>(t0 + term + o) = *reinterpret_cast<uint2*>(h[1]);
-    *reinterpret_cast<uint2*>(t0 + 2 * term + o) = *reinterpret_cast<uint2*>(h[2]);
+    store_terms<3, 4>(t0, term, (f * HW + hw) * 2 * C + (long long)j * C + c4 * 4, a);
   }
 }
 
@@ -90,9 +79,9 @@ using namespace vadc;
 extern "C" size_t vadc_norm_timedebd_workspace_bytes(int64_t N, int C) {
   const size_t n = (size_t)(N > 0 ? N : 1);
   size_t b = 0;
-  b += tc_gemm_split_bytes((long long)n, C);              // z terms
-  b += tc_gemm_split_bytes(2 * C, C);                     // weight terms (either arrangement)
-  b += tc_gemm_split_bytes((long long)n, 2 * C);          // gYm terms (backward)
+  b += tc_terms_bytes(3, (long long)n, C);              // z terms
+  b += tc_terms_bytes(3, 2 * C, C);                     // weight terms (either arrangement)
+  b += tc_terms_bytes(3, (long long)n, 2 * C);          // gYm terms (backward)
   b += align_up(n * C * sizeof(float), 256);              // gZ (backward)
   b += align_up((size_t)timedebd_splits(N) * C * 2 * C * sizeof(float), 256);
   b += align_up((size_t)ln_bwd_blocks(N) * 2 * C * sizeof(float), 256);
@@ -113,12 +102,12 @@ extern "C" int vadc_norm_timedebd_fwd(const float* x, const float* ln_w, const f
   VADC_REQUIRE(tc_gemm_shape_ok(N, 2 * C, C, false), VADC_ERR_UNSUPPORTED);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Carver ws(workspace, workspace_bytes);
-  void* zs = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-  void* wsplit = ws.take<uint8_t>(tc_gemm_split_bytes(2 * C, C));
+  void* zs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* wsplit = ws.take<uint8_t>(tc_terms_bytes(3, 2 * C, C));
   int rc;
   if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, nullptr, mu, rstd, nullptr, st, nullptr, zs))) return rc;
-  if ((rc = tc_split3(wt, 2 * C, C, wsplit, st))) return rc;
-  return launch_tc_gemm<false>(zs, wsplit, N, 2 * C, C, TcTimeDebedEpi{out, bias, HW, C}, st);
+  if ((rc = tc_split<3>(wt, 2 * C, C, nullptr, wsplit, st))) return rc;
+  return tc_gemm<3, false, false>({zs, wsplit, N, 2 * C, C}, TcTimeDebedEpi{out, bias, HW, C}, st);
 }
 
 extern "C" int vadc_norm_timedebd_bwd(const float* x, const float* mu, const float* rstd, const float* ln_w,
@@ -140,9 +129,9 @@ extern "C" int vadc_norm_timedebd_bwd(const float* x, const float* mu, const flo
   VADC_REQUIRE(aligned16(x) && aligned16(gout) && aligned16(wk) && aligned16(gx), VADC_ERR_MISALIGNED);
   VADC_REQUIRE(workspace_bytes >= vadc_norm_timedebd_workspace_bytes(N, C), VADC_ERR_WORKSPACE);
   Carver ws(workspace, workspace_bytes);
-  void* zs = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-  void* wsplit = ws.take<uint8_t>(tc_gemm_split_bytes(2 * C, C));
-  void* gys = ws.take<uint8_t>(tc_gemm_split_bytes(N, 2 * C));
+  void* zs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* wsplit = ws.take<uint8_t>(tc_terms_bytes(3, 2 * C, C));
+  void* gys = ws.take<uint8_t>(tc_terms_bytes(3, N, 2 * C));
   float* gz = ws.take<float>((size_t)N * C);
   const int sk = timedebd_splits(N);
   float* q = ws.take<float>((size_t)sk * C * 2 * C);
@@ -154,18 +143,18 @@ extern "C" int vadc_norm_timedebd_bwd(const float* x, const float* mu, const flo
   {
     const long long total4 = (long long)N * 2 * (C / 4);
     const int grid = (int)std::min<long long>((total4 + 255) / 256, (long long)sm_count() * 8);
-    split3_frames_kernel<<<grid, 256, 0, st>>>(gout, N, C, HW, static_cast<__nv_bfloat16*>(gys));
+    split3_frames_kernel<<<grid, 256, 0, st>>>(gout, N, C, HW, gys);
     VADC_CHECK_LAUNCH("split3_frames_kernel");
     colsum32_kernel<<<(C + 31) / 32, 256, 0, st>>>(gout, 2 * (long long)N, C, gbias);
     VADC_CHECK_LAUNCH("colsum32_kernel");
   }
   // gZ [N, C] = gYm [N, 2C] . Wk^T,  Wk [C rows = ci, 2C cols = j*C + co] is the K-major B operand
-  if ((rc = tc_split3(wk, C, 2 * C, wsplit, st))) return rc;
-  if ((rc = launch_tc_gemm<false>(gys, wsplit, N, C, 2 * C, TcStoreEpi{gz, C}, st))) return rc;
+  if ((rc = tc_split<3>(wk, C, 2 * C, nullptr, wsplit, st))) return rc;
+  if ((rc = tc_gemm<3, false, false>({gys, wsplit, N, C, 2 * C}, TcStoreEpi{gz, C}, st))) return rc;
   // z again (LayerNorm of x: its terms are the A operand of the weight-gradient contraction)
   if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, nullptr, mu2, rstd2, nullptr, st, nullptr, zs))) return rc;
   // gWk [C, 2C] = Z^T gYm: both operands given as [tokens, .] (MN-major), split over the tokens
-  if ((rc = launch_tc_gemm_ex<true, true>(zs, gys, C, 2 * C, N, sk, TcPartialEpi{q, 2 * C, (long long)C * 2 * C}, st))) return rc;
+  if ((rc = tc_gemm<3, true, true>({zs, gys, C, 2 * C, N, nullptr, sk}, TcPartialEpi{q, 2 * C, (long long)C * 2 * C}, st))) return rc;
   {
     const long long n = (long long)C * 2 * C;
     sum_partials_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(q, sk, n, gwk);
@@ -189,7 +178,7 @@ static int pair_terms(const float* x, const float* ln_w, const float* ln_b, int6
   if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, z, mu, rstd, nullptr, st))) return rc;
   const long long total4 = (long long)N * (C / 4);
   const int grid = (int)std::min<long long>((total4 + 255) / 256, (long long)sm_count() * 8);
-  split3_frames_kernel<<<grid, 256, 0, st>>>(z, N / 2, C, HW, static_cast<__nv_bfloat16*>(zp));
+  split3_frames_kernel<<<grid, 256, 0, st>>>(z, N / 2, C, HW, zp);
   VADC_CHECK_LAUNCH("split3_frames_kernel");
   return VADC_OK;
 }
@@ -206,16 +195,16 @@ extern "C" int vadc_norm_timeconv_fwd(const float* x, const float* ln_w, const f
   VADC_REQUIRE(tc_gemm_shape_ok(N / 2, C, 2 * C, false), VADC_ERR_UNSUPPORTED);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Carver ws(workspace, workspace_bytes);
-  void* zp = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-  void* wsplit = ws.take<uint8_t>(tc_gemm_split_bytes(2 * C, C));
-  (void)ws.take<uint8_t>(tc_gemm_split_bytes(N, 2 * C));
+  void* zp = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* wsplit = ws.take<uint8_t>(tc_terms_bytes(3, 2 * C, C));
+  (void)ws.take<uint8_t>(tc_terms_bytes(3, N, 2 * C));
   float* z = ws.take<float>((size_t)N * C);                                  // the gZ slot of the backward
   int rc;
   if ((rc = pair_terms(x, ln_w, ln_b, N, C, HW, eps, z, mu, rstd, zp, st))) return rc;
-  if ((rc = tc_split3(wk, C, 2 * C, wsplit, st))) return rc;
+  if ((rc = tc_split<3>(wk, C, 2 * C, nullptr, wsplit, st))) return rc;
   // rows = output channels, columns = (frame pair, position): coalesced channel-last stores (a handful of rows: row form)
-  if (N / 2 >= 128) return launch_tc_gemm<false>(wsplit, zp, C, N / 2, 2 * C, TcBiasTEpi{out, bias, C}, st);
-  return launch_tc_gemm<false>(zp, wsplit, N / 2, C, 2 * C, TcBiasEpi{out, bias, C}, st);
+  if (N / 2 >= 128) return tc_gemm<3, false, false>({wsplit, zp, C, N / 2, 2 * C}, TcBiasTEpi{out, bias, C}, st);
+  return tc_gemm<3, false, false>({zp, wsplit, N / 2, C, 2 * C}, TcBiasEpi{out, bias, C}, st);
 }
 
 extern "C" int vadc_norm_timeconv_bwd(const float* x, const float* mu, const float* rstd, const float* ln_w,
@@ -237,9 +226,9 @@ extern "C" int vadc_norm_timeconv_bwd(const float* x, const float* mu, const flo
   VADC_REQUIRE(aligned16(x) && aligned16(gout) && aligned16(wk) && aligned16(gx), VADC_ERR_MISALIGNED);
   VADC_REQUIRE(workspace_bytes >= vadc_norm_timedebd_workspace_bytes(N, C), VADC_ERR_WORKSPACE);
   Carver ws(workspace, workspace_bytes);
-  void* zp = ws.take<uint8_t>(tc_gemm_split_bytes(N, C));
-  void* wsplit = ws.take<uint8_t>(tc_gemm_split_bytes(2 * C, C));
-  void* gys = ws.take<uint8_t>(tc_gemm_split_bytes(N, 2 * C));
+  void* zp = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* wsplit = ws.take<uint8_t>(tc_terms_bytes(3, 2 * C, C));
+  void* gys = ws.take<uint8_t>(tc_terms_bytes(3, N, 2 * C));
   float* gz = ws.take<float>((size_t)N * C);
   const int sk = timedebd_splits(N);
   float* q = ws.take<float>((size_t)sk * C * 2 * C);
@@ -249,15 +238,15 @@ extern "C" int vadc_norm_timeconv_bwd(const float* x, const float* mu, const flo
   float* z = ws.take<float>((size_t)N * C);
   const long long Nh = N / 2;
   int rc;
-  if ((rc = tc_split3(gout, Nh, C, gys, st))) return rc;
+  if ((rc = tc_split<3>(gout, Nh, C, nullptr, gys, st))) return rc;
   colsum32_kernel<<<(C + 31) / 32, 256, 0, st>>>(gout, Nh, C, gbias);
   VADC_CHECK_LAUNCH("colsum32_kernel");
   // gZp [N/2, 2C] = gY [N/2, C] . Wk (Wk [co rows, 2C cols] read MN-major), column half j -> the rows of frame 2f + j
-  if ((rc = tc_split3(wk, C, 2 * C, wsplit, st))) return rc;
-  if ((rc = launch_tc_gemm<true>(gys, wsplit, Nh, 2 * C, C, TcTimeDebedEpi{gz, nullptr, HW, C}, st))) return rc;
+  if ((rc = tc_split<3>(wk, C, 2 * C, nullptr, wsplit, st))) return rc;
+  if ((rc = tc_gemm<3, false, true>({gys, wsplit, Nh, 2 * C, C}, TcTimeDebedEpi{gz, nullptr, HW, C}, st))) return rc;
   // Zp again: gWk [C, 2C] = gY^T Zp, both operands given as [pair rows, .] (MN-major), split over the rows
   if ((rc = pair_terms(x, ln_w, ln_b, N, C, HW, eps, z, mu2, rstd2, zp, st))) return rc;
-  if ((rc = launch_tc_gemm_ex<true, true>(gys, zp, C, 2 * C, Nh, sk, TcPartialEpi{q, 2 * C, (long long)C * 2 * C}, st))) return rc;
+  if ((rc = tc_gemm<3, true, true>({gys, zp, C, 2 * C, Nh, nullptr, sk}, TcPartialEpi{q, 2 * C, (long long)C * 2 * C}, st))) return rc;
   {
     const long long n = (long long)C * 2 * C;
     sum_partials_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(q, sk, n, gwk);

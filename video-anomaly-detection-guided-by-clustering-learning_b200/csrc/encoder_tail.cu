@@ -195,10 +195,10 @@ extern "C" size_t vadc_downsample_gelu_workspace_bytes(int B, int Cin, int D, in
   const long long NT = (long long)std::max(B, 1) * std::max(D, 1) * std::max(H, 1) * std::max(W, 1);
   const int K4 = Cin * 4;
   size_t b = 0;
-  b += tc_gemm_split_bytes(NT, K4);                                   // A terms
-  b += tc_gemm_split_bytes(Cout, K4);                                 // W terms
+  b += tc_terms_bytes(3, NT, K4);                                   // A terms
+  b += tc_terms_bytes(3, Cout, K4);                                 // W terms
   b += align_up((size_t)NT * Cout * sizeof(float), 256);              // g_pre
-  b += tc_gemm_split_bytes(NT, Cout);                                 // g_pre terms
+  b += tc_terms_bytes(3, NT, Cout);                                 // g_pre terms
   b += align_up((size_t)NT * K4 * sizeof(float), 256);                // g_A
   b += align_up((size_t)tail_splits(NT, Cout, K4) * Cout * K4 * sizeof(float), 256);
   b += align_up((size_t)tail_colsum_chunks(NT) * Cout * sizeof(float), 256);
@@ -218,13 +218,13 @@ extern "C" int vadc_downsample_gelu_fwd(const float* x, const float* weight, con
   const long long NT = (long long)B * D * H * W;
   const int K4 = Cin * 4;
   Carver ws(workspace, workspace_bytes);
-  void* as = ws.take<uint8_t>(tc_gemm_split_bytes(NT, K4));
-  void* wsp = ws.take<uint8_t>(tc_gemm_split_bytes(Cout, K4));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(3, NT, K4));
+  void* wsp = ws.take<uint8_t>(tc_terms_bytes(3, Cout, K4));
   int rc;
   if ((rc = launch_patchify(x, B, Cin, D, H, W, as, st))) return rc;
-  if ((rc = tc_split3(weight, Cout, K4, wsp, st))) return rc;
+  if ((rc = tc_split<3>(weight, Cout, K4, nullptr, wsp, st))) return rc;
   // rows = output channels, columns = tokens: out[token, co] stored 128 contiguous bytes per warp
-  return launch_tc_gemm<false>(wsp, as, Cout, NT, K4, TcBiasGeluTEpi{out, pre, bias, Cout}, st);
+  return tc_gemm<3, false, false>({wsp, as, Cout, NT, K4}, TcBiasGeluTEpi{out, pre, bias, Cout}, st);
 }
 
 extern "C" int vadc_downsample_gelu_bwd(const float* x, const float* weight, const float* pre, const float* gout, int B,
@@ -239,10 +239,10 @@ extern "C" int vadc_downsample_gelu_bwd(const float* x, const float* weight, con
   const int K4 = Cin * 4;
   const int sk = tail_splits(NT, Cout, K4), cch = tail_colsum_chunks(NT);
   Carver ws(workspace, workspace_bytes);
-  void* as = ws.take<uint8_t>(tc_gemm_split_bytes(NT, K4));
-  void* wsp = ws.take<uint8_t>(tc_gemm_split_bytes(Cout, K4));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(3, NT, K4));
+  void* wsp = ws.take<uint8_t>(tc_terms_bytes(3, Cout, K4));
   float* gpre = ws.take<float>((size_t)NT * Cout);
-  __nv_bfloat16* gps = reinterpret_cast<__nv_bfloat16*>(ws.take<uint8_t>(tc_gemm_split_bytes(NT, Cout)));
+  __nv_bfloat16* gps = reinterpret_cast<__nv_bfloat16*>(ws.take<uint8_t>(tc_terms_bytes(3, NT, Cout)));
   float* ga = ws.take<float>((size_t)NT * K4);
   float* part = ws.take<float>((size_t)sk * Cout * K4);
   float* cpart = ws.take<float>((size_t)cch * Cout);
@@ -261,8 +261,8 @@ extern "C" int vadc_downsample_gelu_bwd(const float* x, const float* weight, con
     VADC_CHECK_LAUNCH("tail_colsum_stage2_kernel");
   }
   // g_A[token, k] = sum_co g_pre[token, co] W[co, k]: rows = k (W [Cout, K4] is the MN-major A operand), columns = tokens
-  if ((rc = tc_split3(weight, Cout, K4, wsp, st))) return rc;
-  if ((rc = launch_tc_gemm_ex<true, false>(wsp, gps, K4, NT, Cout, 1, TcStoreTEpi{ga, K4}, st))) return rc;
+  if ((rc = tc_split<3>(weight, Cout, K4, nullptr, wsp, st))) return rc;
+  if ((rc = tc_gemm<3, true, false>({wsp, gps, K4, NT, Cout}, TcStoreTEpi{ga, K4}, st))) return rc;
   {
     const size_t smem = (size_t)kPatchTok * (K4 + 1) * sizeof(float);
     if (smem > 48 * 1024) VADC_CUDA(cudaFuncSetAttribute(unpatchify_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -272,7 +272,7 @@ extern "C" int vadc_downsample_gelu_bwd(const float* x, const float* weight, con
   }
   // g_W [Cout, K4] = g_pre^T A: both operands given as [tokens, .] (MN-major), split over the tokens
   if ((rc = launch_patchify(x, B, Cin, D, H, W, as, st))) return rc;
-  if ((rc = launch_tc_gemm_ex<true, true>(gps, as, Cout, K4, NT, sk, TcPartialEpi{part, K4, (long long)Cout * K4}, st))) return rc;
+  if ((rc = tc_gemm<3, true, true>({gps, as, Cout, K4, NT, nullptr, sk}, TcPartialEpi{part, K4, (long long)Cout * K4}, st))) return rc;
   {
     const long long n = (long long)Cout * K4;
     tail_sum_partials_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part, sk, n, gweight);

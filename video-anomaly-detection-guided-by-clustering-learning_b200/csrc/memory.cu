@@ -361,11 +361,7 @@ row_softmax_top2_reg_kernel(const float* __restrict__ logits, long long N, int m
       reinterpret_cast<float4*>(orow)[i] = p;
       if (terms) {                             // the operand split of the read GEMM, written in the same pass
         const float a[4] = {p.x * 8192.0f, p.y * 8192.0f, p.z * 8192.0f, p.w * 8192.0f};
-        __half h[2][4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { h[0][j] = __float2half_rn(a[j]); h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j])); }
-        reinterpret_cast<uint2*>(terms + row * m)[i] = *reinterpret_cast<uint2*>(h[0]);
-        reinterpret_cast<uint2*>(terms + N * m + row * m)[i] = *reinterpret_cast<uint2*>(h[1]);
+        store_terms<2, 4>(terms, N * m, row * m + 4 * i, a);
       }
     }
   }
@@ -412,11 +408,7 @@ row_softmax_top2_kernel(const float* __restrict__ logits, long long N, int m,
       reinterpret_cast<float4*>(orow)[i] = p;
       if (terms) {                             // the operand split of the read GEMM, written in the same pass
         const float a[4] = {p.x * 8192.0f, p.y * 8192.0f, p.z * 8192.0f, p.w * 8192.0f};
-        __half h[2][4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { h[0][j] = __float2half_rn(a[j]); h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j])); }
-        reinterpret_cast<uint2*>(terms + row * m)[i] = *reinterpret_cast<uint2*>(h[0]);
-        reinterpret_cast<uint2*>(terms + N * m + row * m)[i] = *reinterpret_cast<uint2*>(h[1]);
+        store_terms<2, 4>(terms, N * m, row * m + 4 * i, a);
       }
     }
     if (lane == 0) {
@@ -428,14 +420,10 @@ row_softmax_top2_kernel(const float* __restrict__ logits, long long N, int m,
   for (int i = lane; i < m; i += 32) s += expf(lr[i] - b1);
   s = warp_sum(s);
   if (terms) {                                 // the operand split of the read GEMM, written in the same pass
-    __half* t0 = terms + row * m;
-    __half* t1 = t0 + N * m;
     for (int i = lane; i < m; i += 32) {
       const float p = expf(lr[i] - b1) / s;
       orow[i] = p;
-      const float ps = p * 8192.0f;
-      const __half h = __float2half_rn(ps);
-      t0[i] = h; t1[i] = __float2half_rn(ps - __half2float(h));
+      store_terms<2>(terms, N * m, row * m + i, p * 8192.0f);
     }
   } else {
     for (int i = lane; i < m; i += 32) orow[i] = expf(lr[i] - b1) / s;
@@ -813,33 +801,6 @@ sum_all_kernel(const float* __restrict__ a, long long n, double scale, float* __
 // tokens: score_memory is the A operand read MN-major ([tokens, slots] = [Kd, M]), G_r the K-major B operand
 // ([channels, tokens]).  Both are split into their operand terms with row pitches padded to eight elements (TMA: 16-byte
 // pitches) and zeros in the padding, so any m and any token count take the tensor-core path.
-template <int TERMS>
-__device__ __forceinline__ void split_terms(float a, __half (&h)[2], __nv_bfloat16 (&b)[3]) {
-  if constexpr (TERMS == 2) {
-    h[0] = __float2half_rn(a);
-    h[1] = __float2half_rn(a - __half2float(h[0]));
-  } else {
-    b[0] = __float2bfloat16_rn(a);
-    const float r1 = a - __bfloat162float(b[0]);
-    b[1] = __float2bfloat16_rn(r1);
-    b[2] = __float2bfloat16_rn(r1 - __bfloat162float(b[1]));
-  }
-}
-
-template <int TERMS>
-__device__ __forceinline__ void store_terms(void* dst, long long plane, long long i, float a) {
-  __half h[2];
-  __nv_bfloat16 b[3];
-  split_terms<TERMS>(a, h, b);
-  if constexpr (TERMS == 2) {
-    __half* o = static_cast<__half*>(dst) + i;
-    o[0] = h[0]; o[plane] = h[1];
-  } else {
-    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(dst) + i;
-    o[0] = b[0]; o[plane] = b[1]; o[2 * plane] = b[2];
-  }
-}
-
 // score_memory [N, m] -> terms [TERMS][Np][m8] of score_memory * scale (fp16 x2: scale = 2^13, bf16 x3: 1)
 template <int TERMS>
 __global__ void __launch_bounds__(256)
@@ -927,30 +888,6 @@ score_coldot_stage2_kernel(const float* __restrict__ part, int chunks, int m, fl
   }
 }
 
-template <int TERMS>
-__device__ __forceinline__ void store4_terms(void* dst, long long plane, long long i, const float (&a)[4]) {
-  if constexpr (TERMS == 2) {
-    __half h[2][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { h[0][j] = __float2half_rn(a[j]); h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j])); }
-    __half* o = static_cast<__half*>(dst) + i;
-    *reinterpret_cast<uint2*>(o) = *reinterpret_cast<uint2*>(h[0]);
-    *reinterpret_cast<uint2*>(o + plane) = *reinterpret_cast<uint2*>(h[1]);
-  } else {
-    __nv_bfloat16 b[3][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      b[0][j] = __float2bfloat16_rn(a[j]);
-      const float r1 = a[j] - __bfloat162float(b[0][j]);
-      b[1][j] = __float2bfloat16_rn(r1);
-      b[2][j] = __float2bfloat16_rn(r1 - __bfloat162float(b[1][j]));
-    }
-    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(dst) + i;
-#pragma unroll
-    for (int t = 0; t < 3; ++t) *reinterpret_cast<uint2*>(o + t * plane) = *reinterpret_cast<uint2*>(b[t]);
-  }
-}
-
 // g_s in one pass, one warp per token row, written straight as operand terms [TERMS][Np][m8] of g_s * scale[0]
 // (scale == NULL: 1; rows N..Np-1 and columns m..m8-1 zero).  Gq / Gm == NULL: that term is absent.
 // V4 > 0 (m % 4 == 0, m <= 128 V4, 16-byte aligned rows): the row of sm and Gm stays in registers between the row dot
@@ -1004,7 +941,7 @@ scores_bwd_gs_kernel(const float* __restrict__ sq, const float* __restrict__ sm,
       }
 #pragma unroll
       for (int j = 0; j < 4; ++j) a[j] *= s;
-      store4_terms<TERMS>(dst, plane, row * m8 + 4 * i, a);
+      store_terms<TERMS, 4>(dst, plane, row * m8 + 4 * i, a);
     }
   } else {
     float r = 0.f;
@@ -1042,28 +979,8 @@ rows_transpose_terms_kernel(const float* __restrict__ q, long long N, int d, lon
   const long long plane = (long long)d * Np, n = n0 + 2 * lane;
   if (n >= Np) return;                         // Np is a multiple of eight: both tokens of a pair are in or out
   for (int i = wid; i < 32 && c0 + i < d; i += 8) {
-    const float a0 = tile[i][2 * lane] * s, a1 = tile[i][2 * lane + 1] * s;
-    const long long o = (long long)(c0 + i) * Np + n;
-    if constexpr (TERMS == 2) {
-      const __half h0 = __float2half_rn(a0), h1 = __float2half_rn(a1);
-      __half2* t = reinterpret_cast<__half2*>(static_cast<__half*>(dst) + o);
-      t[0] = __halves2half2(h0, h1);
-      *reinterpret_cast<__half2*>(static_cast<__half*>(dst) + plane + o) =
-          __halves2half2(__float2half_rn(a0 - __half2float(h0)), __float2half_rn(a1 - __half2float(h1)));
-    } else {
-      __nv_bfloat16 b[2][3];
-      const float a[2] = {a0, a1};
-#pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        b[k][0] = __float2bfloat16_rn(a[k]);
-        const float r1 = a[k] - __bfloat162float(b[k][0]);
-        b[k][1] = __float2bfloat16_rn(r1);
-        b[k][2] = __float2bfloat16_rn(r1 - __bfloat162float(b[k][1]));
-      }
-      __nv_bfloat16* t = static_cast<__nv_bfloat16*>(dst) + o;
-#pragma unroll
-      for (int k = 0; k < 3; ++k) *reinterpret_cast<__nv_bfloat162*>(t + k * plane) = __halves2bfloat162(b[0][k], b[1][k]);
-    }
+    const float a[2] = {tile[i][2 * lane] * s, tile[i][2 * lane + 1] * s};
+    store_terms<TERMS, 2>(dst, plane, (long long)(c0 + i) * Np + n, a);
   }
 }
 
@@ -1192,8 +1109,70 @@ extern "C" size_t vadc_memory_score_workspace_bytes(int64_t N, int m, int d) {
   const size_t groups = std::max<size_t>((n + 31) / 32, (size_t)col_chunks(N));      // 32-token groups of the GEMM epilogue
   return align_up(n * m * sizeof(float), 256) + 2 * align_up(groups * m * sizeof(float), 256) +
          2 * align_up(((groups + 63) / 64) * m * sizeof(float), 256) +               // second level of the statistics tree
-         tc_gemm_split_bytes((long long)n, d) + tc_gemm_split_bytes(m, d) + 1024;     // operand terms of q and keys, scales
+         tc_terms_bytes(3, (long long)n, d) + tc_terms_bytes(3, m, d) + 1024;     // operand terms of q and keys, scales
 }
+
+namespace vadc {
+// q . keys^T on tcgen05 (m = 2000, d = 768 is tensor-bound: 244 flop/B).  TERMS = 3: fp32-faithful, six products.
+// TERMS = 2: two fp16 terms of the operands scaled by a power of two from their measured bounds (unit-norm rows in the
+// module: Memory.py:148, :222), three products, 22 significant bits: 2/3 of the operand bytes, half the MMAs.
+// col_stats: score_query is wanted (fp16 x2 from m = 128 up: the epilogue leaves per-32-token column statistics in
+// pmax / psum and sets have_groups)
+template <int TERMS>
+static int memory_score_tc(const float* q, const float* keys, long long N, int m, int d, bool col_stats, float* logits,
+                           float* pmax, float* psum, bool& have_groups, Carver& ws, cudaStream_t st) {
+  void* qs = ws.take<uint8_t>(tc_terms_bytes(3, N, d));
+  void* ks = ws.take<uint8_t>(tc_terms_bytes(3, m, d));
+  float* sc = nullptr;
+  int rc;
+  if constexpr (TERMS == 2) {
+    unsigned* bits = ws.take<unsigned>(64);
+    sc = ws.take<float>(64);
+    if ((rc = tc_absmax_bits(q, (long long)N * d, bits, st))) return rc;
+    if ((rc = tc_absmax_bits(keys, (long long)m * d, bits + 1, st))) return rc;
+    if ((rc = tc_pair_scales(bits, 0.f, bits + 1, 0.f, sc, st))) return rc;
+  }
+  if ((rc = tc_split<TERMS>(q, N, d, sc, qs, st))) return rc;
+  if ((rc = tc_split<TERMS>(keys, m, d, sc ? sc + 1 : nullptr, ks, st))) return rc;
+  if constexpr (TERMS == 2) {
+    // fp16 x2 only: operands swapped from m = 128 up (rows = memory slots): coalesced stores of the logits
+    if (m >= 128) {
+      have_groups = col_stats;
+      if (col_stats) return tc_gemm<2, false, false>({ks, qs, m, N, d, sc + 2}, TcLogitsColStatsTEpi{logits, m, pmax, psum}, st);
+      return tc_gemm<2, false, false>({ks, qs, m, N, d, sc + 2}, TcStoreTEpi{logits, m}, st);
+    }
+  }
+  return tc_gemm<TERMS, false, false>({qs, ks, N, m, d, sc ? sc + 2 : nullptr}, TcStoreEpi{logits, m}, st);
+}
+
+// score_memory [N,m] . keys [m,d] (keys read MN-major) on tcgen05.  fp16 x2: the softmax weights (in [0, 1],
+// Memory.py:139) scaled by 2^13 so that small weights stay normal numbers; their terms sm_terms may have been written by
+// vadc_memory_score next to score_memory, else they are split here
+template <int TERMS>
+static int memory_read_tc(const float* q, const float* score_memory, const void* sm_terms, const float* keys, long long N,
+                          int m, int d, float* updated_query, Carver& ws, cudaStream_t st) {
+  void* ss = ws.take<uint8_t>(tc_terms_bytes(3, N, m));
+  void* ks = ws.take<uint8_t>(tc_terms_bytes(3, m, d));
+  float* sc = nullptr;
+  int rc;
+  if constexpr (TERMS == 2) {
+    unsigned* bits = ws.take<unsigned>(64);
+    sc = ws.take<float>(64);
+    if ((rc = tc_absmax_bits(keys, (long long)m * d, bits, st))) return rc;
+    if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
+  }
+  if (!sm_terms) {
+    if ((rc = tc_split<TERMS>(score_memory, N, m, sc, ss, st))) return rc;
+    sm_terms = ss;
+  }
+  if ((rc = tc_split<TERMS>(keys, m, d, sc ? sc + 1 : nullptr, ks, st))) return rc;
+  if constexpr (TERMS == 2) {
+    if (d >= 128)   // fp16 x2 only: rows = channels (keys [m,d] as the MN-major A operand): coalesced output
+      return tc_gemm<2, true, false>({ks, sm_terms, d, N, m, sc + 2}, TcReadTEpi{updated_query, q, d}, st);
+  }
+  return tc_gemm<TERMS, false, true>({sm_terms, ks, N, d, m, sc ? sc + 2 : nullptr}, TcReadEpi{updated_query, q, d}, st);
+}
+}  // namespace vadc
 
 extern "C" int vadc_memory_score(const float* q, const float* keys, int64_t N, int m, int d,
                                  float* score_query, float* score_memory, float* colmax,
@@ -1217,31 +1196,11 @@ extern "C" int vadc_memory_score(const float* q, const float* keys, int64_t N, i
   bool have_groups = false;                    // the GEMM epilogue left per-32-token column statistics in pmax / psum
   if (tc_gemm_shape_ok(N, m, d, false) && !env_on("VADC_NO_TC_GEMM")) {
     // q . keys^T on tcgen05 (m = 2000, d = 768 is tensor-bound: 244 flop/B)
-    void* qs = ws.take<uint8_t>(tc_gemm_split_bytes(N, d));
-    void* ks = ws.take<uint8_t>(tc_gemm_split_bytes(m, d));
     int rc;
-    if (env_int("VADC_MEMORY_TERMS", 2) == 3) {            // fp32-faithful three-term bf16 split, six products
-      if ((rc = tc_split3(q, N, d, qs, st))) return rc;
-      if ((rc = tc_split3(keys, m, d, ks, st))) return rc;
-      if ((rc = launch_tc_gemm<false>(qs, ks, N, m, d, TcStoreEpi{logits, m}, st))) return rc;
-    } else {
-      // two fp16 terms of the operands scaled by a power of two from their measured bounds (unit-norm rows in the
-      // module: Memory.py:148, :222), three products, 22 significant bits: 2/3 of the operand bytes, half the MMAs
-      unsigned* bits = ws.take<unsigned>(64);
-      float* sc = ws.take<float>(64);
-      if ((rc = tc_absmax_bits(q, (long long)N * d, bits, st))) return rc;
-      if ((rc = tc_absmax_bits(keys, (long long)m * d, bits + 1, st))) return rc;
-      if ((rc = tc_pair_scales(bits, 0.f, bits + 1, 0.f, sc, st))) return rc;
-      if ((rc = tc_split2h(q, N, d, sc, qs, st))) return rc;
-      if ((rc = tc_split2h(keys, m, d, sc + 1, ks, st))) return rc;
-      // operands swapped from m = 128 up (rows = memory slots): coalesced stores of the logits
-      if (m >= 128) {
-        if (score_query) {
-          if ((rc = launch_tc_gemm_h2<false>(ks, qs, m, N, d, sc + 2, TcLogitsColStatsTEpi{logits, m, pmax, psum}, st))) return rc;
-          have_groups = true;
-        } else if ((rc = launch_tc_gemm_h2<false>(ks, qs, m, N, d, sc + 2, TcStoreTEpi{logits, m}, st))) return rc;
-      } else if ((rc = launch_tc_gemm_h2<false>(qs, ks, N, m, d, sc + 2, TcStoreEpi{logits, m}, st))) return rc;
-    }
+    if ((rc = env_int("VADC_MEMORY_TERMS", 2) == 3
+                  ? memory_score_tc<3>(q, keys, N, m, d, score_query != nullptr, logits, pmax, psum, have_groups, ws, st)
+                  : memory_score_tc<2>(q, keys, N, m, d, score_query != nullptr, logits, pmax, psum, have_groups, ws, st)))
+      return rc;
   } else {
     Operand Aop{q, d, 1}, Bop{keys, 1, d};
     StoreLogits epi{logits, m};
@@ -1298,7 +1257,7 @@ extern "C" int vadc_memory_score(const float* q, const float* keys, int64_t N, i
 
 extern "C" size_t vadc_memory_read_workspace_bytes(int64_t N, int m, int d) {
   size_t n = (size_t)(N > 0 ? N : 1);
-  return tc_gemm_split_bytes((long long)n, m) + tc_gemm_split_bytes(m, d) + 1024;     // operand terms of score_memory and keys, scales
+  return tc_terms_bytes(3, (long long)n, m) + tc_terms_bytes(3, m, d) + 1024;     // operand terms of score_memory and keys, scales
 }
 
 extern "C" int vadc_memory_read(const float* q, const float* score_memory, const void* score_memory_terms,
@@ -1313,28 +1272,9 @@ extern "C" int vadc_memory_read(const float* q, const float* score_memory, const
       !env_on("VADC_NO_TC_GEMM")) {
     // score_memory [N,m] . keys [m,d] (keys read MN-major) on tcgen05
     Carver ws(workspace, workspace_bytes);
-    void* ss = ws.take<uint8_t>(tc_gemm_split_bytes(N, m));
-    void* ks = ws.take<uint8_t>(tc_gemm_split_bytes(m, d));
-    int rc;
-    if (env_int("VADC_MEMORY_TERMS", 2) == 3) {
-      if ((rc = tc_split3(score_memory, N, m, ss, st))) return rc;
-      if ((rc = tc_split3(keys, m, d, ks, st))) return rc;
-      return launch_tc_gemm<true>(ss, ks, N, d, m, TcReadEpi{updated_query, q, d}, st);
-    }
-    // fp16 x2: the softmax weights (in [0, 1], Memory.py:139) scaled by 2^13 so that small weights stay normal numbers
-    unsigned* bits = ws.take<unsigned>(64);
-    float* sc = ws.take<float>(64);
-    if ((rc = tc_absmax_bits(keys, (long long)m * d, bits, st))) return rc;
-    if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
-    const void* sst = score_memory_terms;              // written by vadc_memory_score next to score_memory, or split here
-    if (!sst) {
-      if ((rc = tc_split2h(score_memory, N, m, sc, ss, st))) return rc;
-      sst = ss;
-    }
-    if ((rc = tc_split2h(keys, m, d, sc + 1, ks, st))) return rc;
-    if (d >= 128)   // rows = channels (keys [m,d] as the MN-major A operand): coalesced output
-      return launch_tc_gemm_ex_h2<true, false>(ks, sst, d, N, m, 1, sc + 2, TcReadTEpi{updated_query, q, d}, st);
-    return launch_tc_gemm_h2<true>(sst, ks, N, d, m, sc + 2, TcReadEpi{updated_query, q, d}, st);
+    return env_int("VADC_MEMORY_TERMS", 2) == 3
+               ? memory_read_tc<3>(q, score_memory, nullptr, keys, N, m, d, updated_query, ws, st)
+               : memory_read_tc<2>(q, score_memory, score_memory_terms, keys, N, m, d, updated_query, ws, st);
   }
   Operand Aop{score_memory, m, 1}, Bop{keys, d, 1};
   ReadEpilogue epi{updated_query, q, d};
@@ -1485,8 +1425,33 @@ static long long pad8(long long v) { return (v + 7) / 8 * 8; }
 extern "C" size_t vadc_memory_keys_bwd_workspace_bytes(int B, int d, int64_t HW, int m) {
   const long long Np = pad8((long long)(B > 0 ? B : 1) * (HW > 0 ? HW : 1)), m8 = pad8(m > 0 ? m : 1);
   const int dd = d > 0 ? d : 1;
-  return tc_gemm_split_bytes(Np, m8) + tc_gemm_split_bytes(dd, Np) +       // operand terms (room for three)
+  return tc_terms_bytes(3, Np, m8) + tc_terms_bytes(3, dd, Np) +       // operand terms (room for three)
          align_up((size_t)keys_bwd_splits(Np, (int)m8, dd) * m8 * dd * sizeof(float), 256) + 1024;   // partials, scales
+}
+
+// g_keys partials = score_memory^T G_r.  TERMS = 3: fp32-faithful, six products.  TERMS = 2: the softmax weights scaled
+// by 2^13 as in vadc_memory_read, G_r by the power of two of its measured bound (over the channels d..2d-1 of every batch)
+template <int TERMS>
+static int keys_bwd_tc(const float* score_memory, const float* g_updated_query, int B, int d, int64_t HW, int m, void* sms,
+                       void* gs, int sk, const TcPartialEpi& epi, Carver& ws, cudaStream_t st) {
+  const long long N = (long long)B * HW, Np = pad8(N);
+  const int m8 = (int)pad8(m);
+  const unsigned srows = (unsigned)std::min<long long>(Np, 16ll * sm_count());
+  const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
+  float* sc = nullptr;
+  int rc;
+  if constexpr (TERMS == 2) {
+    unsigned* bits = ws.take<unsigned>(64);
+    sc = ws.take<float>(64);
+    if ((rc = tc_absmax_bits_seg(g_updated_query + (long long)d * HW, (long long)d * HW, B, 2ll * d * HW, bits, st))) return rc;
+    if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
+  }
+  keys_bwd_split_scores_kernel<TERMS><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, TERMS == 2 ? 8192.0f : 1.0f, sms);
+  VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
+  keys_bwd_split_grad_kernel<TERMS><<<ggrid, 256, 0, st>>>(g_updated_query, B, 2 * d, d, d, HW, Np, sc ? sc + 1 : nullptr,
+                                                           nullptr, gs);
+  VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+  return tc_gemm<TERMS, true, false>({sms, gs, m8, d, Np, sc ? sc + 2 : nullptr, sk}, epi, st);
 }
 
 extern "C" int vadc_memory_keys_bwd(const float* score_memory, const float* g_updated_query, int B, int d, int64_t HW,
@@ -1506,32 +1471,13 @@ extern "C" int vadc_memory_keys_bwd(const float* score_memory, const float* g_up
   const int m8 = (int)pad8(m);
   const int sk = keys_bwd_splits(Np, m8, d);
   Carver ws(workspace, workspace_bytes);
-  void* sms = ws.take<uint8_t>(tc_gemm_split_bytes(Np, m8));
-  void* gs = ws.take<uint8_t>(tc_gemm_split_bytes(d, Np));
+  void* sms = ws.take<uint8_t>(tc_terms_bytes(3, Np, m8));
+  void* gs = ws.take<uint8_t>(tc_terms_bytes(3, d, Np));
   float* part = ws.take<float>((size_t)sk * m8 * d);
   const TcPartialEpi epi{part, d, (long long)m8 * d};
-  const unsigned srows = (unsigned)std::min<long long>(Np, 16ll * sm_count());
-  const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
-  int rc;
-  if (env_int("VADC_MEMORY_TERMS", 2) == 3) {            // fp32-faithful three-term bf16 split, six products
-    keys_bwd_split_scores_kernel<3><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 1.0f, sms);
-    VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
-    keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(g_updated_query, B, 2 * d, d, d, HW, Np, nullptr, nullptr, gs);
-    VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
-    rc = launch_tc_gemm_ex<true, false>(sms, gs, m8, d, Np, sk, epi, st);
-  } else {
-    // two fp16 terms: the softmax weights scaled by 2^13 as in vadc_memory_read, G_r by the power of two of its measured
-    // bound (over the channels d..2d-1 of every batch)
-    unsigned* bits = ws.take<unsigned>(64);
-    float* sc = ws.take<float>(64);
-    if ((rc = tc_absmax_bits_seg(g_updated_query + (long long)d * HW, (long long)d * HW, B, 2ll * d * HW, bits, st))) return rc;
-    if ((rc = tc_pair_scales(nullptr, 8192.0f, bits, 0.f, sc, st))) return rc;
-    keys_bwd_split_scores_kernel<2><<<srows, 256, 0, st>>>(score_memory, N, m, Np, m8, 8192.0f, sms);
-    VADC_CHECK_LAUNCH("keys_bwd_split_scores_kernel");
-    keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(g_updated_query, B, 2 * d, d, d, HW, Np, sc + 1, nullptr, gs);
-    VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
-    rc = launch_tc_gemm_ex_h2<true, false>(sms, gs, m8, d, Np, sk, sc + 2, epi, st);
-  }
+  const int rc = env_int("VADC_MEMORY_TERMS", 2) == 3
+                     ? keys_bwd_tc<3>(score_memory, g_updated_query, B, d, HW, m, sms, gs, sk, epi, ws, st)
+                     : keys_bwd_tc<2>(score_memory, g_updated_query, B, d, HW, m, sms, gs, sk, epi, ws, st);
   if (rc) return rc;
   const long long md = (long long)m * d;
   keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
@@ -1593,9 +1539,93 @@ extern "C" int vadc_memory_score_coldot(const float* score_query, const float* g
 extern "C" size_t vadc_memory_scores_bwd_workspace_bytes(int B, int d, int64_t HW, int m) {
   const long long Np = pad8((long long)(B > 0 ? B : 1) * (HW > 0 ? HW : 1)), m8 = pad8(m > 0 ? m : 1);
   const int dd = d > 0 ? d : 1;
-  return tc_gemm_split_bytes(Np, m8) + tc_gemm_split_bytes(m8, pad8(dd)) + tc_gemm_split_bytes(dd, Np) +  // terms
+  return tc_terms_bytes(3, Np, m8) + tc_terms_bytes(3, m8, pad8(dd)) + tc_terms_bytes(3, dd, Np) +  // terms
          align_up((size_t)Np * sizeof(float), 256) +                                                     // 1 / |x|
          align_up((size_t)keys_bwd_splits(Np, (int)m8, dd) * m8 * dd * sizeof(float), 256) + 1024;        // partials, scales
+}
+
+// the g_s pass and the two contractions of scores_bwd_impl.  TERMS = 3: fp32-faithful three-term bf16 split, six
+// products.  TERMS = 2: g_s scaled from the bounds of the incoming gradients (no host sync), K from its measured max, and
+// an unnormalised q (rows) from its measured max
+template <int TERMS>
+static int scores_bwd_tc(const float* query, bool rows, const float* keys, const float* score_query,
+                         const float* score_memory, const float* g_score_query, const float* g_score_memory,
+                         const float* coldot, int B, int d, int64_t HW, int m, float* g_q, float* g_keys, Carver& ws,
+                         cudaStream_t st) {
+  const long long N = (long long)B * HW, Np = pad8(N);
+  const int m8 = (int)pad8(m), d8 = (int)pad8(d);
+  const int sk = keys_bwd_splits(Np, m8, d);
+  void* gst = ws.take<uint8_t>(tc_terms_bytes(3, Np, m8));
+  void* kst = ws.take<uint8_t>(tc_terms_bytes(3, m8, d8));
+  void* qst = ws.take<uint8_t>(tc_terms_bytes(3, d, Np));
+  float* inv = ws.take<float>(Np);
+  float* part = ws.take<float>((size_t)sk * m8 * d);
+  unsigned* bits = ws.take<unsigned>(64);
+  float* sc = ws.take<float>(64);
+  auto at = [&](int i) -> const float* { return TERMS == 2 ? sc + i : nullptr; };
+  int rc;
+  if constexpr (TERMS == 2) {
+    VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
+    if (g_score_query) {
+      if ((rc = tc_absmax_bits(g_score_query, N * m, bits, st))) return rc;
+      if ((rc = tc_absmax_bits(coldot, m, bits + 2, st))) return rc;
+    }
+    if (g_score_memory && (rc = tc_absmax_bits(g_score_memory, N * m, bits + 1, st))) return rc;
+    if (g_q && (rc = tc_absmax_bits(keys, (long long)m * d, bits + 3, st))) return rc;
+    const bool q_measured = rows && g_keys;
+    if (q_measured && (rc = tc_absmax_bits(query, N * d, bits + 4, st))) return rc;
+    scores_bwd_scales_kernel<<<1, 1, 0, st>>>(bits, q_measured, sc);
+    VADC_CHECK_LAUNCH("scores_bwd_scales_kernel");
+  }
+  {
+    const unsigned rg = (unsigned)((Np + 7) / 8);
+    const bool regs = (m % 4) == 0 && m <= 2048 && (!score_query || aligned16(score_query)) &&
+                      (!score_memory || aligned16(score_memory)) && (!g_score_query || aligned16(g_score_query)) &&
+                      (!g_score_memory || aligned16(g_score_memory)) && (!coldot || aligned16(coldot));
+    const float* sq = g_score_query ? score_query : nullptr;
+    const int V4 = !regs ? 0 : (m <= 512 ? 4 : (m <= 1024 ? 8 : 16));
+#define VADC_GS_LAUNCH(V)                                                                                              \
+  scores_bwd_gs_kernel<TERMS, V><<<rg, 256, 0, st>>>(sq, score_memory, g_score_query, g_score_memory, coldot, N, m, Np, \
+                                                     m8, at(0), gst)
+    if (V4 == 4) VADC_GS_LAUNCH(4); else if (V4 == 8) VADC_GS_LAUNCH(8);
+    else if (V4 == 16) VADC_GS_LAUNCH(16); else VADC_GS_LAUNCH(0);
+#undef VADC_GS_LAUNCH
+    VADC_CHECK_LAUNCH("scores_bwd_gs_kernel");
+  }
+  if (g_q) {
+    // g_q = g_s [Np, m8] . K [m8, d8].  Channel-first query: rows = tokens (g_s the K-major A operand, K the MN-major B),
+    // stored into [B, d, HW].  Channel-last (rows): rows = channels (K the MN-major A operand, g_s the K-major B), stored
+    // into [N, d] one 128-byte line of a token row per warp.
+    const unsigned kr = (unsigned)std::min<long long>(m8, 16ll * sm_count());
+    scores_bwd_split_keys_kernel<TERMS><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, at(1), kst);
+    VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
+    rc = rows ? tc_gemm<TERMS, true, false>({kst, gst, d8, Np, m8, at(2)}, ScoresQRowsTEpi{g_q, N, d}, st)
+              : tc_gemm<TERMS, false, true>({gst, kst, Np, d8, m8, at(2)}, ScoresQhatEpi{g_q, N, HW, d}, st);
+    if (rc) return rc;
+  }
+  if (g_keys) {
+    // g_keys [m8, d] += g_s^T q: g_s [Np, m8] the MN-major A operand, q^T [d, Np] (K-major B) written straight from the
+    // query (channel-first: times 1 / |x|, i.e. q-hat; rows: one transposing pass); split-K over the tokens, the
+    // partials then added to g_keys in slot order
+    if (rows) {
+      const dim3 tgrid((unsigned)((Np + 63) / 64), (unsigned)((d + 31) / 32));
+      rows_transpose_terms_kernel<TERMS><<<tgrid, 256, 0, st>>>(query, N, d, Np, at(3), qst);
+      VADC_CHECK_LAUNCH("rows_transpose_terms_kernel");
+    } else {
+      query_norm_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, st>>>(query, d, HW, inv);
+      VADC_CHECK_LAUNCH("query_norm_kernel");
+      const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
+      keys_bwd_split_grad_kernel<TERMS><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, at(3), inv, qst);
+      VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
+    }
+    if ((rc = tc_gemm<TERMS, true, false>({gst, qst, m8, d, Np, at(4), sk}, TcPartialEpi{part, d, (long long)m8 * d}, st)))
+      return rc;
+    const long long md = (long long)m * d;
+    keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
+        part, sk, (long long)m8 * d, md, true, g_keys);
+    VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
+  }
+  return VADC_OK;
 }
 
 // shared by vadc_memory_scores_bwd (query [B, d, HW], normalised where its operand terms are written) and
@@ -1616,101 +1646,12 @@ static int scores_bwd_impl(const float* query, bool rows, const float* keys, con
   if (!vadc_device_ok()) return VADC_ERR_NO_DEVICE;
   if (B == 0) return VADC_OK;                            // no tokens: nothing to add to g_keys, g_q is empty
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const long long N = (long long)B * HW, Np = pad8(N);
-  const int m8 = (int)pad8(m), d8 = (int)pad8(d);
-  const int sk = keys_bwd_splits(Np, m8, d);
-  const bool three = env_int("VADC_MEMORY_TERMS", 2) == 3;   // fp32-faithful three-term bf16 split, six products
   Carver ws(workspace, workspace_bytes);
-  void* gst = ws.take<uint8_t>(tc_gemm_split_bytes(Np, m8));
-  void* kst = ws.take<uint8_t>(tc_gemm_split_bytes(m8, d8));
-  void* qst = ws.take<uint8_t>(tc_gemm_split_bytes(d, Np));
-  float* inv = ws.take<float>(Np);
-  float* part = ws.take<float>((size_t)sk * m8 * d);
-  unsigned* bits = ws.take<unsigned>(64);
-  float* sc = ws.take<float>(64);
-  int rc;
-  if (!three) {
-    // fp16 x2: g_s scaled from the bounds of the incoming gradients (no host sync), K from its measured max, and an
-    // unnormalised q (rows) from its measured max
-    VADC_CUDA(cudaMemsetAsync(bits, 0, 4 * sizeof(unsigned), st));
-    if (g_score_query) {
-      if ((rc = tc_absmax_bits(g_score_query, N * m, bits, st))) return rc;
-      if ((rc = tc_absmax_bits(coldot, m, bits + 2, st))) return rc;
-    }
-    if (g_score_memory && (rc = tc_absmax_bits(g_score_memory, N * m, bits + 1, st))) return rc;
-    if (g_q && (rc = tc_absmax_bits(keys, (long long)m * d, bits + 3, st))) return rc;
-    const bool q_measured = rows && g_keys;
-    if (q_measured && (rc = tc_absmax_bits(query, N * d, bits + 4, st))) return rc;
-    scores_bwd_scales_kernel<<<1, 1, 0, st>>>(bits, q_measured, sc);
-    VADC_CHECK_LAUNCH("scores_bwd_scales_kernel");
-  }
-  const float* s_g = three ? nullptr : sc;
-  {
-    const unsigned rg = (unsigned)((Np + 7) / 8);
-    const bool regs = (m % 4) == 0 && m <= 2048 && (!score_query || aligned16(score_query)) &&
-                      (!score_memory || aligned16(score_memory)) && (!g_score_query || aligned16(g_score_query)) &&
-                      (!g_score_memory || aligned16(g_score_memory)) && (!coldot || aligned16(coldot));
-    const float* sq = g_score_query ? score_query : nullptr;
-    const int V4 = !regs ? 0 : (m <= 512 ? 4 : (m <= 1024 ? 8 : 16));
-#define VADC_GS_LAUNCH(T, V)                                                                                       \
-  scores_bwd_gs_kernel<T, V><<<rg, 256, 0, st>>>(sq, score_memory, g_score_query, g_score_memory, coldot, N, m, Np, \
-                                                 m8, s_g, gst)
-    if (three) {
-      if (V4 == 4) VADC_GS_LAUNCH(3, 4); else if (V4 == 8) VADC_GS_LAUNCH(3, 8);
-      else if (V4 == 16) VADC_GS_LAUNCH(3, 16); else VADC_GS_LAUNCH(3, 0);
-    } else {
-      if (V4 == 4) VADC_GS_LAUNCH(2, 4); else if (V4 == 8) VADC_GS_LAUNCH(2, 8);
-      else if (V4 == 16) VADC_GS_LAUNCH(2, 16); else VADC_GS_LAUNCH(2, 0);
-    }
-#undef VADC_GS_LAUNCH
-    VADC_CHECK_LAUNCH("scores_bwd_gs_kernel");
-  }
-  if (g_q) {
-    // g_q = g_s [Np, m8] . K [m8, d8].  Channel-first query: rows = tokens (g_s the K-major A operand, K the MN-major B),
-    // stored into [B, d, HW].  Channel-last (rows): rows = channels (K the MN-major A operand, g_s the K-major B), stored
-    // into [N, d] one 128-byte line of a token row per warp.
-    const unsigned kr = (unsigned)std::min<long long>(m8, 16ll * sm_count());
-    if (three) {
-      scores_bwd_split_keys_kernel<3><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, nullptr, kst);
-      VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
-      rc = rows ? launch_tc_gemm_ex<true, false>(kst, gst, d8, Np, m8, 1, ScoresQRowsTEpi{g_q, N, d}, st)
-                : launch_tc_gemm_ex<false, true>(gst, kst, Np, d8, m8, 1, ScoresQhatEpi{g_q, N, HW, d}, st);
-    } else {
-      scores_bwd_split_keys_kernel<2><<<kr, 256, 0, st>>>(keys, m, d, m8, d8, sc + 1, kst);
-      VADC_CHECK_LAUNCH("scores_bwd_split_keys_kernel");
-      rc = rows ? launch_tc_gemm_ex_h2<true, false>(kst, gst, d8, Np, m8, 1, sc + 2, ScoresQRowsTEpi{g_q, N, d}, st)
-                : launch_tc_gemm_ex_h2<false, true>(gst, kst, Np, d8, m8, 1, sc + 2, ScoresQhatEpi{g_q, N, HW, d}, st);
-    }
-    if (rc) return rc;
-  }
-  if (g_keys) {
-    // g_keys [m8, d] += g_s^T q: g_s [Np, m8] the MN-major A operand, q^T [d, Np] (K-major B) written straight from the
-    // query (channel-first: times 1 / |x|, i.e. q-hat; rows: one transposing pass); split-K over the tokens, the
-    // partials then added to g_keys in slot order
-    const float* s_q = three ? nullptr : sc + 3;
-    if (rows) {
-      const dim3 tgrid((unsigned)((Np + 63) / 64), (unsigned)((d + 31) / 32));
-      if (three) rows_transpose_terms_kernel<3><<<tgrid, 256, 0, st>>>(query, N, d, Np, s_q, qst);
-      else rows_transpose_terms_kernel<2><<<tgrid, 256, 0, st>>>(query, N, d, Np, s_q, qst);
-      VADC_CHECK_LAUNCH("rows_transpose_terms_kernel");
-    } else {
-      query_norm_kernel<<<dim3((unsigned)((HW + 31) / 32), B), 256, 0, st>>>(query, d, HW, inv);
-      VADC_CHECK_LAUNCH("query_norm_kernel");
-      const dim3 ggrid((unsigned)((HW + (Np - N) + 255) / 256), (unsigned)d, (unsigned)B);
-      if (three) keys_bwd_split_grad_kernel<3><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, s_q, inv, qst);
-      else keys_bwd_split_grad_kernel<2><<<ggrid, 256, 0, st>>>(query, B, d, 0, d, HW, Np, s_q, inv, qst);
-      VADC_CHECK_LAUNCH("keys_bwd_split_grad_kernel");
-    }
-    const TcPartialEpi epi{part, d, (long long)m8 * d};
-    if (three) rc = launch_tc_gemm_ex<true, false>(gst, qst, m8, d, Np, sk, epi, st);
-    else rc = launch_tc_gemm_ex_h2<true, false>(gst, qst, m8, d, Np, sk, sc + 4, epi, st);
-    if (rc) return rc;
-    const long long md = (long long)m * d;
-    keys_bwd_sum_partials_kernel<<<(unsigned)std::min<long long>((md + 255) / 256, 8ll * sm_count()), 256, 0, st>>>(
-        part, sk, (long long)m8 * d, md, true, g_keys);
-    VADC_CHECK_LAUNCH("keys_bwd_sum_partials_kernel");
-  }
-  return VADC_OK;
+  return env_int("VADC_MEMORY_TERMS", 2) == 3
+             ? scores_bwd_tc<3>(query, rows, keys, score_query, score_memory, g_score_query, g_score_memory, coldot, B, d, HW,
+                                m, g_q, g_keys, ws, st)
+             : scores_bwd_tc<2>(query, rows, keys, score_query, score_memory, g_score_query, g_score_memory, coldot, B, d, HW,
+                                m, g_q, g_keys, ws, st);
 }
 
 extern "C" int vadc_memory_scores_bwd(const float* query, const float* keys, const float* score_query,

@@ -5,6 +5,7 @@
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
 #include "common.cuh"
+#include "tc_terms.cuh"
 
 namespace vadc {
 
@@ -72,29 +73,10 @@ ln_rows_kernel(const float* __restrict__ x, const float* __restrict__ w, const f
       }
       if (split && hscale) {
         const float a[4] = {o.x * hs, o.y * hs, o.z * hs, o.w * hs};
-        __half h[2][4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          h[0][j] = __float2half_rn(a[j]);
-          h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j]));
-        }
-        uint2* sp = reinterpret_cast<uint2*>(split + row * C) + c4;
-        sp[0] = *reinterpret_cast<uint2*>(h[0]);
-        sp[term / 4] = *reinterpret_cast<uint2*>(h[1]);
+        store_terms<2, 4>(split, term, row * C + 4 * c4, a);
       } else if (split) {
         const float a[4] = {o.x, o.y, o.z, o.w};
-        __nv_bfloat16 h[3][4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          h[0][j] = __float2bfloat16_rn(a[j]);
-          const float r1 = a[j] - __bfloat162float(h[0][j]);
-          h[1][j] = __float2bfloat16_rn(r1);
-          h[2][j] = __float2bfloat16_rn(r1 - __bfloat162float(h[1][j]));
-        }
-        uint2* sp = reinterpret_cast<uint2*>(split + row * C) + c4;
-        sp[0] = *reinterpret_cast<uint2*>(h[0]);
-        sp[term / 4] = *reinterpret_cast<uint2*>(h[1]);
-        sp[term / 2] = *reinterpret_cast<uint2*>(h[2]);
+        store_terms<3, 4>(split, term, row * C + 4 * c4, a);
       }
     }
   }
@@ -198,12 +180,7 @@ softmin_rows_kernel(const float* __restrict__ D, long long R, int K, int k_valid
       ar[i] = a;
       if (terms) {                          // the operand split of the x_rec GEMM, written in the same pass
         const float b[4] = {a.x * sa, a.y * sa, a.z * sa, a.w * sa};
-        __half h[2][4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { h[0][j] = __float2half_rn(b[j]); h[1][j] = __float2half_rn(b[j] - __half2float(h[0][j])); }
-        uint2* t = reinterpret_cast<uint2*>(terms + row * K) + i;
-        t[0] = *reinterpret_cast<uint2*>(h[0]);
-        reinterpret_cast<uint2*>(terms + R * K + row * K)[i] = *reinterpret_cast<uint2*>(h[1]);
+        store_terms<2, 4>(terms, R * K, row * K + 4 * i, b);
       }
       l += (da_sq(v.x, a.x) + da_sq(v.y, a.y)) + (da_sq(v.z, a.z) + da_sq(v.w, a.w));
     }

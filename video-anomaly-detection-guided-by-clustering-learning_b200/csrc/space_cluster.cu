@@ -48,12 +48,7 @@ ln_transpose_kernel(const float* __restrict__ x, const float* __restrict__ w,
       const float v = tile[lane * ld + c];
       const long long i = (long long)c * T + row;
       if (zt) zt[i] = v;
-      if (terms) {                                // the operand split of the batched tcgen05 GEMM, written in the same pass
-        const __nv_bfloat16 h0 = __float2bfloat16_rn(v);
-        const float r1 = v - __bfloat162float(h0);
-        const __nv_bfloat16 h1 = __float2bfloat16_rn(r1);
-        terms[i] = h0; terms[n + i] = h1; terms[2 * n + i] = __float2bfloat16_rn(r1 - __bfloat162float(h1));
-      }
+      if (terms) store_terms<3>(terms, n, i, v);  // the operand split of the batched tcgen05 GEMM, written in the same pass
     }
   }
 }
@@ -532,6 +527,21 @@ extern "C" size_t vadc_space_cluster_fwd_workspace_bytes(int64_t M, int P, int C
   return b + 256;
 }
 
+// the forward's batched distance GEMM (batch c: A = zt[c] [M,P], B = centers[c]^T; out Ds[m, c, k]) and, from the same
+// terms and norms, cdist(centers, centers) (model/cluster.py:134); fp16 x2 scales in sc (tc_fwd_scales_from_bits)
+template <int TERMS>
+static int space_dist_tc(const void* zs, const float* centers, void* cs, const float* sc, int64_t M, int P, int C, int K,
+                         const float* zz, const float* cc, float* Ds, float* selfdist, cudaStream_t st) {
+  const long long CM = (long long)C * M, CK = (long long)C * K;
+  int rc;
+  if ((rc = tc_split<TERMS>(centers, CK, P, TERMS == 2 ? sc + 1 : nullptr, cs, st))) return rc;
+  if ((rc = tc_gemm<TERMS, false, false>({zs, cs, M, K, P, TERMS == 2 ? sc + 2 : nullptr, 1, C, {(int)M, 0, K, 0}, CM, P, CK, P},
+                                         TcBatchDistEpi{Ds, zz, cc, CK, K, M, K}, st))) return rc;
+  if (!selfdist) return VADC_OK;
+  return tc_gemm<TERMS, false, false>({cs, cs, K, K, P, TERMS == 2 ? sc + 5 : nullptr, 1, C, {K, 0, K, 0}, CK, P, CK, P},
+                                      TcBatchDistEpi{selfdist, cc, cc, K, (long long)K * K, K, K}, st);
+}
+
 static int space_cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b,
                                   const float* centers, int64_t M, int P, int C, int K, int k_valid,
                                   float alpha, float eps, float* Ds, float* As, float* selfdist, void* zt_state,
@@ -587,23 +597,8 @@ static int space_cluster_fwd_impl(const float* x, const float* ln_w, const float
     if ((rc = launch_row_sqnorm(centers, (long long)C * K, P, cc, st))) return rc;
     // batch c: A = zt[c] [M,P], B = centers[c]^T; out Ds[m, c, k]
     if (tc) {
-      TcBatchDistEpi epi{Ds, zz, cc, (long long)C * K, K, M, K};
-      TcBatchDistEpi eps_{selfdist, cc, cc, K, (long long)K * K, K, K};
-      const TcBatchOffsets od{(int)M, 0, K, 0}, os{K, 0, K, 0};
-      if (nt == 2) {
-        if ((rc = tc_split2h(centers, (long long)C * K, P, sc + 1, cs, st))) return rc;
-        if ((rc = launch_tc_gemm_batched_h2<false, false>(zs, (long long)C * M, P, cs, (long long)C * K, P, M, K, P, C, od,
-                                                          sc + 2, epi, st))) return rc;
-        // cdist(centers, centers) (model/cluster.py:134) from the same terms and norms
-        if (selfdist && (rc = launch_tc_gemm_batched_h2<false, false>(cs, (long long)C * K, P, cs, (long long)C * K, P, K, K, P, C,
-                                                                      os, sc + 5, eps_, st))) return rc;
-      } else {
-        if ((rc = tc_split3(centers, (long long)C * K, P, cs, st))) return rc;
-        if ((rc = launch_tc_gemm_batched<false, false>(zs, (long long)C * M, P, cs, (long long)C * K, P, M, K, P, C, od, epi, st)))
-          return rc;
-        if (selfdist && (rc = launch_tc_gemm_batched<false, false>(cs, (long long)C * K, P, cs, (long long)C * K, P, K, K, P, C,
-                                                                   os, eps_, st))) return rc;
-      }
+      if ((rc = nt == 2 ? space_dist_tc<2>(zs, centers, cs, sc, M, P, C, K, zz, cc, Ds, selfdist, st)
+                        : space_dist_tc<3>(zs, centers, cs, sc, M, P, C, K, zz, cc, Ds, selfdist, st))) return rc;
       selfdist_done = true;
     } else {
       Operand Aop{zt, P, 1}, Bop{centers, 1, P};
@@ -648,9 +643,32 @@ extern "C" size_t vadc_space_cluster_bwd_workspace_bytes(int64_t M, int P, int C
   b += align_up((size_t)space_colsum_chunks(M, (long long)C * K) * C * K * sizeof(float), 256);
   b += align_up((size_t)C * K * sizeof(float), 256);                   // rcol
   b += align_up((size_t)std::max(space_ln_bwd_blocks(M * (int64_t)P, C, true), space_ln_bwd_blocks(M * (int64_t)P, C, false)) * 2 * C * sizeof(float), 256);
-  if ((P % 8) == 0 && (K % 64) == 0) b += tc_gemm_split_bytes((long long)m, (long long)C * K) + 512;     // r terms, scales
+  if ((P % 8) == 0 && (K % 64) == 0) b += tc_terms_bytes(3, (long long)m, (long long)C * K) + 512;     // r terms, scales
   return b + 512;
 }
+
+namespace vadc {
+// the backward's two batched contractions on the tcgen05 GEMM (terms of zt and centers from the forward, r split here);
+// fp16 x2: r has no a-priori bound, its scale comes from its measured max (device-side, no host sync)
+template <int TERMS>
+static int space_bwd_tc(const float* r, void* rs, const unsigned* rbits, const float* fsc, const void* zs, const void* cs,
+                        const float* centers, int64_t M, int P, int C, int K, float* gzt, const float* rcol, float* gcenters,
+                        Carver& ws, cudaStream_t st) {
+  const float* bsc = nullptr;
+  int rc;
+  if constexpr (TERMS == 2) {
+    float* s = ws.take<float>(64);
+    if ((rc = tc_space_bwd_scales(rbits, fsc, s, st))) return rc;
+    bsc = s;
+  }
+  if ((rc = tc_split<TERMS>(r, M, (long long)C * K, bsc, rs, st))) return rc;
+  // gzt <- r centers; the LayerNorm backward forms zt rsum - that
+  if ((rc = tc_gemm<TERMS, true, false>({cs, rs, P, M, K, bsc ? bsc + 1 : nullptr, 1, C, {0, K, 0, K}, (long long)C * K, P, M,
+                                         (long long)C * K}, TcSpaceGzEpi{gzt, (long long)M * P, P}, st))) return rc;
+  return tc_gemm<TERMS, true, true>({rs, zs, K, P, M, bsc ? bsc + 2 : nullptr, 1, C, {K, 0, 0, (int)M}, M, (long long)C * K,
+                                     (long long)C * M, P}, TcSpaceGcEpi{gcenters, centers, rcol, (long long)K * P, P, K}, st);
+}
+}  // namespace vadc
 
 extern "C" int vadc_space_cluster_bwd(const float* x, const float* mu, const float* rstd,
                                       const void* zt_state, const float* ln_w, const float* ln_b,
@@ -688,32 +706,15 @@ extern "C" int vadc_space_cluster_bwd(const float* x, const float* mu, const flo
     //   acc[c]^T = centers[c]^T r[:,c,:]^T   (gzt = zt rsum - acc is formed by the LayerNorm backward)   rows = positions p:
     //                                        A = centers MN-major, B = r K-major
     //   gcenters[c] = centers[c] rcol[c] - r[:,c,:]^T zt[c]    A MN-major (window offset along m), B MN-major
-    void* rs = ws.take<uint8_t>(tc_gemm_split_bytes(M, (long long)C * K));
+    void* rs = ws.take<uint8_t>(tc_terms_bytes(3, M, (long long)C * K));
     const int nt = space_nt(C);
     const void* zs = zt_state;
     const uint8_t* cs = static_cast<const uint8_t*>(zt_state) + space_zt_bytes(M, P, C);
     const float* fsc = reinterpret_cast<const float*>(cs + space_cen_bytes(P, C, K));
-    TcSpaceGzEpi egz{gzt, T, P};                   // gzt <- r centers; the LayerNorm backward below forms zt rsum - that
-    TcSpaceGcEpi egc{gcenters, centers, rcol, (long long)K * P, P, K};
-    const TcBatchOffsets oz{0, K, 0, K}, oc{K, 0, 0, (int)M};
     e = launch_space_colsum(r, M, C * K, cpart, rcol, st);
     if (e != cudaSuccess) return record_cuda_error(e, "space colsum r");
-    if (nt == 2) {
-      // r has no a-priori bound: scale from its measured max (device-side, no host sync)
-      float* bsc = ws.take<float>(64);
-      if ((rc = tc_space_bwd_scales(rbits, fsc, bsc, st))) return rc;
-      if ((rc = tc_split2h(r, M, (long long)C * K, bsc, rs, st))) return rc;
-      if ((rc = launch_tc_gemm_batched_h2<true, false>(cs, (long long)C * K, P, rs, M, (long long)C * K, P, M, K, C, oz, bsc + 1,
-                                                       egz, st))) return rc;
-      if ((rc = launch_tc_gemm_batched_h2<true, true>(rs, M, (long long)C * K, zs, (long long)C * M, P, K, P, M, C, oc, bsc + 2,
-                                                      egc, st))) return rc;
-    } else {
-      if ((rc = tc_split3(r, M, (long long)C * K, rs, st))) return rc;
-      if ((rc = launch_tc_gemm_batched<true, false>(cs, (long long)C * K, P, rs, M, (long long)C * K, P, M, K, C, oz, egz, st)))
-        return rc;
-      if ((rc = launch_tc_gemm_batched<true, true>(rs, M, (long long)C * K, zs, (long long)C * M, P, K, P, M, C, oc, egc, st)))
-        return rc;
-    }
+    if ((rc = nt == 2 ? space_bwd_tc<2>(r, rs, rbits, fsc, zs, cs, centers, M, P, C, K, gzt, rcol, gcenters, ws, st)
+                      : space_bwd_tc<3>(r, rs, rbits, fsc, zs, cs, centers, M, P, C, K, gzt, rcol, gcenters, ws, st))) return rc;
   } else {
     const float* zt = static_cast<const float*>(zt_state);
     // gzt[c] = zt[c] * rsum[:,c] - r[:,c,:] @ centers[c]

@@ -5,8 +5,8 @@
 //
 //   C[m,n] = sum_k A[m,k] B(n,k)      A [M,Kd] row-major;  B [N,Kd] row-major (K-major) or [Kd,N] row-major (MN-major)
 //
-// fp32 inputs are first split into THREE bf16 terms v = t0 + t1 + t2 (exact: 3 x 8 mantissa bits),
-// written once as bf16 matrices of the same layout (split3_kernel: 6 bytes per element of workspace);
+// fp32 inputs are first split into THREE bf16 terms v = t0 + t1 + t2 (exact: 3 x 8 mantissa bits; tc_terms.cuh),
+// written once as bf16 matrices of the same layout (6 bytes per element of workspace);
 // the GEMM keeps the six products t0t0, t0t1, t1t0, t0t2, t1t1, t2t0 in the fp32 TMEM accumulator
 // (dropped terms <= 2^-24 relative), which is what keeps argmin bit-exact against the fp32 reference.
 //
@@ -31,23 +31,15 @@ namespace tg {
 constexpr int BM = 128, BK = 64;
 constexpr int kThreads = 320;            // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue
 
+// fp32 [n4 * 4] -> its TERMS term planes (tc_terms.cuh); fp16 x2: of src * scale[0]
+template <int TERMS>
 __global__ void __launch_bounds__(256)
-split3_kernel(const float* __restrict__ src, long long n4, __nv_bfloat16* __restrict__ t0,
-              __nv_bfloat16* __restrict__ t1, __nv_bfloat16* __restrict__ t2) {
+split_kernel(const float* __restrict__ src, long long n4, const float* __restrict__ scale, void* __restrict__ dst) {
+  const float s = TERMS == 2 ? __ldg(scale) : 1.0f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
     const float4 v = reinterpret_cast<const float4*>(src)[i];
-    const float a[4] = {v.x, v.y, v.z, v.w};
-    __nv_bfloat16 h[3][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      h[0][j] = __float2bfloat16_rn(a[j]);
-      const float r1 = a[j] - __bfloat162float(h[0][j]);
-      h[1][j] = __float2bfloat16_rn(r1);
-      h[2][j] = __float2bfloat16_rn(r1 - __bfloat162float(h[1][j]));
-    }
-    reinterpret_cast<uint2*>(t0)[i] = *reinterpret_cast<uint2*>(h[0]);
-    reinterpret_cast<uint2*>(t1)[i] = *reinterpret_cast<uint2*>(h[1]);
-    reinterpret_cast<uint2*>(t2)[i] = *reinterpret_cast<uint2*>(h[2]);
+    const float a[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
+    store_terms<TERMS, 4>(dst, 4 * n4, 4 * i, a);
   }
 }
 
@@ -265,98 +257,97 @@ bool tc_gemm_shape_ok(long long M, long long N, long long Kd, bool b_mn) {
   return vadc_device_ok() != 0;
 }
 
-size_t tc_gemm_split_bytes(long long rows, long long cols) {
-  return align_up((size_t)3 * rows * cols * sizeof(__nv_bfloat16), 256);
+size_t tc_terms_bytes(int terms, long long rows, long long cols) {
+  return align_up((size_t)terms * rows * cols * sizeof(uint16_t), 256);
 }
 
-int tc_split3(const float* src, long long rows, long long cols, void* dst, cudaStream_t st) {
+template <int TERMS>
+int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st) {
+  static_assert(TERMS == 2 || TERMS == 3, "operand terms: fp16 x2 or bf16 x3");
   const long long n = rows * cols;
   if (n % 4) return VADC_ERR_BAD_SHAPE;
-  __nv_bfloat16* t0 = static_cast<__nv_bfloat16*>(dst);
+  if (TERMS == 2 && !scale) return VADC_ERR_NULL_POINTER;
   const long long n4 = n / 4;
   const int grid = (int)std::min<long long>((n4 + 255) / 256, (long long)sm_count() * 8);
-  tg::split3_kernel<<<grid, 256, 0, st>>>(src, n4, t0, t0 + n, t0 + 2 * n);
-  VADC_CHECK_LAUNCH("split3_kernel");
+  tg::split_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst);
+  VADC_CHECK_LAUNCH("split_kernel");
   return VADC_OK;
 }
+template int tc_split<2>(const float*, long long, long long, const float*, void*, cudaStream_t);
+template int tc_split<3>(const float*, long long, long long, const float*, void*, cudaStream_t);
 
-// The launch of every front-end: nz slices along z of an [M, N] output on min(work items, SMs) persistent CTAs with three
-// 64 KB (fp16 x2) or two 96 KB (bf16 x3) operand stages.  The split matrices are a_rows x a_cols and b_rows x b_cols
-// (MN-major: [Kd rows, M / N cols], boxes of 64 k-rows x 64 cols; K-major: [M / N rows, Kd cols], boxes of 128 rows x
-// 64 k-cols).  kb_per_split > 0: split-K slots of kb_per_split k-blocks; 0: nz problems, operands zo further along.
+// nz work slices along z of an [M, N] output on min(work items, SMs) persistent CTAs with three 64 KB (fp16 x2) or two
+// 96 KB (bf16 x3) operand stages.  Split matrices MN-major: [Kd rows, M / N cols], boxes of 64 k-rows x 64 cols; K-major:
+// [M / N rows, Kd cols], boxes of 128 rows x 64 k-cols.  Split-K: kb_per_split k-blocks per slot; batched: 0.
 template <int TERMS, bool A_MN, bool B_MN, class Epi>
-static int launch_tc_gemm_t(const void* a_split, long long a_rows, long long a_cols, const void* b_split, long long b_rows,
-                            long long b_cols, long long M, long long N, long long Kd, int nz, int kb_per_split,
-                            TcBatchOffsets zo, const float* acc_scale, Epi epi, cudaStream_t st) {
+int tc_gemm(const TcGemm& g, Epi epi, cudaStream_t st) {
   constexpr int BN = 128, kStages = TERMS == 2 ? 3 : 2;
-  if (TERMS == 2 && !acc_scale) return VADC_ERR_NULL_POINTER;
+  if (TERMS == 2 && !g.acc_scale) return VADC_ERR_NULL_POINTER;
+  if (g.nbatch < 1 || g.nbatch > 65535) return VADC_ERR_UNSUPPORTED;
+  const int splits = g.splits < 1 ? 1 : g.splits;
+  if (splits > 1 && g.nbatch > 1) return VADC_ERR_UNSUPPORTED;
+  const long long M = g.M, N = g.N, Kd = g.Kd;
+  const int nkb = (int)((Kd + tg::BK - 1) / tg::BK);
+  const int kb_per_split = splits > 1 ? (nkb + splits - 1) / splits : 0;
+  const int nz = splits > 1 ? splits : g.nbatch;
+  const long long a_rows = g.a_rows ? g.a_rows : (A_MN ? Kd : M), a_cols = g.a_cols ? g.a_cols : (A_MN ? M : Kd);
+  const long long b_rows = g.b_rows ? g.b_rows : (B_MN ? Kd : N), b_cols = g.b_cols ? g.b_cols : (B_MN ? N : Kd);
   CUtensorMap mA, mB;
   int rc;
-  if ((rc = tg::make_map3(&mA, a_split, a_rows, a_cols, A_MN ? 64 : tg::BM, TERMS))) return rc;
-  if ((rc = tg::make_map3(&mB, b_split, b_rows, b_cols, B_MN ? 64 : BN, TERMS))) return rc;
+  if ((rc = tg::make_map3(&mA, g.a, a_rows, a_cols, A_MN ? 64 : tg::BM, TERMS))) return rc;
+  if ((rc = tg::make_map3(&mB, g.b, b_rows, b_cols, B_MN ? 64 : BN, TERMS))) return rc;
   const int mt = (int)((M + tg::BM - 1) / tg::BM), nt = (int)((N + BN - 1) / BN);
   const int grid = (int)std::min<long long>((long long)mt * nt * nz, sm_count());
   const size_t smem = (size_t)kStages * TERMS * (tg::BM * 128 + BN * 128) + 1024;
   auto kern = tg::tc_gemm_persist_kernel<BN, TERMS, kStages, A_MN, B_MN, Epi>;
   VADC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<grid, tg::kThreads, smem, st>>>(mA, mB, (int)M, (int)N, (int)Kd, mt, nt, nz, mt < nt ? 1 : 0, kb_per_split, zo,
-                                         acc_scale, epi);
+  kern<<<grid, tg::kThreads, smem, st>>>(mA, mB, (int)M, (int)N, (int)Kd, mt, nt, nz, mt < nt ? 1 : 0, kb_per_split, g.off,
+                                         g.acc_scale, epi);
   VADC_CHECK_LAUNCH("tc_gemm_persist_kernel");
   return VADC_OK;
 }
 
-// one problem; splits > 1 slots along the contraction, each handing its index to the epilogue (split-K partials)
-template <int TERMS, bool A_MN, bool B_MN, class Epi>
-static int launch_tc_gemm_ex_t(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                               const float* acc_scale, Epi epi, cudaStream_t st) {
-  if (splits < 1) splits = 1;
-  const int nkb = (int)((Kd + tg::BK - 1) / tg::BK);
-  const int per = splits > 1 ? (nkb + splits - 1) / splits : 0;          // k-blocks per slot
-  return launch_tc_gemm_t<TERMS, A_MN, B_MN, Epi>(a_split, A_MN ? Kd : M, A_MN ? M : Kd, b_split, B_MN ? Kd : N,
-                                                  B_MN ? N : Kd, M, N, Kd, splits, per, TcBatchOffsets{0, 0, 0, 0},
-                                                  acc_scale, epi, st);
-}
-
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_ex(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                      Epi epi, cudaStream_t st) {
-  return launch_tc_gemm_ex_t<3, A_MN, B_MN, Epi>(a_split, b_split, M, N, Kd, splits, nullptr, epi, st);
-}
-
-// the same with fp16 x2 operands (tc_split2h) and the accumulators scaled by *acc_scale
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_ex_h2(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                         const float* acc_scale, Epi epi, cudaStream_t st) {
-  return launch_tc_gemm_ex_t<2, A_MN, B_MN, Epi>(a_split, b_split, M, N, Kd, splits, acc_scale, epi, st);
-}
-
-// nbatch independent [M,N,Kd] problems in ONE launch (z = batch): the operands of batch z start
-// z * off.{m,k} coordinates further along tensors of the given full extents (rows x cols of the split matrices)
-// TERMS = 3: bf16 x3 operands from tc_split3; TERMS = 2: fp16 x2 operands from tc_split2h, accumulators scaled by *acc_scale
-template <int TERMS, bool A_MN, bool B_MN, class Epi>
-static int launch_tc_gemm_batched_t(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                                    long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                                    TcBatchOffsets off, const float* acc_scale, Epi epi, cudaStream_t st) {
-  if (nbatch < 1 || nbatch > 65535) return VADC_ERR_UNSUPPORTED;
-  return launch_tc_gemm_t<TERMS, A_MN, B_MN, Epi>(a_split, a_rows, a_cols, b_split, b_rows, b_cols, M, N, Kd, nbatch, 0, off,
-                                                  acc_scale, epi, st);
-}
-
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_batched(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                           long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                           TcBatchOffsets off, Epi epi, cudaStream_t st) {
-  return launch_tc_gemm_batched_t<3, A_MN, B_MN, Epi>(a_split, a_rows, a_cols, b_split, b_rows, b_cols, M, N, Kd, nbatch, off,
-                                                      nullptr, epi, st);
-}
-
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_batched_h2(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                              long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                              TcBatchOffsets off, const float* acc_scale, Epi epi, cudaStream_t st) {
-  return launch_tc_gemm_batched_t<2, A_MN, B_MN, Epi>(a_split, a_rows, a_cols, b_split, b_rows, b_cols, M, N, Kd, nbatch, off,
-                                                      acc_scale, epi, st);
-}
+// one line per (terms, operand layouts, epilogue) the library launches
+#define VADC_TC_GEMM(TERMS, A_MN, B_MN, EPI) template int tc_gemm<TERMS, A_MN, B_MN, EPI>(const TcGemm&, EPI, cudaStream_t);
+VADC_TC_GEMM(2, false, false, TcDistEpi)
+VADC_TC_GEMM(2, false, true, TcStoreEpi)
+VADC_TC_GEMM(2, false, false, TcStoreEpi)
+VADC_TC_GEMM(2, false, true, TcReadEpi)
+VADC_TC_GEMM(2, false, false, TcLogitsColStatsTEpi)
+VADC_TC_GEMM(2, false, false, TcStoreTEpi)
+VADC_TC_GEMM(2, false, false, TcDistTEpi)
+VADC_TC_GEMM(2, false, true, TcGzEpi)
+VADC_TC_GEMM(2, true, false, TcStoreTEpi)
+VADC_TC_GEMM(2, true, false, TcReadTEpi)
+VADC_TC_GEMM(2, true, false, TcGzTEpi)
+VADC_TC_GEMM(2, true, false, TcPartialEpi)
+VADC_TC_GEMM(2, true, true, TcPartialEpi)
+VADC_TC_GEMM(2, false, true, ScoresQhatEpi)
+VADC_TC_GEMM(2, true, false, ScoresQRowsTEpi)
+VADC_TC_GEMM(2, false, false, TcBatchDistEpi)
+VADC_TC_GEMM(2, true, false, TcSpaceGzEpi)
+VADC_TC_GEMM(2, true, true, TcSpaceGcEpi)
+VADC_TC_GEMM(2, true, false, TcCdistGaTEpi)
+VADC_TC_GEMM(3, false, false, TcStoreEpi)
+VADC_TC_GEMM(3, false, true, TcStoreEpi)
+VADC_TC_GEMM(3, false, false, TcDistEpi)
+VADC_TC_GEMM(3, false, true, TcReadEpi)
+VADC_TC_GEMM(3, false, true, TcGzEpi)
+VADC_TC_GEMM(3, false, false, TcTimeDebedEpi)
+VADC_TC_GEMM(3, false, true, TcTimeDebedEpi)
+VADC_TC_GEMM(3, true, false, TcPartialEpi)
+VADC_TC_GEMM(3, true, true, TcPartialEpi)
+VADC_TC_GEMM(3, false, true, ScoresQhatEpi)
+VADC_TC_GEMM(3, true, false, ScoresQRowsTEpi)
+VADC_TC_GEMM(3, true, false, TcStoreTEpi)
+VADC_TC_GEMM(3, false, false, TcBiasEpi)
+VADC_TC_GEMM(3, false, false, TcBiasTEpi)
+VADC_TC_GEMM(3, false, false, TcBiasGeluTEpi)
+VADC_TC_GEMM(3, false, false, TcBatchDistEpi)
+VADC_TC_GEMM(3, true, false, TcSpaceGzEpi)
+VADC_TC_GEMM(3, true, true, TcSpaceGcEpi)
+VADC_TC_GEMM(3, true, false, TcCdistGaTEpi)
+#undef VADC_TC_GEMM
 
 // ---- two-term fp16 mode -------------------------------------------------------------------------
 namespace tg {
@@ -401,44 +392,12 @@ fwd_scales_kernel(const float* __restrict__ centers, const float* __restrict__ l
   }
 }
 
-__global__ void __launch_bounds__(256)
-split2h_kernel(const float* __restrict__ src, long long n4, const float* __restrict__ scale, __half* __restrict__ t0,
-               __half* __restrict__ t1) {
-  const float s = __ldg(scale);
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
-    const float4 v = reinterpret_cast<const float4*>(src)[i];
-    const float a[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
-    __half h[2][4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      h[0][j] = __float2half_rn(a[j]);
-      h[1][j] = __float2half_rn(a[j] - __half2float(h[0][j]));
-    }
-    reinterpret_cast<uint2*>(t0)[i] = *reinterpret_cast<uint2*>(h[0]);
-    reinterpret_cast<uint2*>(t1)[i] = *reinterpret_cast<uint2*>(h[1]);
-  }
-}
 }  // namespace tg
-
-size_t tc_gemm_split2_bytes(long long rows, long long cols) {
-  return align_up((size_t)2 * rows * cols * sizeof(__half), 256);
-}
 
 int tc_fwd_scales(const float* centers, const float* ln_w, const float* ln_b, long long KC, int C, float* out,
                   cudaStream_t st) {
   tg::fwd_scales_kernel<<<1, 1024, 0, st>>>(centers, ln_w, ln_b, KC, C, out);
   VADC_CHECK_LAUNCH("fwd_scales_kernel");
-  return VADC_OK;
-}
-
-int tc_split2h(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st) {
-  const long long n = rows * cols;
-  if (n % 4) return VADC_ERR_BAD_SHAPE;
-  __half* t0 = static_cast<__half*>(dst);
-  const long long n4 = n / 4;
-  const int grid = (int)std::min<long long>((n4 + 255) / 256, (long long)sm_count() * 8);
-  tg::split2h_kernel<<<grid, 256, 0, st>>>(src, n4, scale, t0, t0 + n);
-  VADC_CHECK_LAUNCH("split2h_kernel");
   return VADC_OK;
 }
 
@@ -549,75 +508,13 @@ int tc_pair_scales(const unsigned* a_bits, float a_given, const unsigned* b_bits
   return VADC_OK;
 }
 
-template <bool B_MN, class Epi>
-int launch_tc_gemm_h2(const void* a_split, const void* b_split, long long M, long long N, long long Kd,
-                      const float* acc_scale, Epi epi, cudaStream_t st) {
-  return launch_tc_gemm_ex_t<2, false, B_MN, Epi>(a_split, b_split, M, N, Kd, 1, acc_scale, epi, st);
-}
-template int launch_tc_gemm_h2<false, TcDistEpi>(const void*, const void*, long long, long long, long long, const float*, TcDistEpi, cudaStream_t);
-template int launch_tc_gemm_h2<true, TcStoreEpi>(const void*, const void*, long long, long long, long long, const float*, TcStoreEpi, cudaStream_t);
-template int launch_tc_gemm_h2<false, TcStoreEpi>(const void*, const void*, long long, long long, long long, const float*, TcStoreEpi, cudaStream_t);
-template int launch_tc_gemm_h2<true, TcReadEpi>(const void*, const void*, long long, long long, long long, const float*, TcReadEpi, cudaStream_t);
-template int launch_tc_gemm_h2<false, TcLogitsColStatsTEpi>(const void*, const void*, long long, long long, long long, const float*, TcLogitsColStatsTEpi, cudaStream_t);
-template int launch_tc_gemm_h2<false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, const float*, TcStoreTEpi, cudaStream_t);
-template int launch_tc_gemm_h2<false, TcDistTEpi>(const void*, const void*, long long, long long, long long, const float*, TcDistTEpi, cudaStream_t);
-template int launch_tc_gemm_h2<true, TcGzEpi>(const void*, const void*, long long, long long, long long, const float*, TcGzEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcStoreTEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, false, TcReadTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcReadTEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, false, TcGzTEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcGzTEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, const float*, TcPartialEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<false, true, ScoresQhatEpi>(const void*, const void*, long long, long long, long long, int, const float*, ScoresQhatEpi, cudaStream_t);
-template int launch_tc_gemm_ex_h2<true, false, ScoresQRowsTEpi>(const void*, const void*, long long, long long, long long, int, const float*, ScoresQRowsTEpi, cudaStream_t);
-
-template <bool B_MN, class Epi>
-int launch_tc_gemm(const void* a_split, const void* b_split, long long M, long long N, long long Kd, Epi epi,
-                   cudaStream_t st) {
-  return launch_tc_gemm_ex<false, B_MN, Epi>(a_split, b_split, M, N, Kd, 1, epi, st);
-}
-
-// explicit instantiations for the epilogues of the path
-template int launch_tc_gemm<false, TcStoreEpi>(const void*, const void*, long long, long long, long long, TcStoreEpi, cudaStream_t);
-template int launch_tc_gemm<true, TcStoreEpi>(const void*, const void*, long long, long long, long long, TcStoreEpi, cudaStream_t);
-template int launch_tc_gemm<false, TcDistEpi>(const void*, const void*, long long, long long, long long, TcDistEpi, cudaStream_t);
-template int launch_tc_gemm<true, TcReadEpi>(const void*, const void*, long long, long long, long long, TcReadEpi, cudaStream_t);
-template int launch_tc_gemm<true, TcGzEpi>(const void*, const void*, long long, long long, long long, TcGzEpi, cudaStream_t);
-template int launch_tc_gemm<false, TcTimeDebedEpi>(const void*, const void*, long long, long long, long long, TcTimeDebedEpi, cudaStream_t);
-template int launch_tc_gemm_ex<true, false, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
-template int launch_tc_gemm_ex<true, true, TcPartialEpi>(const void*, const void*, long long, long long, long long, int, TcPartialEpi, cudaStream_t);
-template int launch_tc_gemm_ex<false, true, ScoresQhatEpi>(const void*, const void*, long long, long long, long long, int, ScoresQhatEpi, cudaStream_t);
-template int launch_tc_gemm_ex<true, false, ScoresQRowsTEpi>(const void*, const void*, long long, long long, long long, int, ScoresQRowsTEpi, cudaStream_t);
-template int launch_tc_gemm_ex<true, false, TcStoreTEpi>(const void*, const void*, long long, long long, long long, int, TcStoreTEpi, cudaStream_t);
-template int launch_tc_gemm<false, TcBiasEpi>(const void*, const void*, long long, long long, long long, TcBiasEpi, cudaStream_t);
-template int launch_tc_gemm<false, TcBiasTEpi>(const void*, const void*, long long, long long, long long, TcBiasTEpi, cudaStream_t);
-template int launch_tc_gemm<true, TcTimeDebedEpi>(const void*, const void*, long long, long long, long long, TcTimeDebedEpi, cudaStream_t);
-template int launch_tc_gemm<false, TcBiasGeluTEpi>(const void*, const void*, long long, long long, long long, TcBiasGeluTEpi, cudaStream_t);
-#define VADC_TC_BATCHED(AMN, BMN, EPI)                                                                               \
-  template int launch_tc_gemm_batched<AMN, BMN, EPI>(const void*, long long, long long, const void*, long long,       \
-                                                     long long, long long, long long, long long, int, TcBatchOffsets, \
-                                                     EPI, cudaStream_t);
-VADC_TC_BATCHED(false, false, TcBatchDistEpi)
-VADC_TC_BATCHED(true, false, TcSpaceGzEpi)
-VADC_TC_BATCHED(true, true, TcSpaceGcEpi)
-VADC_TC_BATCHED(true, false, TcCdistGaTEpi)
-#undef VADC_TC_BATCHED
-#define VADC_TC_BATCHED_H2(AMN, BMN, EPI)                                                                              \
-  template int launch_tc_gemm_batched_h2<AMN, BMN, EPI>(const void*, long long, long long, const void*, long long,      \
-                                                        long long, long long, long long, long long, int, TcBatchOffsets, \
-                                                        const float*, EPI, cudaStream_t);
-VADC_TC_BATCHED_H2(false, false, TcBatchDistEpi)
-VADC_TC_BATCHED_H2(true, false, TcSpaceGzEpi)
-VADC_TC_BATCHED_H2(true, true, TcSpaceGcEpi)
-VADC_TC_BATCHED_H2(true, false, TcCdistGaTEpi)
-#undef VADC_TC_BATCHED_H2
-
 }  // namespace vadc
 
 // ---------------------------------------------------------------------------
 // self-test entry: out[M,N] = A[M,Kd] . B^T  (b_mn = 0: B is [N,Kd]; b_mn = 1: B is [Kd,N])
 // ---------------------------------------------------------------------------
 extern "C" size_t vadc_debug_tc_gemm_workspace_bytes(int64_t M, int64_t N, int64_t Kd) {
-  return vadc::tc_gemm_split_bytes(M, Kd) + vadc::tc_gemm_split_bytes(N, Kd) + 256;
+  return vadc::tc_terms_bytes(3, M, Kd) + vadc::tc_terms_bytes(3, N, Kd) + 256;
 }
 
 extern "C" int vadc_debug_tc_gemm(const float* A, const float* B, int64_t M, int64_t N, int64_t Kd, int b_mn,
@@ -628,11 +525,12 @@ extern "C" int vadc_debug_tc_gemm(const float* A, const float* B, int64_t M, int
   VADC_REQUIRE(workspace_bytes >= vadc_debug_tc_gemm_workspace_bytes(M, N, Kd), VADC_ERR_WORKSPACE);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Carver ws(workspace, workspace_bytes);
-  void* as = ws.take<uint8_t>(tc_gemm_split_bytes(M, Kd));
-  void* bs = ws.take<uint8_t>(tc_gemm_split_bytes(N, Kd));
+  void* as = ws.take<uint8_t>(tc_terms_bytes(3, M, Kd));
+  void* bs = ws.take<uint8_t>(tc_terms_bytes(3, N, Kd));
   int rc;
-  if ((rc = tc_split3(A, M, Kd, as, st))) return rc;
-  if ((rc = b_mn ? tc_split3(B, Kd, N, bs, st) : tc_split3(B, N, Kd, bs, st))) return rc;
+  if ((rc = tc_split<3>(A, M, Kd, nullptr, as, st))) return rc;
+  if ((rc = b_mn ? tc_split<3>(B, Kd, N, nullptr, bs, st) : tc_split<3>(B, N, Kd, nullptr, bs, st))) return rc;
+  const TcGemm g{as, bs, M, N, Kd};
   TcStoreEpi epi{out, N};
-  return b_mn ? launch_tc_gemm<true>(as, bs, M, N, Kd, epi, st) : launch_tc_gemm<false>(as, bs, M, N, Kd, epi, st);
+  return b_mn ? tc_gemm<3, false, true>(g, epi, st) : tc_gemm<3, false, false>(g, epi, st);
 }

@@ -3,33 +3,43 @@
 #pragma once
 #include <cuda_bf16.h>
 #include "common.cuh"
+#include "tc_terms.cuh"
 
 namespace vadc {
 
+// ---- operands: each fp32 operand is first split into its terms (format: tc_terms.cuh), TERMS matrices of its shape
+// stored back to back — tc_split<3> (bf16 x3, fp32-faithful for any data) or tc_split<2> (fp16 x2 of the operand times a
+// power-of-two scale held in device memory, for bounded data).  Row kernels that already hold the data write the terms
+// themselves (store_terms).  Workspace of one operand's terms: tc_terms_bytes.
+size_t tc_terms_bytes(int terms, long long rows, long long cols);
+template <int TERMS>
+int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st);
+
+// ---- the GEMM: C[m,n] = sum_k A[m,k] B(n,k), handed to the epilogue in 32-column pieces: epi(m, n, v[32], nvalid, z).
+// A's terms are [M, Kd] (A_MN: [Kd, M], e.g. a transposed token matrix), B's [N, Kd] (B_MN: [Kd, N]).
+// TERMS = 3: six bf16 products.  TERMS = 2: three fp16 products, the accumulators multiplied by *acc_scale
+// (= 1 / (s_a s_b), required) before the epilogue.
+// z, handed to the epilogue, is either a split-K slot (splits > 1: slot z contracts its share of the k-blocks and writes
+// a partial; an empty slot writes zeros) or a batch (nbatch problems in one launch, the operands of batch z starting
+// z * off coordinates further along the split matrices — a_m / b_n along the output-row / output-column dimension,
+// a_k / b_k along the contraction; a_rows x a_cols, b_rows x b_cols are then the full split matrices).
+struct TcBatchOffsets { int a_m, a_k, b_n, b_k; };
+struct TcGemm {
+  const void* a; const void* b;
+  long long M, N, Kd;
+  const float* acc_scale = nullptr;
+  int splits = 1;
+  int nbatch = 1;
+  TcBatchOffsets off = {0, 0, 0, 0};
+  long long a_rows = 0, a_cols = 0, b_rows = 0, b_cols = 0;     // 0: one problem's extents from M, N, Kd
+};
 bool tc_gemm_shape_ok(long long M, long long N, long long Kd, bool b_mn);
-size_t tc_gemm_split_bytes(long long rows, long long cols);     // workspace of one operand's three bf16 terms
-int tc_split3(const float* src, long long rows, long long cols, void* dst, cudaStream_t st);
+template <int TERMS, bool A_MN, bool B_MN, class Epi>
+int tc_gemm(const TcGemm& g, Epi epi, cudaStream_t st);
 
-// C[m,n] = sum_k A[m,k] B(n,k); a_split / b_split from tc_split3 ([M,Kd]; [N,Kd] or, with B_MN, [Kd,N])
-template <bool B_MN, class Epi>
-int launch_tc_gemm(const void* a_split, const void* b_split, long long M, long long N, long long Kd, Epi epi,
-                   cudaStream_t st);
-// general form: A_MN = A given as [Kd, M] (e.g. a transposed token matrix), `splits` slots along the contraction,
-// each handing its index to the epilogue (split-K partials for the centroid-gradient GEMMs, Kd = tokens)
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_ex(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                      Epi epi, cudaStream_t st);
-
-// two-term fp16 mode for bounded operands (tc_gemm.cu): operands pre-scaled by powers of two held in device memory,
-// accumulators multiplied by *acc_scale before the epilogue
-size_t tc_gemm_split2_bytes(long long rows, long long cols);
+// scales of the fp16 x2 mode, all in device memory (no host sync)
 int tc_fwd_scales(const float* centers, const float* ln_w, const float* ln_b, long long KC, int C, float* out5,
                   cudaStream_t st);     // out (6 floats) = {s_z, s_c, 1/(s_z s_c), s_a, 1/(s_a s_c), 1/(s_c s_c)}
-int tc_split2h(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st);
-template <bool B_MN, class Epi>
-int launch_tc_gemm_h2(const void* a_split, const void* b_split, long long M, long long N, long long Kd,
-                      const float* acc_scale, Epi epi, cudaStream_t st);
-
 // scales for operands whose bound has to be measured: max |src| as float bits (memset + atomicMax), then
 // out3 = {s_a, s_b, 1 / (s_a s_b)} with s = the power of two that puts the bound in [4, 8), or the given constant
 int tc_absmax_bits(const float* src, long long n, unsigned* out, cudaStream_t st);
@@ -39,23 +49,6 @@ int tc_pair_scales(const unsigned* a_bits, float a_given, const unsigned* b_bits
 int tc_fwd_scales_from_bits(const unsigned* cen_bits, const float* ln_w, const float* ln_b, int C, float* out6, cudaStream_t st);
 int tc_cluster_bwd_scales(const unsigned* bits4, int stage, float* out9, cudaStream_t st);   // see tc_gemm.cu
 int tc_space_bwd_scales(const unsigned* r_bits, const float* fwd_sc, float* out3, cudaStream_t st);   // {s_r, 1/(s_c s_r), 1/(s_r s_z)}
-
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_ex_h2(const void* a_split, const void* b_split, long long M, long long N, long long Kd, int splits,
-                         const float* acc_scale, Epi epi, cudaStream_t st);
-
-// batched form (z = batch, handed to the epilogue): per-batch coordinate offsets along the operands' tensors — a_m / b_n along the
-// output-row / output-column dimension, a_k / b_k along the contraction dimension
-struct TcBatchOffsets { int a_m, a_k, b_n, b_k; };
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_batched(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                           long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                           TcBatchOffsets off, Epi epi, cudaStream_t st);
-
-template <bool A_MN, bool B_MN, class Epi>
-int launch_tc_gemm_batched_h2(const void* a_split, long long a_rows, long long a_cols, const void* b_split,
-                              long long b_rows, long long b_cols, long long M, long long N, long long Kd, int nbatch,
-                              TcBatchOffsets off, const float* acc_scale, Epi epi, cudaStream_t st);
 
 __device__ __forceinline__ void tc_store_row32(float* o, const float (&v)[32], int nvalid) {
   if (nvalid == 32 && (reinterpret_cast<uintptr_t>(o) & 15u) == 0) {

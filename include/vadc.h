@@ -82,7 +82,9 @@ int vadc_timing_read(int slot, float* mean_ms, int* count);
  *   rowstats = per-token sums the backward's closed-form LayerNorm statistics use, [N,4]:
  *              |f|^2, sum_c f gamma, sum_c f gamma xhat, 0   (may be NULL: not produced)
  *   loss_sq = sum (D*A)^2                           [1]     (sqrt of it is the cluster loss)
- * Constraints: C % 4 == 0, K % 4 == 0.
+ * Constraints: 1 <= C <= 4096 (VADC_ERR_UNSUPPORTED above), K % 4 == 0.  Any C: rows of C % 4 != 0 are read without
+ * assuming 16-byte alignment (the base pointers still need it); the tensor-core contractions run over C rounded up to 8
+ * with zero padding.  The same holds for vadc_cluster_fwd_padded and vadc_cluster_bwd.
  * ------------------------------------------------------------------------ */
 size_t vadc_cluster_fwd_workspace_bytes(int64_t N, int C, int K, int impl);
 int vadc_cluster_fwd(const float* x, const float* ln_w, const float* ln_b,
@@ -127,7 +129,7 @@ int vadc_cdist_bwd(const float* a, const float* b, const float* dist, const floa
  * two [N,K] tensors.  The caller derives g_loss_sq from whatever it did with
  * loss_sq (local sqrt, or all-reduce over ranks then sqrt: SURVEY.md §8e).
  * Outputs: gx [N,C]; gcenters [K,C]; g_ln_w, g_ln_b [C] (overwritten, not
- * accumulated).
+ * accumulated).  Shapes as vadc_cluster_fwd: 1 <= C <= 4096, K % 4 == 0.
  * ------------------------------------------------------------------------ */
 size_t vadc_cluster_bwd_workspace_bytes(int64_t N, int C, int K);
 int vadc_cluster_bwd(const float* x, const float* mu, const float* rstd, const float* rowstats,

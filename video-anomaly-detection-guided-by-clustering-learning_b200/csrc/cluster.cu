@@ -98,6 +98,21 @@ int launch_ln_rows(const float* x, const float* w, const float* b, long long N, 
                    float* z, float* mu, float* rstd, float* zz, cudaStream_t st, float* rowstats, void* split3,
                    const float* hscale) {
   if (N == 0) return VADC_OK;
+  if (ln_any_width(C)) {
+    if (C > 4096) return VADC_ERR_UNSUPPORTED;
+#define LA_CASE(E, WPR)                                                                                      \
+  ln_rows_any_kernel<E, WPR><<<(unsigned)((N + 8 / WPR - 1) / (8 / WPR)), 256, 0, st>>>(                     \
+      x, w, b, N, C, eps, z, mu, rstd, zz, rowstats, static_cast<__nv_bfloat16*>(split3), hscale, tc_pitch(C))
+    if (C <= 128) LA_CASE(4, 1);
+    else if (C <= 256) LA_CASE(8, 1);
+    else if (C <= 512) LA_CASE(16, 1);
+    else if (C <= 1024) LA_CASE(16, 2);
+    else if (C <= 2048) LA_CASE(16, 4);
+    else LA_CASE(16, 8);
+#undef LA_CASE
+    VADC_CHECK_LAUNCH("ln_rows_any_kernel");
+    return VADC_OK;
+  }
   const int wpb = 8;
   dim3 grid((unsigned)((N + wpb - 1) / wpb));
 #define LN_CASE(V) ln_rows_kernel<V><<<grid, wpb * 32, 0, st>>>(x, w, b, N, C, eps, z, mu, rstd, zz, rowstats, \
@@ -189,6 +204,21 @@ int launch_ln_bwd(const float* gz, const float* x, const float* mu, const float*
                   const float* w, long long N, int C, float* gx, float* partial, float* gw,
                   float* gb, cudaStream_t st) {
   int nb = ln_bwd_blocks(N);
+  if (ln_any_width(C)) {
+    if (C > 4096) return VADC_ERR_UNSUPPORTED;
+#define LA_CASE(E, WPR) ln_bwd_any_kernel<E, WPR><<<nb, 256, 0, st>>>(gz, x, mu, rstd, w, N, C, gx, partial)
+    if (C <= 128) LA_CASE(4, 1);
+    else if (C <= 256) LA_CASE(8, 1);
+    else if (C <= 512) LA_CASE(16, 1);
+    else if (C <= 1024) LA_CASE(16, 2);
+    else if (C <= 2048) LA_CASE(16, 4);
+    else LA_CASE(16, 8);
+#undef LA_CASE
+    VADC_CHECK_LAUNCH("ln_bwd_any_kernel");
+    ln_bwd_finalize_kernel<<<(2 * C + 31) / 32, 256, 0, st>>>(partial, nb, C, gw, gb);
+    VADC_CHECK_LAUNCH("ln_bwd_finalize_kernel");
+    return VADC_OK;
+  }
   size_t smem = (size_t)8 * 2 * C * sizeof(float);
 #define LB_CASE(V)                                                                              \
   do {                                                                                          \
@@ -274,21 +304,24 @@ extern "C" size_t vadc_cluster_fwd_workspace_bytes(int64_t N, int C, int K, int 
   b += align_up((size_t)(softmin_blocks(N, K) + 1) * sizeof(double), 256);
   b += std::max(vadc_cluster_tc_extra_workspace_bytes(N, C, K), vadc_cluster_ws_extra_workspace_bytes(N, C, K));
   if (impl != VADC_IMPL_SIMT && N > 0)                                   // term copies for the tcgen05 GEMMs + scales
-    b += tc_terms_bytes(3, N, C) + tc_terms_bytes(3, K, C) + tc_terms_bytes(3, N, K) + 256;
+    b += tc_terms_bytes(3, N, tc_pitch(C)) + tc_terms_bytes(3, K, tc_pitch(C)) + tc_terms_bytes(3, N, K) + 256;
   return b + 256;
 }
 
 // the generic forward's two contractions on the tcgen05 GEMM.  TERMS = 3: bf16 x3 (fp32-faithful).  TERMS = 2: every
 // operand is bounded (LayerNorm output, centroids, softmin weights in [0, 1]), so two fp16 terms after a power-of-two
 // scaling carry 22 significant bits (the fused K = 32 kernel's recipe): 2/3 of the operand bytes and half the MMAs; the
-// scales stay in device memory (no host sync)
+// scales stay in device memory (no host sync).  The [., C] operands' terms have row pitch Cp = tc_pitch(C) (C rounded up to
+// 8 for the any-width shapes, zero padding): the contractions over C run over Cp, the x_rec GEMM's C dimension reads the
+// centroid terms at pitch Cp and its epilogue stops at C.
 template <int TERMS>
 static int cluster_fwd_tc(const float* x, const float* ln_w, const float* ln_b, const float* centers, int64_t N, int C,
                           int K, int k_valid, float alpha, float eps, float* D, float* A, float* x_rec, float* feature,
                           int64_t* label, float* mu, float* rstd, float* rowstats, float* loss_sq, float* zz, float* cc,
                           double* partial, Carver& ws, cudaStream_t st) {
-  void* fs = ws.take<uint8_t>(tc_terms_bytes(TERMS, N, C));
-  void* cs = ws.take<uint8_t>(tc_terms_bytes(TERMS, K, C));
+  const long long Cp = tc_pitch(C);
+  void* fs = ws.take<uint8_t>(tc_terms_bytes(TERMS, N, Cp));
+  void* cs = ws.take<uint8_t>(tc_terms_bytes(TERMS, K, Cp));
   void* as = ws.take<uint8_t>(tc_terms_bytes(TERMS, N, K));
   float* sc = nullptr;
   int rc;
@@ -298,23 +331,24 @@ static int cluster_fwd_tc(const float* x, const float* ln_w, const float* ln_b, 
   }
   if ((rc = launch_ln_rows(x, ln_w, ln_b, N, C, eps, feature, mu, rstd, zz, st, rowstats, fs, sc))) return rc;
   if ((rc = launch_row_sqnorm(centers, K, C, cc, st))) return rc;
-  if ((rc = tc_split<TERMS>(centers, K, C, sc ? sc + 1 : nullptr, cs, st))) return rc;
+  if ((rc = tc_split<TERMS>(centers, K, C, sc ? sc + 1 : nullptr, cs, st, Cp))) return rc;
   const float* sc2 = sc ? sc + 2 : nullptr;
   if constexpr (TERMS == 2) {
     // fp16 x2 only: from K = 128 up the distance GEMM runs with the operands swapped (rows = centroids): coalesced stores of D
     if (K >= 128) {
-      if ((rc = tc_gemm<2, false, false>({cs, fs, K, N, C, sc2}, TcDistTEpi{D, cc, zz, K}, st))) return rc;
-    } else if ((rc = tc_gemm<2, false, false>({fs, cs, N, K, C, sc2}, TcDistEpi{D, zz, cc, K}, st))) return rc;
+      if ((rc = tc_gemm<2, false, false>({cs, fs, K, N, Cp, sc2}, TcDistTEpi{D, cc, zz, K}, st))) return rc;
+    } else if ((rc = tc_gemm<2, false, false>({fs, cs, N, K, Cp, sc2}, TcDistEpi{D, zz, cc, K}, st))) return rc;
     // softmin writes A and, in the same pass, its two fp16 terms scaled by s_a = 2^13 (the value fwd_scales_kernel puts in sc[3])
     if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid, as, 8192.0f))) return rc;
     if (C >= 128)   // rows = channels (centers [K,C] as the MN-major A operand): coalesced x_rec
-      return tc_gemm<2, true, false>({cs, as, C, N, K, sc + 4}, TcStoreTEpi{x_rec, C}, st);
+      return tc_gemm<2, true, false>({cs, as, C, N, K, sc + 4, 1, 1, {0, 0, 0, 0}, K, Cp}, TcStoreTEpi{x_rec, C}, st);
   } else {
-    if ((rc = tc_gemm<3, false, false>({fs, cs, N, K, C}, TcDistEpi{D, zz, cc, K}, st))) return rc;
+    if ((rc = tc_gemm<3, false, false>({fs, cs, N, K, Cp}, TcDistEpi{D, zz, cc, K}, st))) return rc;
     if ((rc = launch_softmin_rows(D, N, K, alpha, A, (long long*)label, partial, loss_sq, st, k_valid))) return rc;
     if ((rc = tc_split<3>(A, N, K, nullptr, as, st))) return rc;
   }
-  return tc_gemm<TERMS, false, true>({as, cs, N, C, K, sc ? sc + 4 : nullptr}, TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
+  return tc_gemm<TERMS, false, true>({as, cs, N, C, K, sc ? sc + 4 : nullptr, 1, 1, {0, 0, 0, 0}, 0, 0, K, Cp},
+                                     TcStoreEpi{x_rec, C}, st);    // centers [K,C] read MN-major
 }
 
 static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b,
@@ -322,8 +356,8 @@ static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b
                             float eps, float* D, float* A, float* x_rec, float* feature,
                             int64_t* label, float* mu, float* rstd, float* rowstats, float* loss_sq,
                             void* workspace, size_t workspace_bytes, int impl, void* stream) {
-  VADC_REQUIRE(N >= 0 && C > 0 && K > 0 && (C % 4) == 0 && (K % 4) == 0, VADC_ERR_BAD_SHAPE);
-  VADC_REQUIRE(N < (1ll << 31) && C <= 1024, VADC_ERR_UNSUPPORTED);
+  VADC_REQUIRE(N >= 0 && C > 0 && K > 0 && (K % 4) == 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(N < (1ll << 31) && C <= 4096, VADC_ERR_UNSUPPORTED);
   VADC_REQUIRE(ln_w && ln_b && centers && loss_sq && workspace, VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(N == 0 || (x && D && A && x_rec && feature && label && mu && rstd), VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(aligned16(rowstats), VADC_ERR_MISALIGNED);
@@ -349,9 +383,10 @@ static int cluster_fwd_impl(const float* x, const float* ln_w, const float* ln_b
   int rc;
   // shapes outside the fused kernels (C = 768, K = 16 / 64 / 256 / 1024): the two contractions run on the
   // tcgen05 GEMM (three-term bf16 split: fp32-faithful); LayerNorm (+ rowstats + the split of z) and softmin
-  // stay row kernels
+  // stay row kernels.  Any-width C (C % 4 != 0, C > 1024) contracts over its padded pitch tc_pitch(C).
+  const int Cp = tc_pitch(C);
   const bool use_tc = impl != VADC_IMPL_SIMT && N > 0 && !env_on("VADC_NO_TC_GEMM") &&
-                      tc_gemm_shape_ok(N, K, C, false) && tc_gemm_shape_ok(N, C, K, true);
+                      tc_gemm_shape_ok(N, K, Cp, false) && tc_gemm_shape_ok(N, Cp, K, true);
   if (use_tc)
     return env_on("VADC_TC_BF16X3")
                ? cluster_fwd_tc<3>(x, ln_w, ln_b, centers, N, C, K, k_valid, alpha, eps, D, A, x_rec, feature, label, mu,
@@ -502,13 +537,13 @@ static int cluster_bwd_tc(const float* x, const float* mu, const float* rstd, co
                           const float* gR, const float* gF, const float* g_loss_sq, int64_t N, int C, int K, float alpha,
                           float* gx, float* gcenters, float* g_ln_w, float* g_ln_b, float* gemm, float* r, float* rsum,
                           float* gz, float* cpart, float* rcol, float* lnpart, Carver& ws, cudaStream_t st) {
-  const long long KC = (long long)K * C;
+  const long long KC = (long long)K * C, Cp = tc_pitch(C);     // terms of gR, feature, centers at row pitch Cp
   const int sk = bwd_tc_splits(N, C, K);
-  void* gRs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
-  void* fs = ws.take<uint8_t>(tc_terms_bytes(3, N, C));
+  void* gRs = ws.take<uint8_t>(tc_terms_bytes(3, N, Cp));
+  void* fs = ws.take<uint8_t>(tc_terms_bytes(3, N, Cp));
   void* as = ws.take<uint8_t>(tc_terms_bytes(3, N, K));
   void* rs = ws.take<uint8_t>(tc_terms_bytes(3, N, K));
-  void* cs = ws.take<uint8_t>(tc_terms_bytes(3, K, C));
+  void* cs = ws.take<uint8_t>(tc_terms_bytes(3, K, Cp));
   float* q1 = ws.take<float>((size_t)sk * KC);
   float* q2 = ws.take<float>((size_t)sk * KC);
   unsigned* bits = nullptr;
@@ -526,15 +561,15 @@ static int cluster_bwd_tc(const float* x, const float* mu, const float* rstd, co
     if ((rc = tc_absmax_bits(feature, (long long)N * C, bits + 2, st))) return rc;
     if ((rc = tc_cluster_bwd_scales(bits, 0, sc, st))) return rc;
   }
-  if ((rc = tc_split<TERMS>(centers, K, C, at(1), cs, st))) return rc;
+  if ((rc = tc_split<TERMS>(centers, K, C, at(1), cs, st, Cp))) return rc;
   if (gR) {
-    if ((rc = tc_split<TERMS>(gR, N, C, at(0), gRs, st))) return rc;
+    if ((rc = tc_split<TERMS>(gR, N, C, at(0), gRs, st, Cp))) return rc;
     // fp16 x2 only: from K = 128 up the operands are swapped (rows = centroids): coalesced stores
     if constexpr (TERMS == 2) {
-      if (K >= 128) rc = tc_gemm<2, false, false>({cs, gRs, K, N, C, at(5)}, TcStoreTEpi{gemm, K}, st);
-      else rc = tc_gemm<2, false, false>({gRs, cs, N, K, C, at(5)}, TcStoreEpi{gemm, K}, st);
+      if (K >= 128) rc = tc_gemm<2, false, false>({cs, gRs, K, N, Cp, at(5)}, TcStoreTEpi{gemm, K}, st);
+      else rc = tc_gemm<2, false, false>({gRs, cs, N, K, Cp, at(5)}, TcStoreEpi{gemm, K}, st);
     } else {
-      rc = tc_gemm<3, false, false>({gRs, cs, N, K, C}, TcStoreEpi{gemm, K}, st);
+      rc = tc_gemm<3, false, false>({gRs, cs, N, K, Cp}, TcStoreEpi{gemm, K}, st);
     }
     if (rc) return rc;
   }
@@ -546,18 +581,22 @@ static int cluster_bwd_tc(const float* x, const float* mu, const float* rstd, co
   if ((rc = tc_split<TERMS>(r, N, K, at(4), rs, st))) return rc;
   // fp16 x2 only: from C = 128 up rows = channels, coalesced loads of feature / gF and stores of gz
   if constexpr (TERMS == 2) {
-    if (C >= 128) rc = tc_gemm<2, true, false>({cs, rs, C, N, K, at(7)}, TcGzTEpi{gz, feature, rsum, gF, C}, st);
-    else rc = tc_gemm<2, false, true>({rs, cs, N, C, K, at(7)}, TcGzEpi{gz, feature, rsum, gF, C}, st);
+    if (C >= 128)
+      rc = tc_gemm<2, true, false>({cs, rs, C, N, K, at(7), 1, 1, {0, 0, 0, 0}, K, Cp}, TcGzTEpi{gz, feature, rsum, gF, C}, st);
+    else
+      rc = tc_gemm<2, false, true>({rs, cs, N, C, K, at(7), 1, 1, {0, 0, 0, 0}, 0, 0, K, Cp}, TcGzEpi{gz, feature, rsum, gF, C}, st);
   } else {
-    rc = tc_gemm<3, false, true>({rs, cs, N, C, K}, TcGzEpi{gz, feature, rsum, gF, C}, st);
+    rc = tc_gemm<3, false, true>({rs, cs, N, C, K, nullptr, 1, 1, {0, 0, 0, 0}, 0, 0, K, Cp}, TcGzEpi{gz, feature, rsum, gF, C}, st);
   }
   if (rc) return rc;
   if (gR) {
     if ((rc = tc_split<TERMS>(A, N, K, at(3), as, st))) return rc;
-    if ((rc = tc_gemm<TERMS, true, true>({as, gRs, K, C, N, at(6), sk}, TcPartialEpi{q1, C, KC}, st))) return rc;
+    if ((rc = tc_gemm<TERMS, true, true>({as, gRs, K, C, N, at(6), sk, 1, {0, 0, 0, 0}, 0, 0, N, Cp}, TcPartialEpi{q1, C, KC}, st)))
+      return rc;
   }
-  if ((rc = tc_split<TERMS>(feature, N, C, at(2), fs, st))) return rc;
-  if ((rc = tc_gemm<TERMS, true, true>({rs, fs, K, C, N, at(8), sk}, TcPartialEpi{q2, C, KC}, st))) return rc;
+  if ((rc = tc_split<TERMS>(feature, N, C, at(2), fs, st, Cp))) return rc;
+  if ((rc = tc_gemm<TERMS, true, true>({rs, fs, K, C, N, at(8), sk, 1, {0, 0, 0, 0}, 0, 0, N, Cp}, TcPartialEpi{q2, C, KC}, st)))
+    return rc;
   cudaError_t e2 = launch_colsum(r, N, K, cpart, rcol, st);
   if (e2 != cudaSuccess) return record_cuda_error(e2, "colsum r");
   gcenters_finalize_kernel<<<(unsigned)((KC + 255) / 256), 256, 0, st>>>(gR ? q1 : nullptr, q2, sk, centers, rcol, K, C, gcenters);
@@ -566,22 +605,36 @@ static int cluster_bwd_tc(const float* x, const float* mu, const float* rstd, co
 }
 }  // namespace vadc
 
+namespace vadc {
+// split-K partials of the backward: [splits, K, C] for each of the two centroid-gradient contractions, SIMT and tcgen05.
+// The slot count falls as C adds tiles, so for the any-width shapes this is the maximum over every width up to C (the
+// product is largest at the end of a 64-wide tile band): a workspace sized for one head also serves every narrower one.
+static size_t bwd_partial_bytes(long long N, int C, int K) {
+  auto at = [&](int c) {
+    const int tiles = ((K + 63) / 64) * ((c + 63) / 64);
+    return 2 * align_up((size_t)split_count(N, tiles) * K * c * sizeof(float), 256) +
+           2 * align_up((size_t)bwd_tc_splits(N, c, K) * K * c * sizeof(float), 256);
+  };
+  size_t b = at(C);
+  if (ln_any_width(C))
+    for (int c = 64; c < C; c += 64) b = std::max(b, at(c));
+  return b;
+}
+}  // namespace vadc
+
 extern "C" size_t vadc_cluster_bwd_workspace_bytes(int64_t N, int C, int K) {
   size_t n = (size_t)(N > 0 ? N : 1);
-  int tiles = ((K + 63) / 64) * ((C + 63) / 64);
-  int splits = split_count(N, tiles);
   size_t b = 0;
   b += align_up(n * K * sizeof(float), 256);                 // gR.c^T
   b += align_up(n * K * sizeof(float), 256);                 // r
   b += align_up(n * sizeof(float), 256);                     // rsum
   b += align_up(n * C * sizeof(float), 256);                 // gz
-  b += 2 * align_up((size_t)splits * K * C * sizeof(float), 256);   // split-K partials
   b += align_up((size_t)colsum_chunks(N) * K * sizeof(float), 256); // colsum partial
   b += align_up((size_t)K * sizeof(float), 256);             // rcol
   b += align_up((size_t)ln_bwd_blocks(N) * 2 * C * sizeof(float), 256);
   // generic path on the tcgen05 GEMM: bf16 term copies of gR, feature, A, r and the centroids + split-K partials
-  b += 2 * tc_terms_bytes(3, (long long)n, C) + 2 * tc_terms_bytes(3, (long long)n, K) + tc_terms_bytes(3, K, C) + 1024;
-  b += 2 * align_up((size_t)bwd_tc_splits(N, C, K) * K * C * sizeof(float), 256);
+  b += 2 * tc_terms_bytes(3, (long long)n, tc_pitch(C)) + 2 * tc_terms_bytes(3, (long long)n, K) + tc_terms_bytes(3, K, tc_pitch(C)) + 1024;
+  b += bwd_partial_bytes(N, C, K);                           // split-K partials
   return std::max(std::max(b + 256, bwd_fused_workspace_bytes(N, C, K)), bwd_tc2_workspace_bytes(N, C, K));
 }
 
@@ -593,8 +646,8 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
                                 int64_t N, int C, int K, float alpha,
                                 float* gx, float* gcenters, float* g_ln_w, float* g_ln_b,
                                 void* workspace, size_t workspace_bytes, void* stream) {
-  VADC_REQUIRE(N >= 0 && C > 0 && K > 0 && (C % 4) == 0 && (K % 4) == 0, VADC_ERR_BAD_SHAPE);
-  VADC_REQUIRE(N < (1ll << 31) && C <= 1024, VADC_ERR_UNSUPPORTED);
+  VADC_REQUIRE(N >= 0 && C > 0 && K > 0 && (K % 4) == 0, VADC_ERR_BAD_SHAPE);
+  VADC_REQUIRE(N < (1ll << 31) && C <= 4096, VADC_ERR_UNSUPPORTED);
   VADC_REQUIRE(ln_w && centers && gcenters && g_ln_w && g_ln_b && workspace, VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(N == 0 || (x && mu && rstd && feature && D && A && gx), VADC_ERR_NULL_POINTER);
   VADC_REQUIRE(workspace_bytes >= vadc_cluster_bwd_workspace_bytes(N, C, K), VADC_ERR_WORKSPACE);
@@ -628,7 +681,9 @@ extern "C" int vadc_cluster_bwd(const float* x, const float* mu, const float* rs
   float* cpart = ws.take<float>((size_t)colsum_chunks(N) * K);
   float* rcol = ws.take<float>(K);
   float* lnpart = ws.take<float>((size_t)ln_bwd_blocks(N) * 2 * C);
-  if (!env_on("VADC_NO_TC_GEMM") && vadc_device_ok() && (K % 8) == 0 && (C % 8) == 0 && K >= 8 && C >= 8) {
+  // any-width C (C % 4 != 0, C > 1024) contracts over its padded pitch tc_pitch(C); C % 8 == 4 up to 1024 stays SIMT
+  if (!env_on("VADC_NO_TC_GEMM") && vadc_device_ok() && (K % 8) == 0 && K >= 8 &&
+      (((C % 8) == 0 && C >= 8) || ln_any_width(C))) {
     return env_on("VADC_TC_BF16X3")
                ? cluster_bwd_tc<3>(x, mu, rstd, feature, ln_w, centers, D, A, gD, gA, gR, gF, g_loss_sq, N, C, K, alpha,
                                    gx, gcenters, g_ln_w, g_ln_b, gemm, r, rsum, gz, cpart, rcol, lnpart, ws, st)

@@ -90,6 +90,101 @@ ln_rows_kernel(const float* __restrict__ x, const float* __restrict__ w, const f
   }
 }
 
+// ---------------------------------------------------------------------------
+// Rows of any width (the cluster head at C % 4 != 0 or C > 1024; ln_rows_kernel / ln_bwd_rows_kernel keep the rest).
+// WPR warps share a row (one block = 8 / WPR rows), each lane holds E elements c = t + 32 WPR i (t = lane index within
+// the row), loaded one float at a time: a row of pitch C % 4 != 0 is not 16-byte aligned.  Row sums go through the warp
+// shuffles and, for WPR > 1, through shared memory in fixed warp order (deterministic).
+// ---------------------------------------------------------------------------
+inline bool ln_any_width(int C) { return (C % 4) != 0 || C > 1024; }
+// row pitch of the operand terms of a [rows, C] matrix: C, or for the any-width shapes C rounded up to 8 (tc_gemm's TMA
+// row pitch is a multiple of 16 bytes); the padding columns hold zeros, so a contraction over the padded pitch is exact
+inline int tc_pitch(int C) { return ln_any_width(C) ? (C + 7) & ~7 : C; }
+
+// sums NV values over the WPR warps of a row; red: 32 floats of shared memory.  Every thread of the block calls it.
+template <int WPR, int NV>
+__device__ __forceinline__ void row_sums(float (&v)[NV], float* red) {
+#pragma unroll
+  for (int i = 0; i < NV; ++i) v[i] = warp_sum(v[i]);
+  if constexpr (WPR > 1) {
+    const int wid = threadIdx.x >> 5, w0 = wid - wid % WPR;
+    if ((threadIdx.x & 31) == 0)
+#pragma unroll
+      for (int i = 0; i < NV; ++i) red[wid * 4 + i] = v[i];
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+      float s = 0.f;
+#pragma unroll
+      for (int k = 0; k < WPR; ++k) s += red[(w0 + k) * 4 + i];
+      v[i] = s;
+    }
+    __syncthreads();
+  }
+}
+
+// LayerNorm rows of any width: ln_rows_kernel's outputs (two-pass statistics from the E values a lane holds); the
+// operand terms of z go to pitch ldt = tc_pitch(C) with zeros in columns C..ldt-1
+template <int E, int WPR>
+__global__ void __launch_bounds__(256)
+ln_rows_any_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ b,
+                   long long N, int C, float eps, float* __restrict__ z, float* __restrict__ mu,
+                   float* __restrict__ rstd, float* __restrict__ zz, float* __restrict__ rowstats,
+                   __nv_bfloat16* __restrict__ split, const float* __restrict__ hscale, int ldt) {
+  __shared__ float red[32];
+  const float hs = hscale ? __ldg(hscale) : 1.0f;
+  const int t = (threadIdx.x >> 5) % WPR * 32 + (threadIdx.x & 31);
+  const long long row = (long long)blockIdx.x * (8 / WPR) + (threadIdx.x >> 5) / WPR;
+  const bool live = row < N;
+  if (WPR == 1 && !live) return;
+  const float* xr = x + row * C;
+  float v[E];
+  float s[1] = {0.f};
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    const int c = t + 32 * WPR * i;
+    v[i] = (live && c < C) ? __ldcs(xr + c) : 0.f;
+    s[0] += v[i];
+  }
+  row_sums<WPR, 1>(s, red);
+  const float mean = s[0] / (float)C;
+  float q[1] = {0.f};
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    const float d = v[i] - mean;
+    if (t + 32 * WPR * i < C) q[0] = fmaf(d, d, q[0]);
+  }
+  row_sums<WPR, 1>(q, red);
+  const float rs = 1.0f / sqrtf(q[0] / (float)C + eps);
+  float st[3] = {0.f, 0.f, 0.f};                  // |z|^2, sum z gamma, sum z gamma xhat
+  const long long plane = N * (long long)ldt;
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    const int c = t + 32 * WPR * i;
+    if (live && c < C) {
+      const float g = __ldg(w + c), xh = (v[i] - mean) * rs;
+      const float o = xh * g + __ldg(b + c);
+      if (z) z[row * C + c] = o;
+      st[0] = fmaf(o, o, st[0]);
+      st[1] += o * g;
+      st[2] = fmaf(o * g, xh, st[2]);
+      if (split && hscale) store_terms<2>(split, plane, row * ldt + c, o * hs);
+      else if (split) store_terms<3>(split, plane, row * ldt + c, o);
+    }
+  }
+  if (split && live && t < ldt - C) {
+    if (hscale) store_terms<2>(split, plane, row * ldt + C + t, 0.f);
+    else store_terms<3>(split, plane, row * ldt + C + t, 0.f);
+  }
+  row_sums<WPR, 3>(st, red);
+  if (live && t == 0) {
+    mu[row] = mean;
+    rstd[row] = rs;
+    if (zz) zz[row] = st[0];
+    if (rowstats) reinterpret_cast<float4*>(rowstats)[row] = make_float4(st[0], st[1], st[2], 0.f);
+  }
+}
+
 // |row|^2 for a [R, C] matrix, one warp per row (any C).
 static __global__ void __launch_bounds__(256)
 row_sqnorm_kernel(const float* __restrict__ a, long long R, int C, float* __restrict__ out) {
@@ -411,6 +506,72 @@ ln_bwd_rows_kernel(const float* __restrict__ gz, const float* __restrict__ x,
     float s = 0.f;
     for (int ww = 0; ww < nw; ++ww) s += sm[(size_t)ww * 2 * C + c];
     partial[(size_t)blockIdx.x * 2 * C + c] = s;
+  }
+}
+
+// LayerNorm backward of any width (layout as ln_rows_any_kernel): a block's row groups walk the rows together, every
+// lane carries the gamma / beta partials of its E columns in registers; at the end the block's 8 / WPR row groups are
+// summed column slice by column slice through 2 KB of shared memory (not [8][2C] floats: 256 KB at C = 4096) into the
+// same partial [grid, 2C] ln_bwd_finalize_kernel reduces
+template <int E, int WPR>
+__global__ void __launch_bounds__(256)
+ln_bwd_any_kernel(const float* __restrict__ gz, const float* __restrict__ x, const float* __restrict__ mu,
+                  const float* __restrict__ rstd, const float* __restrict__ w, long long N, int C,
+                  float* __restrict__ gx, float* __restrict__ partial /*[grid,2C]*/) {
+  constexpr int G = 8 / WPR, RT = 32 * WPR;      // row groups per block, threads per row
+  __shared__ float red[32];
+  __shared__ float cs[2][256];
+  const int t = (threadIdx.x >> 5) % WPR * 32 + (threadIdx.x & 31), grp = (threadIdx.x >> 5) / WPR;
+  float gw[E], gb[E], wv[E];
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    const int c = t + RT * i;
+    gw[i] = 0.f; gb[i] = 0.f;
+    wv[i] = c < C ? __ldg(w + c) : 0.f;
+  }
+  for (long long r0 = (long long)blockIdx.x * G; r0 < N; r0 += (long long)gridDim.x * G) {   // uniform over the block
+    const long long row = r0 + grp;
+    const bool live = row < N;
+    const float m = live ? __ldg(mu + row) : 0.f, rs = live ? __ldg(rstd + row) : 0.f;
+    float g[E], xh[E];
+    float s[2] = {0.f, 0.f};
+#pragma unroll
+    for (int i = 0; i < E; ++i) {
+      const int c = t + RT * i;
+      g[i] = 0.f; xh[i] = 0.f;
+      if (live && c < C) {
+        const float gv = __ldcs(gz + row * C + c), xv = __ldcs(x + row * C + c);
+        xh[i] = (xv - m) * rs;
+        gw[i] = fmaf(gv, xh[i], gw[i]);
+        gb[i] += gv;
+        g[i] = gv * wv[i];
+        s[0] += g[i];
+        s[1] = fmaf(g[i], xh[i], s[1]);
+      }
+    }
+    row_sums<WPR, 2>(s, red);
+    const float s1 = s[0] / (float)C, s2 = s[1] / (float)C;
+#pragma unroll
+    for (int i = 0; i < E; ++i) {
+      const int c = t + RT * i;
+      if (live && c < C) gx[row * C + c] = (g[i] - s1 - xh[i] * s2) * rs;
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < E; ++i) {
+    if (RT * i >= C) break;                      // uniform
+    cs[0][grp * RT + t] = gw[i];
+    cs[1][grp * RT + t] = gb[i];
+    __syncthreads();
+    const int c = (int)threadIdx.x + RT * i;
+    if ((int)threadIdx.x < RT && c < C) {
+      float a = 0.f, e = 0.f;
+#pragma unroll
+      for (int k = 0; k < G; ++k) { a += cs[0][k * RT + threadIdx.x]; e += cs[1][k * RT + threadIdx.x]; }
+      partial[(size_t)blockIdx.x * 2 * C + c] = a;
+      partial[(size_t)blockIdx.x * 2 * C + C + c] = e;
+    }
+    __syncthreads();
   }
 }
 

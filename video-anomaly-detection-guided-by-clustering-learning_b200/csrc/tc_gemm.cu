@@ -31,14 +31,28 @@ namespace tg {
 constexpr int BM = 128, BK = 64;
 constexpr int kThreads = 320;            // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue
 
-// fp32 [n4 * 4] -> its TERMS term planes (tc_terms.cuh); fp16 x2: of src * scale[0]
+// fp32 [n4 * 4] -> its TERMS term planes (tc_terms.cuh); fp16 x2: of src * scale[0].  ld > cols: src is [rows, cols]
+// (any cols, any alignment), the terms [rows, ld] (n4 = rows ld / 4) with zeros in columns cols..ld-1
 template <int TERMS>
 __global__ void __launch_bounds__(256)
-split_kernel(const float* __restrict__ src, long long n4, const float* __restrict__ scale, void* __restrict__ dst) {
+split_kernel(const float* __restrict__ src, long long n4, const float* __restrict__ scale, void* __restrict__ dst,
+             long long cols, long long ld) {
   const float s = TERMS == 2 ? __ldg(scale) : 1.0f;
+  if (ld == cols) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+      const float4 v = reinterpret_cast<const float4*>(src)[i];
+      const float a[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
+      store_terms<TERMS, 4>(dst, 4 * n4, 4 * i, a);
+    }
+    return;
+  }
+  const long long q = ld / 4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
-    const float4 v = reinterpret_cast<const float4*>(src)[i];
-    const float a[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
+    const long long r = i / q, c = 4 * (i - r * q);
+    const float* p = src + r * cols + c;
+    float a[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) a[j] = c + j < cols ? __ldg(p + j) * s : 0.f;
     store_terms<TERMS, 4>(dst, 4 * n4, 4 * i, a);
   }
 }
@@ -262,19 +276,22 @@ size_t tc_terms_bytes(int terms, long long rows, long long cols) {
 }
 
 template <int TERMS>
-int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st) {
+int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st,
+             long long ld) {
   static_assert(TERMS == 2 || TERMS == 3, "operand terms: fp16 x2 or bf16 x3");
-  const long long n = rows * cols;
+  if (ld == 0) ld = cols;
+  if (ld < cols || (ld != cols && ld % 8)) return VADC_ERR_BAD_SHAPE;
+  const long long n = rows * ld;
   if (n % 4) return VADC_ERR_BAD_SHAPE;
   if (TERMS == 2 && !scale) return VADC_ERR_NULL_POINTER;
   const long long n4 = n / 4;
   const int grid = (int)std::min<long long>((n4 + 255) / 256, (long long)sm_count() * 8);
-  tg::split_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst);
+  tg::split_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst, cols, ld);
   VADC_CHECK_LAUNCH("split_kernel");
   return VADC_OK;
 }
-template int tc_split<2>(const float*, long long, long long, const float*, void*, cudaStream_t);
-template int tc_split<3>(const float*, long long, long long, const float*, void*, cudaStream_t);
+template int tc_split<2>(const float*, long long, long long, const float*, void*, cudaStream_t, long long);
+template int tc_split<3>(const float*, long long, long long, const float*, void*, cudaStream_t, long long);
 
 // nz work slices along z of an [M, N] output on min(work items, SMs) persistent CTAs with three 64 KB (fp16 x2) or two
 // 96 KB (bf16 x3) operand stages.  Split matrices MN-major: [Kd rows, M / N cols], boxes of 64 k-rows x 64 cols; K-major:

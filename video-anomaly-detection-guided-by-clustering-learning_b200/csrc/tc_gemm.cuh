@@ -11,9 +11,12 @@ namespace vadc {
 // stored back to back — tc_split<3> (bf16 x3, fp32-faithful for any data) or tc_split<2> (fp16 x2 of the operand times a
 // power-of-two scale held in device memory, for bounded data).  Row kernels that already hold the data write the terms
 // themselves (store_terms).  Workspace of one operand's terms: tc_terms_bytes.
+// ld (0: = cols): row pitch of the terms, a multiple of 8 above cols for a source of any cols (rows of cols % 4 != 0 are
+// read without assuming alignment); the padding columns cols..ld-1 are written as zeros.
 size_t tc_terms_bytes(int terms, long long rows, long long cols);
 template <int TERMS>
-int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st);
+int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st,
+             long long ld = 0);
 
 // ---- the GEMM: C[m,n] = sum_k A[m,k] B(n,k), handed to the epilogue in 32-column pieces: epi(m, n, v[32], nvalid, z).
 // A's terms are [M, Kd] (A_MN: [Kd, M], e.g. a transposed token matrix), B's [N, Kd] (B_MN: [Kd, N]).
@@ -54,6 +57,9 @@ __device__ __forceinline__ void tc_store_row32(float* o, const float (&v)[32], i
   if (nvalid == 32 && (reinterpret_cast<uintptr_t>(o) & 15u) == 0) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) reinterpret_cast<float4*>(o)[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+  } else if (nvalid == 32) {           // a full piece of a row that is not 16-byte aligned (row pitch C % 4 != 0)
+#pragma unroll
+    for (int j = 0; j < 32; ++j) o[j] = v[j];
   } else {
 #pragma unroll
     for (int j = 0; j < 32; ++j) if (j < nvalid) o[j] = v[j];

@@ -14,14 +14,22 @@
 
 namespace vadc {
 
+// Operand terms of the tensor-core path, for any P and any K (a multiple of 4): zt [C, M, Pp], centroids [C, Kp, Pp]
+// (channel c's rows from c Kp), r [M, C Kp] (channel c's columns from c Kp).  Pp = P rounded up to 8: the TMA row pitch
+// is a multiple of 16 bytes.  Kp = K rounded up to 64: channel c's window of the r·centers contraction ends on a k-block,
+// so no column of channel c + 1 enters its sum.  The padding is written as zeros; the epilogues stop at P and K.
+__host__ __device__ __forceinline__ int space_pp(int P) { return (P + 7) & ~7; }
+static int space_kp(int K) { return (K + 63) & ~63; }
+
 // LayerNorm + transpose: x [T, C] tokens -> zt [C, T].  A block normalises 32
 // tokens (one warp per 4 tokens), parks them in shared memory and writes 32
 // consecutive tokens per channel (128-byte segments) so both sides coalesce.
+// terms (instead of zt): the three bf16 terms of zt [C, T / P, Pp], the frame's last token also writing the zero columns
 __global__ void __launch_bounds__(256)
 ln_transpose_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                    const float* __restrict__ b, long long T, int C, float eps,
+                    const float* __restrict__ b, long long T, int P, int C, float eps,
                     float* __restrict__ zt, float* __restrict__ mu, float* __restrict__ rstd,
-                    __nv_bfloat16* __restrict__ terms /* optional: the three bf16 terms of zt, [3][C*T] */) {
+                    __nv_bfloat16* __restrict__ terms) {
   extern __shared__ float tile[];            // [32][C+1]
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const long long t0 = (long long)blockIdx.x * 32;
@@ -43,12 +51,17 @@ ln_transpose_kernel(const float* __restrict__ x, const float* __restrict__ w,
   __syncthreads();
   const long long row = t0 + lane;
   if (row < T) {
-    const long long n = (long long)C * T;
-    for (int c = wid; c < C; c += 8) {
-      const float v = tile[lane * ld + c];
-      const long long i = (long long)c * T + row;
-      if (zt) zt[i] = v;
-      if (terms) store_terms<3>(terms, n, i, v);  // the operand split of the batched tcgen05 GEMM, written in the same pass
+    if (zt) {
+      for (int c = wid; c < C; c += 8) zt[(long long)c * T + row] = tile[lane * ld + c];
+    } else {                                   // the operand split of the batched tcgen05 GEMM, written in the same pass
+      const int Pp = space_pp(P);
+      const long long f = row / P, p = row - f * P, Tp = T / P * Pp, n = (long long)C * Tp;
+      for (int c = wid; c < C; c += 8) {
+        const long long i = (long long)c * Tp + f * Pp + p;
+        store_terms<3>(terms, n, i, tile[lane * ld + c]);
+        if (p == P - 1)
+          for (int j = 1; j <= Pp - P; ++j) store_terms<3>(terms, n, i + j, 0.f);
+      }
     }
   }
 }
@@ -136,8 +149,9 @@ constexpr int kTileTok = 64, kTileLd = kTileTok + 1, kMaxCpl = 8, kTokPerWarp = 
 // LayerNorm + transpose of one (frame m, 64-token chunk j) tile.  Phase 1: a warp owns eight tokens and issues ALL
 // their loads before the first reduction (the whole 48 KB tile of a block is in flight at once), normalises them in
 // registers and parks them in the transposed shared tile [C][65].  Phase 2 writes a channel's 64 tokens per warp
-// instruction — either fp32 zt (SIMT contraction path) or the three bf16 operand terms of the batched tcgen05 GEMM plus
-// the chunk's share of |zt[c,m,:]|^2 (sqpart [C*M, chunks]; fp32 zt is then never materialised).
+// instruction — either fp32 zt (SIMT contraction path) or the operand terms of the batched tcgen05 GEMM at row pitch Pp
+// (the frame's last chunk also writes the zero columns P..Pp-1, from tile columns it zeroes first) plus the chunk's
+// share of |zt[c,m,:]|^2 (sqpart [C*M, chunks]; fp32 zt is then never materialised).
 // CPL = channels per lane (C <= 32 CPL).
 // NT = 0: fp32 zt; 3: three bf16 terms; 2: two fp16 terms of zt * *scale (a power of two from the LayerNorm bound).
 // FULL: C == 32 CPL, no per-channel predicates.
@@ -188,19 +202,22 @@ ln_transpose_tile_kernel(const float* __restrict__ x, const float* __restrict__ 
       if (lane == 0) { mu[t0 + rr] = mean; rstd[t0 + rr] = rs; }
     }
   }
+  const int Pp = space_pp(P), npp = min(kTileTok, Pp - p0);       // npp > np: the frame's last chunk, P % 8 != 0
+  if (NT != 0 && npp > np)
+    for (int c = wid; c < C; c += 8) if (lane < npp - np) tile[c * kTileLd + np + lane] = 0.f;
   __syncthreads();
   if constexpr (NT != 0) {
-    // half a warp per channel, four tokens per lane (np is a multiple of 8 on this path: P % 8 == 0): 8-byte stores
-    const long long n = (long long)C * T;
+    // half a warp per channel, four tokens per lane (the padded pitch Pp is a multiple of 8): 8-byte stores
+    const long long Tp = (long long)M * Pp, n = (long long)C * Tp;
     const int half = lane >> 4, l16 = lane & 15;
-    const bool tok = 4 * l16 < np;
-    uint16_t* const tbase = static_cast<uint16_t*>(terms_) + t0 + 4 * l16;
+    const bool tok = 4 * l16 < npp;
+    uint16_t* const tbase = static_cast<uint16_t*>(terms_) + (long long)m * Pp + p0 + 4 * l16;
     const float sc = NT == 2 ? __ldg(scale) : 1.0f;
     // pointers advance by 16 channels per iteration (no per-iteration 64-bit multiplies)
-    uint16_t* d = tbase + (long long)(2 * wid + half) * T;
+    uint16_t* d = tbase + (long long)(2 * wid + half) * Tp;
     float* sp = sqpart + ((long long)(2 * wid + half) * M + m) * chunks + j;
     const float* tp = tile + (2 * wid + half) * kTileLd + 4 * l16;
-    const long long dstep = 16 * T, sstep = 16ll * M * chunks;
+    const long long dstep = 16 * Tp, sstep = 16ll * M * chunks;
 #pragma unroll 2
     for (int cc = 2 * wid; cc < C; cc += 16, d += dstep, sp += sstep, tp += 16 * kTileLd) {
       const int c = cc + half;
@@ -386,13 +403,11 @@ struct SpaceGzEpilogue {
 };
 
 
-// The three contractions of the head as batched tcgen05 GEMMs (three-term bf16 split, fp32-faithful): worth it
-// from a few GFLOP up; P, K multiples of 8 for the TMA row pitches, K a multiple of 64 so that a batch's window
-// of the contraction over centroids ends on a k-block boundary (the next batch's columns must not leak in).
+// The three contractions of the head as batched tcgen05 GEMMs: worth it from a few GFLOP up, for any P and K (the
+// operand terms are padded to Pp, Kp: space_pp, space_kp); the batch offsets of the launches fit in int.
 static bool space_tc_ok(long long M, int P, int C, int K) {
-  return M >= 1 && (P % 8) == 0 && (K % 64) == 0 && C <= 65535 && (long long)C * M < (1ll << 31) &&
-         (long long)C * K < (1ll << 31) && (double)M * P * K * C >= (double)(1ll << 28) && vadc_device_ok() != 0 &&
-         !env_on("VADC_NO_TC_GEMM");
+  return M >= 1 && C <= 65535 && (long long)C * M < (1ll << 31) && (long long)C * space_kp(K) < (1ll << 31) &&
+         (double)M * P * K * C >= (double)(1ll << 28) && vadc_device_ok() != 0 && !env_on("VADC_NO_TC_GEMM");
 }
 
 static int space_ln_bwd_blocks(long long T, int C, bool tiled) {
@@ -409,8 +424,9 @@ __global__ void __launch_bounds__(256)
 row_sqnorm_terms_kernel(const __nv_bfloat16* __restrict__ t, long long n, long long R, int P, float* __restrict__ out) {
   const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (row >= R) return;
+  const long long base = row * space_pp(P);
   float s = 0.f;
-  for (int p = threadIdx.x & 31; p < P; p += 32) { const float v = terms_value(t, n, row * P + p); s += v * v; }
+  for (int p = threadIdx.x & 31; p < P; p += 32) { const float v = terms_value(t, n, base + p); s += v * v; }
   s = warp_sum(s);
   if ((threadIdx.x & 31) == 0) out[row] = s;
 }
@@ -421,9 +437,13 @@ static int space_chunks(int P) { return (P + kTileTok - 1) / kTileTok; }
 // the bytes, half the MMAs) unless VADC_SPACE_TERMS=3 asks for the fp32-faithful three bf16 terms; the untiled
 // LayerNorm kernels (C > 256) only write the latter
 static int space_nt(int C) { return (C > 32 * kMaxCpl || env_int("VADC_SPACE_TERMS", 2) == 3) ? 3 : 2; }
-// saved state of the tensor-core path: [ zt terms | centroid terms | forward scales (256 bytes) ]
-static size_t space_zt_bytes(long long M, int P, int C) { return align_up((size_t)C * M * P * space_nt(C) * 2, 256); }
-static size_t space_cen_bytes(int P, int C, int K) { return align_up((size_t)C * K * P * space_nt(C) * 2, 256); }
+// saved state of the tensor-core path: [ zt terms [C, M, Pp] | centroid terms [C, Kp, Pp] | forward scales (256 bytes) ]
+static size_t space_zt_bytes(long long M, int P, int C) {
+  return align_up((size_t)C * M * space_pp(P) * space_nt(C) * 2, 256);
+}
+static size_t space_cen_bytes(int P, int C, int K) {
+  return align_up((size_t)C * space_kp(K) * space_pp(P) * space_nt(C) * 2, 256);
+}
 
 // column sums of r [M, C K]: few rows, many columns — split the rows so that the grid covers the SMs a few times
 static int space_colsum_chunks(long long R, long long W) {
@@ -506,9 +526,9 @@ static int launch_ln_bwd_tile(const float* gzt, const float* x, const float* mu,
 
 using namespace vadc;
 
-// The LayerNorm output in the batched-cdist layout [C, M, P], kept from the forward for the backward: the three bf16
-// operand terms of the tcgen05 GEMMs when those run (6 bytes per element, fp32 zt = their exact sum is never
-// written) followed by the terms of the centroids, fp32 zt otherwise.  Opaque to the caller; forward and backward must
+// The LayerNorm output in the batched-cdist layout [C, M, P], kept from the forward for the backward: the operand
+// terms of the tcgen05 GEMMs when those run (at the padded pitches of space_pp / space_kp; fp32 zt = their exact sum is
+// never written) followed by the terms of the centroids, fp32 zt otherwise.  Opaque to the caller; forward and backward must
 // see the same environment.
 extern "C" size_t vadc_space_cluster_saved_bytes(int64_t M, int P, int C, int K) {
   const size_t n = (size_t)C * (size_t)(M > 0 ? M : 1) * P;
@@ -532,13 +552,14 @@ extern "C" size_t vadc_space_cluster_fwd_workspace_bytes(int64_t M, int P, int C
 template <int TERMS>
 static int space_dist_tc(const void* zs, const float* centers, void* cs, const float* sc, int64_t M, int P, int C, int K,
                          const float* zz, const float* cc, float* Ds, float* selfdist, cudaStream_t st) {
-  const long long CM = (long long)C * M, CK = (long long)C * K;
+  const int Pp = space_pp(P), Kp = space_kp(K);
+  const long long CM = (long long)C * M, CK = (long long)C * K, CKp = (long long)C * Kp;
   int rc;
-  if ((rc = tc_split<TERMS>(centers, CK, P, TERMS == 2 ? sc + 1 : nullptr, cs, st))) return rc;
-  if ((rc = tc_gemm<TERMS, false, false>({zs, cs, M, K, P, TERMS == 2 ? sc + 2 : nullptr, 1, C, {(int)M, 0, K, 0}, CM, P, CK, P},
+  if ((rc = tc_split<TERMS>(centers, CK, P, TERMS == 2 ? sc + 1 : nullptr, cs, st, Pp, K, Kp))) return rc;
+  if ((rc = tc_gemm<TERMS, false, false>({zs, cs, M, K, P, TERMS == 2 ? sc + 2 : nullptr, 1, C, {(int)M, 0, Kp, 0}, CM, Pp, CKp, Pp},
                                          TcBatchDistEpi{Ds, zz, cc, CK, K, M, K}, st))) return rc;
   if (!selfdist) return VADC_OK;
-  return tc_gemm<TERMS, false, false>({cs, cs, K, K, P, TERMS == 2 ? sc + 5 : nullptr, 1, C, {K, 0, K, 0}, CK, P, CK, P},
+  return tc_gemm<TERMS, false, false>({cs, cs, K, K, P, TERMS == 2 ? sc + 5 : nullptr, 1, C, {Kp, 0, Kp, 0}, CKp, Pp, CKp, Pp},
                                       TcBatchDistEpi{selfdist, cc, cc, K, (long long)K * K, K, K}, st);
 }
 
@@ -586,11 +607,11 @@ static int space_cluster_fwd_impl(const float* x, const float* ln_w, const float
       size_t smem = (size_t)32 * (C + 1) * sizeof(float);
       if (smem > 48 * 1024)
         VADC_CUDA(cudaFuncSetAttribute(ln_transpose_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      ln_transpose_kernel<<<(unsigned)((T + 31) / 32), 256, smem, st>>>(x, ln_w, ln_b, T, C, eps, zt, mu, rstd, zs);
+      ln_transpose_kernel<<<(unsigned)((T + 31) / 32), 256, smem, st>>>(x, ln_w, ln_b, T, P, C, eps, zt, mu, rstd, zs);
       VADC_CHECK_LAUNCH("ln_transpose_kernel");
       if (tc) {
         const long long rows = (long long)C * M;
-        row_sqnorm_terms_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(zs, rows * P, rows, P, zz);
+        row_sqnorm_terms_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(zs, rows * space_pp(P), rows, P, zz);
         VADC_CHECK_LAUNCH("row_sqnorm_terms_kernel");
       } else if ((rc = launch_row_sqnorm(zt, (long long)C * M, P, zz, st))) return rc;
     }
@@ -643,7 +664,7 @@ extern "C" size_t vadc_space_cluster_bwd_workspace_bytes(int64_t M, int P, int C
   b += align_up((size_t)space_colsum_chunks(M, (long long)C * K) * C * K * sizeof(float), 256);
   b += align_up((size_t)C * K * sizeof(float), 256);                   // rcol
   b += align_up((size_t)std::max(space_ln_bwd_blocks(M * (int64_t)P, C, true), space_ln_bwd_blocks(M * (int64_t)P, C, false)) * 2 * C * sizeof(float), 256);
-  if ((P % 8) == 0 && (K % 64) == 0) b += tc_terms_bytes(3, (long long)m, (long long)C * K) + 512;     // r terms, scales
+  b += tc_terms_bytes(3, (long long)m, (long long)C * space_kp(K)) + 512;     // r terms [M, C Kp], scales
   return b + 512;
 }
 
@@ -661,12 +682,16 @@ static int space_bwd_tc(const float* r, void* rs, const unsigned* rbits, const f
     if ((rc = tc_space_bwd_scales(rbits, fsc, s, st))) return rc;
     bsc = s;
   }
-  if ((rc = tc_split<TERMS>(r, M, (long long)C * K, bsc, rs, st))) return rc;
+  const int Pp = space_pp(P), Kp = space_kp(K);
+  const long long CKp = (long long)C * Kp;
+  // r [M, C, K] as M C rows of K columns: its terms [M, C Kp], channel c's columns from c Kp
+  if ((rc = tc_split<TERMS>(r, M * (long long)C, K, bsc, rs, st, Kp))) return rc;
   // gzt <- r centers; the LayerNorm backward forms zt rsum - that
-  if ((rc = tc_gemm<TERMS, true, false>({cs, rs, P, M, K, bsc ? bsc + 1 : nullptr, 1, C, {0, K, 0, K}, (long long)C * K, P, M,
-                                         (long long)C * K}, TcSpaceGzEpi{gzt, (long long)M * P, P}, st))) return rc;
-  return tc_gemm<TERMS, true, true>({rs, zs, K, P, M, bsc ? bsc + 2 : nullptr, 1, C, {K, 0, 0, (int)M}, M, (long long)C * K,
-                                     (long long)C * M, P}, TcSpaceGcEpi{gcenters, centers, rcol, (long long)K * P, P, K}, st);
+  if ((rc = tc_gemm<TERMS, true, false>({cs, rs, P, M, Kp, bsc ? bsc + 1 : nullptr, 1, C, {0, Kp, 0, Kp}, CKp, Pp, M, CKp},
+                                        TcSpaceGzEpi{gzt, (long long)M * P, P}, st))) return rc;
+  // output rows K..Kp-1 of a channel are not computed (M = K): they would land in the next channel's gcenters
+  return tc_gemm<TERMS, true, true>({rs, zs, K, P, M, bsc ? bsc + 2 : nullptr, 1, C, {Kp, 0, 0, (int)M}, M, CKp,
+                                     (long long)C * M, Pp}, TcSpaceGcEpi{gcenters, centers, rcol, (long long)K * P, P, K}, st);
 }
 }  // namespace vadc
 
@@ -702,11 +727,11 @@ extern "C" int vadc_space_cluster_bwd(const float* x, const float* mu, const flo
   if ((rc = launch_bwd_rows(Ds, As, nullptr, gD, gA, g_loss_sq, M * (long long)C, K, alpha, r, rsum, st,
                             (tc && space_nt(C) == 2) ? rbits : nullptr))) return rc;
   if (tc) {
-    // r as [M, C K] (batch c = its K-column window), centers as [C K, P] and zt as [C M, P] (terms the forward kept):
+    // r as [M, C Kp] (batch c = its Kp-column window), centers as [C Kp, Pp] and zt as [C M, Pp] (terms the forward kept):
     //   acc[c]^T = centers[c]^T r[:,c,:]^T   (gzt = zt rsum - acc is formed by the LayerNorm backward)   rows = positions p:
     //                                        A = centers MN-major, B = r K-major
     //   gcenters[c] = centers[c] rcol[c] - r[:,c,:]^T zt[c]    A MN-major (window offset along m), B MN-major
-    void* rs = ws.take<uint8_t>(tc_terms_bytes(3, M, (long long)C * K));
+    void* rs = ws.take<uint8_t>(tc_terms_bytes(3, M, (long long)C * space_kp(K)));
     const int nt = space_nt(C);
     const void* zs = zt_state;
     const uint8_t* cs = static_cast<const uint8_t*>(zt_state) + space_zt_bytes(M, P, C);

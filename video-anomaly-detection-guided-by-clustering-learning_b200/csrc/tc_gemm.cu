@@ -57,6 +57,25 @@ split_kernel(const float* __restrict__ src, long long n4, const float* __restric
   }
 }
 
+// split_kernel for row groups (tc_split's group < gpitch): term row g gpitch + k [.., ld] holds source row g group + k
+// [.., cols] for k < group; the other rows and columns cols..ld-1 are zeros (a kernel of its own, so that the ungrouped
+// splits keep their instruction stream)
+template <int TERMS>
+__global__ void __launch_bounds__(256)
+split_groups_kernel(const float* __restrict__ src, long long n4, const float* __restrict__ scale, void* __restrict__ dst,
+                    long long cols, long long ld, long long group, long long gpitch) {
+  const float s = TERMS == 2 ? __ldg(scale) : 1.0f;
+  const long long q = ld / 4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i / q, c = 4 * (i - r * q), g = r / gpitch, k = r - g * gpitch;
+    const float* p = src + (g * group + k) * cols + c;
+    float a[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) a[j] = k < group && c + j < cols ? __ldg(p + j) * s : 0.f;
+    store_terms<TERMS, 4>(dst, 4 * n4, 4 * i, a);
+  }
+}
+
 __device__ __forceinline__ void tma_load_3d(const void* tmap, uint32_t smem_dst, uint64_t* bar, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
                ::"r"(smem_dst), "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
@@ -277,21 +296,29 @@ size_t tc_terms_bytes(int terms, long long rows, long long cols) {
 
 template <int TERMS>
 int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st,
-             long long ld) {
+             long long ld, long long group, long long gpitch) {
   static_assert(TERMS == 2 || TERMS == 3, "operand terms: fp16 x2 or bf16 x3");
   if (ld == 0) ld = cols;
   if (ld < cols || (ld != cols && ld % 8)) return VADC_ERR_BAD_SHAPE;
-  const long long n = rows * ld;
+  if (group == 0 && gpitch == 0) group = gpitch = 1;
+  if (group < 1 || gpitch < group || rows % group) return VADC_ERR_BAD_SHAPE;
+  if (gpitch != group && ld % 4) return VADC_ERR_BAD_SHAPE;
+  const long long n = rows / group * gpitch * ld;
   if (n % 4) return VADC_ERR_BAD_SHAPE;
   if (TERMS == 2 && !scale) return VADC_ERR_NULL_POINTER;
   const long long n4 = n / 4;
   const int grid = (int)std::min<long long>((n4 + 255) / 256, (long long)sm_count() * 8);
-  tg::split_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst, cols, ld);
-  VADC_CHECK_LAUNCH("split_kernel");
+  if (gpitch == group) {
+    tg::split_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst, cols, ld);
+    VADC_CHECK_LAUNCH("split_kernel");
+  } else {
+    tg::split_groups_kernel<TERMS><<<grid, 256, 0, st>>>(src, n4, scale, dst, cols, ld, group, gpitch);
+    VADC_CHECK_LAUNCH("split_groups_kernel");
+  }
   return VADC_OK;
 }
-template int tc_split<2>(const float*, long long, long long, const float*, void*, cudaStream_t, long long);
-template int tc_split<3>(const float*, long long, long long, const float*, void*, cudaStream_t, long long);
+template int tc_split<2>(const float*, long long, long long, const float*, void*, cudaStream_t, long long, long long, long long);
+template int tc_split<3>(const float*, long long, long long, const float*, void*, cudaStream_t, long long, long long, long long);
 
 // nz work slices along z of an [M, N] output on min(work items, SMs) persistent CTAs with three 64 KB (fp16 x2) or two
 // 96 KB (bf16 x3) operand stages.  Split matrices MN-major: [Kd rows, M / N cols], boxes of 64 k-rows x 64 cols; K-major:

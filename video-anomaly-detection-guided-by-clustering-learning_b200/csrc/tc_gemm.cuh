@@ -13,10 +13,13 @@ namespace vadc {
 // themselves (store_terms).  Workspace of one operand's terms: tc_terms_bytes.
 // ld (0: = cols): row pitch of the terms, a multiple of 8 above cols for a source of any cols (rows of cols % 4 != 0 are
 // read without assuming alignment); the padding columns cols..ld-1 are written as zeros.
+// group, gpitch (0: none): the source rows come in groups of `group` (rows a multiple of it), and group g lands at term
+// rows g gpitch .. g gpitch + group - 1, with rows group..gpitch-1 of every group written as zeros (rows / group * gpitch
+// term rows in all) — e.g. a batch's block of rows padded to whole k-blocks.
 size_t tc_terms_bytes(int terms, long long rows, long long cols);
 template <int TERMS>
 int tc_split(const float* src, long long rows, long long cols, const float* scale, void* dst, cudaStream_t st,
-             long long ld = 0);
+             long long ld = 0, long long group = 0, long long gpitch = 0);
 
 // ---- the GEMM: C[m,n] = sum_k A[m,k] B(n,k), handed to the epilogue in 32-column pieces: epi(m, n, v[32], nvalid, z).
 // A's terms are [M, Kd] (A_MN: [Kd, M], e.g. a transposed token matrix), B's [N, Kd] (B_MN: [Kd, N]).
